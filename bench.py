@@ -4,6 +4,7 @@ enclosure, kappa = sigma_s = 0.5, 1e10 rays per step — sharded over the N GPUs
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference on the host cores
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's tallies to DIR/*.npy
 
 A "step" is one full exchange-factor trace of the workload: zero the UInt64 count matrix, trace rays_total rays (every
 emitter row, all bands), land the rows of all GPUs in one matrix on rank 0.  `value` is device-resident whole-job rays/s
@@ -62,7 +63,16 @@ def parse_args():
     ap.add_argument("--cpu-mode", default="faithful", choices=["faithful", "philox"],
                     help="CPU arm: faithful = per-thread xoshiro256++ and a Dict-like row tally, as the reference does (SURVEY.md 8(d)); "
                          "philox = the parity oracle itself (counter-based RNG, dense row)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64): lost [bands, N] whole "
+                         "and a fixed seeded sample of emitter rows of the count matrix [bands, N, N]; the same arguments give the same "
+                         "inputs, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "rthx":
+        ap.error("--dump-outputs applies to --impl rthx")
+    return args
 
 
 # DRAM bytes per launch of the trace kernel measured by ncu --set full (dram__bytes_read.sum + dram__bytes_write.sum)
@@ -295,6 +305,24 @@ def matrix_hash(t):
     return acc
 
 
+DUMP_COUNT_BYTES = 48 << 20     # count-matrix sample of --dump-outputs (900 MB whole for cfg3); lost and the row ids stay small
+
+
+def dump_outputs(out_dir, counts, lost):
+    """Write the last step's `lost` [nb, N] whole and the rows of `counts` [nb, N, N] of a fixed seeded sample of emitters (all
+    rows when they fit DUMP_COUNT_BYTES) with their indices, as float64 (exact: every count is below 2^53)."""
+    import numpy as np
+    import torch
+    nb, N, _ = counts.shape
+    k = max(1, min(N, DUMP_COUNT_BYTES // (8 * nb * N)))
+    rows = np.sort(np.random.default_rng(0).choice(N, size=k, replace=False))
+    sample = counts.index_select(1, torch.from_numpy(rows).to(counts.device))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "counts_rows.npy"), sample.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "counts_row_ids.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "lost.npy"), lost.cpu().numpy().astype(np.float64))
+
+
 def main():
     args = parse_args()
     if args.impl == "reference":
@@ -378,6 +406,8 @@ def main():
     lost_total = int(sh.lost.sum().item()) if rank == 0 else 0
     tallied = int(sh.counts.sum().item()) if rank == 0 else 0
     flag_timeouts = sh.wait_errors()
+    if args.dump_outputs and rank == 0:      # before anything else traces into sh: it still holds the last timed step
+        dump_outputs(args.dump_outputs, sh.counts, sh.lost)
 
     # the other scaling mode, short (N > 1): weak next to the strong headline, or the reverse
     other_scaling = None

@@ -1,9 +1,12 @@
-"""bench.py's CPU-runnable contract: the reference arm (`--impl reference`) prints one JSON line with the keys the driver reads,
-runs on rank 0 only under torchrun, and ignores the OMP_NUM_THREADS=1 that torchrun exports to its workers."""
+"""bench.py's contract: the reference arm (`--impl reference`) prints one JSON line with the keys the driver reads,
+runs on rank 0 only under torchrun, and ignores the OMP_NUM_THREADS=1 that torchrun exports to its workers; `--dump-outputs`
+writes what the last timed step computed."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -72,3 +75,66 @@ def test_reference_faithful_mode_is_statistically_the_same_tracer(oracle_mod=Non
     fa = a["counts"][0][:ns, ns:].sum() / a["counts"][0][:ns].sum()
     fb = b["counts"][0][:ns, ns:].sum() / b["counts"][0][:ns].sum()
     assert abs(fa - fb) < 5e-3 and not np.array_equal(a["counts"], b["counts"])
+
+
+def _bench_module():
+    sys.path.insert(0, ROOT)
+    import bench
+    return bench
+
+
+def test_steps_must_be_positive_and_dump_needs_the_rthx_path():
+    bench = _bench_module()
+    old = sys.argv
+    try:
+        for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"]):
+            sys.argv = ["bench.py"] + argv
+            with pytest.raises(SystemExit):
+                bench.parse_args()
+        sys.argv = ["bench.py", "--steps", "3", "--dump-outputs", "d"]
+        args = bench.parse_args()
+    finally:
+        sys.argv = old
+    assert args.steps == 3 and args.dump_outputs == "d"
+
+
+def test_dump_outputs_writes_float64_rows_of_a_fixed_sample(tmp_path, monkeypatch):
+    """--dump-outputs: lost whole, the count rows of a seeded emitter sample that depends on the shape only, all rows when they fit."""
+    import numpy as np
+    import torch
+    bench = _bench_module()
+    nb, N = 2, 50
+    counts = torch.arange(nb * N * N, dtype=torch.int64).reshape(nb, N, N)
+    lost = torch.arange(nb * N, dtype=torch.int64).reshape(nb, N)
+
+    def dump(d):
+        bench.dump_outputs(str(d), counts, lost)
+        return {n: np.load(d / f"{n}.npy") for n in ("counts_rows", "counts_row_ids", "lost")}
+
+    whole = dump(tmp_path / "whole")
+    assert all(a.dtype == np.float64 for a in whole.values())
+    assert np.array_equal(whole["counts_row_ids"], np.arange(N)) and np.array_equal(whole["counts_rows"], counts.numpy())
+    assert np.array_equal(whole["lost"], lost.numpy())
+    monkeypatch.setattr(bench, "DUMP_COUNT_BYTES", 7 * 8 * nb * N)
+    a, b = dump(tmp_path / "a"), dump(tmp_path / "b")
+    ids = a["counts_row_ids"].astype(np.int64)
+    assert len(ids) == 7 and np.all(np.diff(ids) > 0) and np.array_equal(a["counts_row_ids"], b["counts_row_ids"])
+    assert np.array_equal(a["counts_rows"], counts.numpy()[:, ids]) and np.array_equal(a["lost"], lost.numpy())
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(tmp_path, rthx_mod, cuda_lib):
+    """The dumped tallies are those of the last timed step (seed 1000 + 1000 + steps - 1), identical to a plain trace of that seed."""
+    import numpy as np
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cfg1", "--steps", "2", "--warmup", "1",
+                        "--no-extras", "--no-e2e", "--no-smoothing", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2
+    flat = rthx_mod.flatten_domain(rthx_mod.meshes.cfg1())
+    want = rthx_mod.DeviceTracer(flat, device=0).trace(line["config"]["rays_per_emitter"], seed=2001)
+    ids = np.load(tmp_path / "counts_row_ids.npy").astype(np.int64)
+    assert np.array_equal(ids, np.arange(flat.n_elements))
+    assert np.array_equal(np.load(tmp_path / "counts_rows.npy"), want["counts"][:, ids].astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "lost.npy"), want["lost"].astype(np.float64))
