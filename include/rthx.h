@@ -269,6 +269,35 @@ int rthx_smooth_F(rthx_handle* h, int source, const void* src_host, int bin, int
 int rthx_smooth_DkAP(rthx_handle* h, int source, const void* src_host, int bin, int n, const double* w, int k_dykstra,
                      int max_iters, double target, int measure_pass, double* F_out, rthx_smooth_stats* stats);
 
+/* Reciprocity smoothing of a SPARSE exchange-factor matrix on the device: the sparse branch of smooth_F (density <= 0.25,
+ * smoothExchangeFactors.jl:432-434), i.e. AP (:548-612) on the non-zero pattern.  X = (W F + (W F)')/2 is built on the union
+ * pattern of F and F' and is exactly symmetric; each iteration is one pass over its non-zeros; the stopping rule is that of
+ * rthx_smooth_F.  The result F_smooth keeps that pattern and stays on the device; *nnz_out receives its number of non-zeros and
+ * rthx_smooth_sparse_csc copies it out.
+ *   source RTHX_SMOOTH_FROM_LAST_TRACE: the UInt64 counts of traced bin `bin` still resident from the last full trace on this
+ *          handle (single-device, or rthx_trace_exchange_multi with counts_out == NULL on hs[0]); n <= N crops to the leading
+ *          block, row totals are taken over the crop and F_ij = count / row total exactly as rthx_counts_csc computes it;
+ *   source RTHX_SMOOTH_FROM_CSC: F given by the host as 0-based CSC, used as given — colptr [n+1] int64, rowval [nnz] int32
+ *          strictly ascending within each column, nzval [nnz] float64 (a SparseMatrixCSC, e.g. an F_raw traced in row tiles).
+ *          Checked on the host before anything is uploaded: colptr[0] != 0, a decreasing colptr, or a rowval outside [0, n) or
+ *          not strictly ascending within its column is RTHX_ERR_ARG.  colptr, rowval and nzval are ignored for FROM_LAST_TRACE.
+ * The FROM_CSC result for the F_raw that rthx_counts_csc returns is bit-identical to the FROM_LAST_TRACE result, and
+ * repeated calls are bit-identical (fixed summation orders throughout).
+ *   w, max_iters, target as for rthx_smooth_F.  stats: the Dykstra fields are 0; measure_pass != 0 times the scaling pass alone,
+ *   pass_gbs = (20 nnz_X + 8 (n + 1)) bytes / pass_ms (value read + write, column index, row pointers of X).
+ * A sparse smoothing replaces any dense F_smooth on the handle: rthx_solve_grey(RTHX_SOLVE_FROM_LAST_SMOOTH) then fails with
+ * RTHX_ERR_ARG until the next rthx_smooth_F; solve a sparse F_smooth with RTHX_SOLVE_FROM_CSC.                            [0.3+] */
+enum { RTHX_SMOOTH_FROM_CSC = 3 };
+int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n,
+                       const int64_t* colptr, const int32_t* rowval, const double* nzval,
+                       const double* w, int max_iters, double target, int measure_pass,
+                       int64_t* nnz_out, rthx_smooth_stats* stats);
+/* The F_smooth of the last rthx_smooth_sparse on this handle as CSC, with the conventions of rthx_counts_csc: colptr [n+1] int64,
+ * rowval [nnz] int64 (rowval_is_i64 != 0) or int32, rows ascending within each column, nzval [nnz]; index_base 0 or 1 is added
+ * to colptr and rowval.  RTHX_ERR_ARG when no sparse smoothing has run on the handle.                                     [0.3+] */
+int rthx_smooth_sparse_csc(rthx_handle* h, int index_base, int rowval_is_i64,
+                           int64_t* colptr, void* rowval, double* nzval);
+
 /* Grey GERT equilibrium solve on the device (next-stage row of the hot path: the consumer of F).  Restates the
  * linear-algebra core of src/HeatTransfer/equilibrium/equilibriumGrey2D.jl:80-211:
  *     M = I - Diagonal(coeff) * F'   (:148-149; coeff = ifelse(Q_known, 1, b), never formed explicitly)

@@ -15,7 +15,7 @@ import numpy as np
 
 from ._abi import (rthx_mesh, rthx_trace_args, rthx_rec_out, rthx_stats, rthx_info, rthx_smooth_stats, c_i32p, c_f64p, c_u64p,
                    rthx_solve_args, rthx_solve_stats, c_i64p,
-                   RTHX_SMOOTH_FROM_LAST_TRACE, RTHX_SMOOTH_FROM_COUNTS, RTHX_SMOOTH_FROM_F,
+                   RTHX_SMOOTH_FROM_LAST_TRACE, RTHX_SMOOTH_FROM_COUNTS, RTHX_SMOOTH_FROM_F, RTHX_SMOOTH_FROM_CSC,
                    RTHX_SOLVE_FROM_LAST_SMOOTH, RTHX_SOLVE_FROM_DENSE, RTHX_SOLVE_FROM_CSC, RTHX_ROW_MAJOR, RTHX_COL_MAJOR,
                    RTHX_FIRST_INTERACTION, RTHX_LOCATOR_AUTO, RTHX_LOCATOR_GENERIC, EXPORTED_SYMBOLS)
 
@@ -104,6 +104,11 @@ def load_library():
     L.rthx_smooth_DkAP.restype = C.c_int
     L.rthx_smooth_DkAP.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, c_f64p, C.c_int, C.c_int, C.c_double, C.c_int,
                                    c_f64p, C.POINTER(rthx_smooth_stats)]
+    L.rthx_smooth_sparse.restype = C.c_int
+    L.rthx_smooth_sparse.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_i64p, c_i32p, c_f64p, c_f64p, C.c_int, C.c_double, C.c_int,
+                                     C.POINTER(C.c_int64), C.POINTER(rthx_smooth_stats)]
+    L.rthx_smooth_sparse_csc.restype = C.c_int
+    L.rthx_smooth_sparse_csc.argtypes = [C.c_void_p, C.c_int, C.c_int, c_i64p, C.c_void_p, c_f64p]
     L.rthx_solve_grey.restype = C.c_int
     L.rthx_solve_grey.argtypes = [C.c_void_p, C.POINTER(rthx_solve_args), c_f64p, c_f64p, C.POINTER(rthx_solve_stats)]
     L.rthx_release_cached.restype = C.c_int
@@ -394,6 +399,44 @@ class DeviceTracer:
                                              int(max_iters), float(target), 1 if measure_pass else 0,
                                              F_out.ctypes.data_as(c_f64p), C.byref(st)))
         return F_out.reshape(n, n), st.as_dict()
+
+    def smooth_sparse(self, w, n: Optional[int] = None, F=None, bin: int = 0, max_iters: int = 1000, target: float = 0.0,
+                      measure_pass: bool = False):
+        """Sparse reciprocity smoothing on the device (rthx_smooth_sparse: AP on the union pattern of F and F', the sparse branch
+        of smooth_F).  Source: `F`, a scipy.sparse matrix (sent as CSC; its rows must be sorted within each column), or — without
+        it — the counts of traced bin `bin` still resident from the last `trace()`, cropped to the leading n x n block.  `w` must
+        already be renormalised (w / min(w)).  Returns (F_smooth as scipy.sparse.csc_matrix over page-locked arrays, stats dict)."""
+        import scipy.sparse as sp
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        n = len(w) if n is None else int(n)
+        assert len(w) == n
+        self._resident_F = None        # a dense F_smooth an earlier smooth() left on the device is replaced
+        keep = (None, None, None)
+        source = RTHX_SMOOTH_FROM_LAST_TRACE
+        if F is not None:
+            Fc = F.tocsc() if sp.issparse(F) else sp.csc_matrix(F)
+            assert Fc.shape == (n, n)
+            keep = (np.ascontiguousarray(Fc.indptr, dtype=np.int64), np.ascontiguousarray(Fc.indices, dtype=np.int32),
+                    np.ascontiguousarray(Fc.data, dtype=np.float64))
+            source = RTHX_SMOOTH_FROM_CSC
+        ptrs = [a.ctypes.data_as(t) if a is not None else None for a, t in zip(keep, (c_i64p, c_i32p, c_f64p))]
+        nnz = C.c_int64(0)
+        st = rthx_smooth_stats()
+        self._check(self._L.rthx_smooth_sparse(self._h, source, int(bin), n, *ptrs, w.ctypes.data_as(c_f64p), int(max_iters),
+                                               float(target), 1 if measure_pass else 0, C.byref(nnz), C.byref(st)))
+        nz = nnz.value
+        k = max(1, nz)
+        alloc = pinned_empty if k > (1 << 16) else (lambda shape, dtype: np.empty(shape, dtype))
+        colptr = np.empty(n + 1, np.int64)
+        rowval = alloc(k, np.int32 if nz < 2 ** 31 else np.int64)
+        nzval = alloc(k, np.float64)
+        self._check(self._L.rthx_smooth_sparse_csc(self._h, 0, 0 if nz < 2 ** 31 else 1, colptr.ctypes.data_as(c_i64p),
+                                                   rowval.ctypes.data_as(C.c_void_p), nzval.ctypes.data_as(c_f64p)))
+        if nz < 2 ** 31:
+            colptr = colptr.astype(np.int32)           # scipy wants one index type; N + 1 entries, the big array stays as it is
+        Fs = sp.csc_matrix((nzval[:nz], rowval[:nz], colptr), shape=(n, n), copy=False)
+        Fs.has_sorted_indices = True                   # rows ascend within each column by construction
+        return Fs, st.as_dict()
 
     def solve_grey(self, coeff, rhs, F=None, col_major: bool = False, memory: int = 50, max_iters: int = 0,
                    rtol: float = 1e-12, atol: float = -1.0, measure_pass: bool = False):

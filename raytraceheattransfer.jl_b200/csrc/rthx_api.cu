@@ -48,6 +48,15 @@ struct DevRes {
   double* smooth_vec = nullptr;             size_t smooth_vec_cap = 0; // w, rs, r, u, part (5 n doubles)
   void* smooth_src = nullptr;               size_t smooth_src_cap = 0; // staged host matrix (FROM_COUNTS / FROM_F)
   double* dyk_buf = nullptr;                size_t dyk_cap = 0;        // Dykstra rounds: Xbar / F iterate (+ second iterate and P for k > 1)
+  // sparse smoothing (rthx_smooth_sparse): F as CSC and as sorted transpose keys, the CSR iterate X, work vectors, sort scratch
+  long long* sp_ptr = nullptr;              size_t sp_ptr_cap = 0;     // colptr of F | row pointers of F | row pointers of X (3 (n+1))
+  int* sp_rowval = nullptr;                 size_t sp_rowval_cap = 0;  // rowval of F
+  double* sp_val = nullptr;                 size_t sp_val_cap = 0;     // values of F as CSC | in row order (2 nnz_F)
+  unsigned long long* sp_keys = nullptr;    size_t sp_keys_cap = 0;    // transpose keys | sorted keys (2 nnz_F); index read-out scratch
+  int* sp_xcol = nullptr;                   size_t sp_xcol_cap = 0;    // X / F_smooth: column indices
+  double* sp_xval = nullptr;                size_t sp_xval_cap = 0;    // X / F_smooth: values
+  double* sp_vec = nullptr;                 size_t sp_vec_cap = 0;     // w, r, u, u', part (5 n) + 8 scalars
+  void* sp_tmp = nullptr;                   size_t sp_tmp_cap = 0;     // radix-sort scratch (bytes)
   double* solve_buf = nullptr;              size_t solve_cap = 0;      // Krylov basis + work vectors + matvec partials
   double* solve_mat = nullptr;              size_t solve_mat_cap = 0;  // staged host F of rthx_solve_grey (dense padded / CSC)
   void* stage[2] = {nullptr, nullptr};      size_t stage_cap = 0;      // pinned staging for pageable destinations
@@ -77,6 +86,7 @@ struct rthx_handle : DevRes {
   int last_trace_bins = 0; size_t last_trace_rows = 0;    // resident counts: bins, rows per bin (N, or the rows of a shard)
   int last_rank = 0, last_world = 1;                      // ... row y of the resident matrix is element last_rank + y * last_world
   int smooth_n = 0; size_t smooth_ldx = 0;                // F_smooth resident in smooth_X after rthx_smooth_F (0: none)
+  int sparse_n = 0; long long sparse_nnz = 0;             // sparse F_smooth resident in sp_* after rthx_smooth_sparse (0: none)
   int csr_bin = -1; long long csr_total = 0;              // bin whose row pointers are prepared on the device
   int csc_bin = -1;                                       // bin whose column pointers are prepared on the device
   double csr_chi = 0.0;                                   // surface-gas cross-coupling of that bin's row-normalised F
@@ -100,6 +110,7 @@ bool g_kernels_configured[64] = {};   // cudaFuncSetAttribute(max dynamic smem) 
 
 void devres_free(DevRes& r) {
   cudaFree(r.smooth_X); cudaFree(r.smooth_vec); cudaFree(r.smooth_src); cudaFree(r.solve_buf); cudaFree(r.solve_mat); cudaFree(r.dyk_buf);
+  cudaFree(r.sp_ptr); cudaFree(r.sp_rowval); cudaFree(r.sp_val); cudaFree(r.sp_keys); cudaFree(r.sp_xcol); cudaFree(r.sp_xval); cudaFree(r.sp_vec); cudaFree(r.sp_tmp);
   cudaFree(r.csr_nnz); cudaFree(r.csr_rowsum); cudaFree(r.csr_rowptr); cudaFree(r.csr_out); cudaFree(r.csr_cross); cudaFree(r.csc_partial); cudaFree(r.csc_colptr); cudaFree(r.row_done_dev);
   cudaFree(r.arena); cudaFree(r.generic_arena); cudaFree(r.counts_dev); cudaFree(r.rec_pts_dev); cudaFree(r.rec_valid_dev); cudaFree(r.peak_dev);
   for (auto& e : r.ev) if (e) cudaEventDestroy(e);
@@ -2053,6 +2064,140 @@ extern "C" int rthx_smooth_DkAP(rthx_handle* h, int source, const void* src_host
     st->launches += dres.launches;
     st->converged = res.converged; st->pad_ = 0;
   }
+  return RTHX_OK;
+}
+
+namespace rthx {
+size_t sparse_sort_temp_bytes(int nnz, int n);
+cudaError_t sparse_transpose(int n, int nnz, const long long* colptr, const int* rowval, const double* val, unsigned long long* keys,
+                             unsigned long long* keys_sorted, double* val_sorted, long long* rptr, void* temp, size_t temp_bytes, cudaStream_t st);
+cudaError_t launch_x_count(int n, const long long* colptr, const int* rowval, const long long* rptr, const unsigned long long* keys_sorted, long long* xptr,
+                           cudaStream_t st);
+cudaError_t launch_x_fill(int n, const long long* colptr, const int* rowval, const double* val, const long long* rptr, const unsigned long long* keys_sorted,
+                          const double* val_sorted, const double* w, long long* xptr, int* xcol, double* xval, cudaStream_t st);
+cudaError_t run_ap_sparse(int n, long long nnz_f, long long nnz_x, const long long* xptr, const int* xcol, double* xval, const double* w, double* vec,
+                          int max_iters, double target, cudaStream_t st, SmoothResult* out);
+cudaError_t time_sparse_pass(int n, const long long* xptr, const int* xcol, double* xval, const double* w, double* vec, int reps, cudaStream_t st,
+                             cudaEvent_t e0, cudaEvent_t e1, double* ms_per_pass);
+cudaError_t launch_index_out(const int* col, long long nnz, int base, void* out, bool i64, cudaStream_t st);
+}  // namespace rthx
+
+extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, const int64_t* colptr, const int32_t* rowval, const double* nzval,
+                                  const double* w, int max_iters, double target, int measure_pass, int64_t* nnz_out, rthx_smooth_stats* st) {
+  if (!h) return RTHX_ERR_ARG;
+  if (n < 1 || !w || !nnz_out || max_iters < 0) return fail(h, RTHX_ERR_ARG, "smooth_sparse: bad argument");
+  long long nnz_f = 0;
+  if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
+    if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev || n > h->N || h->last_world != 1 || (int)h->last_trace_rows != h->N)
+      return fail(h, RTHX_ERR_ARG, "smooth_sparse: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
+  } else if (source == RTHX_SMOOTH_FROM_CSC) {
+    // the whole matrix is checked here, before anything is uploaded: a bad index must never reach a kernel
+    if (!colptr) return fail(h, RTHX_ERR_ARG, "smooth_sparse: colptr is NULL");
+    if (colptr[0] != 0) return fail(h, RTHX_ERR_ARG, "smooth_sparse: colptr[0] must be 0 (0-based CSC)");
+    for (int j = 0; j < n; ++j)
+      if (colptr[j + 1] < colptr[j]) return fail(h, RTHX_ERR_ARG, "smooth_sparse: colptr decreases at column " + std::to_string(j));
+    nnz_f = colptr[n];
+    if (nnz_f > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "smooth_sparse: more than 2^31 - 1 non-zeros");
+    if (nnz_f > 0 && (!rowval || !nzval)) return fail(h, RTHX_ERR_ARG, "smooth_sparse: rowval / nzval is NULL");
+    for (int j = 0; j < n; ++j)
+      for (long long p = colptr[j]; p < colptr[j + 1]; ++p)
+        if (rowval[p] < 0 || rowval[p] >= n || (p > colptr[j] && rowval[p] <= rowval[p - 1]))
+          return fail(h, RTHX_ERR_ARG, "smooth_sparse: rowval out of [0, n) or not strictly ascending in column " + std::to_string(j));
+  } else {
+    return fail(h, RTHX_ERR_ARG, "smooth_sparse: unknown source");
+  }
+  CU(h, cudaSetDevice(h->device));
+  h->smooth_n = 0;                 // a dense F_smooth left by rthx_smooth_F is no longer the handle's smoothing result
+  h->sparse_n = 0;
+  const size_t n1 = (size_t)n + 1;
+  CU(h, ensure(&h->sp_ptr, &h->sp_ptr_cap, 3 * n1));
+  CU(h, ensure(&h->sp_vec, &h->sp_vec_cap, 5 * (size_t)n + 8));
+  long long *cp = h->sp_ptr, *rptr = cp + n1, *xptr = rptr + n1;
+  double* w_dev = h->sp_vec;
+  double* vec = w_dev + n;                                     // r | u | u' | part | scalars
+  CU(h, cudaMemcpyAsync(w_dev, w, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
+  CU(h, cudaEventRecord(h->ev[0], h->stream));
+  if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
+    // F = counts / row total over the crop, compacted to CSC by the read-out kernels of rthx_counts_csc
+    const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * h->N;
+    const size_t ld = (size_t)h->N;
+    unsigned long long* rowsum = reinterpret_cast<unsigned long long*>(vec + n);   // u and u' are free until the iteration
+    int* row_nnz = reinterpret_cast<int*>(vec + 2 * (size_t)n);
+    CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)((n + 63) / 64) * (size_t)n));
+    CU(h, rthx::launch_row_nnz(c, n, n, ld, h->ns, 0, 1, row_nnz, rowsum, nullptr, h->stream));
+    CU(h, rthx::launch_csc_count(c, n, ld, h->csc_partial, cp, h->stream));
+    CU(h, cudaMemcpyAsync(&nnz_f, cp + n, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    CU(h, cudaStreamSynchronize(h->stream));
+    if (nnz_f > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "smooth_sparse: more than 2^31 - 1 non-zeros");
+    CU(h, ensure(&h->sp_rowval, &h->sp_rowval_cap, (size_t)std::max<long long>(nnz_f, 1)));
+    CU(h, ensure(&h->sp_val, &h->sp_val_cap, 2 * (size_t)std::max<long long>(nnz_f, 1)));
+    CU(h, rthx::launch_csc_fill(c, n, ld, h->csc_partial, cp, rowsum, 0, h->sp_rowval, false, nullptr, h->sp_val, h->stream));
+  } else {
+    CU(h, ensure(&h->sp_rowval, &h->sp_rowval_cap, (size_t)std::max<long long>(nnz_f, 1)));
+    CU(h, ensure(&h->sp_val, &h->sp_val_cap, 2 * (size_t)std::max<long long>(nnz_f, 1)));
+    CU(h, cudaMemcpyAsync(cp, colptr, sizeof(long long) * n1, cudaMemcpyHostToDevice, h->stream));
+    if (nnz_f > 0) {
+      CU(h, cudaMemcpyAsync(h->sp_rowval, rowval, sizeof(int) * (size_t)nnz_f, cudaMemcpyHostToDevice, h->stream));
+      CU(h, cudaMemcpyAsync(h->sp_val, nzval, sizeof(double) * (size_t)nnz_f, cudaMemcpyHostToDevice, h->stream));
+    }
+  }
+  // transpose (CSR of F), then X on the union pattern
+  const size_t nz1 = (size_t)std::max<long long>(nnz_f, 1);
+  CU(h, ensure(&h->sp_keys, &h->sp_keys_cap, 2 * nz1));
+  const size_t tmp_bytes = rthx::sparse_sort_temp_bytes((int)nnz_f, n);
+  CU(h, ensure(reinterpret_cast<char**>(&h->sp_tmp), &h->sp_tmp_cap, tmp_bytes));
+  double* val_sorted = h->sp_val + nz1;
+  unsigned long long* keys_sorted = h->sp_keys + nz1;
+  CU(h, rthx::sparse_transpose(n, (int)nnz_f, cp, h->sp_rowval, h->sp_val, h->sp_keys, keys_sorted, val_sorted, rptr, h->sp_tmp, tmp_bytes, h->stream));
+  CU(h, rthx::launch_x_count(n, cp, h->sp_rowval, rptr, keys_sorted, xptr, h->stream));
+  long long nnz_x = 0;
+  CU(h, cudaMemcpyAsync(&nnz_x, xptr + n, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  CU(h, ensure(&h->sp_xcol, &h->sp_xcol_cap, (size_t)std::max<long long>(nnz_x, 1)));
+  CU(h, ensure(&h->sp_xval, &h->sp_xval_cap, (size_t)std::max<long long>(nnz_x, 1)));
+  CU(h, rthx::launch_x_fill(n, cp, h->sp_rowval, h->sp_val, rptr, keys_sorted, val_sorted, w_dev, xptr, h->sp_xcol, h->sp_xval, h->stream));
+  rthx::SmoothResult res{};
+  const double tgt = target > 0 ? target : 8 * 2.220446049250313e-16;
+  CU(h, rthx::run_ap_sparse(n, nnz_f, nnz_x, xptr, h->sp_xcol, h->sp_xval, w_dev, vec, max_iters, tgt, h->stream, &res));
+  CU(h, cudaEventRecord(h->ev[1], h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  float ms = 0;
+  CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]));
+  h->sparse_n = n; h->sparse_nnz = nnz_x;
+  *nnz_out = nnz_x;
+  double pass_ms = 0;
+  if (measure_pass) CU(h, rthx::time_sparse_pass(n, xptr, h->sp_xcol, h->sp_xval, w_dev, vec, 20, h->stream, h->ev[0], h->ev[1], &pass_ms));
+  if (st) {
+    std::memset(st, 0, sizeof(*st));
+    st->iterations = res.iters; st->launches = res.launches; st->delta_init = res.delta_init; st->delta = res.delta;
+    st->total_ms = ms; st->ms_per_iteration = res.iters > 0 ? ms / res.iters : 0.0; st->pass_ms = pass_ms;
+    st->pass_gbs = pass_ms > 0 ? (20.0 * (double)nnz_x + 8.0 * (double)n1) / (pass_ms * 1e-3) / 1e9 : 0.0;
+    st->converged = res.converged;
+  }
+  return RTHX_OK;
+}
+
+extern "C" int rthx_smooth_sparse_csc(rthx_handle* h, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, double* nzval) {
+  if (!h) return RTHX_ERR_ARG;
+  if (!colptr || !rowval || !nzval || (index_base != 0 && index_base != 1)) return fail(h, RTHX_ERR_ARG, "smooth_sparse_csc: bad argument");
+  if (h->sparse_n < 1) return fail(h, RTHX_ERR_ARG, "smooth_sparse_csc: no sparse F_smooth on this handle (run rthx_smooth_sparse first)");
+  CU(h, cudaSetDevice(h->device));
+  const int n = h->sparse_n;
+  const long long nnz = h->sparse_nnz;
+  const long long* xptr = h->sp_ptr + 2 * ((size_t)n + 1);
+  int rc = copy_out(h, colptr, xptr, sizeof(long long) * ((size_t)n + 1), h->stream);
+  if (rc) return rc;
+  if (index_base) for (int i = 0; i <= n; ++i) colptr[i] += index_base;
+  if (nnz > 0) {
+    const void* idx = h->sp_xcol;
+    if (index_base || rowval_is_i64) {         // the key buffers (>= 16 bytes per entry of F, >= 8 per entry of F_smooth) are free now
+      CU(h, rthx::launch_index_out(h->sp_xcol, nnz, index_base, h->sp_keys, rowval_is_i64 != 0, h->stream));
+      idx = h->sp_keys;
+    }
+    if ((rc = copy_out(h, rowval, idx, (rowval_is_i64 ? sizeof(long long) : sizeof(int)) * (size_t)nnz, h->stream))) return rc;
+    if ((rc = copy_out(h, nzval, h->sp_xval, sizeof(double) * (size_t)nnz, h->stream))) return rc;
+  }
+  CU(h, cudaStreamSynchronize(h->stream));
   return RTHX_OK;
 }
 

@@ -14,11 +14,14 @@
 //                         system R lambda = b (DualSolver :1-37, Jacobi-PCG, rtol 1e-14), then max(., 0) with the
 //                         Dykstra correction P                         -> op_xbar / y_matvec / pcg_* / op_finalize kernels
 // Every pass is HBM-bound: 16 B per matrix element per iteration (read + write of X), 8 B for a delta check.
+// The sparse branch (density <= 0.25, :432-434) runs the same AP on the non-zero pattern: see "Sparse AP" at the end of this file.
 #include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <string>
 #include <vector>
+
+#include <cub/device/device_radix_sort.cuh>
 
 #include "rthx_internal.h"
 
@@ -315,6 +318,41 @@ __global__ void __launch_bounds__(256) nnz_count_kernel(const T* __restrict__ sr
   if (lane == 0 && cnt) atomicAdd(out, (unsigned long long)cnt);
 }
 
+// The AP iteration with the reference's stopping rule (smoothExchangeFactors.jl:548-612), shared by the dense and the sparse
+// form: `step()` enqueues one iteration (scaling pass + u = w ./ r), `delta_now(&d)` returns delta_R_X of the current iterate.
+// `guard` is the floor below which a stalled contraction is accepted.  Returns the iterations run and the final delta.
+struct ApLoop { int iters; double delta, delta_init; bool floor_accepted; };
+template <class Step, class Delta>
+static cudaError_t ap_loop(int max_iters, double target, double guard, Step step, Delta delta_now, ApLoop* out) {
+  cudaError_t e;
+  double delta = 0;
+  if ((e = delta_now(&delta)) != cudaSuccess) return e;
+  const double delta_init = delta;
+  double best = delta, delta_prev = delta, rho_est = 0.5;
+  int k = 0, k_next = 1, flat = 0, checks = 0, k_prev = 0;
+  bool floor_accepted = false;
+  while (k < max_iters && delta > target) {
+    if ((e = step()) != cudaSuccess) return e;
+    ++k;
+    if (k >= k_next || k == max_iters) {
+      if ((e = delta_now(&delta)) != cudaSuccess) return e;
+      // the reference's stopping rule (smoothExchangeFactors.jl:578-590): contraction estimate and the flat count start with
+      // the third check; a stalled contraction is accepted only below the guard, otherwise the loop runs to max_iters
+      ++checks;
+      if (checks >= 3) {
+        rho_est = std::min(std::max(std::pow(delta / delta_prev, 1.0 / std::max(k - k_prev, 1)), 0.5), 0.9999);
+        flat = delta >= best * (1 - 1e-3) ? flat + 1 : 0;
+      }
+      best = std::min(best, delta);
+      if (delta < guard && (rho_est > 0.99 || flat >= 3)) { floor_accepted = true; break; }
+      k_prev = k; delta_prev = delta;
+      k_next = k + std::min(32, std::max(1, k));             // 1,2,4,...,32 then every 32 iterations
+    }
+  }
+  out->iters = k; out->delta = delta; out->delta_init = delta_init; out->floor_accepted = floor_accepted;
+  return cudaSuccess;
+}
+
 // Runs AP on the device.  `src_counts` (u64, leading dimension ld) or `src_F` (doubles; `src_rs` = its row sums when it
 // still has to be row-normalised, else nullptr) is a DEVICE pointer; X (n*ldx doubles) and the work vectors are device
 // scratch owned by the caller.  On return X holds F_smooth.
@@ -360,41 +398,24 @@ cudaError_t run_ap(const unsigned long long* src_counts, const double* src_F, co
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
     if (nz > 0) guard = target * std::sqrt((double)n * (double)n / (double)nz);
   }
-  double delta = 0;
-  if ((e = delta_now(&delta)) != cudaSuccess) return e;
-  const double delta_init = delta;
-  double best = delta, delta_prev = delta, rho_est = 0.5;
-  int k = 0, k_next = 1, flat = 0, checks = 0, k_prev = 0;
-  bool floor_accepted = false;
-  while (k < max_iters && delta > target) {
+  auto step = [&]() -> cudaError_t {
     scale_rows_kernel<<<n, ROW_THREADS, 0, st>>>(X, u, ldx, r);
     u_kernel<<<(unsigned)((ldx + 255) / 256), 256, 0, st>>>(w_dev, r, n, (int)ldx, u);
     launches += 2;
-    ++k;
-    if (k >= k_next || k == max_iters) {
-      if ((e = delta_now(&delta)) != cudaSuccess) return e;
-      // the reference's stopping rule (smoothExchangeFactors.jl:578-590): contraction estimate and the flat count start with
-      // the third check; a stalled contraction is accepted only below the guard, otherwise the loop runs to max_iters
-      ++checks;
-      if (checks >= 3) {
-        rho_est = std::min(std::max(std::pow(delta / delta_prev, 1.0 / std::max(k - k_prev, 1)), 0.5), 0.9999);
-        flat = delta >= best * (1 - 1e-3) ? flat + 1 : 0;
-      }
-      best = std::min(best, delta);
-      if (delta < guard && (rho_est > 0.99 || flat >= 3)) { floor_accepted = true; break; }
-      k_prev = k; delta_prev = delta;
-      k_next = k + std::min(32, std::max(1, k));             // 1,2,4,...,32 then every 32 iterations
-    }
-  }
+    return cudaSuccess;
+  };
+  ApLoop lp{};
+  if ((e = ap_loop(max_iters, target, guard, step, delta_now, &lp)) != cudaSuccess) return e;
   recover_kernel<<<n, ROW_THREADS, 0, st>>>(X, r, ldx);
   ++launches;
   if ((e = cudaEventRecord(e1, st)) != cudaSuccess) return e;
   if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
   float ms = 0;
   cudaEventElapsedTime(&ms, e0, e1);
-  out->iters = k; out->delta = delta; out->delta_init = delta_init; out->ms_total = ms;
+  const int k = lp.iters;
+  out->iters = k; out->delta = lp.delta; out->delta_init = lp.delta_init; out->ms_total = ms;
   out->ms_per_iter = k > 0 ? ms / k : 0.0; out->launches = launches;
-  out->converged = (delta <= target || floor_accepted) ? 1 : 0;     // else the reference warns "AP reached max_iters" (:605-607)
+  out->converged = (lp.delta <= target || lp.floor_accepted) ? 1 : 0;     // else the reference warns "AP reached max_iters" (:605-607)
   return cudaGetLastError();
 }
 
@@ -616,6 +637,225 @@ cudaError_t time_scale_pass(double* X, double* u, double* r, int n, size_t ldx, 
   float ms = 0;
   cudaEventElapsedTime(&ms, e0, e1);
   *ms_per_pass = ms / reps;
+  return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Sparse AP: the branch of smooth_F for density <= 0.25 (smoothExchangeFactors.jl:432-434, AP :548-612 on the non-zero
+// pattern).  F arrives as CSC (uploaded, or compacted from the resident counts by csc_count / csc_fill); its transpose (the
+// CSR of F) comes from a radix sort of (row, column) keys, so the order within a row is fixed.  X = (W F + (W F)')/2 lives on
+// the union pattern of F and F' as CSR with ascending columns and is exactly symmetric, so F_smooth = X ./ r leaves as CSC
+// without a transpose: colptr = X's row pointers, rowval = X's columns, nzval[p] = X[p] / r[col[p]].
+// One iteration is one pass over X: 8 B value read + 8 B write + 4 B column index per entry, plus the row pointers; u
+// (8 n bytes) is gathered from L2.
+// ---------------------------------------------------------------------------------------------------------------
+
+// CSC of F -> transpose keys (row << 32 | column) and the non-zeros per row of F (atomic counts: the totals are deterministic)
+__global__ void __launch_bounds__(256) csc_keys_kernel(const long long* __restrict__ colptr, const int* __restrict__ rowval, int n,
+                                                       unsigned long long* __restrict__ keys, unsigned long long* __restrict__ row_cnt) {
+  const int j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (j >= n) return;
+  for (long long p = colptr[j] + lane; p < colptr[j + 1]; p += 32) {
+    const int i = rowval[p];
+    keys[p] = ((unsigned long long)i << 32) | (unsigned)j;
+    atomicAdd(row_cnt + i, 1ull);
+  }
+}
+
+// Row i of X is the union of row i of F (sorted keys [rptr[i], rptr[i+1]), column in the low word) and column i of F (rowval
+// [colptr[i], colptr[i+1]), ascending); one thread per row merges the two lists.  FILL == false counts the union into xptr[i];
+// FILL == true writes X_ij = (w_i F_ij + w_j F_ji) / 2.  X_ji is the same expression with the two products swapped; the
+// products are rounded on their own (no FMA contraction) so that the sum, and with it X, is exactly symmetric.
+template <bool FILL>
+__global__ void __launch_bounds__(256) x_merge_kernel(int n, const long long* __restrict__ colptr, const int* __restrict__ rowval,
+                                                      const double* __restrict__ val, const long long* __restrict__ rptr,
+                                                      const unsigned long long* __restrict__ keys, const double* __restrict__ kval,
+                                                      const double* __restrict__ w, long long* __restrict__ xptr, int* __restrict__ xcol,
+                                                      double* __restrict__ xval) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  long long a = rptr[i], b = colptr[i], k = FILL ? xptr[i] : 0;
+  const long long ae = rptr[i + 1], be = colptr[i + 1];
+  const double wi = FILL ? w[i] : 0.0;
+  while (a < ae || b < be) {
+    const int ja = a < ae ? (int)(keys[a] & 0xffffffffull) : 0x7fffffff;
+    const int jb = b < be ? rowval[b] : 0x7fffffff;
+    const int j = min(ja, jb);
+    if (FILL) {
+      const double fij = ja == j ? kval[a] : 0.0, fji = jb == j ? val[b] : 0.0;
+      xcol[k] = j;
+      xval[k] = 0.5 * __dadd_rn(__dmul_rn(wi, fij), __dmul_rn(w[j], fji));
+    }
+    ++k;
+    a += ja == j;
+    b += jb == j;
+  }
+  if (!FILL) xptr[i] = k;
+}
+
+// One warp per row of X: (SCALE) X_p *= (u_i + u_col(p))/2, then r_i = sum of the row — lane-strided partial sums and a fixed
+// shuffle tree, so the order is the same on every call — and u'_i = w_i / r_i (1 for an empty row) into the OTHER u buffer:
+// the rows still being scaled keep reading the old u.  SCALE == false: the first hunger! (row sums of X as built).
+template <bool SCALE>
+__global__ void __launch_bounds__(256) csr_scale_kernel(int n, const long long* __restrict__ xptr, const int* __restrict__ xcol,
+                                                        double* __restrict__ xval, const double* __restrict__ u, const double* __restrict__ w,
+                                                        double* __restrict__ r, double* __restrict__ u_next) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (row >= n) return;
+  const long long e = xptr[row + 1];
+  const double hui = SCALE ? 0.5 * u[row] : 0.0;
+  double s = 0.0;
+  for (long long p = xptr[row] + lane; p < e; p += 32) {
+    double v = xval[p];
+    if (SCALE) {
+      v *= fma(0.5, u[xcol[p]], hui);       // = (u_i + u_j)/2 rounded once: the same factor for X_ij and X_ji
+      xval[p] = v;
+    }
+    s += v;
+  }
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+  if (lane == 0) { r[row] = s; u_next[row] = s > 0.0 ? w[row] / s : 1.0; }
+}
+
+// delta_R_X^2 per row over the stored upper-triangle entries: sum_{j>i} (X_ij (u_i - u_j))^2 / (w_i^2 + w_j^2) -> part[row]
+__global__ void __launch_bounds__(256) csr_delta_kernel(int n, const long long* __restrict__ xptr, const int* __restrict__ xcol,
+                                                        const double* __restrict__ xval, const double* __restrict__ u, const double* __restrict__ w,
+                                                        double* __restrict__ part) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (row >= n) return;
+  const double ui = u[row], wi2 = w[row] * w[row];
+  const long long e = xptr[row + 1];
+  double s = 0.0;
+  for (long long p = xptr[row] + lane; p < e; p += 32) {
+    const int j = xcol[p];
+    if (j > row) {
+      const double d = xval[p] * (ui - u[j]);
+      s += d * d / (wi2 + w[j] * w[j]);
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+  if (lane == 0) part[row] = s;
+}
+
+// *out = sum of part[0..n) in a fixed order (one block): the delta check moves 8 bytes to the host, not n partial sums
+__global__ void __launch_bounds__(1024) sum_kernel(const double* __restrict__ part, int n, double* __restrict__ out) {
+  __shared__ double red[32];
+  double s = 0.0;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) s += part[i];
+  s = block_allsum_1024(s, red);
+  if (threadIdx.x == 0) *out = s;
+}
+
+// recover_F (:537-546) written straight as the CSC of F_smooth: nzval[p] = X[p] / r[col[p]], in place
+__global__ void __launch_bounds__(256) csr_recover_kernel(long long nnz, const int* __restrict__ xcol, const double* __restrict__ r, double* __restrict__ xval) {
+  for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < nnz; p += (long long)gridDim.x * blockDim.x) {
+    const double d = r[xcol[p]];
+    xval[p] = d > 0.0 ? xval[p] / d : 0.0;
+  }
+}
+
+template <class IDX>
+__global__ void __launch_bounds__(256) index_out_kernel(const int* __restrict__ col, long long nnz, int base, IDX* __restrict__ out) {
+  for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < nnz; p += (long long)gridDim.x * blockDim.x) out[p] = (IDX)col[p] + base;
+}
+
+static unsigned flat_blocks(long long nnz) { return (unsigned)std::max<long long>(1, std::min<long long>((nnz + 255) / 256, 148 * 32)); }
+static int sort_end_bit(int n) { int b = 1; while ((1ll << b) < (long long)n) ++b; return 32 + b; }
+
+size_t sparse_sort_temp_bytes(int nnz, int n) {
+  size_t bytes = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr, (const double*)nullptr,
+                                  (double*)nullptr, nnz, 0, sort_end_bit(n));
+  return bytes;
+}
+
+// CSR of F from its CSC: rptr [n+1] (row pointers), keys_sorted / val_sorted [nnz] (row-major order, ascending columns)
+cudaError_t sparse_transpose(int n, int nnz, const long long* colptr, const int* rowval, const double* val, unsigned long long* keys,
+                             unsigned long long* keys_sorted, double* val_sorted, long long* rptr, void* temp, size_t temp_bytes, cudaStream_t st) {
+  cudaError_t e;
+  if ((e = cudaMemsetAsync(rptr, 0, sizeof(long long) * ((size_t)n + 1), st)) != cudaSuccess) return e;
+  csc_keys_kernel<<<(n + 7) / 8, 256, 0, st>>>(colptr, rowval, n, keys, reinterpret_cast<unsigned long long*>(rptr));
+  exclusive_scan_kernel<<<1, 1024, 0, st>>>(rptr, n, rptr);
+  if (nnz > 0 && (e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys, keys_sorted, val, val_sorted, nnz, 0, sort_end_bit(n), st)) != cudaSuccess)
+    return e;
+  return cudaGetLastError();
+}
+
+// row pointers of X (union pattern) into xptr [n+1]
+cudaError_t launch_x_count(int n, const long long* colptr, const int* rowval, const long long* rptr, const unsigned long long* keys_sorted, long long* xptr,
+                           cudaStream_t st) {
+  x_merge_kernel<false><<<(n + 255) / 256, 256, 0, st>>>(n, colptr, rowval, nullptr, rptr, keys_sorted, nullptr, nullptr, xptr, nullptr, nullptr);
+  exclusive_scan_kernel<<<1, 1024, 0, st>>>(xptr, n, xptr);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_x_fill(int n, const long long* colptr, const int* rowval, const double* val, const long long* rptr, const unsigned long long* keys_sorted,
+                          const double* val_sorted, const double* w, long long* xptr, int* xcol, double* xval, cudaStream_t st) {
+  x_merge_kernel<true><<<(n + 255) / 256, 256, 0, st>>>(n, colptr, rowval, val, rptr, keys_sorted, val_sorted, w, xptr, xcol, xval);
+  return cudaGetLastError();
+}
+
+// AP on the CSR iterate X (n rows, nnz_x entries); nnz_f = non-zeros of F for the floor guard.  vec: r, u0, u1, part [n each]
+// + 8 scalars.  On return xval holds the values of F_smooth as CSC (see above).  Timing is the caller's.
+cudaError_t run_ap_sparse(int n, long long nnz_f, long long nnz_x, const long long* xptr, const int* xcol, double* xval, const double* w, double* vec,
+                          int max_iters, double target, cudaStream_t st, SmoothResult* out) {
+  cudaError_t e;
+  double *r = vec, *u = r + n, *un = u + n, *part = un + n, *sc = part + n;
+  const unsigned rb = (unsigned)((n + 7) / 8);
+  int launches = 1;
+  csr_scale_kernel<false><<<rb, 256, 0, st>>>(n, xptr, xcol, xval, nullptr, w, r, u);     // r = X 1, u = w ./ r
+  auto delta_now = [&](double* d) -> cudaError_t {
+    csr_delta_kernel<<<rb, 256, 0, st>>>(n, xptr, xcol, xval, u, w, part);
+    sum_kernel<<<1, 1024, 0, st>>>(part, n, sc);
+    launches += 2;
+    double s = 0;
+    cudaError_t ee = cudaMemcpyAsync(&s, sc, sizeof(double), cudaMemcpyDeviceToHost, st);
+    if (ee != cudaSuccess) return ee;
+    if ((ee = cudaStreamSynchronize(st)) != cudaSuccess) return ee;
+    *d = std::sqrt(s);
+    return cudaSuccess;
+  };
+  auto step = [&]() -> cudaError_t {
+    csr_scale_kernel<true><<<rb, 256, 0, st>>>(n, xptr, xcol, xval, u, w, r, un);
+    std::swap(u, un);
+    ++launches;
+    return cudaSuccess;
+  };
+  // floor-aware acceptance (smoothExchangeFactors.jl:558-560): guard = target * sqrt(n^2 / nnz_F)
+  const double guard = nnz_f > 0 ? target * std::sqrt((double)n * (double)n / (double)nnz_f) : target;
+  ApLoop lp{};
+  if ((e = ap_loop(max_iters, target, guard, step, delta_now, &lp)) != cudaSuccess) return e;
+  if (nnz_x > 0) { csr_recover_kernel<<<flat_blocks(nnz_x), 256, 0, st>>>(nnz_x, xcol, r, xval); ++launches; }
+  out->iters = lp.iters; out->delta = lp.delta; out->delta_init = lp.delta_init; out->launches = launches;
+  out->converged = (lp.delta <= target || lp.floor_accepted) ? 1 : 0;
+  out->ms_total = out->ms_per_iter = 0.0;
+  return cudaGetLastError();
+}
+
+// timing helper: `reps` back-to-back sparse scaling passes with u = 1 (the factor is exactly 1: X is unchanged)
+cudaError_t time_sparse_pass(int n, const long long* xptr, const int* xcol, double* xval, const double* w, double* vec, int reps, cudaStream_t st,
+                             cudaEvent_t e0, cudaEvent_t e1, double* ms_per_pass) {
+  cudaError_t e;
+  double *r = vec, *u = r + n, *un = u + n;
+  std::vector<double> ones((size_t)n, 1.0);
+  if ((e = cudaMemcpyAsync(u, ones.data(), sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st)) != cudaSuccess) return e;
+  const unsigned rb = (unsigned)((n + 7) / 8);
+  csr_scale_kernel<true><<<rb, 256, 0, st>>>(n, xptr, xcol, xval, u, w, r, un);
+  if ((e = cudaEventRecord(e0, st)) != cudaSuccess) return e;
+  for (int i = 0; i < reps; ++i) csr_scale_kernel<true><<<rb, 256, 0, st>>>(n, xptr, xcol, xval, u, w, r, un);
+  if ((e = cudaEventRecord(e1, st)) != cudaSuccess) return e;
+  if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
+  float ms = 0;
+  cudaEventElapsedTime(&ms, e0, e1);
+  *ms_per_pass = ms / reps;
+  return cudaGetLastError();
+}
+
+// column indices of the resident F_smooth for the caller: + index_base, as int32 or int64
+cudaError_t launch_index_out(const int* col, long long nnz, int base, void* out, bool i64, cudaStream_t st) {
+  if (nnz <= 0) return cudaSuccess;
+  if (i64) index_out_kernel<long long><<<flat_blocks(nnz), 256, 0, st>>>(col, nnz, base, (long long*)out);
+  else index_out_kernel<int><<<flat_blocks(nnz), 256, 0, st>>>(col, nnz, base, (int*)out);
   return cudaGetLastError();
 }
 

@@ -244,18 +244,42 @@ def get_b(rtm) -> np.ndarray:
     return b
 
 
-def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: bool, k_dykstra=None):
-    """Dense branch of smooth_F (density > 0.25, smoothExchangeFactors.jl:432-434) on the GPU, straight from the counts of
-    traced bin number `k` (0-based position in the last launch) that the trace left on the device; returns None when the
-    sparse host path applies (sparsity must be preserved)."""
+def _warn_smoothing(st, max_iters: int):
     import warnings
+    if not st["converged"]:          # the reference @warns here (smoothExchangeFactors.jl:605-607)
+        warnings.warn(f"AP reached max_iters = {max_iters}. Final delta_R = {st['delta']:.3e}")
+    if st["delta"] > max(st["delta_init"], 16 * np.finfo(np.float64).eps):       # :608-610
+        warnings.warn("Smoothing increased the distance to the target manifold; use F_raw instead of F_smooth.")
+
+
+def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: bool, k_dykstra=None):
+    """smooth_F on the GPU for traced bin number `k` (0-based position in the last launch).  Dense branch (density > 0.25,
+    smoothExchangeFactors.jl:432-434): straight from the counts the trace left on the device.  Sparse branch with AP only
+    (k_dykstra nothing or 0): AP on the non-zero pattern, from the resident counts, or from the host CSC F_raw after a trace
+    in row tiles (only the last tile is resident).  Returns None where the host path applies: sparse Dykstra rounds, or a dense
+    F traced in row tiles."""
     tr = getattr(rtm, "_device", None)
     n = F_raw.shape[0]
-    if tr is None or max_iters <= 0 or F_raw.nnz / float(n * n) <= 0.25:
+    if tr is None or max_iters <= 0:
         return None
-    if (getattr(rtm, "last_trace_stats", None) or {}).get("row_tiles", 1) > 1:
-        return None                                          # traced in row tiles: only the last tile is resident
+    row_tiled = (getattr(rtm, "last_trace_stats", None) or {}).get("row_tiles", 1) > 1
     wn = w[:n] / np.min(w[:n])
+    if F_raw.nnz / float(n * n) <= 0.25:
+        if k_dykstra not in (None, 0):
+            return None
+        verbose and print(f"Matrix size: {n}x{n}; sparse smoothing on the device (AP, {F_raw.nnz} non-zeros)")
+        if row_tiled:
+            F_smooth, st = tr.smooth_sparse(wn, F=F_raw, max_iters=max_iters)
+        else:
+            F_smooth, st = tr.smooth_sparse(wn, n=n, bin=k, max_iters=max_iters)
+        st["path"] = "device_sparse"
+        rtm.last_smooth_stats = st
+        _warn_smoothing(st, max_iters)
+        verbose and print(f"AP: {st['iterations']} iterations, delta_R {st['delta_init']:.3e} -> {st['delta']:.3e}, "
+                          f"{st['total_ms']:.1f} ms on the device")
+        return F_smooth
+    if row_tiled:
+        return None                                          # a dense F traced in row tiles: only the last tile is resident
     if k_dykstra is None:       # smooth_F :441-450: one Dykstra round when surfaces and gas are strongly coupled, else AP only
         stats = getattr(rtm, "last_counts_stats", None)
         if rtm.surfaces_only:
@@ -268,11 +292,9 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
         k_dykstra = 1 if chi >= 0.4 else 0
     verbose and print(f"Matrix size: {n}x{n}; dense smoothing on the device ({k_dykstra} Dykstra rounds + AP)")
     F_smooth, st = tr.smooth(wn, n=n, bin=k, max_iters=max_iters, k_dykstra=int(k_dykstra))
+    st["path"] = "device_dense"
     rtm.last_smooth_stats = st
-    if not st["converged"]:          # the reference @warns here (smoothExchangeFactors.jl:605-607)
-        warnings.warn(f"AP reached max_iters = {max_iters}. Final delta_R = {st['delta']:.3e}")
-    if st["delta"] > max(st["delta_init"], 16 * np.finfo(np.float64).eps):       # :608-610
-        warnings.warn("Smoothing increased the distance to the target manifold; use F_raw instead of F_smooth.")
+    _warn_smoothing(st, max_iters)
     # the smoothed matrix also stays on the device: solveEquilibrium reads it there when handed this very array
     from .equilibrium import _sample_of
     tr._resident_F = (F_smooth, _sample_of(F_smooth))
@@ -296,12 +318,13 @@ def exchangeRayTracing(rtm, rays_tot: int, nudge: float, max_iters: int, k_dykst
         F_raw = F_raw[:ns, :ns]
 
     def smooth_one(k, F, spectral_bin):
-        # the device path where the reference would take its dense branch, the reference's sparse host iteration otherwise
+        # the device path for both branches of the reference; the host iteration for what the device does not cover
         w = get_w(rtm, spectral_bin=spectral_bin)
         Fs = _smooth_on_device(rtm, k, F, w, ns, max_iters, verbose, k_dykstra=k_dykstra)
         if Fs is None:
             Fs = smooth_F(F, w, ns, max_iters=max_iters, k_dykstra=k_dykstra, verbose=verbose,
                           smooth_surfaces_only=rtm.surfaces_only)
+            rtm.last_smooth_stats = {"path": "host"}
         return Fs
 
     if not smooth:
