@@ -374,6 +374,29 @@ int rthx_counts_csr(rthx_handle* h, int bin, int64_t* row_ptr, int32_t* cols, ui
 int rthx_counts_stats(rthx_handle* h, int bin, int64_t* nnz_out, double* chi_out);
 int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, uint64_t* vals, double* F_vals);
 
+/* Blocking trace whose counts never exist in dense form: a hashed row tally for meshes whose 8 N^2-byte count matrix does not fit
+ * (N >> 57 k elements).  Each thread block tallies its row in a shared-memory hash table and flushes it as (row, column, count)
+ * pairs into a pair buffer; the pairs are radix-sorted and reduced by key into u64 totals that stay on the device.  Device memory
+ * is O(non-zeros), not O(rows x N).  The pair buffer holds at most half the free device memory; a group of rows whose pairs
+ * overrun it is traced again split in two (exact: counts are a pure function of seed, ray id and emitter).
+ * Same arguments, lost_out, rec and stats as rthx_trace_exchange with counts_out == NULL; sharded traces (emitter_rank/world),
+ * ray_id_offset, batched bins, both locators and the recorder work as there.  RTHX_MULTI_BOUNCE[_SPECULAR] is RTHX_ERR_ARG.
+ * Afterwards rthx_counts_nnz / _csr / _stats / _csc and rthx_smooth_sparse(RTHX_SMOOTH_FROM_LAST_TRACE) return what they return
+ * after rthx_trace_exchange(counts_out == NULL) with the same arguments, bit for bit; rthx_smooth_F / rthx_smooth_DkAP
+ * (RTHX_SMOOTH_FROM_LAST_TRACE) fail with RTHX_ERR_ARG until the next dense trace, which in turn discards the sparse form.
+ * sparse_stats (may be NULL) reports the tally.                                                                           [0.3+] */
+typedef struct rthx_sparse_stats {
+  int64_t pairs;                /* pairs flushed by the launches that completed */
+  int64_t nnz;                  /* non-zeros of all traced bins after the reduction */
+  int64_t flushes;              /* hash-table flushes of those launches (one per block at least) */
+  int64_t pair_capacity;        /* pair-buffer capacity in pairs */
+  int32_t row_groups;           /* launches that completed: 1 + the number of splits after an overflow */
+  int32_t hash_slots;           /* hash-table slots per block */
+  double  reduce_ms;            /* device time of sort + reduce-by-key */
+} rthx_sparse_stats;
+int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args* args, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* stats,
+                               rthx_sparse_stats* sparse_stats);
+
 /* Peer-memory plumbing for the fused flush in one-process-per-GPU runs: rank 0 allocates the UInt64 count matrix
  * with rthx_shared_alloc and publishes the 64-byte CUDA IPC handle; every other rank maps it with rthx_shared_open
  * (peer access over NVLink is enabled lazily) and passes the mapped pointer as `counts_dev` to

@@ -66,6 +66,14 @@ class rthx_smooth_stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class rthx_sparse_stats(C.Structure):
+    _fields_ = [("pairs", C.c_int64), ("nnz", C.c_int64), ("flushes", C.c_int64), ("pair_capacity", C.c_int64),
+                ("row_groups", C.c_int32), ("hash_slots", C.c_int32), ("reduce_ms", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 RTHX_SMOOTH_FROM_LAST_TRACE, RTHX_SMOOTH_FROM_COUNTS, RTHX_SMOOTH_FROM_F, RTHX_SMOOTH_FROM_CSC = 0, 1, 2, 3
 RTHX_SOLVE_FROM_LAST_SMOOTH, RTHX_SOLVE_FROM_DENSE, RTHX_SOLVE_FROM_CSC = 0, 1, 2
 RTHX_ROW_MAJOR, RTHX_COL_MAJOR = 0, 1
@@ -106,5 +114,5 @@ EXPORTED_SYMBOLS = (
     "rthx_trace_exchange_multi", "rthx_measure_fp64_peak", "rthx_last_error", "rthx_version",
     "rthx_shared_alloc", "rthx_shared_open", "rthx_shared_close", "rthx_shared_free", "rthx_release_cached",
     "rthx_smooth_F", "rthx_smooth_DkAP", "rthx_solve_grey", "rthx_flag_signal", "rthx_flag_wait", "rthx_host_register", "rthx_host_unregister", "rthx_host_alloc", "rthx_host_free", "rthx_set_copy_helpers", "rthx_counts_nnz", "rthx_counts_csr", "rthx_counts_stats", "rthx_counts_csc",
-    "rthx_smooth_sparse", "rthx_smooth_sparse_csc",
+    "rthx_smooth_sparse", "rthx_smooth_sparse_csc", "rthx_trace_exchange_sparse",
 )

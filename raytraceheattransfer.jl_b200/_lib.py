@@ -13,7 +13,7 @@ from typing import Optional, Sequence
 
 import numpy as np
 
-from ._abi import (rthx_mesh, rthx_trace_args, rthx_rec_out, rthx_stats, rthx_info, rthx_smooth_stats, c_i32p, c_f64p, c_u64p,
+from ._abi import (rthx_mesh, rthx_trace_args, rthx_rec_out, rthx_stats, rthx_info, rthx_smooth_stats, rthx_sparse_stats, c_i32p, c_f64p, c_u64p,
                    rthx_solve_args, rthx_solve_stats, c_i64p,
                    RTHX_SMOOTH_FROM_LAST_TRACE, RTHX_SMOOTH_FROM_COUNTS, RTHX_SMOOTH_FROM_F, RTHX_SMOOTH_FROM_CSC,
                    RTHX_SOLVE_FROM_LAST_SMOOTH, RTHX_SOLVE_FROM_DENSE, RTHX_SOLVE_FROM_CSC, RTHX_ROW_MAJOR, RTHX_COL_MAJOR,
@@ -84,6 +84,9 @@ def load_library():
     L.rthx_trace_exchange.restype = C.c_int
     L.rthx_trace_exchange.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_u64p, c_u64p,
                                       C.POINTER(rthx_rec_out), C.POINTER(rthx_stats)]
+    L.rthx_trace_exchange_sparse.restype = C.c_int
+    L.rthx_trace_exchange_sparse.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_u64p, C.POINTER(rthx_rec_out), C.POINTER(rthx_stats),
+                                             C.POINTER(rthx_sparse_stats)]
     L.rthx_trace_exchange_device.restype = C.c_int
     L.rthx_trace_exchange_device.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int, C.POINTER(rthx_stats)]
@@ -295,18 +298,31 @@ class DeviceTracer:
         assert counts is None or (counts.dtype == np.uint64 and counts.size == nb * N * N and counts.flags["C_CONTIGUOUS"])
         lost = np.empty((nb, N), np.uint64)
         st = rthx_stats()
-        rec = None
-        origins = endpoints = None
-        if rec_ids:
-            cap = len(rec_ids) * int(rays_per_emitter)
-            origins = np.zeros((max(cap, 1), 2))
-            endpoints = np.zeros((max(cap, 1), 2))
-            rec = rthx_rec_out(cap, origins.ctypes.data_as(c_f64p), endpoints.ctypes.data_as(c_f64p), 0)
+        rec, origins, endpoints = _recorder(rec_ids, rays_per_emitter)
         self._check(self._L.rthx_trace_exchange(self._h, C.byref(args), counts.ctypes.data_as(c_u64p) if counts is not None else None,
                                                 lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                 C.byref(st)))
         self._last_shard = (int(args.emitter_rank), int(args.emitter_world))     # rows resident on the device: e = rank + y * world
         out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
+        if rec is not None:
+            out["origins"] = origins[: rec.n_recorded].copy()
+            out["endpoints"] = endpoints[: rec.n_recorded].copy()
+        return out
+
+    def trace_sparse(self, rays_per_emitter: int, **kw):
+        """Blocking trace with the hashed row tally (rthx_trace_exchange_sparse): the counts never exist in dense form and stay on
+        the device as sorted (row, column, total) triplets, so device memory is O(non-zeros).  Same keywords and result as
+        `trace(dense=False)` (counts is None; `counts_csr()`, `counts_csc()`, `counts_stats()` and `smooth_sparse()` read the
+        resident counts and return what they return after it, bit for bit), plus `sparse_stats` (pairs, flushes, row groups).
+        FIRST_INTERACTION only."""
+        args, keep = make_trace_args(rays_per_emitter, **kw)
+        lost = np.empty((args.n_bins, self.n_elements), np.uint64)
+        st, sst = rthx_stats(), rthx_sparse_stats()
+        rec, origins, endpoints = _recorder(kw.get("rec_ids"), rays_per_emitter)
+        self._check(self._L.rthx_trace_exchange_sparse(self._h, C.byref(args), lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
+                                                       C.byref(st), C.byref(sst)))
+        self._last_shard = (int(args.emitter_rank), int(args.emitter_world))
+        out = dict(counts=None, lost=lost, stats=st.as_dict(), sparse_stats=sst.as_dict())
         if rec is not None:
             out["origins"] = origins[: rec.n_recorded].copy()
             out["endpoints"] = endpoints[: rec.n_recorded].copy()
@@ -482,6 +498,16 @@ class DeviceTracer:
         return v.value
 
 
+def _recorder(rec_ids, rays_per_emitter: int):
+    """rthx_rec_out over fresh host arrays for `rec_ids` (None when recording is off): (rec, origins, endpoints)."""
+    if not rec_ids:
+        return None, None, None
+    cap = len(rec_ids) * int(rays_per_emitter)
+    origins = np.zeros((max(cap, 1), 2))
+    endpoints = np.zeros((max(cap, 1), 2))
+    return rthx_rec_out(cap, origins.ctypes.data_as(c_f64p), endpoints.ctypes.data_as(c_f64p), 0), origins, endpoints
+
+
 def create_multi(flat, devices: Sequence[int]):
     """One DeviceTracer per device from ONE host-side mesh preparation (rthx_create_multi)."""
     L = load_library()
@@ -514,13 +540,7 @@ def trace_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, counts_o
     lost = np.empty((nb, N), np.uint64)
     st = rthx_stats()
     hs = (C.c_void_p * len(tracers))(*[t._h for t in tracers])
-    rec = None
-    origins = endpoints = None
-    if rec_ids:
-        cap = len(rec_ids) * int(rays_per_emitter)
-        origins = np.zeros((max(cap, 1), 2))
-        endpoints = np.zeros((max(cap, 1), 2))
-        rec = rthx_rec_out(cap, origins.ctypes.data_as(c_f64p), endpoints.ctypes.data_as(c_f64p), 0)
+    rec, origins, endpoints = _recorder(rec_ids, rays_per_emitter)
     rc = L.rthx_trace_exchange_multi(hs, len(tracers), C.byref(args), counts.ctypes.data_as(c_u64p) if counts is not None else None,
                                      lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None, C.byref(st))
     if rc != 0:
@@ -534,6 +554,50 @@ def trace_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, counts_o
     return out
 
 
+def merge_row_tiles(tiles, N: int, n_bins: int):
+    """Merge the CSR read-outs of interleaved row tiles (tile t holds the rows e = t (mod n_tiles), in order) into one CSR matrix per
+    traced bin.  tiles[t][k] = (row_ptr, cols, F_vals) of bin k.  Returns a list of (row_ptr [N+1], cols, F_vals)."""
+    n_tiles = len(tiles)
+    mats = []
+    for k in range(n_bins):
+        nnz_row = np.zeros(N, np.int64)
+        for t in range(n_tiles):
+            nnz_row[t::n_tiles] = np.diff(tiles[t][k][0])
+        row_ptr = np.zeros(N + 1, np.int64)
+        np.cumsum(nnz_row, out=row_ptr[1:])
+        cols = np.empty(int(row_ptr[-1]), np.int32)
+        vals = np.empty(int(row_ptr[-1]), np.float64)
+        for t in range(n_tiles):
+            rp, c_t, f_t = tiles[t][k]
+            rows = np.arange(t, N, n_tiles)
+            lens = np.diff(rp)
+            # destination of every entry of the tile: start of its global row + offset inside the row
+            dst = np.repeat(row_ptr[rows] - rp[:-1], lens) + np.arange(int(rp[-1]), dtype=np.int64)
+            cols[dst] = c_t
+            vals[dst] = f_t
+        mats.append((row_ptr, cols, vals))
+    return mats
+
+
+def _tile_readout(tracer: DeviceTracer, n_bins: int, divide: bool = False):
+    """(per-bin CSR pieces, per-bin chi share) of the rows resident on `tracer` after a sharded trace.  F = count * (1 / row total)
+    as rthx_counts_csr forms it, or with `divide` count / row total as rthx_counts_csc does (IEEE division of exact integers: the
+    same bits as the device's CSC read-out of an unsharded trace)."""
+    parts, chi = [], np.zeros(n_bins)
+    for k in range(n_bins):
+        chi[k] = tracer.counts_stats(k)[1]
+        if divide:
+            rp, cols, vals, _ = tracer.counts_csr(k, values=True, normalised=False)
+            cs = np.zeros(len(vals) + 1, np.uint64)
+            np.cumsum(vals, out=cs[1:])
+            total = cs[rp[1:]] - cs[rp[:-1]]
+            fv = vals.astype(np.float64) / np.repeat(total, np.diff(rp)).astype(np.float64)
+        else:
+            rp, cols, _, fv = tracer.counts_csr(k, values=False, normalised=True)
+        parts.append((rp, cols.copy(), fv.copy()))
+    return parts, chi
+
+
 def trace_row_tiles(tracer: DeviceTracer, rays_per_emitter: int, n_tiles: int, **kw):
     """Exchange factors of a mesh whose dense 8 N^2-byte count matrix does not fit (N >> 57 k elements, SURVEY.md section 5): the
     emitter rows are traced in `n_tiles` interleaved tiles (rows e = t (mod n_tiles) — the multi-GPU partition, run in sequence on
@@ -542,37 +606,57 @@ def trace_row_tiles(tracer: DeviceTracer, rays_per_emitter: int, n_tiles: int, *
     id and emitter).  Returns a list of (row_ptr [N+1], cols, F_vals) per traced bin, plus lost [nb, N] and chi per bin."""
     N = tracer.n_elements
     n_tiles = max(1, min(int(n_tiles), N))
-    bins = kw.get("bins", (0,))
-    nb = len(bins)
-    nnz_row = [np.zeros(N, np.int64) for _ in range(nb)]
-    parts = [[None] * n_tiles for _ in range(nb)]
+    nb = len(kw.get("bins", (0,)))
+    tiles = []
     lost = np.zeros((nb, N), np.uint64)
     chi = np.zeros(nb)
     for t in range(n_tiles):
         out = tracer.trace(rays_per_emitter, dense=False, emitter_rank=t, emitter_world=n_tiles, **kw)
         stats = out["stats"]
         lost += out["lost"]
-        for k in range(nb):
-            chi[k] += tracer.counts_stats(k)[1]
-            rp, cols, _, fv = tracer.counts_csr(k, values=False, normalised=True)
-            nnz_row[k][t::n_tiles] = np.diff(rp)
-            parts[k][t] = (rp, cols.copy(), fv.copy())
-    mats = []
-    for k in range(nb):
-        row_ptr = np.zeros(N + 1, np.int64)
-        np.cumsum(nnz_row[k], out=row_ptr[1:])
-        cols = np.empty(int(row_ptr[-1]), np.int32)
-        vals = np.empty(int(row_ptr[-1]), np.float64)
-        for t in range(n_tiles):
-            rp, c_t, f_t = parts[k][t]
-            rows = np.arange(t, N, n_tiles)
-            lens = np.diff(rp)
-            # destination of every entry of the tile: start of its global row + offset inside the row
-            dst = np.repeat(row_ptr[rows] - rp[:-1], lens) + np.arange(int(rp[-1]), dtype=np.int64)
-            cols[dst] = c_t
-            vals[dst] = f_t
-        mats.append((row_ptr, cols, vals))
-    return dict(csr=mats, lost=lost, chi=chi, stats=stats)
+        parts, c = _tile_readout(tracer, nb)
+        tiles.append(parts)
+        chi += c
+    return dict(csr=merge_row_tiles(tiles, N, nb), lost=lost, chi=chi, stats=stats)
+
+
+def trace_sparse_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, **kw):
+    """The hashed-tally trace (DeviceTracer.trace_sparse) on several devices at once: device r traces the emitters e = r (mod n)
+    (one host thread per handle; the ctypes call releases the GIL), its rows stay on its device and only their non-zeros come back;
+    the host merges them into ONE row-normalised CSR matrix per traced bin (merge_row_tiles).  Counts are those of a single-device
+    trace bit for bit, and F = count / row total is the F_raw of a single-device trace bit for bit.  Returns dict(csr=[(row_ptr, cols, F_vals)] per bin, lost [nb, N], chi per bin, stats, sparse_stats), plus
+    origins / endpoints with rec_ids: the points of device 0's recorded emitters first, then device 1's, ... (each in ascending
+    (emitter, ray) order)."""
+    from concurrent.futures import ThreadPoolExecutor
+    n = len(tracers)
+    N = tracers[0].n_elements
+    nb = len(kw.get("bins", (0,)))
+    rec_ids = kw.pop("rec_ids", None)
+
+    def run(r):
+        own = [e for e in (rec_ids or []) if e % n == r]
+        out = tracers[r].trace_sparse(rays_per_emitter, emitter_rank=r, emitter_world=n, rec_ids=own or None, **kw)
+        parts, chi = _tile_readout(tracers[r], nb, divide=True)
+        return out, parts, chi
+
+    with ThreadPoolExecutor(max_workers=n) as ex:
+        res = list(ex.map(run, range(n)))
+    lost = np.zeros((nb, N), np.uint64)
+    chi = np.zeros(nb)
+    for out, _, c in res:
+        lost += out["lost"]
+        chi += c
+    stats = dict(res[0][0]["stats"])
+    stats["kernel_ms"] = max(o["stats"]["kernel_ms"] for o, _, _ in res)
+    stats["total_ms"] = max(o["stats"]["total_ms"] for o, _, _ in res)
+    stats["rays_traced"] = sum(o["stats"]["rays_traced"] for o, _, _ in res)
+    stats["rays_lost"] = sum(o["stats"]["rays_lost"] for o, _, _ in res)
+    sparse_stats = {k: sum(o["sparse_stats"][k] for o, _, _ in res) for k in ("pairs", "nnz", "flushes", "row_groups")}
+    result = dict(csr=merge_row_tiles([p for _, p, _ in res], N, nb), lost=lost, chi=chi, stats=stats, sparse_stats=sparse_stats)
+    if rec_ids:
+        result["origins"] = np.concatenate([o.get("origins", np.zeros((0, 2))) for o, _, _ in res], axis=0)
+        result["endpoints"] = np.concatenate([o.get("endpoints", np.zeros((0, 2))) for o, _, _ in res], axis=0)
+    return result
 
 
 class SharedDeviceBuffer:

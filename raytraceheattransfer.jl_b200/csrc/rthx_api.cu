@@ -57,6 +57,14 @@ struct DevRes {
   double* sp_xval = nullptr;                size_t sp_xval_cap = 0;    // X / F_smooth: values
   double* sp_vec = nullptr;                 size_t sp_vec_cap = 0;     // w, r, u, u', part (5 n) + 8 scalars
   void* sp_tmp = nullptr;                   size_t sp_tmp_cap = 0;     // radix-sort scratch (bytes)
+  // hashed row tally (rthx_trace_exchange_sparse): pair buffer (keys | alternate keys | counts | alternate counts, 24 bytes a pair),
+  // control words, reduction scratch, and the resident counts as sorted unique keys, u64 totals and row pointers
+  void* sk_pairs = nullptr;                 size_t sk_pairs_cap = 0;   // in pairs
+  unsigned long long* sk_ctl = nullptr;     size_t sk_ctl_cap = 0;     // [0] pairs, [1] overflow, [2] flushes, [3] unique keys of a group
+  void* sk_tmp = nullptr;                   size_t sk_tmp_cap = 0;     // bytes
+  unsigned long long* sk_keys = nullptr;    size_t sk_keys_cap = 0;
+  unsigned long long* sk_vals = nullptr;    size_t sk_vals_cap = 0;
+  long long* sk_rowptr = nullptr;           size_t sk_rowptr_cap = 0;
   double* solve_buf = nullptr;              size_t solve_cap = 0;      // Krylov basis + work vectors + matvec partials
   double* solve_mat = nullptr;              size_t solve_mat_cap = 0;  // staged host F of rthx_solve_grey (dense padded / CSC)
   void* stage[2] = {nullptr, nullptr};      size_t stage_cap = 0;      // pinned staging for pageable destinations
@@ -85,6 +93,8 @@ struct rthx_handle : DevRes {
   TraceParams base{};          // mesh pointers filled once
   int last_trace_bins = 0; size_t last_trace_rows = 0;    // resident counts: bins, rows per bin (N, or the rows of a shard)
   int last_rank = 0, last_world = 1;                      // ... row y of the resident matrix is element last_rank + y * last_world
+  bool sparse_counts = false;                             // the resident counts are the hashed tally's (sk_*), not counts_dev
+  long long sk_nnz = 0;                                   // ... its non-zeros over all traced bins
   int smooth_n = 0; size_t smooth_ldx = 0;                // F_smooth resident in smooth_X after rthx_smooth_F (0: none)
   int sparse_n = 0; long long sparse_nnz = 0;             // sparse F_smooth resident in sp_* after rthx_smooth_sparse (0: none)
   int csr_bin = -1; long long csr_total = 0;              // bin whose row pointers are prepared on the device
@@ -110,6 +120,7 @@ bool g_kernels_configured[64] = {};   // cudaFuncSetAttribute(max dynamic smem) 
 
 void devres_free(DevRes& r) {
   cudaFree(r.smooth_X); cudaFree(r.smooth_vec); cudaFree(r.smooth_src); cudaFree(r.solve_buf); cudaFree(r.solve_mat); cudaFree(r.dyk_buf);
+  cudaFree(r.sk_pairs); cudaFree(r.sk_ctl); cudaFree(r.sk_tmp); cudaFree(r.sk_keys); cudaFree(r.sk_vals); cudaFree(r.sk_rowptr);
   cudaFree(r.sp_ptr); cudaFree(r.sp_rowval); cudaFree(r.sp_val); cudaFree(r.sp_keys); cudaFree(r.sp_xcol); cudaFree(r.sp_xval); cudaFree(r.sp_vec); cudaFree(r.sp_tmp);
   cudaFree(r.csr_nnz); cudaFree(r.csr_rowsum); cudaFree(r.csr_rowptr); cudaFree(r.csr_out); cudaFree(r.csr_cross); cudaFree(r.csc_partial); cudaFree(r.csc_colptr); cudaFree(r.row_done_dev);
   cudaFree(r.arena); cudaFree(r.generic_arena); cudaFree(r.counts_dev); cudaFree(r.rec_pts_dev); cudaFree(r.rec_valid_dev); cudaFree(r.peak_dev);
@@ -940,7 +951,8 @@ int queue_variant_bits(const rthx_handle* h, const LaunchPlan& pl) {
   return h->queue_general ? 8 : 0;
 }
 
-LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, int world) {
+// hash_slots > 0: the hashed row tally (no histogram, no SQ / queue kernels; the table takes hash_table_bytes(hash_slots))
+LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, int world, int hash_slots = 0) {
   LaunchPlan pl{};
   pl.n_owned = (h->N - rank + world - 1) / world;
   if (pl.n_owned < 0) pl.n_owned = 0;
@@ -957,6 +969,7 @@ LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, i
   const size_t hist_bytes = sizeof(uint32_t) * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;   // emitter block + log table
   pl.hist_in_smem = (coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin) ? 1 : 0;
   if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) pl.hist_in_smem = 0; }   // test knob: the N > ~57k path
+  if (hash_slots > 0) pl.hist_in_smem = 0;
   pl.sq = (h->single_quad && a->locator != RTHX_LOCATOR_GENERIC && pl.hist_in_smem) ? 1 : 0;
   if (const char* ev = std::getenv("RTHX_NO_SQ")) { if (std::atoi(ev)) pl.sq = 0; }   // test / tuning knob
   // MULTI_BOUNCE on any mesh with analytic locators runs in the queue kernel's MULTI variant (lanes refill when their ray is
@@ -972,7 +985,7 @@ LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, i
     // tuning knob: 3 = the shared-loop SQ branch of the general kernel (A/B reference)
     if (const char* ev = std::getenv("RTHX_MINB")) { const int v = std::atoi(ev); if (v == 3) pl.minb = v; }
   }
-  pl.smem_bytes = coarse_bytes + em_bytes + (pl.hist_in_smem ? hist_bytes : 0);
+  pl.smem_bytes = coarse_bytes + em_bytes + (pl.hist_in_smem ? hist_bytes : 0) + (hash_slots > 0 ? hash_table_bytes(hash_slots) : 0);
   // Multi-face FAST meshes: the queue kernel (per-warp ray queue in shared memory, 40 bytes per parked ray).  Depth = as many
   // rays per lane as still leave 4 resident blocks per SM, at most 8; RTHX_QUEUE_DEPTH overrides (0 = the lock-step kernel).
   // The same kernel's general variant also takes multi-face meshes through the GENERIC locator (faces without a verified lattice,
@@ -1005,7 +1018,8 @@ LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, i
   long long chunks = a->row_chunks;
   if (chunks <= 0) {
     // enough blocks for ~32 waves of the resident set, but keep >= 2048 rays (and >= N/2, the flush scan) per block
-    const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.block_threads, pl.smem_bytes, pl.hist_in_smem != 0, pl.fast != 0, pl.minb, pl.multi != 0, pl.sq != 0, pl.queue_depth + queue_variant_bits(h, pl)));
+    const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.block_threads, pl.smem_bytes, pl.hist_in_smem != 0, pl.fast != 0, pl.minb, pl.multi != 0, pl.sq != 0, pl.queue_depth + queue_variant_bits(h, pl),
+                                                                  hash_slots > 0));
     const long long target = (long long)h->prop.multiProcessorCount * per_sm * 32;
     chunks = rows > 0 ? (target + rows - 1) / rows : 1;
     const long long min_rays = std::max<long long>(2048, h->N / 2);
@@ -1122,7 +1136,7 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
   unsigned long long* stage_counts = nullptr;
   unsigned int* row_done = nullptr;
   if (staged) {
-    h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1;            // counts_dev becomes the staging matrix
+    h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false;   // counts_dev becomes the staging matrix
     const size_t n_rows = (size_t)a->n_bins * (size_t)pl.n_owned;
     if (pl.row_chunks > 1) {
       CU(h, ensure(&h->counts_dev, &h->counts_cap, n_rows * (size_t)h->N));
@@ -1192,7 +1206,7 @@ int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, int rank, int worl
   const int n_owned = (N - rank + world - 1) / world;
   // counts_dev is about to be overwritten: whatever view an earlier trace left behind (resident bins, CSR row pointers) is void
   // until the caller re-validates it (rthx_trace_exchange does, for a complete single-device trace)
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1;
+  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false;
   CU(h, ensure(&h->counts_dev, &h->counts_cap, (size_t)a->n_bins * (size_t)n_owned * N));
   LaunchPlan pl = make_plan(h, a, rank, world);
   if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
@@ -1413,6 +1427,172 @@ extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args*
 }
 
 namespace {
+// grow a device array to >= need elements, keeping its first `keep`
+template <class T>
+cudaError_t grow_keep(T** ptr, size_t* cap, size_t need, size_t keep, cudaStream_t st) {
+  if (*cap >= need && *ptr) return cudaSuccess;
+  size_t nc = std::max(need, *cap + *cap / 2);
+  T* np = nullptr;
+  if (cudaMalloc((void**)&np, std::max<size_t>(nc, 1) * sizeof(T)) != cudaSuccess) {
+    cudaGetLastError();
+    nc = need;
+    cudaError_t e = cudaMalloc((void**)&np, std::max<size_t>(nc, 1) * sizeof(T));
+    if (e != cudaSuccess) return e;
+  }
+  cudaError_t e = cudaSuccess;
+  if (keep && *ptr) e = cudaMemcpyAsync(np, *ptr, keep * sizeof(T), cudaMemcpyDeviceToDevice, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) { cudaFree(np); return e; }
+  cudaFree(*ptr);
+  *ptr = np; *cap = nc;
+  return cudaSuccess;
+}
+}  // namespace
+
+extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st,
+                                          rthx_sparse_stats* sst) {
+  if (!h) return RTHX_ERR_ARG;
+  int rc = check_args(h, a);
+  if (rc) return rc;
+  if (a->mode != RTHX_FIRST_INTERACTION)
+    return fail(h, RTHX_ERR_ARG, "trace_sparse: the hashed tally supports RTHX_FIRST_INTERACTION only (trace MULTI_BOUNCE with rthx_trace_exchange)");
+  CU(h, cudaSetDevice(h->device));
+  const int N = h->N, nb = a->n_bins, rank = a->emitter_rank, world = a->emitter_world;
+  // whatever counts were resident (dense or sparse) are void from here on
+  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false; h->sk_nnz = 0;
+  const int bt = a->block_threads ? a->block_threads : 256;
+  int log2s = 12;                                            // 4096 slots: 32 KB of table
+  int min_log2s = 1;
+  while ((1 << min_log2s) < 2 * bt) ++min_log2s;             // a round of blockDim.x inserts must fit below half full
+  bool forced = false;
+  if (const char* ev = std::getenv("RTHX_SPARSE_HASH_SLOTS")) {   // test knob: small tables flush many times
+    const long long v = std::atoll(ev);
+    if (v > 0) { log2s = 0; while ((1ll << log2s) < v) ++log2s; forced = true; }
+  }
+  log2s = std::max(log2s, min_log2s);
+  LaunchPlan pl = make_plan(h, a, rank, world, 1 << log2s);
+  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
+  if (!forced) {                                             // a block with few rays needs no large table: clearing and scanning it is the cost
+    const long long per_block = (a->rays_per_emitter + pl.row_chunks - 1) / pl.row_chunks;
+    const long long distinct = std::min<long long>(per_block, N);
+    const int old = log2s;
+    while (log2s > min_log2s && (1ll << (log2s - 1)) >= 2 * distinct) --log2s;
+    pl.smem_bytes = pl.smem_bytes - hash_table_bytes(1 << old) + hash_table_bytes(1 << log2s);
+  }
+  if (pl.smem_bytes > h->prop.sharedMemPerBlockOptin) return fail(h, RTHX_ERR_ARG, "trace_sparse: hash table does not fit in shared memory");
+  if (!pl.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }
+  // pair buffer: at most one pair per tallied ray, and at most half the free device memory (24 bytes a pair with the sort's
+  // alternate buffers); the other half is left for the resident totals
+  long long cap = 0x7FFFFFFFll;
+  {
+    size_t free_b = 0, total_b = 0;
+    CU(h, cudaMemGetInfo(&free_b, &total_b));
+    const double rays = (double)pl.n_owned * nb * (double)a->rays_per_emitter;
+    cap = (long long)std::min<double>((double)cap, std::min(rays, (double)(free_b / 2 + h->sk_pairs_cap * 24) / 24.0));
+    if (const char* ev = std::getenv("RTHX_SPARSE_PAIR_CAP")) { const long long v = std::atoll(ev); if (v > 0) cap = std::min(cap, v); }   // test knob: forces row-group splits
+    cap = std::max<long long>(cap, 1);
+  }
+  if ((size_t)cap > h->sk_pairs_cap) {
+    cudaFree(h->sk_pairs); h->sk_pairs = nullptr; h->sk_pairs_cap = 0;
+    CU(h, cudaMalloc(&h->sk_pairs, (size_t)cap * 24));
+    h->sk_pairs_cap = (size_t)cap;
+  }
+  CU(h, ensure(&h->sk_ctl, &h->sk_ctl_cap, 4));
+  const size_t tmp_bytes = tally_temp_bytes(cap);
+  CU(h, ensure(reinterpret_cast<char**>(&h->sk_tmp), &h->sk_tmp_cap, tmp_bytes));
+  unsigned long long* keys = (unsigned long long*)h->sk_pairs;
+  unsigned long long* keys_alt = keys + cap;
+  uint32_t* cnt = (uint32_t*)(keys_alt + cap);
+  uint32_t* cnt_alt = cnt + cap;
+  const long long n_rows = (long long)pl.n_owned * nb;       // row key y * n_bins + bi
+  int end_bit = 32;
+  while ((1ll << (end_bit - 32)) < n_rows) ++end_bit;
+
+  int n_slots = 0, n_launches = 0;
+  CU(h, cudaEventRecord(h->ev[0], h->stream));
+  rc = prepare_recorder(h, a, rec, &n_slots, h->stream);
+  if (rc) return rc;
+  CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)nb, cudaMemcpyHostToDevice, h->stream));
+  CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)nb * N, h->stream));
+  n_launches += 1;
+  TraceParams P;
+  fill_params(h, a, pl, rank, world, true, nullptr, h->lost_dev, P);
+  if (n_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
+  P.sk_keys = keys; P.sk_cnt = cnt; P.sk_ctl = h->sk_ctl; P.sk_cap = (unsigned long long)cap; P.sk_slots_log2 = log2s;
+
+  // row groups in ascending order: a group whose pairs overran the buffer is traced again as two halves
+  std::vector<std::pair<int, int>> todo{{0, pl.n_owned}};
+  long long total = 0, pairs = 0, flushes = 0;
+  int groups = 0;
+  double kernel_ms = 0, reduce_ms = 0;
+  while (!todo.empty()) {
+    const auto [y0, y1] = todo.front();
+    todo.erase(todo.begin());
+    if (y1 <= y0) continue;
+    CU(h, cudaMemsetAsync(h->sk_ctl, 0, 4 * sizeof(unsigned long long), h->stream));
+    P.y_offset = y0;
+    CU(h, cudaEventRecord(h->ev[1], h->stream));
+    CU(h, launch_trace_exchange(P, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, pl.fast != 0, pl.minb, false, h->stream));
+    CU(h, cudaEventRecord(h->ev[2], h->stream));
+    n_launches += 2;
+    unsigned long long ctl[4];
+    CU(h, cudaMemcpyAsync(ctl, h->sk_ctl, sizeof(ctl), cudaMemcpyDeviceToHost, h->stream));
+    CU(h, cudaStreamSynchronize(h->stream));
+    float ms = 0;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); kernel_ms += ms;
+    if (ctl[1]) {
+      if (y1 - y0 == 1) return fail(h, RTHX_ERR_NOMEM, "trace_sparse: the pairs of one emitter row exceed the pair buffer (" + std::to_string(cap) + " pairs)");
+      for (int b = 0; b < nb; ++b)                          // the lost rays of the group are counted again
+        CU(h, cudaMemset2DAsync(h->lost_dev + (size_t)b * N + rank + (size_t)y0 * world, sizeof(unsigned long long) * world, 0,
+                                sizeof(unsigned long long), (size_t)(y1 - y0), h->stream));
+      const int mid = y0 + (y1 - y0) / 2;
+      todo.insert(todo.begin(), {{y0, mid}, {mid, y1}});
+      continue;
+    }
+    const long long n = (long long)ctl[0];
+    ++groups; pairs += n; flushes += (long long)ctl[2];
+    CU(h, grow_keep(&h->sk_keys, &h->sk_keys_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
+    CU(h, grow_keep(&h->sk_vals, &h->sk_vals_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
+    CU(h, cudaEventRecord(h->ev[1], h->stream));
+    CU(h, tally_reduce(keys, cnt, keys_alt, cnt_alt, n, end_bit, h->sk_keys + total, h->sk_vals + total, (long long*)(h->sk_ctl + 3), h->sk_tmp,
+                       h->sk_tmp_cap, h->stream));
+    CU(h, cudaEventRecord(h->ev[2], h->stream));
+    long long uniq = 0;
+    CU(h, cudaMemcpyAsync(&uniq, h->sk_ctl + 3, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    CU(h, cudaStreamSynchronize(h->stream));
+    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); reduce_ms += ms;
+    total += uniq;
+  }
+  CU(h, ensure(&h->sk_rowptr, &h->sk_rowptr_cap, (size_t)n_rows + 1));
+  CU(h, tally_row_ptr(h->sk_keys, total, n_rows, h->sk_rowptr, h->stream));
+  std::vector<uint64_t> lost_host((size_t)nb * N);
+  CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaEventRecord(h->ev[3], h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  h->sparse_counts = true; h->sk_nnz = total;
+  h->last_trace_bins = nb; h->last_trace_rows = (size_t)pl.n_owned; h->last_rank = rank; h->last_world = world;
+  if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
+  rc = collect_recorder(h, a, rec, n_slots, h->stream, false);
+  if (rc) return rc;
+  if (st) {
+    fill_stats(st, pl, a);
+    st->kernel_ms = kernel_ms;
+    float ms = 0;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3])); st->total_ms = ms;
+    int64_t nl = 0;
+    for (uint64_t v : lost_host) nl += (int64_t)v;
+    st->rays_lost = nl;
+    st->n_launches = n_launches;
+  }
+  if (sst) {
+    std::memset(sst, 0, sizeof(*sst));
+    sst->pairs = pairs; sst->nnz = total; sst->flushes = flushes; sst->pair_capacity = cap;
+    sst->row_groups = groups; sst->hash_slots = 1 << log2s; sst->reduce_ms = reduce_ms;
+  }
+  return RTHX_OK;
+}
+
+namespace {
 
 // Per-device outcome of rthx_trace_exchange_multi (one host thread drives each device).
 struct MultiJob {
@@ -1485,11 +1665,11 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
   if (gather) {
     // the full matrix lives on hs[0]; the other devices need peer access to it
     CU(h0, cudaSetDevice(h0->device));
-    h0->last_trace_bins = 0; h0->csr_bin = -1; h0->csc_bin = -1;
+    h0->last_trace_bins = 0; h0->csr_bin = -1; h0->csc_bin = -1; h0->sparse_counts = false;
     CU(h0, ensure(&h0->counts_dev, &h0->counts_cap, (size_t)a->n_bins * (size_t)N * N));
     shared_counts = h0->counts_dev;
     for (int i = 1; i < n; ++i) {
-      hs[i]->last_trace_bins = 0; hs[i]->csr_bin = -1; hs[i]->csc_bin = -1;
+      hs[i]->last_trace_bins = 0; hs[i]->csr_bin = -1; hs[i]->csc_bin = -1; hs[i]->sparse_counts = false;
       if (hs[i]->device == h0->device) continue;
       int can = 0;
       CU(h0, cudaDeviceCanAccessPeer(&can, hs[i]->device, h0->device));
@@ -1854,8 +2034,8 @@ int copy_out(rthx_handle* h, void* dst, const void* src_dev, size_t bytes, cudaS
 // cross-coupling chi of the row-normalised F (cross_coupling_chi, smoothExchangeFactors.jl:212-241).  After a sharded trace
 // (emitter_world > 1: one row tile of a matrix too large to hold at once) the rows are those of the shard and chi is their share.
 int prepare_rows(rthx_handle* h, int bin) {
-  if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev)
-    return fail(h, RTHX_ERR_ARG, "counts: no resident counts for that bin (run rthx_trace_exchange with counts_out == NULL, or rthx_trace_exchange_multi with counts_out == NULL, first)");
+  if (bin < 0 || bin >= h->last_trace_bins || (!h->counts_dev && !h->sparse_counts))
+    return fail(h, RTHX_ERR_ARG, "counts: no resident counts for that bin (run rthx_trace_exchange with counts_out == NULL, rthx_trace_exchange_multi with counts_out == NULL, or rthx_trace_exchange_sparse first)");
   if (h->csr_bin == bin) return RTHX_OK;
   CU(h, cudaSetDevice(h->device));
   const int N = h->N, R = (int)h->last_trace_rows;
@@ -1868,8 +2048,13 @@ int prepare_rows(rthx_handle* h, int bin) {
     CU(h, cudaMalloc(&h->csr_rowptr, sizeof(long long) * ((size_t)N + 1)));
     h->csr_cap = (size_t)N + 1;
   }
-  const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
-  CU(h, rthx::launch_row_nnz(c, R, N, (size_t)N, h->ns, h->last_rank, h->last_world, h->csr_nnz, h->csr_rowsum, h->csr_cross, h->stream));
+  if (h->sparse_counts) {
+    CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, R, N, h->ns, h->last_rank, h->last_world, h->csr_nnz,
+                                h->csr_rowsum, h->csr_cross, h->stream));
+  } else {
+    const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
+    CU(h, rthx::launch_row_nnz(c, R, N, (size_t)N, h->ns, h->last_rank, h->last_world, h->csr_nnz, h->csr_rowsum, h->csr_cross, h->stream));
+  }
   std::vector<int> nnz(std::max(R, 1));
   std::vector<unsigned long long> rowsum(std::max(R, 1)), cross(std::max(R, 1));
   if (R > 0) {
@@ -1890,6 +2075,74 @@ int prepare_rows(rthx_handle* h, int bin) {
   return RTHX_OK;
 }
 
+}  // namespace
+
+namespace rthx {
+size_t sparse_sort_temp_bytes(int nnz, int n);
+cudaError_t sparse_transpose(int n, int nnz, const long long* colptr, const int* rowval, const double* val, unsigned long long* keys,
+                             unsigned long long* keys_sorted, double* val_sorted, long long* rptr, void* temp, size_t temp_bytes, cudaStream_t st);
+}  // namespace rthx
+
+namespace {
+// Leading n x n block of the hashed tally's rows (bin `bin`, all emitters) as CSC in the sparse smoothing's scratch: colptr -> cp [n+1],
+// rowval -> sp_rowval, F = count / row total over the block -> sp_val (the values rthx_counts_csc computes); *nnz_out its non-zeros.
+// The CSR of the block is transposed by the radix sort of rthx_smooth_sparse (sparse_transpose), so rows ascend within each column.
+// With counts != nullptr the count of every entry (as bits) is sorted along instead of F.  vec: 3 n scratch words.
+int sparse_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long long* rptr, void* vec, bool counts, long long* nnz_out) {
+  unsigned long long* rowsum = reinterpret_cast<unsigned long long*>(vec);
+  int* row_nnz = reinterpret_cast<int*>(rowsum + n);
+  CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, n, n, h->ns, 0, 1, row_nnz, rowsum, nullptr, h->stream));
+  std::vector<int> rn((size_t)n);
+  CU(h, cudaMemcpyAsync(rn.data(), row_nnz, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  std::vector<long long> rp((size_t)n + 1, 0);
+  for (int i = 0; i < n; ++i) rp[i + 1] = rp[i] + rn[i];
+  const long long nnz = rp[n];
+  if (nnz > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "sparse counts: more than 2^31 - 1 non-zeros in one column view");
+  CU(h, cudaMemcpyAsync(rptr, rp.data(), sizeof(long long) * ((size_t)n + 1), cudaMemcpyHostToDevice, h->stream));
+  const size_t nz1 = (size_t)std::max<long long>(nnz, 1);
+  CU(h, ensure(&h->sp_rowval, &h->sp_rowval_cap, nz1));
+  CU(h, ensure(&h->sp_val, &h->sp_val_cap, 2 * nz1));
+  CU(h, ensure(&h->sp_keys, &h->sp_keys_cap, 2 * nz1));
+  const size_t tmp_bytes = rthx::sparse_sort_temp_bytes((int)nnz, n);
+  CU(h, ensure(reinterpret_cast<char**>(&h->sp_tmp), &h->sp_tmp_cap, tmp_bytes));
+  CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, n, n, rptr, rowsum, true, h->sp_rowval,
+                             counts ? reinterpret_cast<unsigned long long*>(h->sp_val) : nullptr, counts ? nullptr : h->sp_val, h->stream));
+  CU(h, rthx::sparse_transpose(n, (int)nnz, rptr, h->sp_rowval, h->sp_val, h->sp_keys, h->sp_keys + nz1, h->sp_val + nz1, cp, h->sp_tmp, tmp_bytes,
+                               h->stream));
+  *nnz_out = nnz;
+  return RTHX_OK;
+}
+
+// rthx_counts_csc after a sparse trace: sorted transpose keys -> rowval (+ base), sorted values -> F_vals / vals
+int counts_csc_sparse(rthx_handle* h, int bin, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, uint64_t* vals, double* F_vals) {
+  const int N = h->N;
+  CU(h, ensure(&h->csc_colptr, &h->csc_colptr_cap, (size_t)N + 1));
+  const size_t need = (3 * (size_t)N + 1) * sizeof(unsigned long long);   // row pointers + row totals / non-zeros scratch
+  if (h->csr_out_cap < need) {
+    cudaFree(h->csr_out); h->csr_out = nullptr; h->csr_out_cap = 0;
+    CU(h, cudaMalloc(&h->csr_out, need));
+    h->csr_out_cap = need;
+  }
+  long long* rptr = reinterpret_cast<long long*>(h->csr_out);
+  void* vec = rptr + (size_t)N + 1;
+  long long nnz = 0;
+  int rc = sparse_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, false, &nnz);
+  if (rc) return rc;
+  if (F_vals && nnz && (rc = copy_out(h, F_vals, h->sp_val + std::max<long long>(nnz, 1), sizeof(double) * (size_t)nnz, h->stream))) return rc;
+  if (vals) {                                                // the counts ride along a second sort of the same keys
+    if ((rc = sparse_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, true, &nnz))) return rc;
+    if (nnz && (rc = copy_out(h, vals, h->sp_val + std::max<long long>(nnz, 1), sizeof(uint64_t) * (size_t)nnz, h->stream))) return rc;
+  }
+  const size_t nz1 = (size_t)std::max<long long>(nnz, 1);
+  // the indices: low words of the sorted keys, written over the unsorted keys
+  CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz, index_base, h->sp_keys, rowval_is_i64 != 0, h->stream));
+  if (index_base) CU(h, rthx::launch_add_base(h->csc_colptr, N + 1, (long long)index_base, h->stream));
+  if ((rc = copy_out(h, colptr, h->csc_colptr, sizeof(long long) * ((size_t)N + 1), h->stream))) return rc;
+  if (nnz && (rc = copy_out(h, rowval, h->sp_keys, (rowval_is_i64 ? sizeof(long long) : sizeof(int)) * (size_t)nnz, h->stream))) return rc;
+  CU(h, cudaStreamSynchronize(h->stream));
+  return RTHX_OK;
+}
 }  // namespace
 
 extern "C" int rthx_counts_nnz(rthx_handle* h, int bin, int64_t* nnz_out) {
@@ -1925,9 +2178,14 @@ extern "C" int rthx_counts_csr(rthx_handle* h, int bin, int64_t* row_ptr, int32_
   unsigned long long* d_vals = (unsigned long long*)h->csr_out;
   double* d_f = (double*)(d_vals + std::max<size_t>(1, nnz));
   int* d_cols = (int*)(d_f + std::max<size_t>(1, nnz));
-  const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
   const int R = (int)h->last_trace_rows;
-  CU(h, rthx::launch_row_fill(c, R, N, (size_t)N, h->csr_rowptr, h->csr_rowsum, d_cols, d_vals, F_vals ? d_f : nullptr, h->stream));
+  if (h->sparse_counts) {
+    CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, R, N, h->csr_rowptr, h->csr_rowsum, false, d_cols, d_vals,
+                               F_vals ? d_f : nullptr, h->stream));
+  } else {
+    const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
+    CU(h, rthx::launch_row_fill(c, R, N, (size_t)N, h->csr_rowptr, h->csr_rowsum, d_cols, d_vals, F_vals ? d_f : nullptr, h->stream));
+  }
   rc = copy_out(h, row_ptr, h->csr_rowptr, sizeof(long long) * ((size_t)R + 1), h->stream);
   if (rc) return rc;
   if (nnz) {
@@ -1949,6 +2207,7 @@ extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowv
   const int N = h->N;
   const size_t nnz = (size_t)h->csr_total, nz1 = std::max<size_t>(1, nnz);
   if (!rowval_is_i64 && (size_t)N + (size_t)index_base > 0x7FFFFFFFull) return fail(h, RTHX_ERR_ARG, "counts_csc: 32-bit row indices overflow");
+  if (h->sparse_counts) { rc = counts_csc_sparse(h, bin, index_base, rowval_is_i64, colptr, rowval, vals, F_vals); if (rc) return rc; h->csc_bin = bin; return RTHX_OK; }
   const int n_tiles = (N + 63) / 64;
   CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)n_tiles * (size_t)N));
   CU(h, ensure(&h->csc_colptr, &h->csc_colptr_cap, (size_t)N + 1));
@@ -2006,6 +2265,8 @@ extern "C" int rthx_smooth_DkAP(rthx_handle* h, int source, const void* src_host
   const double* src_F = nullptr;
   size_t ld = (size_t)n;
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
+    if (h->sparse_counts)
+      return fail(h, RTHX_ERR_ARG, "smooth: the resident counts are the sparse form of rthx_trace_exchange_sparse (smooth them with rthx_smooth_sparse)");
     if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev || n > h->N || h->last_world != 1 || (int)h->last_trace_rows != h->N)
       return fail(h, RTHX_ERR_ARG, "smooth: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
     src_counts = h->counts_dev + (size_t)bin * h->last_trace_rows * h->N;
@@ -2088,7 +2349,7 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
   if (n < 1 || !w || !nnz_out || max_iters < 0) return fail(h, RTHX_ERR_ARG, "smooth_sparse: bad argument");
   long long nnz_f = 0;
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
-    if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev || n > h->N || h->last_world != 1 || (int)h->last_trace_rows != h->N)
+    if (bin < 0 || bin >= h->last_trace_bins || (!h->counts_dev && !h->sparse_counts) || n > h->N || h->last_world != 1 || (int)h->last_trace_rows != h->N)
       return fail(h, RTHX_ERR_ARG, "smooth_sparse: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
   } else if (source == RTHX_SMOOTH_FROM_CSC) {
     // the whole matrix is checked here, before anything is uploaded: a bad index must never reach a kernel
@@ -2117,7 +2378,14 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
   double* vec = w_dev + n;                                     // r | u | u' | part | scalars
   CU(h, cudaMemcpyAsync(w_dev, w, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
   CU(h, cudaEventRecord(h->ev[0], h->stream));
-  if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
+  if (source == RTHX_SMOOTH_FROM_LAST_TRACE && h->sparse_counts) {
+    // the hashed tally's rows cropped to n, F = count / row total over the crop, transposed to CSC (same values and order as below)
+    int rc = sparse_counts_to_csc(h, bin, n, cp, rptr, vec + n, false, &nnz_f);
+    if (rc) return rc;
+    const size_t nz1 = (size_t)std::max<long long>(nnz_f, 1);
+    CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz_f, 0, h->sp_rowval, false, h->stream));
+    if (nnz_f) CU(h, cudaMemcpyAsync(h->sp_val, h->sp_val + nz1, sizeof(double) * (size_t)nnz_f, cudaMemcpyDeviceToDevice, h->stream));
+  } else if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
     // F = counts / row total over the crop, compacted to CSC by the read-out kernels of rthx_counts_csc
     const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * h->N;
     const size_t ld = (size_t)h->N;

@@ -125,6 +125,13 @@ struct TraceParams {
   int32_t sq_pad_;
   uint32_t rk[20];  // Philox round keys (key + r*W), two per round
   CoarseDev face0;  // SQ kernels: the single coarse face, read from the parameter bank
+  // Hashed row tally (rthx_trace_exchange_sparse).  Kept behind everything else so that no field the other kernels read moves.
+  unsigned long long* sk_keys; // [sk_cap] pair keys (row key << 32) | column, row key = y * n_bins + bi; nullptr: no hashed tally
+  uint32_t* sk_cnt;            // [sk_cap] pair counts
+  unsigned long long* sk_ctl;  // [0] pairs reserved, [1] overflow flag, [2] flushes
+  unsigned long long sk_cap;   // pair-buffer capacity
+  int32_t sk_slots_log2;       // hash slots per block = 1 << sk_slots_log2 (>= 2 blockDim.x)
+  int32_t sk_pad_;
 };
 
 static_assert(offsetof(TraceParams, rays_per_emitter) % 16 == 0 && offsetof(TraceParams, k_u52) % 16 == 0 && offsetof(TraceParams, rk) % 16 == 0,
@@ -135,7 +142,29 @@ cudaError_t launch_trace_exchange(const TraceParams& p, int n_blocks, int block_
                                   cudaStream_t stream);   // minb == 6: the queue kernel with p.queue_depth in {1, 2, 4}
 cudaError_t configure_trace_kernel(size_t smem_bytes);
 cudaError_t launch_fp64_peak(double* out, int n_blocks, int block_threads, int iters, cudaStream_t stream);
-int trace_kernel_max_blocks_per_sm(int block_threads, size_t smem_bytes, bool hist, bool fast, int minb, bool multi, bool sq, int queue_depth = 0);
+int trace_kernel_max_blocks_per_sm(int block_threads, size_t smem_bytes, bool hist, bool fast, int minb, bool multi, bool sq, int queue_depth = 0,
+                                   bool hash = false);
+constexpr size_t hash_table_bytes(int slots) { return 8 * (size_t)slots + 16; }   // keys + counts (u32 each) + occupied / fill / base words
+
+// hashed row tally, host side of the reduction (rthx_sparse_tally.cu)
+size_t tally_temp_bytes(long long n_pairs);
+// sort the pairs of one row group and append (unique key, u64 total) to out_keys / out_vals at out_off; *n_unique_dev receives the count
+cudaError_t tally_reduce(unsigned long long* keys, uint32_t* cnt, unsigned long long* keys_alt, uint32_t* cnt_alt, long long n_pairs, int end_bit,
+                         unsigned long long* out_keys, unsigned long long* out_vals, long long* n_unique_dev, void* temp, size_t temp_bytes,
+                         cudaStream_t st);
+// row pointers [n_rows + 1] of the sorted unique keys (row key in the high word)
+cudaError_t tally_row_ptr(const unsigned long long* keys, long long nnz, long long n_rows, long long* row_ptr, cudaStream_t st);
+// rows of bin `bin` (row key y * n_bins + bin, y < n_rows): non-zeros, total and surface-gas cross tallies over the columns < n_cols
+cudaError_t tally_row_stats(const unsigned long long* keys, const unsigned long long* vals, const long long* row_ptr, int n_bins, int bin, int n_rows,
+                            int n_cols, int n_surf, int row_first, int row_stride, int* nnz, unsigned long long* rowsum, unsigned long long* cross,
+                            cudaStream_t st);
+// the same rows as CSR at out_ptr[row]: columns < n_cols, counts, and F = count * (1 / total) (divide == false, the CSR read-out) or
+// count / total (divide == true, the CSC read-out)
+cudaError_t tally_row_fill(const unsigned long long* keys, const unsigned long long* vals, const long long* row_ptr, int n_bins, int bin, int n_rows,
+                           int n_cols, const long long* out_ptr, const unsigned long long* rowsum, bool divide, int* cols, unsigned long long* cnt_out,
+                           double* fvals, cudaStream_t st);
+// low words of sorted transpose keys (the rows of a CSC) + base as int32 / int64
+cudaError_t tally_key_index(const unsigned long long* keys_sorted, long long nnz, int base, void* out, bool i64, cudaStream_t st);
 
 // ---- grey equilibrium solve (rthx_solve.cu) ---------------------------------------------------------------------
 struct SolveMatrix {

@@ -121,16 +121,27 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
     t0 = time.perf_counter()
     kw = dict(seed=seed, bins=[b - 1 for b in spectral_bins], nudge=nudge, rec_ids=rec_ids, rec_bin=rec_bin, locator=locator)
     n_tiles = auto_row_tiles(tr.n_elements, len(spectral_bins)) if row_tiles is None else int(row_tiles)
-    if n_tiles > 1:
-        # N >> 57 k elements: the dense count matrix is the limit, not the tally (SURVEY.md section 5) — trace the rows in tiles,
-        # keep only each tile's non-zeros.  One device; the recorder is not available on this path.
-        if rec is not None:
-            raise ValueError("RayRecorder is not supported together with row tiles")
-        from ._lib import trace_row_tiles
-        kw.pop("rec_ids"); kw.pop("rec_bin")
-        res = trace_row_tiles(tr, rays_per_emitter, n_tiles, **kw)
+    sparse_multi = row_tiles is None and n_tiles > 1 and len(trs) > 1
+    if n_tiles > 1 and (row_tiles is not None or sparse_multi):
+        # N >> 57 k elements: the dense count matrix is the limit, not the tally (SURVEY.md section 5).  Several devices: each traces
+        # its emitter shard with the hashed row tally and only the non-zeros come back.  An explicit row_tiles: the rows are traced in
+        # tiles on one device, keeping only each tile's non-zeros; the recorder is not available there.
+        if sparse_multi:
+            from ._lib import trace_sparse_multi
+            res = trace_sparse_multi(trs, rays_per_emitter, **kw)
+            stats = dict(res["stats"], tally="sparse", devices=len(trs), sparse=res["sparse_stats"])
+            if rec is not None and "origins" in res:
+                rec.origins[0] = np.concatenate([rec.origins[0], res["origins"]], axis=0)
+                rec.endpoints[0] = np.concatenate([rec.endpoints[0], res["endpoints"]], axis=0)
+        else:
+            if rec is not None:
+                raise ValueError("RayRecorder is not supported together with row tiles")
+            from ._lib import trace_row_tiles
+            kw.pop("rec_ids"); kw.pop("rec_bin")
+            res = trace_row_tiles(tr, rays_per_emitter, n_tiles, **kw)
+            stats = dict(res["stats"], row_tiles=n_tiles)
         t1 = time.perf_counter()
-        rtm.last_trace_stats = dict(res["stats"], row_tiles=n_tiles)
+        rtm.last_trace_stats = stats
         rtm.last_lost = res["lost"]
         N = tr.n_elements
         mats = []
@@ -142,7 +153,11 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
             mats.append(sp.csr_matrix((vals, cols, row_ptr), shape=(N, N)).tocsc())
         rtm.last_phase_ms.update({"trace": 1e3 * (t1 - t0), "csc_F_raw": 1e3 * (time.perf_counter() - t1), "row_tiles": n_tiles})
         return mats
-    if len(trs) == 1:
+    if n_tiles > 1:
+        # one device, dense matrix beyond the budget: the hashed row tally keeps the counts on the device in sparse form
+        out = tr.trace_sparse(rays_per_emitter, **kw)
+        out["stats"] = dict(out["stats"], tally="sparse", sparse=out["sparse_stats"])
+    elif len(trs) == 1:
         out = tr.trace(rays_per_emitter, dense=False, **kw)
     else:
         from ._lib import trace_multi
@@ -255,20 +270,23 @@ def _warn_smoothing(st, max_iters: int):
 def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: bool, k_dykstra=None):
     """smooth_F on the GPU for traced bin number `k` (0-based position in the last launch).  Dense branch (density > 0.25,
     smoothExchangeFactors.jl:432-434): straight from the counts the trace left on the device.  Sparse branch with AP only
-    (k_dykstra nothing or 0): AP on the non-zero pattern, from the resident counts, or from the host CSC F_raw after a trace
-    in row tiles (only the last tile is resident).  Returns None where the host path applies: sparse Dykstra rounds, or a dense
-    F traced in row tiles."""
+    (k_dykstra nothing or 0): AP on the non-zero pattern, from the resident counts (dense, or the hashed tally's of a single-device
+    trace), or from the host CSC F_raw after a trace in row tiles or a multi-device hashed-tally trace (only one shard is resident).  Returns None where the host path applies: sparse Dykstra rounds, or a dense
+    F traced in row tiles or with the hashed row tally."""
     tr = getattr(rtm, "_device", None)
     n = F_raw.shape[0]
     if tr is None or max_iters <= 0:
         return None
-    row_tiled = (getattr(rtm, "last_trace_stats", None) or {}).get("row_tiles", 1) > 1
+    trace_stats = getattr(rtm, "last_trace_stats", None) or {}
+    row_tiled = trace_stats.get("row_tiles", 1) > 1
+    sparse_tally = trace_stats.get("tally") == "sparse"
+    resident = not row_tiled and not (sparse_tally and trace_stats.get("devices", 1) > 1)   # all rows of F_raw on this device
     wn = w[:n] / np.min(w[:n])
     if F_raw.nnz / float(n * n) <= 0.25:
         if k_dykstra not in (None, 0):
             return None
         verbose and print(f"Matrix size: {n}x{n}; sparse smoothing on the device (AP, {F_raw.nnz} non-zeros)")
-        if row_tiled:
+        if not resident:
             F_smooth, st = tr.smooth_sparse(wn, F=F_raw, max_iters=max_iters)
         else:
             F_smooth, st = tr.smooth_sparse(wn, n=n, bin=k, max_iters=max_iters)
@@ -278,8 +296,8 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
         verbose and print(f"AP: {st['iterations']} iterations, delta_R {st['delta_init']:.3e} -> {st['delta']:.3e}, "
                           f"{st['total_ms']:.1f} ms on the device")
         return F_smooth
-    if row_tiled:
-        return None                                          # a dense F traced in row tiles: only the last tile is resident
+    if row_tiled or sparse_tally:
+        return None                                          # a dense F traced in row tiles or with the hashed tally: no dense counts resident
     if k_dykstra is None:       # smooth_F :441-450: one Dykstra round when surfaces and gas are strongly coupled, else AP only
         stats = getattr(rtm, "last_counts_stats", None)
         if rtm.surfaces_only:
