@@ -397,6 +397,32 @@ typedef struct rthx_sparse_stats {
 int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args* args, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* stats,
                                rthx_sparse_stats* sparse_stats);
 
+/* Continue the trace whose counts are resident: add the rays [ray_id_offset, ray_id_offset + rays_per_emitter) of every owned emitter
+ * to them, in the form they are in (dense or hashed).  The resident counts are always those of ONE trace of a contiguous ray-id range
+ * [lo, hi) with one seed, so k continuations give, bit for bit, what one trace of the whole range gives: rthx_counts_nnz / _csr / _stats
+ * / _csc, rthx_smooth_sparse(RTHX_SMOOTH_FROM_LAST_TRACE) and, for the dense form, rthx_smooth_F / _DkAP(RTHX_SMOOTH_FROM_LAST_TRACE).
+ * Preconditions (RTHX_ERR_ARG naming the mismatch, the resident state untouched): counts are resident from rthx_trace_exchange with
+ * counts_out == NULL or from rthx_trace_exchange_sparse (not from a host-output trace, nor from rthx_trace_exchange_multi, whose peer
+ * hand-over stores rows instead of adding them); seed, nudge, mode, locator, bins (in the same order) and emitter_rank / emitter_world
+ * are those of that trace; ray_id_offset == hi.  rays_per_emitter, block_threads and row_chunks are free: counts do not depend on the
+ * launch shape.  Afterwards hi has advanced by rays_per_emitter.
+ *   dense form : the launches of rthx_trace_exchange(counts_out == NULL) without clearing the counts (MULTI_BOUNCE too);
+ *   hashed form: the new rays are tallied and reduced into a sorted set of their own (row groups and splits as rthx_trace_exchange_sparse),
+ *                which a merge-path kernel merges into the resident set, summing equal keys; the merged set then replaces it.
+ *                Device memory at its peak, 16 bytes a key: while the new rays are tallied, the resident set, the pair buffer (24 bytes a
+ *                pair, as rthx_trace_exchange_sparse sizes it) and the new set (up to 2.5x it while it grows: the old and the grown copy);
+ *                during the merge, the resident, the new and the merged set (old nnz + new nnz), with the pair buffer released first
+ *                when the merged set would not fit beside it.  The old and the new set are freed after the merge.
+ * lost_out [n_bins*N] (may be NULL) and stats->rays_lost are cumulative over [lo, hi); stats->rays_traced and the kernel times are this
+ * call's.  The recorder records this call's rays only, as a plain trace with this ray_id_offset would.  sparse_stats (may be NULL;
+ * zeroed for the dense form): this call's pairs, flushes and row groups, nnz after the merge, reduce_ms including the merge.
+ * The prepared row / column pointers of the read-outs are rebuilt on the next read-out; an F_smooth left on the device by an earlier
+ * rthx_smooth_F / rthx_smooth_sparse is NOT updated (smooth again).  A call that fails after its checks leaves no counts resident, with
+ * one exception: a hashed continuation that fails before its merged set is complete (e.g. RTHX_ERR_NOMEM, RTHX_ERR_CUDA from an
+ * allocation) leaves the resident set and its lost counters as they were.                                               [0.3+] */
+int rthx_trace_exchange_continue(rthx_handle* h, const rthx_trace_args* args, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* stats,
+                                 rthx_sparse_stats* sparse_stats);
+
 /* Peer-memory plumbing for the fused flush in one-process-per-GPU runs: rank 0 allocates the UInt64 count matrix
  * with rthx_shared_alloc and publishes the 64-byte CUDA IPC handle; every other rank maps it with rthx_shared_open
  * (peer access over NVLink is enabled lazily) and passes the mapped pointer as `counts_dev` to

@@ -114,5 +114,5 @@ EXPORTED_SYMBOLS = (
     "rthx_trace_exchange_multi", "rthx_measure_fp64_peak", "rthx_last_error", "rthx_version",
     "rthx_shared_alloc", "rthx_shared_open", "rthx_shared_close", "rthx_shared_free", "rthx_release_cached",
     "rthx_smooth_F", "rthx_smooth_DkAP", "rthx_solve_grey", "rthx_flag_signal", "rthx_flag_wait", "rthx_host_register", "rthx_host_unregister", "rthx_host_alloc", "rthx_host_free", "rthx_set_copy_helpers", "rthx_counts_nnz", "rthx_counts_csr", "rthx_counts_stats", "rthx_counts_csc",
-    "rthx_smooth_sparse", "rthx_smooth_sparse_csc", "rthx_trace_exchange_sparse",
+    "rthx_smooth_sparse", "rthx_smooth_sparse_csc", "rthx_trace_exchange_sparse", "rthx_trace_exchange_continue",
 )

@@ -87,6 +87,9 @@ def load_library():
     L.rthx_trace_exchange_sparse.restype = C.c_int
     L.rthx_trace_exchange_sparse.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_u64p, C.POINTER(rthx_rec_out), C.POINTER(rthx_stats),
                                              C.POINTER(rthx_sparse_stats)]
+    L.rthx_trace_exchange_continue.restype = C.c_int
+    L.rthx_trace_exchange_continue.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_u64p, C.POINTER(rthx_rec_out), C.POINTER(rthx_stats),
+                                               C.POINTER(rthx_sparse_stats)]
     L.rthx_trace_exchange_device.restype = C.c_int
     L.rthx_trace_exchange_device.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int, C.POINTER(rthx_stats)]
@@ -303,6 +306,7 @@ class DeviceTracer:
                                                 lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                 C.byref(st)))
         self._last_shard = (int(args.emitter_rank), int(args.emitter_world))     # rows resident on the device: e = rank + y * world
+        self._record_resident(rays_per_emitter, kw, sparse=False)
         out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
         if rec is not None:
             out["origins"] = origins[: rec.n_recorded].copy()
@@ -322,7 +326,39 @@ class DeviceTracer:
         self._check(self._L.rthx_trace_exchange_sparse(self._h, C.byref(args), lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                        C.byref(st), C.byref(sst)))
         self._last_shard = (int(args.emitter_rank), int(args.emitter_world))
+        self._record_resident(rays_per_emitter, kw, sparse=True)
         out = dict(counts=None, lost=lost, stats=st.as_dict(), sparse_stats=sst.as_dict())
+        if rec is not None:
+            out["origins"] = origins[: rec.n_recorded].copy()
+            out["endpoints"] = endpoints[: rec.n_recorded].copy()
+        return out
+
+    # keywords that fix the resident trace's ray stream; trace_continue repeats them unless given
+    _STREAM_KW = ("seed", "bins", "nudge", "mode", "locator", "emitter_rank", "emitter_world")
+
+    def _record_resident(self, rays_per_emitter: int, kw, sparse: bool):
+        lo = int(kw.get("ray_id_offset", 0))
+        self._resident = dict(kw={k: kw[k] for k in self._STREAM_KW if k in kw}, hi=lo + int(rays_per_emitter), sparse=sparse)
+
+    def trace_continue(self, rays_per_emitter: int, **kw):
+        """Add `rays_per_emitter` rays per owned emitter to the counts resident from the last `trace(dense=False)`, `trace_sparse()` or
+        `trace_continue()` (rthx_trace_exchange_continue), in their dense or hashed form.  The seed, bins, nudge, mode, locator and
+        shard of that trace are repeated unless given (the library rejects any that differ), and ray_id_offset is the end of the
+        resident ray-id range.  Afterwards every read-out of the resident counts equals, bit for bit, the read-out after ONE trace of
+        the whole range.  Returns the dict of the trace that left the counts resident (sparse_stats after a hashed one), with lost
+        cumulative over the whole range; origins / endpoints hold this call's recorded rays."""
+        res = getattr(self, "_resident", None) or dict(kw={}, hi=0, sparse=False)
+        kw = {**res["kw"], "ray_id_offset": res["hi"], **kw}
+        args, keep = make_trace_args(rays_per_emitter, **kw)
+        lost = np.empty((args.n_bins, self.n_elements), np.uint64)
+        st, sst = rthx_stats(), rthx_sparse_stats()
+        rec, origins, endpoints = _recorder(kw.get("rec_ids"), rays_per_emitter)
+        self._check(self._L.rthx_trace_exchange_continue(self._h, C.byref(args), lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
+                                                         C.byref(st), C.byref(sst)))
+        res["hi"] = int(args.ray_id_offset) + int(rays_per_emitter)
+        out = dict(counts=None, lost=lost, stats=st.as_dict())
+        if res["sparse"]:
+            out["sparse_stats"] = sst.as_dict()
         if rec is not None:
             out["origins"] = origins[: rec.n_recorded].copy()
             out["endpoints"] = endpoints[: rec.n_recorded].copy()
@@ -547,6 +583,7 @@ def trace_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, counts_o
         msg = L.rthx_last_error(tracers[0]._h)
         raise RthxError(f"rthx_trace_exchange_multi failed ({rc}): {msg.decode() if msg else ''}")
     tracers[0]._last_shard = (0, 1)
+    tracers[0]._record_resident(rays_per_emitter, kw, sparse=False)
     out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
     if rec is not None:
         out["origins"] = origins[: rec.n_recorded].copy()
@@ -620,13 +657,14 @@ def trace_row_tiles(tracer: DeviceTracer, rays_per_emitter: int, n_tiles: int, *
     return dict(csr=merge_row_tiles(tiles, N, nb), lost=lost, chi=chi, stats=stats)
 
 
-def trace_sparse_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, **kw):
+def trace_sparse_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, refine: bool = False, **kw):
     """The hashed-tally trace (DeviceTracer.trace_sparse) on several devices at once: device r traces the emitters e = r (mod n)
     (one host thread per handle; the ctypes call releases the GIL), its rows stay on its device and only their non-zeros come back;
     the host merges them into ONE row-normalised CSR matrix per traced bin (merge_row_tiles).  Counts are those of a single-device
     trace bit for bit, and F = count / row total is the F_raw of a single-device trace bit for bit.  Returns dict(csr=[(row_ptr, cols, F_vals)] per bin, lost [nb, N], chi per bin, stats, sparse_stats), plus
     origins / endpoints with rec_ids: the points of device 0's recorded emitters first, then device 1's, ... (each in ascending
-    (emitter, ray) order)."""
+    (emitter, ray) order).  refine=True continues the shards left resident by the previous call (DeviceTracer.trace_continue) instead
+    of tracing them afresh; lost is then cumulative."""
     from concurrent.futures import ThreadPoolExecutor
     n = len(tracers)
     N = tracers[0].n_elements
@@ -635,7 +673,8 @@ def trace_sparse_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, *
 
     def run(r):
         own = [e for e in (rec_ids or []) if e % n == r]
-        out = tracers[r].trace_sparse(rays_per_emitter, emitter_rank=r, emitter_world=n, rec_ids=own or None, **kw)
+        trace = tracers[r].trace_continue if refine else tracers[r].trace_sparse
+        out = trace(rays_per_emitter, emitter_rank=r, emitter_world=n, rec_ids=own or None, **kw)
         parts, chi = _tile_readout(tracers[r], nb, divide=True)
         return out, parts, chi
 

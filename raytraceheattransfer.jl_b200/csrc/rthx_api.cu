@@ -95,6 +95,12 @@ struct rthx_handle : DevRes {
   int last_rank = 0, last_world = 1;                      // ... row y of the resident matrix is element last_rank + y * last_world
   bool sparse_counts = false;                             // the resident counts are the hashed tally's (sk_*), not counts_dev
   long long sk_nnz = 0;                                   // ... its non-zeros over all traced bins
+  // The one trace (of the contiguous ray-id range [ray_lo, ray_hi)) the resident counts are those of; rthx_trace_exchange_continue
+  // extends it.  Valid while last_trace_bins > 0.
+  int resident_kind = 0;                                  // RESIDENT_*
+  uint64_t res_seed = 0; double res_nudge = 0.0; int res_mode = 0, res_locator = 0;
+  std::vector<int32_t> res_bins;
+  int64_t ray_lo = 0, ray_hi = 0;
   int smooth_n = 0; size_t smooth_ldx = 0;                // F_smooth resident in smooth_X after rthx_smooth_F (0: none)
   int sparse_n = 0; long long sparse_nnz = 0;             // sparse F_smooth resident in sp_* after rthx_smooth_sparse (0: none)
   int csr_bin = -1; long long csr_total = 0;              // bin whose row pointers are prepared on the device
@@ -945,6 +951,39 @@ int check_args(rthx_handle* h, const rthx_trace_args* a) {
   return RTHX_OK;
 }
 
+// where the resident counts come from
+enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4 };
+
+void record_resident(rthx_handle* h, const rthx_trace_args* a, int kind) {
+  h->resident_kind = kind;
+  h->res_seed = a->seed; h->res_nudge = a->nudge; h->res_mode = a->mode; h->res_locator = a->locator;
+  h->res_bins.assign(a->bins, a->bins + a->n_bins);
+  h->ray_lo = a->ray_id_offset; h->ray_hi = a->ray_id_offset + a->rays_per_emitter;
+}
+
+// Preconditions of rthx_trace_exchange_continue: the resident counts are one trace of [ray_lo, ray_hi) that `a` continues
+int check_continue(rthx_handle* h, const rthx_trace_args* a) {
+  if (h->last_trace_bins <= 0 || h->resident_kind == RESIDENT_NONE)
+    return fail(h, RTHX_ERR_ARG, "trace_continue: no resident counts (run rthx_trace_exchange with counts_out == NULL or rthx_trace_exchange_sparse first)");
+  if (h->resident_kind == RESIDENT_HOST)
+    return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts come from a host-output trace (counts_out != NULL); trace with counts_out == NULL to continue");
+  if (h->resident_kind == RESIDENT_MULTI)
+    return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts were gathered from several devices (rthx_trace_exchange_multi), whose peer hand-over stores rows instead of adding them");
+  if (a->seed != h->res_seed) return fail(h, RTHX_ERR_ARG, "trace_continue: seed differs from the resident trace's");
+  if (a->nudge != h->res_nudge) return fail(h, RTHX_ERR_ARG, "trace_continue: nudge differs from the resident trace's");
+  if (a->mode != h->res_mode) return fail(h, RTHX_ERR_ARG, "trace_continue: mode differs from the resident trace's");
+  if (a->locator != h->res_locator) return fail(h, RTHX_ERR_ARG, "trace_continue: locator differs from the resident trace's");
+  if (a->n_bins != (int)h->res_bins.size() || !std::equal(a->bins, a->bins + a->n_bins, h->res_bins.begin()))
+    return fail(h, RTHX_ERR_ARG, "trace_continue: bins differ from the resident trace's");
+  if (a->emitter_rank != h->last_rank || a->emitter_world != h->last_world)
+    return fail(h, RTHX_ERR_ARG, "trace_continue: emitter shard (emitter_rank / emitter_world) differs from the resident trace's");
+  if (a->ray_id_offset != h->ray_hi)
+    return fail(h, RTHX_ERR_ARG, "trace_continue: ray_id_offset " + std::to_string(a->ray_id_offset) + " does not continue the resident ray-id range [" +
+                                     std::to_string(h->ray_lo) + ", " + std::to_string(h->ray_hi) + ")");
+  if (a->rays_per_emitter > INT64_MAX - h->ray_hi) return fail(h, RTHX_ERR_ARG, "trace_continue: ray ids past 2^63");
+  return RTHX_OK;
+}
+
 // variant bits of the queue kernel (rthx_kernels.cu, kernel_variant): 8 general faces, 16 generic locator (implies 8), 32 its 80-register build
 int queue_variant_bits(const rthx_handle* h, const LaunchPlan& pl) {
   if (pl.queue_gen) return 8 + 16 + (pl.queue_gen == 3 ? 32 : 0);
@@ -1389,6 +1428,7 @@ extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uin
   h->last_trace_bins = a->n_bins;
   h->last_trace_rows = (size_t)pl.n_owned; h->last_rank = a->emitter_rank; h->last_world = a->emitter_world;
   h->csr_bin = -1; h->csc_bin = -1;
+  record_resident(h, a, counts_out ? RESIDENT_HOST : RESIDENT_DENSE);
   std::vector<uint64_t> lost_host((size_t)a->n_bins * N);
   CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->copy_stream));
   CU(h, cudaEventRecord(h->ev[3], h->copy_stream));
@@ -1449,17 +1489,32 @@ cudaError_t grow_keep(T** ptr, size_t* cap, size_t need, size_t keep, cudaStream
 }
 }  // namespace
 
-extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st,
-                                          rthx_sparse_stats* sst) {
-  if (!h) return RTHX_ERR_ARG;
-  int rc = check_args(h, a);
-  if (rc) return rc;
-  if (a->mode != RTHX_FIRST_INTERACTION)
-    return fail(h, RTHX_ERR_ARG, "trace_sparse: the hashed tally supports RTHX_FIRST_INTERACTION only (trace MULTI_BOUNCE with rthx_trace_exchange)");
-  CU(h, cudaSetDevice(h->device));
+namespace {
+// What one hashed-tally pass over the rows of a call did (sparse_trace_rows)
+struct SparseRun {
+  LaunchPlan pl{};
+  int log2s = 0, groups = 0, n_slots = 0, n_launches = 0;
+  long long cap = 0, n_rows = 0, total = 0, pairs = 0, flushes = 0;
+  double kernel_ms = 0, reduce_ms = 0;
+};
+
+// A device array freed when it goes out of scope (scratch of rthx_trace_exchange_continue)
+template <class T>
+struct DevBuf {
+  T* p = nullptr;
+  size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { cudaFree(p); }
+};
+
+// Trace the rows of `a` with the hashed row tally and append the sorted unique (key, u64 total) pairs of every row group to
+// (*out_keys, *out_vals), growing them as needed; lost_dev is cleared first and counts the rays of this call.  A group whose pairs
+// overran the pair buffer is traced again split in two.  ev[0] marks the start of the call's device work.
+int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec, unsigned long long** out_keys, size_t* keys_cap,
+                      unsigned long long** out_vals, size_t* vals_cap, SparseRun& R) {
   const int N = h->N, nb = a->n_bins, rank = a->emitter_rank, world = a->emitter_world;
-  // whatever counts were resident (dense or sparse) are void from here on
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false; h->sk_nnz = 0;
   const int bt = a->block_threads ? a->block_threads : 256;
   int log2s = 12;                                            // 4096 slots: 32 KB of table
   int min_log2s = 1;
@@ -1508,23 +1563,20 @@ extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args*
   int end_bit = 32;
   while ((1ll << (end_bit - 32)) < n_rows) ++end_bit;
 
-  int n_slots = 0, n_launches = 0;
   CU(h, cudaEventRecord(h->ev[0], h->stream));
-  rc = prepare_recorder(h, a, rec, &n_slots, h->stream);
+  int rc = prepare_recorder(h, a, rec, &R.n_slots, h->stream);
   if (rc) return rc;
   CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)nb, cudaMemcpyHostToDevice, h->stream));
   CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)nb * N, h->stream));
-  n_launches += 1;
+  R.n_launches += 1;
   TraceParams P;
   fill_params(h, a, pl, rank, world, true, nullptr, h->lost_dev, P);
-  if (n_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
+  if (R.n_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
   P.sk_keys = keys; P.sk_cnt = cnt; P.sk_ctl = h->sk_ctl; P.sk_cap = (unsigned long long)cap; P.sk_slots_log2 = log2s;
 
   // row groups in ascending order: a group whose pairs overran the buffer is traced again as two halves
   std::vector<std::pair<int, int>> todo{{0, pl.n_owned}};
-  long long total = 0, pairs = 0, flushes = 0;
-  int groups = 0;
-  double kernel_ms = 0, reduce_ms = 0;
+  long long total = 0;
   while (!todo.empty()) {
     const auto [y0, y1] = todo.front();
     todo.erase(todo.begin());
@@ -1534,12 +1586,12 @@ extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args*
     CU(h, cudaEventRecord(h->ev[1], h->stream));
     CU(h, launch_trace_exchange(P, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, pl.fast != 0, pl.minb, false, h->stream));
     CU(h, cudaEventRecord(h->ev[2], h->stream));
-    n_launches += 2;
+    R.n_launches += 2;
     unsigned long long ctl[4];
     CU(h, cudaMemcpyAsync(ctl, h->sk_ctl, sizeof(ctl), cudaMemcpyDeviceToHost, h->stream));
     CU(h, cudaStreamSynchronize(h->stream));
     float ms = 0;
-    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); kernel_ms += ms;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); R.kernel_ms += ms;
     if (ctl[1]) {
       if (y1 - y0 == 1) return fail(h, RTHX_ERR_NOMEM, "trace_sparse: the pairs of one emitter row exceed the pair buffer (" + std::to_string(cap) + " pairs)");
       for (int b = 0; b < nb; ++b)                          // the lost rays of the group are counted again
@@ -1550,46 +1602,192 @@ extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args*
       continue;
     }
     const long long n = (long long)ctl[0];
-    ++groups; pairs += n; flushes += (long long)ctl[2];
-    CU(h, grow_keep(&h->sk_keys, &h->sk_keys_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
-    CU(h, grow_keep(&h->sk_vals, &h->sk_vals_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
+    ++R.groups; R.pairs += n; R.flushes += (long long)ctl[2];
+    CU(h, grow_keep(out_keys, keys_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
+    CU(h, grow_keep(out_vals, vals_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
     CU(h, cudaEventRecord(h->ev[1], h->stream));
-    CU(h, tally_reduce(keys, cnt, keys_alt, cnt_alt, n, end_bit, h->sk_keys + total, h->sk_vals + total, (long long*)(h->sk_ctl + 3), h->sk_tmp,
+    CU(h, tally_reduce(keys, cnt, keys_alt, cnt_alt, n, end_bit, *out_keys + total, *out_vals + total, (long long*)(h->sk_ctl + 3), h->sk_tmp,
                        h->sk_tmp_cap, h->stream));
     CU(h, cudaEventRecord(h->ev[2], h->stream));
     long long uniq = 0;
     CU(h, cudaMemcpyAsync(&uniq, h->sk_ctl + 3, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
     CU(h, cudaStreamSynchronize(h->stream));
-    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); reduce_ms += ms;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); R.reduce_ms += ms;
     total += uniq;
   }
-  CU(h, ensure(&h->sk_rowptr, &h->sk_rowptr_cap, (size_t)n_rows + 1));
-  CU(h, tally_row_ptr(h->sk_keys, total, n_rows, h->sk_rowptr, h->stream));
+  R.pl = pl; R.log2s = log2s; R.cap = cap; R.n_rows = n_rows; R.total = total;
+  return RTHX_OK;
+}
+
+// Second half of a hashed-tally trace or continuation whose sorted unique pairs (R.total of them) are in sk_keys / sk_vals: row
+// pointers, lost read-out, handle state, recorder and statistics.  lost_before (continuation): the lost counts of the resident
+// trace, added to this call's.
+int sparse_finish(rthx_handle* h, const rthx_trace_args* a, const SparseRun& R, const std::vector<uint64_t>* lost_before, uint64_t* lost_out,
+                  rthx_rec_out* rec, rthx_stats* st, rthx_sparse_stats* sst) {
+  const int N = h->N, nb = a->n_bins;
+  CU(h, ensure(&h->sk_rowptr, &h->sk_rowptr_cap, (size_t)R.n_rows + 1));
+  CU(h, tally_row_ptr(h->sk_keys, R.total, R.n_rows, h->sk_rowptr, h->stream));
   std::vector<uint64_t> lost_host((size_t)nb * N);
+  CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->stream));
+  if (lost_before) {
+    CU(h, cudaStreamSynchronize(h->stream));
+    for (size_t k = 0; k < lost_host.size(); ++k) lost_host[k] += (*lost_before)[k];
+    CU(h, cudaMemcpyAsync(h->lost_dev, lost_host.data(), sizeof(uint64_t) * lost_host.size(), cudaMemcpyHostToDevice, h->stream));
+  }
+  CU(h, cudaEventRecord(h->ev[3], h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  h->sparse_counts = true; h->sk_nnz = R.total;
+  h->last_trace_bins = nb; h->last_trace_rows = (size_t)R.pl.n_owned; h->last_rank = a->emitter_rank; h->last_world = a->emitter_world;
+  if (lost_before) h->ray_hi += a->rays_per_emitter;
+  else record_resident(h, a, RESIDENT_SPARSE);
+  if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
+  int rc = collect_recorder(h, a, rec, R.n_slots, h->stream, false);
+  if (rc) return rc;
+  if (st) {
+    fill_stats(st, R.pl, a);
+    st->kernel_ms = R.kernel_ms;
+    float ms = 0;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3])); st->total_ms = ms;
+    int64_t nl = 0;
+    for (uint64_t v : lost_host) nl += (int64_t)v;
+    st->rays_lost = nl;
+    st->n_launches = R.n_launches;
+  }
+  if (sst) {
+    std::memset(sst, 0, sizeof(*sst));
+    sst->pairs = R.pairs; sst->nnz = R.total; sst->flushes = R.flushes; sst->pair_capacity = R.cap;
+    sst->row_groups = R.groups; sst->hash_slots = 1 << R.log2s; sst->reduce_ms = R.reduce_ms;
+  }
+  return RTHX_OK;
+}
+
+// Continuation of a hashed-tally trace, up to the merged set: the new rays' pairs are reduced into a set of their own, which is then
+// merged into the resident set (equal keys summed) and replaces it as the last step.  R.total receives the merged key count.
+int continue_sparse_merge(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec, long long old_nnz, SparseRun& R) {
+  DevBuf<unsigned long long> add_keys, add_vals;
+  int rc = sparse_trace_rows(h, a, rec, &add_keys.p, &add_keys.cap, &add_vals.p, &add_vals.cap, R);
+  if (rc) return rc;
+  // the merge does not use the pair buffer: when device memory is short it makes room for the merged set
+  auto alloc = [h](void** p, size_t bytes) {
+    cudaError_t e = cudaMalloc(p, bytes);
+    if (e == cudaErrorMemoryAllocation && h->sk_pairs) {
+      cudaGetLastError();
+      cudaFree(h->sk_pairs); h->sk_pairs = nullptr; h->sk_pairs_cap = 0;
+      e = cudaMalloc(p, bytes);
+    }
+    return e;
+  };
+  const long long n_out = old_nnz + R.total, n_tiles = tally_merge_tiles(n_out);
+  DevBuf<unsigned long long> mrg_keys, mrg_vals;
+  DevBuf<long long> tiles;
+  CU(h, alloc((void**)&mrg_keys.p, sizeof(unsigned long long) * (size_t)std::max(n_out, 1ll)));
+  CU(h, alloc((void**)&mrg_vals.p, sizeof(unsigned long long) * (size_t)std::max(n_out, 1ll)));
+  CU(h, alloc((void**)&tiles.p, sizeof(long long) * 2 * (size_t)(n_tiles + 1)));
+  mrg_keys.cap = mrg_vals.cap = (size_t)std::max(n_out, 1ll);
+  CU(h, ensure(reinterpret_cast<char**>(&h->sk_tmp), &h->sk_tmp_cap, tally_merge_temp_bytes(n_tiles)));
+  CU(h, cudaEventRecord(h->ev[1], h->stream));
+  CU(h, tally_merge(h->sk_keys, h->sk_vals, old_nnz, add_keys.p, add_vals.p, R.total, mrg_keys.p, mrg_vals.p, tiles.p, h->sk_tmp, h->sk_tmp_cap,
+                    h->stream));
+  CU(h, cudaEventRecord(h->ev[2], h->stream));
+  long long merged = 0;
+  CU(h, cudaMemcpyAsync(&merged, tiles.p + 2 * n_tiles + 1, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  float ms = 0;
+  CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2]));
+  R.reduce_ms += ms;
+  R.n_launches += n_tiles > 0 ? 5 : 3;     // memset, scan (init + scan kernel), and the counting and writing passes
+  R.total = merged;
+  std::swap(h->sk_keys, mrg_keys.p); std::swap(h->sk_keys_cap, mrg_keys.cap);   // the old set is freed with mrg_*
+  std::swap(h->sk_vals, mrg_vals.p); std::swap(h->sk_vals_cap, mrg_vals.cap);
+  return RTHX_OK;
+}
+
+// Continuation of a hashed-tally trace.  Until the merged set replaces it the resident set is untouched, so a failure before that
+// point leaves it resident, with its lost counters restored.
+int continue_sparse(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st, rthx_sparse_stats* sst) {
+  std::vector<uint64_t> lost_before((size_t)a->n_bins * h->N);
+  CU(h, cudaMemcpyAsync(lost_before.data(), h->lost_dev, sizeof(uint64_t) * lost_before.size(), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  const long long old_nnz = h->sk_nnz;
+  const int old_bins = h->last_trace_bins;
+  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1;  // incomplete until the merge has landed
+  SparseRun R;
+  const int rc = continue_sparse_merge(h, a, rec, old_nnz, R);
+  if (rc) {
+    if (cudaMemcpy(h->lost_dev, lost_before.data(), sizeof(uint64_t) * lost_before.size(), cudaMemcpyHostToDevice) == cudaSuccess)
+      h->last_trace_bins = old_bins;
+    else
+      cudaGetLastError();
+    return rc;
+  }
+  return sparse_finish(h, a, R, &lost_before, lost_out, rec, st, sst);
+}
+
+// Continuation of a dense resident trace: the same launches as rthx_trace_exchange(counts_out == NULL) without clearing the counts or
+// the lost counters.  Every flush into a matrix on the handle's own device adds (shared-memory histogram rows, global atomics,
+// row_chunks == 1 alike), so the counts add up to those of one trace of the whole range.
+int continue_dense(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
+  int n_slots = 0, n_launches = 0;
+  CU(h, cudaEventRecord(h->ev[0], h->stream));
+  int rc = prepare_recorder(h, a, rec, &n_slots, h->stream);
+  if (rc) return rc;
+  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1;  // incomplete until the kernels have finished
+  CU(h, cudaEventRecord(h->ev[1], h->stream));
+  LaunchPlan pl{};
+  rc = enqueue_trace(h, a, a->emitter_rank, a->emitter_world, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, rec != nullptr, n_slots,
+                     h->stream, &pl, &n_launches);
+  if (rc) return rc;
+  CU(h, cudaEventRecord(h->ev[2], h->stream));
+  std::vector<uint64_t> lost_host((size_t)a->n_bins * h->N);
   CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaEventRecord(h->ev[3], h->stream));
   CU(h, cudaStreamSynchronize(h->stream));
-  h->sparse_counts = true; h->sk_nnz = total;
-  h->last_trace_bins = nb; h->last_trace_rows = (size_t)pl.n_owned; h->last_rank = rank; h->last_world = world;
+  h->last_trace_bins = a->n_bins;
+  h->ray_hi += a->rays_per_emitter;
   if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
   rc = collect_recorder(h, a, rec, n_slots, h->stream, false);
   if (rc) return rc;
   if (st) {
     fill_stats(st, pl, a);
-    st->kernel_ms = kernel_ms;
     float ms = 0;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); st->kernel_ms = ms;
     CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3])); st->total_ms = ms;
     int64_t nl = 0;
     for (uint64_t v : lost_host) nl += (int64_t)v;
     st->rays_lost = nl;
     st->n_launches = n_launches;
   }
-  if (sst) {
-    std::memset(sst, 0, sizeof(*sst));
-    sst->pairs = pairs; sst->nnz = total; sst->flushes = flushes; sst->pair_capacity = cap;
-    sst->row_groups = groups; sst->hash_slots = 1 << log2s; sst->reduce_ms = reduce_ms;
-  }
   return RTHX_OK;
+}
+}  // namespace
+
+extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st,
+                                          rthx_sparse_stats* sst) {
+  if (!h) return RTHX_ERR_ARG;
+  int rc = check_args(h, a);
+  if (rc) return rc;
+  if (a->mode != RTHX_FIRST_INTERACTION)
+    return fail(h, RTHX_ERR_ARG, "trace_sparse: the hashed tally supports RTHX_FIRST_INTERACTION only (trace MULTI_BOUNCE with rthx_trace_exchange)");
+  CU(h, cudaSetDevice(h->device));
+  // whatever counts were resident (dense or sparse) are void from here on
+  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false; h->sk_nnz = 0;
+  SparseRun R;
+  rc = sparse_trace_rows(h, a, rec, &h->sk_keys, &h->sk_keys_cap, &h->sk_vals, &h->sk_vals_cap, R);
+  if (rc) return rc;
+  return sparse_finish(h, a, R, nullptr, lost_out, rec, st, sst);
+}
+
+extern "C" int rthx_trace_exchange_continue(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st,
+                                            rthx_sparse_stats* sst) {
+  if (!h) return RTHX_ERR_ARG;
+  int rc = check_args(h, a);
+  if (rc) return rc;
+  rc = check_continue(h, a);
+  if (rc) return rc;
+  CU(h, cudaSetDevice(h->device));
+  if (h->sparse_counts) return continue_sparse(h, a, lost_out, rec, st, sst);
+  if (sst) std::memset(sst, 0, sizeof(*sst));
+  return continue_dense(h, a, lost_out, rec, st);
 }
 
 namespace {
@@ -1734,6 +1932,7 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
     CU(h0, cudaSetDevice(h0->device));
     CU(h0, cudaMemcpy(lost_sum.data(), h0->lost_dev, sizeof(uint64_t) * lost_n, cudaMemcpyDeviceToHost));
     h0->last_trace_bins = a->n_bins; h0->last_trace_rows = (size_t)N; h0->last_rank = 0; h0->last_world = 1;
+    record_resident(h0, a, RESIDENT_MULTI);
   } else {
     for (int i = 0; i < n; ++i)
       for (size_t k = 0; k < lost_n; ++k) lost_sum[k] += jobs[i].lost[k];

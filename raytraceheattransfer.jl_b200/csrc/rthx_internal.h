@@ -163,6 +163,13 @@ cudaError_t tally_row_stats(const unsigned long long* keys, const unsigned long 
 cudaError_t tally_row_fill(const unsigned long long* keys, const unsigned long long* vals, const long long* row_ptr, int n_bins, int bin, int n_rows,
                            int n_cols, const long long* out_ptr, const unsigned long long* rowsum, bool divide, int* cols, unsigned long long* cnt_out,
                            double* fvals, cudaStream_t st);
+// merge two sorted unique (key, u64 total) sets into out_keys / out_vals (room for na + nb), summing the totals of equal keys;
+// `tiles` holds 2 (tally_merge_tiles(na + nb) + 1) words, and tiles[2 * n_tiles + 1] receives the number of merged keys
+long long tally_merge_tiles(long long n);
+size_t tally_merge_temp_bytes(long long n_tiles);
+cudaError_t tally_merge(const unsigned long long* a_keys, const unsigned long long* a_vals, long long na, const unsigned long long* b_keys,
+                        const unsigned long long* b_vals, long long nb, unsigned long long* out_keys, unsigned long long* out_vals, long long* tiles,
+                        void* temp, size_t temp_bytes, cudaStream_t st);
 // low words of sorted transpose keys (the rows of a CSC) + base as int32 / int64
 cudaError_t tally_key_index(const unsigned long long* keys_sorted, long long nnz, int base, void* out, bool i64, cudaStream_t st);
 

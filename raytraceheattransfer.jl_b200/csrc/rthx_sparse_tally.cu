@@ -4,7 +4,9 @@
 // and the read-outs of the resident counts (CSR / CSC / row statistics / the sparse smoothing's F) are formed from them with the
 // value formulas of the dense read-outs (rthx_smooth.cu), so that they agree bit for bit.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/block/block_scan.cuh>
 #include <cub/device/device_reduce.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cuda/std/functional>
 #include <thrust/iterator/transform_iterator.h>
 
@@ -85,7 +87,109 @@ __global__ void __launch_bounds__(256) key_index_kernel(const unsigned long long
 }
 
 unsigned flat_grid(long long n) { return (unsigned)std::max<long long>(1, std::min<long long>((n + 255) / 256, 148 * 32)); }
+
+// Merge of two sorted key sets, each key at most once per set (rthx_trace_exchange_continue): merge path over the sequence of all
+// na + nb keys, A before B on equal keys.  Thread t walks the MERGE_ITEMS positions from diagonal t * MERGE_ITEMS on.  A position that
+// takes A[i] emits it plus B[j] when B[j] is the same key; a position that takes B[j] emits it unless A[i-1] was that key (then it was
+// summed there).  Pass 1 counts the emitted keys per tile, pass 2 walks again, stages them in shared memory and writes them at the
+// scanned tile offsets.
+constexpr int MERGE_THREADS = 128, MERGE_ITEMS = 16, MERGE_TILE = MERGE_THREADS * MERGE_ITEMS;
+
+__device__ __forceinline__ long long merge_split(const unsigned long long* __restrict__ a, long long na, const unsigned long long* __restrict__ b,
+                                                 long long nb, long long d) {
+  long long lo = d > nb ? d - nb : 0, hi = d < na ? d : na;   // A elements among the first d positions
+  while (lo < hi) {
+    const long long mid = (lo + hi) >> 1;
+    if (a[mid] <= b[d - 1 - mid]) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+template <bool WRITE>
+__device__ __forceinline__ int merge_walk(const unsigned long long* __restrict__ ak, const unsigned long long* __restrict__ av, long long na,
+                                          const unsigned long long* __restrict__ bk, const unsigned long long* __restrict__ bv, long long nb,
+                                          long long i, long long j, int steps, unsigned long long* __restrict__ ok,
+                                          unsigned long long* __restrict__ ov, long long o) {
+  int n = 0;
+  for (int s = 0; s < steps; ++s) {
+    if (i < na && (j >= nb || ak[i] <= bk[j])) {
+      if (WRITE) {
+        const unsigned long long k = ak[i];
+        ok[o + n] = k;
+        ov[o + n] = av[i] + (j < nb && bk[j] == k ? bv[j] : 0ull);
+      }
+      ++i; ++n;
+    } else {
+      const unsigned long long k = bk[j];
+      if (i == 0 || ak[i - 1] != k) {
+        if (WRITE) { ok[o + n] = k; ov[o + n] = bv[j]; }
+        ++n;
+      }
+      ++j;
+    }
+  }
+  return n;
+}
+
+template <bool WRITE>
+__global__ void __launch_bounds__(MERGE_THREADS) tally_merge_kernel(const unsigned long long* __restrict__ ak, const unsigned long long* __restrict__ av,
+                                                                    long long na, const unsigned long long* __restrict__ bk,
+                                                                    const unsigned long long* __restrict__ bv, long long nb,
+                                                                    long long* __restrict__ tile_cnt, const long long* __restrict__ tile_off,
+                                                                    unsigned long long* __restrict__ ok, unsigned long long* __restrict__ ov) {
+  using Scan = cub::BlockScan<int, MERGE_THREADS>;
+  __shared__ typename Scan::TempStorage scan_tmp;
+  const long long d = ((long long)blockIdx.x * MERGE_THREADS + threadIdx.x) * MERGE_ITEMS;
+  const long long left = na + nb - d;
+  const int steps = left <= 0 ? 0 : (left < MERGE_ITEMS ? (int)left : MERGE_ITEMS);
+  long long i = 0, j = 0;
+  int n = 0;
+  if (steps > 0) {
+    i = merge_split(ak, na, bk, nb, d); j = d - i;
+    n = merge_walk<false>(ak, av, na, bk, bv, nb, i, j, steps, nullptr, nullptr, 0);
+  }
+  int off = 0, sum = 0;
+  Scan(scan_tmp).ExclusiveSum(n, off, sum);
+  if (!WRITE) {
+    if (threadIdx.x == 0) tile_cnt[blockIdx.x] = sum;
+    return;
+  }
+  if constexpr (WRITE) {
+    // each thread's keys are consecutive, so direct stores would be strided across the warp: the tile is staged in shared memory
+    // and written out with coalesced stores
+    __shared__ unsigned long long s_k[MERGE_TILE], s_v[MERGE_TILE];
+    if (steps > 0) merge_walk<true>(ak, av, na, bk, bv, nb, i, j, steps, s_k, s_v, off);
+    __syncthreads();
+    const long long base = tile_off[blockIdx.x];
+    for (int t = threadIdx.x; t < sum; t += MERGE_THREADS) { ok[base + t] = s_k[t]; ov[base + t] = s_v[t]; }
+  }
+}
 }  // namespace
+
+long long tally_merge_tiles(long long n) { return (n + MERGE_TILE - 1) / MERGE_TILE; }
+
+size_t tally_merge_temp_bytes(long long n_tiles) {
+  size_t b = 0;
+  cub::DeviceScan::ExclusiveSum(nullptr, b, (const long long*)nullptr, (long long*)nullptr, (int)(n_tiles + 1));
+  return b;
+}
+
+cudaError_t tally_merge(const unsigned long long* ak, const unsigned long long* av, long long na, const unsigned long long* bk,
+                        const unsigned long long* bv, long long nb, unsigned long long* ok, unsigned long long* ov, long long* tiles,
+                        void* temp, size_t temp_bytes, cudaStream_t st) {
+  const long long n_tiles = tally_merge_tiles(na + nb);
+  long long* cnt = tiles;
+  long long* off = tiles + n_tiles + 1;
+  cudaError_t e;
+  if ((e = cudaMemsetAsync(cnt + n_tiles, 0, sizeof(long long), st)) != cudaSuccess) return e;
+  if (n_tiles > 0) {
+    tally_merge_kernel<false><<<(unsigned)n_tiles, MERGE_THREADS, 0, st>>>(ak, av, na, bk, bv, nb, cnt, nullptr, nullptr, nullptr);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  if ((e = cub::DeviceScan::ExclusiveSum(temp, temp_bytes, (const long long*)cnt, off, (int)(n_tiles + 1), st)) != cudaSuccess) return e;
+  if (n_tiles > 0) tally_merge_kernel<true><<<(unsigned)n_tiles, MERGE_THREADS, 0, st>>>(ak, av, na, bk, bv, nb, nullptr, off, ok, ov);
+  return cudaGetLastError();
+}
 
 size_t tally_temp_bytes(long long n_pairs) {
   const int n = (int)std::max<long long>(n_pairs, 1);

@@ -104,14 +104,46 @@ def auto_row_tiles(n_elements: int, n_bins: int, budget_bytes: float = 48e9) -> 
     return max(1, int(np.ceil(8.0 * n_elements * n_elements * n_bins / budget_bytes)))
 
 
+def _same_flat(a, b) -> bool:
+    keys = [k for k in a.__dict__ if k != "c"]
+    return keys == [k for k in b.__dict__ if k != "c"] and all(np.array_equal(np.asarray(a.__dict__[k]), np.asarray(b.__dict__[k])) for k in keys)
+
+
+def _refine_state(rtm, seed, devices, locator, row_tiles, nudge):
+    """The state of the previous call that `refine=True` continues; ValueError when it cannot be continued with these keywords."""
+    state = getattr(rtm, "_trace_state", None)
+    if state is None or not getattr(rtm, "_devices", None):
+        raise ValueError("refine=True: there is no previous exchange trace on this domain to refine")
+    if state["row_tiles"] is not None:
+        raise ValueError("refine=True: the previous call traced explicit row_tiles, whose tile counts are not kept")
+    if state["dense_multi"]:
+        raise ValueError("refine=True: the previous call gathered dense counts from several devices, which cannot be continued")
+    for name, given in (("seed", seed), ("devices", devices), ("locator", locator), ("row_tiles", row_tiles), ("nudge", nudge)):
+        if given is not None and given != state[name]:
+            raise ValueError(f"refine=True: {name}={given!r} differs from the previous call's {state[name]!r}")
+    if not _same_flat(flatten_domain(rtm), rtm._devices[0].flat):
+        raise ValueError("refine=True: the domain changed since the previous call (its flattened mesh differs)")
+    return state
+
+
 def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectral_bins: Sequence[int],
                                verbose: bool, rec, seed: int, device: int = 0,
-                               locator: int = RTHX_LOCATOR_AUTO, devices=None, row_tiles: Optional[int] = None) -> List[sp.csc_matrix]:
-    """Batched form of computeExchangeFactorsBin: traces every requested (1-based) bin in one launch per device."""
+                               locator: int = RTHX_LOCATOR_AUTO, devices=None, row_tiles: Optional[int] = None,
+                               refine: bool = False) -> List[sp.csc_matrix]:
+    """Batched form of computeExchangeFactorsBin: traces every requested (1-based) bin in one launch per device.  refine=True adds
+    the rays to the counts the previous call left resident (parallelRayTracing checks that it can)."""
     import time
-    devs = resolve_devices(devices if devices is not None else [device], device, 0)
-    trs = _tracers_for(rtm, devs)
+    if refine:
+        state = rtm._trace_state
+        trs = rtm._devices
+        devs = state["devices"]
+        rtm.last_phase_ms = {}
+    else:
+        rtm._trace_state = None
+        devs = resolve_devices(devices if devices is not None else [device], device, 0)
+        trs = _tracers_for(rtm, devs)
     tr = trs[0]
+    rpe_total = rays_per_emitter + (state["rays_per_emitter_total"] if refine else 0)
     rec_ids = [i - 1 for i in rec.ids] if rec is not None else None
     rec_bin = (rec.bin - 1) if rec is not None else 0
     verbose and print(f"  Using CUDA device(s) {devs} for spectral bins {list(spectral_bins)}")
@@ -120,7 +152,12 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
     # returns (parallelRayTracing.jl:144-158 + row_normalize! :161-169) — no N^2 host traffic, no sparse(I, J, V), no transpose.
     t0 = time.perf_counter()
     kw = dict(seed=seed, bins=[b - 1 for b in spectral_bins], nudge=nudge, rec_ids=rec_ids, rec_bin=rec_bin, locator=locator)
-    n_tiles = auto_row_tiles(tr.n_elements, len(spectral_bins)) if row_tiles is None else int(row_tiles)
+    if refine:
+        n_tiles = state["n_tiles"]
+    else:
+        n_tiles = auto_row_tiles(tr.n_elements, len(spectral_bins)) if row_tiles is None else int(row_tiles)
+    new_state = dict(seed=seed, devices=devs, locator=locator, row_tiles=row_tiles, nudge=nudge, n_tiles=n_tiles,
+                     dense_multi=n_tiles == 1 and len(trs) > 1, rays_per_emitter_total=rpe_total)
     sparse_multi = row_tiles is None and n_tiles > 1 and len(trs) > 1
     if n_tiles > 1 and (row_tiles is not None or sparse_multi):
         # N >> 57 k elements: the dense count matrix is the limit, not the tally (SURVEY.md section 5).  Several devices: each traces
@@ -128,8 +165,8 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
         # tiles on one device, keeping only each tile's non-zeros; the recorder is not available there.
         if sparse_multi:
             from ._lib import trace_sparse_multi
-            res = trace_sparse_multi(trs, rays_per_emitter, **kw)
-            stats = dict(res["stats"], tally="sparse", devices=len(trs), sparse=res["sparse_stats"])
+            res = trace_sparse_multi(trs, rays_per_emitter, refine=refine, **kw)
+            stats = dict(res["stats"], tally="sparse", devices=len(trs), sparse=res["sparse_stats"], rays_per_emitter_total=rpe_total)
             if rec is not None and "origins" in res:
                 rec.origins[0] = np.concatenate([rec.origins[0], res["origins"]], axis=0)
                 rec.endpoints[0] = np.concatenate([rec.endpoints[0], res["endpoints"]], axis=0)
@@ -139,8 +176,9 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
             from ._lib import trace_row_tiles
             kw.pop("rec_ids"); kw.pop("rec_bin")
             res = trace_row_tiles(tr, rays_per_emitter, n_tiles, **kw)
-            stats = dict(res["stats"], row_tiles=n_tiles)
+            stats = dict(res["stats"], row_tiles=n_tiles, rays_per_emitter_total=rpe_total)
         t1 = time.perf_counter()
+        rtm._trace_state = new_state
         rtm.last_trace_stats = stats
         rtm.last_lost = res["lost"]
         N = tr.n_elements
@@ -148,23 +186,24 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
         rtm.last_counts_stats = []
         for k in range(len(spectral_bins)):
             row_ptr, cols, vals = res["csr"][k]
-            print(f"Maximum ray tracing ray loss per emitter: {int(res['lost'][k].max()) if N else 0}/{rays_per_emitter}")   # unconditional, :163
+            print(f"Maximum ray tracing ray loss per emitter: {int(res['lost'][k].max()) if N else 0}/{rpe_total}")   # unconditional, :163
             rtm.last_counts_stats.append({"nnz": int(row_ptr[-1]), "chi": float(res["chi"][k]), "density": row_ptr[-1] / float(N * N)})
             mats.append(sp.csr_matrix((vals, cols, row_ptr), shape=(N, N)).tocsc())
         rtm.last_phase_ms.update({"trace": 1e3 * (t1 - t0), "csc_F_raw": 1e3 * (time.perf_counter() - t1), "row_tiles": n_tiles})
         return mats
     if n_tiles > 1:
         # one device, dense matrix beyond the budget: the hashed row tally keeps the counts on the device in sparse form
-        out = tr.trace_sparse(rays_per_emitter, **kw)
+        out = tr.trace_continue(rays_per_emitter, **kw) if refine else tr.trace_sparse(rays_per_emitter, **kw)
         out["stats"] = dict(out["stats"], tally="sparse", sparse=out["sparse_stats"])
     elif len(trs) == 1:
-        out = tr.trace(rays_per_emitter, dense=False, **kw)
+        out = tr.trace_continue(rays_per_emitter, **kw) if refine else tr.trace(rays_per_emitter, dense=False, **kw)
     else:
         from ._lib import trace_multi
         out = trace_multi(trs, rays_per_emitter, dense=False, **kw)
         tr.set_copy_helpers(trs[1:])           # the read-outs below leave through every device's PCIe link
     t1 = time.perf_counter()
-    rtm.last_trace_stats = out["stats"]
+    rtm._trace_state = new_state
+    rtm.last_trace_stats = dict(out["stats"], rays_per_emitter_total=rpe_total)
     rtm.last_lost = out["lost"]
     if rec is not None and "origins" in out:
         # parallelRayTracing.jl:120-123 push into rec.origins[tid]; any slot works for collect_rays
@@ -178,7 +217,7 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
         rtm.last_counts_stats.append({"nnz": nnz, "chi": chi, "density": nnz / float(N * N) if N else 0.0})
         colptr, rowval, _, fvals = tr.counts_csc(k, values=False, normalised=True)
         max_loss = int(out["lost"][k].max()) if N else 0
-        print(f"Maximum ray tracing ray loss per emitter: {max_loss}/{rays_per_emitter}")   # unconditional, :163
+        print(f"Maximum ray tracing ray loss per emitter: {max_loss}/{rpe_total}")   # unconditional, :163
         if nnz < 2 ** 31:
             colptr = colptr.astype(np.int32)          # scipy wants one index type; N + 1 entries, the big array stays as it is
         else:
@@ -198,20 +237,38 @@ def computeExchangeFactorsBin(rtm, rays_per_emitter: int, nudge: float, spectral
                                       locator, devices, row_tiles)[0]
 
 
-def parallelRayTracing(rtm, rays_total: int, nudge: float, verbose: bool, rec=None, seed: Optional[int] = None,
-                       device: int = 0, locator: int = RTHX_LOCATOR_AUTO, devices=None, row_tiles: Optional[int] = None):
-    """parallelRayTracing(rtm, rays_total, nudge, verbose; rec) -> (F_raw, rays_per_emitter)."""
-    if seed is None:
-        seed = secrets.randbits(64)   # the reference is unseeded: a fresh stream per call
+def parallelRayTracing(rtm, rays_total: int, nudge: Optional[float], verbose: bool, rec=None, seed: Optional[int] = None,
+                       device: Optional[int] = None, locator: Optional[int] = None, devices=None, row_tiles: Optional[int] = None,
+                       refine: bool = False):
+    """parallelRayTracing(rtm, rays_total, nudge, verbose; rec) -> (F_raw, rays_per_emitter).  refine=True (new): add
+    rays_total // N rays per emitter to the counts the previous call left on the device(s) — same handles, seed, bins, nudge and
+    locator — and return the F_raw of ONE trace of all rays so far, with their number per emitter.  ValueError when there is no
+    previous call, it traced explicit row_tiles or gathered dense counts from several devices, the flattened mesh changed, or
+    seed / devices / device / locator / row_tiles / nudge are given and differ (`device=d` stands for `devices=[d]`)."""
     num_emitters = rtm.num_elements
     rays_per_emitter = rays_total // num_emitters                        # parallelRayTracing.jl:6
     n_bins = rtm.n_spectral_bins
-    devices = resolve_devices(devices, device, rays_total)
+    if refine:
+        given = resolve_devices(devices, 0, rays_total) if devices is not None else ([int(device)] if device is not None else None)
+        state = _refine_state(rtm, seed, given, locator, row_tiles, nudge)
+        seed, devices, locator, nudge = state["seed"], state["devices"], state["locator"], state["nudge"]
+        device = devices[0]
+    else:
+        if seed is None:
+            seed = secrets.randbits(64)   # the reference is unseeded: a fresh stream per call
+        if locator is None:
+            locator = RTHX_LOCATOR_AUTO
+        if nudge is None:
+            nudge = DEFAULT_NUDGE
+        if device is None:
+            device = 0
+        devices = resolve_devices(devices, device, rays_total)
     if rtm.spectral_mode == "spectral_variable":
         verbose and print(f"Computing {n_bins} separate F matrices for variable spectral extinction")
         groups, reps, nonuniform = group_uniform_bins(rtm.uniform_across_bin)
         to_trace = list(nonuniform) + [g[0] for g in groups]
-        mats = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, to_trace, verbose, rec, seed, device, locator, devices, row_tiles)
+        mats = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, to_trace, verbose, rec, seed, device, locator, devices, row_tiles,
+                                          refine)
         rtm._traced_bins = list(to_trace)
         F_raw_vector: List[Optional[sp.csc_matrix]] = [None] * n_bins
         for b, F in zip(to_trace[: len(nonuniform)], mats[: len(nonuniform)]):
@@ -219,14 +276,14 @@ def parallelRayTracing(rtm, rays_total: int, nudge: float, verbose: bool, rec=No
         for g, F in zip(groups, mats[len(nonuniform):]):
             for j in g:
                 F_raw_vector[j - 1] = F                                  # group members alias one matrix (:38-41)
-        return F_raw_vector, rays_per_emitter
+        return F_raw_vector, rtm._trace_state["rays_per_emitter_total"]
     if rtm.spectral_mode != "grey":
         verbose and print(f"Computing single F matrix for uniform spectral extinction ({n_bins} bins)")
     else:
         verbose and print("Computing single F matrix for grey extinction")
-    F_raw = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, [1], verbose, rec, seed, device, locator, devices, row_tiles)[0]
+    F_raw = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, [1], verbose, rec, seed, device, locator, devices, row_tiles, refine)[0]
     rtm._traced_bins = [1]
-    return F_raw, rays_per_emitter
+    return F_raw, rtm._trace_state["rays_per_emitter_total"]
 
 
 def get_w(rtm, spectral_bin: int = 1) -> np.ndarray:
@@ -321,15 +378,15 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
     return F_smooth
 
 
-def exchangeRayTracing(rtm, rays_tot: int, nudge: float, max_iters: int, k_dykstra, verbose: bool, rec,
-                       seed: Optional[int] = None, device: int = 0, locator: int = RTHX_LOCATOR_AUTO,
-                       smooth: bool = True, devices=None, row_tiles: Optional[int] = None):
+def exchangeRayTracing(rtm, rays_tot: int, nudge: Optional[float], max_iters: int, k_dykstra, verbose: bool, rec,
+                       seed: Optional[int] = None, device: Optional[int] = None, locator: Optional[int] = None,
+                       smooth: bool = True, devices=None, row_tiles: Optional[int] = None, refine: bool = False):
     """exchangeRayTracing!(rtm, rays_tot, nudge, max_iters, k_dykstra, verbose, rec): trace, optional
-    surfaces-only crop (:9-11), smooth (:14-70), store rtm.F_raw / rtm.F_smooth (:73-74)."""
+    surfaces-only crop (:9-11), smooth (:14-70), store rtm.F_raw / rtm.F_smooth (:73-74).  refine=True: see parallelRayTracing."""
     import time
     from .smoothing import smooth_F
     F_raw, rays_per_emitter = parallelRayTracing(rtm, rays_tot, nudge, verbose, rec=rec, seed=seed, device=device,
-                                                 locator=locator, devices=devices, row_tiles=row_tiles)
+                                                 locator=locator, devices=devices, row_tiles=row_tiles, refine=refine)
     t0 = time.perf_counter()
     ns = rtm.num_surfaces
     if rtm.surfaces_only and not isinstance(F_raw, list):
@@ -369,11 +426,11 @@ def exchangeRayTracing(rtm, rays_tot: int, nudge: float, max_iters: int, k_dykst
 
 def dispatch_ray_trace(rtm, rays_tot: int, method: str = "exchange", nudge: Optional[float] = None,
                        k_dykstra=None, max_iters: int = 1000, verbose: bool = True, rec=None, **kw):
-    """(rtm)(rays_tot; method, nudge, k_dykstra, max_iters, verbose, rec) — multiDispatchRayTrace2D.jl:1-18."""
-    trace_nudge = DEFAULT_NUDGE if nudge is None else nudge
+    """(rtm)(rays_tot; method, nudge, k_dykstra, max_iters, verbose, rec) — multiDispatchRayTrace2D.jl:1-18.  New keyword
+    refine=True (method=:exchange): add rays_tot // N rays per emitter to the previous call's trace and smooth again (parallelRayTracing)."""
     method = method.lstrip(":")
     if method == "exchange":
-        return exchangeRayTracing(rtm, rays_tot, trace_nudge, max_iters, k_dykstra, verbose, rec, **kw)
+        return exchangeRayTracing(rtm, rays_tot, nudge, max_iters, k_dykstra, verbose, rec, **kw)
     if method == "direct":
         raise NotImplementedError("method=:direct is outside the scope of this drop-in (exchange path only)")
     raise ValueError(f"Unknown ray tracing method: {method}, must be :exchange or :direct")
