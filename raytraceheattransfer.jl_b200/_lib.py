@@ -32,7 +32,7 @@ class RthxError(RuntimeError):
 
 
 def library_path() -> str:
-    # RTHX_LIBRARY: an alternative build of the same sources (A/B experiments, e.g. tools/gpu_evidence_r2.sh); never a fallback
+    # RTHX_LIBRARY: another build of the library, e.g. of an earlier commit for an A/B run against this one; never a fallback
     return os.environ.get("RTHX_LIBRARY") or os.path.join(_CSRC, "librthx.so")
 
 

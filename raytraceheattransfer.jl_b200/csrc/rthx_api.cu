@@ -932,7 +932,7 @@ extern "C" int rthx_get_info(const rthx_handle* h, rthx_info* info) {
 // ---------------------------------------------------------------------------------------------------------------
 namespace {
 
-struct LaunchPlan { int n_owned, n_blocks, block_threads, row_chunks, hist_in_smem, fast, minb, multi, sq, queue_depth, queue_gen; size_t smem_bytes; };
+struct LaunchPlan { int n_owned, n_blocks, block_threads, row_chunks; size_t smem_bytes; TraceKernelSel kernel; };
 
 int check_args(rthx_handle* h, const rthx_trace_args* a) {
   if (!a) return fail(h, RTHX_ERR_ARG, "trace: args is NULL");
@@ -984,81 +984,53 @@ int check_continue(rthx_handle* h, const rthx_trace_args* a) {
   return RTHX_OK;
 }
 
-// variant bits of the queue kernel (rthx_kernels.cu, kernel_variant): 8 general faces, 16 generic locator (implies 8), 32 its 80-register build
-int queue_variant_bits(const rthx_handle* h, const LaunchPlan& pl) {
-  if (pl.queue_gen) return 8 + 16 + (pl.queue_gen == 3 ? 32 : 0);
-  return h->queue_general ? 8 : 0;
-}
-
-// hash_slots > 0: the hashed row tally (no histogram, no SQ / queue kernels; the table takes hash_table_bytes(hash_slots))
+// hash_slots > 0: the hashed row tally (no histogram; the table takes hash_table_bytes(hash_slots))
 LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, int world, int hash_slots = 0) {
   LaunchPlan pl{};
   pl.n_owned = (h->N - rank + world - 1) / world;
   if (pl.n_owned < 0) pl.n_owned = 0;
   pl.block_threads = a->block_threads ? a->block_threads : 256;
-  pl.fast = (h->fast_ok && a->locator != RTHX_LOCATOR_GENERIC) ? 1 : 0;
-  pl.multi = a->mode != RTHX_FIRST_INTERACTION ? 1 : 0;
-  pl.minb = pl.multi ? 2 : 4;
-  if (const char* ev = std::getenv("RTHX_MINB")) { const int v = std::atoi(ev); if (v >= 2 && v <= 4) pl.minb = v; }   // tuning knob
-  if (!pl.fast && !pl.multi) {     // generic locator kernel: 4 resident blocks (64 registers; +4 % with the sole-bucket locator) unless RTHX_GENERIC_MINB=3 (80 registers)
-    pl.minb = 4;
-    if (const char* ev = std::getenv("RTHX_GENERIC_MINB")) { if (std::atoi(ev) == 3) pl.minb = 3; }
-  }
+  const bool analytic = a->locator != RTHX_LOCATOR_GENERIC;
+  const bool multi = a->mode != RTHX_FIRST_INTERACTION;
   const size_t coarse_bytes = h->coarse_fits_smem ? sizeof(CoarseDev) * (size_t)h->n_coarse : 0;
   const size_t hist_bytes = sizeof(uint32_t) * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;   // emitter block + log table
-  pl.hist_in_smem = (coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin) ? 1 : 0;
-  if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) pl.hist_in_smem = 0; }   // test knob: the N > ~57k path
-  if (hash_slots > 0) pl.hist_in_smem = 0;
-  pl.sq = (h->single_quad && a->locator != RTHX_LOCATOR_GENERIC && pl.hist_in_smem) ? 1 : 0;
-  if (const char* ev = std::getenv("RTHX_NO_SQ")) { if (std::atoi(ev)) pl.sq = 0; }   // test / tuning knob
-  // MULTI_BOUNCE on any mesh with analytic locators runs in the queue kernel's MULTI variant (lanes refill when their ray is
-  // absorbed); RTHX_MULTI_SQ=1 keeps the lock-step loop of the SQ kernel on single-quad domains (A/B knob)
-  bool multi_queue = pl.multi && h->queue_ok && a->locator != RTHX_LOCATOR_GENERIC && pl.hist_in_smem && pl.block_threads == 256;
-  if (const char* ev = std::getenv("RTHX_MULTI_SQ")) { if (std::atoi(ev) && pl.sq) multi_queue = false; }
-  if (const char* ev = std::getenv("RTHX_QUEUE_DEPTH")) { if (std::atoi(ev) == 0 && !pl.sq) multi_queue = false; }
-  if (multi_queue) pl.sq = 0;
-  if (pl.sq && pl.multi) {
-    pl.fast = 1; pl.minb = 4;                        // trace_exchange_sq_kernel<4, MULTI>
-  } else if (pl.sq) {
-    pl.fast = 1; pl.minb = 4;
-    // tuning knob: 3 = the shared-loop SQ branch of the general kernel (A/B reference)
-    if (const char* ev = std::getenv("RTHX_MINB")) { const int v = std::atoi(ev); if (v == 3) pl.minb = v; }
-  }
-  pl.smem_bytes = coarse_bytes + em_bytes + (pl.hist_in_smem ? hist_bytes : 0) + (hash_slots > 0 ? hash_table_bytes(hash_slots) : 0);
-  // Multi-face FAST meshes: the queue kernel (per-warp ray queue in shared memory, 40 bytes per parked ray).  Depth = as many
-  // rays per lane as still leave 4 resident blocks per SM, at most 8; RTHX_QUEUE_DEPTH overrides (0 = the lock-step kernel).
-  // The same kernel's general variant also takes multi-face meshes through the GENERIC locator (faces without a verified lattice,
-  // RTHX_LOCATOR_GENERIC) as long as the coarse descriptors fit in shared memory: a ray crosses several coarse faces there too, and
-  // the lock-step kernel keeps 13 of 32 lanes busy.  RTHX_NO_QUEUE_GENERIC=1 keeps the lock-step kernel (A/B knob).
-  pl.queue_gen = (!pl.multi && (a->locator == RTHX_LOCATOR_GENERIC || !h->queue_ok) && h->coarse_fits_smem && h->n_coarse > 1 &&
-                  pl.hist_in_smem && pl.block_threads == 256) ? 1 : 0;
-  if (const char* ev = std::getenv("RTHX_NO_QUEUE_GENERIC")) { if (std::atoi(ev)) pl.queue_gen = 0; }
-  if (pl.queue_gen) { if (const char* ev = std::getenv("RTHX_GENERIC_MINB")) { if (std::atoi(ev) == 3) pl.queue_gen = 3; } }   // 3: the 80-register build (A/B knob)
-  if (((h->queue_ok && a->locator != RTHX_LOCATOR_GENERIC && (!pl.multi || multi_queue) && (h->n_coarse > 1 || h->queue_general || multi_queue)) || pl.queue_gen) &&
-      !pl.sq && pl.hist_in_smem && pl.block_threads == 256) {
+  bool hist = hash_slots == 0 && coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
+  if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) hist = false; }   // test knob: the N > ~57k path
+  pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0) + (hash_slots > 0 ? hash_table_bytes(hash_slots) : 0);
+  pl.kernel = TraceKernelSel::lockstep(hist, h->fast_ok && analytic, multi);
+  // The queue kernel needs the histogram and 256 threads.  It takes multi-face meshes with analytic locators, and MULTI_BOUNCE on
+  // any of them (lanes refill when their ray is absorbed).  Its generic variant takes multi-face meshes through the GENERIC locator
+  // (faces without a verified lattice, RTHX_LOCATOR_GENERIC) as long as the coarse descriptors fit in shared memory: a ray crosses
+  // several coarse faces there too, and the lock-step kernel keeps 13 of 32 lanes busy.  A single parallelogram takes the SQ
+  // kernel, except for MULTI_BOUNCE at 256 threads.
+  const bool queue_fast = h->queue_ok && analytic && (h->n_coarse > 1 || h->queue_general || multi);
+  const bool queue_gen = !multi && (!analytic || !h->queue_ok) && h->coarse_fits_smem && h->n_coarse > 1;
+  if (hash_slots > 0) {
+    pl.kernel = TraceKernelSel::hash(h->fast_ok && analytic);
+  } else if (h->single_quad && analytic && hist && !(multi && pl.block_threads == 256)) {
+    pl.kernel = TraceKernelSel::sq(multi);
+  } else if (hist && pl.block_threads == 256 && (queue_fast || queue_gen)) {
+    // per-warp ray queue in shared memory.  Depth = as many rays per lane as still leave 4 resident blocks per SM (3 for the MULTI
+    // variant, which is bounded to 85 registers), at most 4 (MULTI: 2); large descriptor tables / histograms settle for fewer
     const size_t base = (pl.smem_bytes + 15) & ~size_t(15);
-    const size_t per_depth = (size_t)pl.block_threads * (multi_queue ? 48 : 40);   // bytes per parked ray: p, d, S (+ ray index and event word for MULTI)
-    // aim at 4 resident blocks per SM (3 for the MULTI variant, which is bounded to 85 registers); large descriptor tables /
-    // histograms settle for fewer
+    const size_t per_depth = (size_t)pl.block_threads * (multi ? 48 : 40);   // bytes per parked ray: p, d, S (+ ray index and event word for MULTI)
     int depth = 0;
-    const size_t max_depth = multi_queue ? 2 : 4;
-    for (int blocks = multi_queue ? 3 : 4; blocks >= 1 && depth == 0; --blocks) {
+    const size_t max_depth = multi ? 2 : 4;
+    for (int blocks = multi ? 3 : 4; blocks >= 1 && depth == 0; --blocks) {
       const size_t budget = std::min((size_t)h->prop.sharedMemPerMultiprocessor / blocks - 1024, (size_t)h->prop.sharedMemPerBlockOptin);
       if (base + per_depth <= budget) depth = (int)std::min<size_t>(max_depth, (budget - base) / per_depth);
     }
-    if (const char* ev = std::getenv("RTHX_QUEUE_DEPTH")) { const int v = std::atoi(ev); if (v >= 0 && v <= (int)max_depth) depth = v; }
-    if (depth == 3) depth = 2;                       // compiled depths: 1, 2, 4 rays per lane and batch (MULTI: 1, 2)
-    if (depth >= (pl.queue_gen ? 2 : 1) && base + depth * per_depth <= h->prop.sharedMemPerBlockOptin) {   // (the generic variant is compiled for depths 2 and 4)
-      pl.fast = 1; pl.minb = 6; pl.queue_depth = depth; pl.smem_bytes = base + depth * per_depth;
+    if (depth == 3) depth = 2;                       // compiled depths: 1, 2, 4 rays per lane and batch (MULTI: 1, 2; generic: 2, 4)
+    if (depth >= (queue_gen ? 2 : 1) && base + depth * per_depth <= h->prop.sharedMemPerBlockOptin) {
+      pl.kernel = TraceKernelSel::queue(!queue_gen, multi, depth, queue_gen || h->queue_general);
+      pl.smem_bytes = base + depth * per_depth;
     }
   }
-  if (!pl.queue_depth) pl.queue_gen = 0;
   const long long rows = (long long)pl.n_owned * a->n_bins;
   long long chunks = a->row_chunks;
   if (chunks <= 0) {
     // enough blocks for ~32 waves of the resident set, but keep >= 2048 rays (and >= N/2, the flush scan) per block
-    const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.block_threads, pl.smem_bytes, pl.hist_in_smem != 0, pl.fast != 0, pl.minb, pl.multi != 0, pl.sq != 0, pl.queue_depth + queue_variant_bits(h, pl),
-                                                                  hash_slots > 0));
+    const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.kernel, pl.block_threads, pl.smem_bytes));
     const long long target = (long long)h->prop.multiProcessorCount * per_sm * 32;
     chunks = rows > 0 ? (target + rows - 1) / rows : 1;
     const long long min_rays = std::max<long long>(2048, h->N / 2);
@@ -1085,14 +1057,10 @@ void fill_params(const rthx_handle* h, const rthx_trace_args* a, const LaunchPla
   P.emitter_rank = rank; P.emitter_world = world; P.n_owned = pl.n_owned; P.y_offset = 0;
   P.compact_rows = compact ? 1 : 0;
   P.row_chunks = pl.row_chunks;
-  P.queue_depth = pl.queue_depth;
-  P.queue_bilinear = queue_variant_bits(h, pl);
   P.queue_refill = 24;
-  if (const char* ev = std::getenv("RTHX_QUEUE_REFILL")) { const int v = std::atoi(ev); if (v >= 0 && v <= 32) P.queue_refill = v; }   // tuning knob
   P.coarse_in_smem = h->coarse_fits_smem ? 1 : 0;
-  P.hist_in_smem = pl.hist_in_smem;
   P.force_generic = a->locator == RTHX_LOCATOR_GENERIC ? 1 : 0;
-  P.multi_bounce = pl.multi; P.specular = a->mode == RTHX_MULTI_BOUNCE_SPECULAR ? 1 : 0;
+  P.specular = a->mode == RTHX_MULTI_BOUNCE_SPECULAR ? 1 : 0;
   // a count matrix that lives on another GPU (fused peer flush) is updated with system-scope reductions
   P.flush_system = 0;
   cudaPointerAttributes pa;
@@ -1122,8 +1090,7 @@ void fill_params(const rthx_handle* h, const rthx_trace_args* a, const LaunchPla
     const bool axis = f.nx[0] == 0.0 && std::fabs(f.ny[0]) == 1.0 && std::fabs(f.nx[1]) == 1.0 && f.ny[1] == 0.0 && f.g1y == 0.0 && f.g2x == 0.0;
     P.sq_axis = axis ? 1 : 0;
     if (const char* ev = std::getenv("RTHX_NO_AXIS")) { if (std::atoi(ev)) P.sq_axis = 0; }   // test knob: the general SQ loop
-    P.queue_sq = (h->single_quad && pl.multi && pl.queue_depth > 0) ? (P.sq_axis ? 1 : 2) : 0;
-    if (const char* ev = std::getenv("RTHX_NO_QUEUE_SQ")) { if (std::atoi(ev)) P.queue_sq = 0; }   // A/B knob: the generic step on a single quad
+    P.queue_sq = (h->single_quad && pl.kernel.family == TraceKernelSel::QUEUE && pl.kernel.multi) ? (P.sq_axis ? 1 : 2) : 0;
     P.sq_cy = f.ny[0] * P.sq_cen0; P.sq_cx = f.nx[1] * P.sq_cen1;
     P.sq_flip0 = f.ny[0] < 0.0 ? 0x80000000u : 0u; P.sq_flip1 = f.nx[1] < 0.0 ? 0x80000000u : 0u;
   }
@@ -1146,7 +1113,7 @@ void fill_stats(rthx_stats* st, const LaunchPlan& pl, const rthx_trace_args* a) 
   std::memset(st, 0, sizeof(*st));
   st->rays_traced = (int64_t)pl.n_owned * a->n_bins * a->rays_per_emitter;
   st->n_blocks = pl.n_blocks; st->block_threads = pl.block_threads; st->row_chunks = pl.row_chunks;
-  st->smem_bytes = (int32_t)pl.smem_bytes; st->hist_in_smem = pl.hist_in_smem;
+  st->smem_bytes = (int32_t)pl.smem_bytes; st->hist_in_smem = pl.kernel.hist;
 }
 
 // Enqueue (zero +) kernel for one handle on `stream`; counts layout compact (owned rows) or full.
@@ -1156,7 +1123,7 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
                   LaunchPlan* plan_out, int* n_launches, int y0 = 0, int y1 = -1, bool upload_bins = true) {
   LaunchPlan pl = make_plan(h, a, rank, world);
   if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
-  if (!pl.fast || pl.queue_gen) { const int rcg = ensure_generic(h); if (rcg) return rcg; }     // the generic kernel reads the reference-faithful locator tables
+  if (!pl.kernel.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }     // the generic locator reads the reference-faithful tables
   if (upload_bins) CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)a->n_bins, cudaMemcpyHostToDevice, stream));
   // A matrix in peer memory (fused multi-GPU flush) is never the target of reductions: the chunks of a row add up in a local
   // compact staging matrix and the finished row is handed over with plain stores (flush_row_hist) — so the peer rows need no
@@ -1169,9 +1136,8 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
     if (counts && cudaPointerGetAttributes(&pa, counts) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device != h->device) peer = true;
     else cudaGetLastError();
     if (const char* ev = std::getenv("RTHX_FLUSH_SYSTEM")) peer = std::atoi(ev) != 0;     // test knob: exercise the hand-over on one GPU
-    if (const char* ev = std::getenv("RTHX_PEER_ATOMICS")) { if (std::atoi(ev)) peer = false; }   // A/B knob: the old red.sys flush
   }
-  const bool staged = peer && pl.hist_in_smem && !compact;
+  const bool staged = peer && pl.kernel.hist && !compact;
   unsigned long long* stage_counts = nullptr;
   unsigned int* row_done = nullptr;
   if (staged) {
@@ -1216,7 +1182,7 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
   if (y1 < 0) y1 = pl.n_owned;
   P.y_offset = y0;
   const long long nb = (long long)(y1 - y0) * a->n_bins * pl.row_chunks;
-  CU(h, launch_trace_exchange(P, (int)nb, pl.block_threads, pl.smem_bytes, pl.fast != 0, pl.minb, pl.sq != 0, stream));
+  CU(h, launch_trace_exchange(P, pl.kernel, (int)nb, pl.block_threads, pl.smem_bytes, stream));
   if (nb > 0) *n_launches += 1;
   *plan_out = pl;
   return RTHX_OK;
@@ -1252,7 +1218,7 @@ int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, int rank, int worl
   // batches: >= ~2 waves of resident blocks each, at most 16 (consecutive batches alternate between two streams, so a batch's
   // draining tail overlaps the next one's head; cfg3 at 1e10 rays: 16 batches, the copy behind the last kernel is 17 MB and the
   // call ends 0.5 ms after the kernel — with 5 even batches it was 180 MB and 3.6 ms)
-  const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.block_threads, pl.smem_bytes, pl.hist_in_smem != 0, pl.fast != 0, pl.minb, pl.multi != 0, pl.sq != 0, pl.queue_depth + queue_variant_bits(h, pl)));
+  const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.kernel, pl.block_threads, pl.smem_bytes));
   const long long resident = (long long)h->prop.multiProcessorCount * per_sm;
   int n_batches = (int)std::min<long long>(16, std::max<long long>(1, pl.n_blocks / (2 * resident)));
   n_batches = std::max(1, std::min(n_batches, n_owned));
@@ -1307,7 +1273,6 @@ int pipeline_copy(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
   cudaPointerAttributes pa;
   bool pinned = cudaPointerGetAttributes(&pa, counts_out) == cudaSuccess && (pa.type == cudaMemoryTypeHost || pa.type == cudaMemoryTypeManaged);
   cudaGetLastError();
-  if (const char* ev = std::getenv("RTHX_FORCE_STAGING")) { if (std::atoi(ev)) pinned = false; }
   const size_t row_bytes = sizeof(uint64_t) * (size_t)N;
   auto batch_rows = [&](int b, int& y0, int& y1) { batch_rows_of(n_owned, n_batches, b, y0, y1); };
   if (pinned) {
@@ -1535,7 +1500,7 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     pl.smem_bytes = pl.smem_bytes - hash_table_bytes(1 << old) + hash_table_bytes(1 << log2s);
   }
   if (pl.smem_bytes > h->prop.sharedMemPerBlockOptin) return fail(h, RTHX_ERR_ARG, "trace_sparse: hash table does not fit in shared memory");
-  if (!pl.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }
+  if (!pl.kernel.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }
   // pair buffer: at most one pair per tallied ray, and at most half the free device memory (24 bytes a pair with the sort's
   // alternate buffers); the other half is left for the resident totals
   long long cap = 0x7FFFFFFFll;
@@ -1584,7 +1549,7 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     CU(h, cudaMemsetAsync(h->sk_ctl, 0, 4 * sizeof(unsigned long long), h->stream));
     P.y_offset = y0;
     CU(h, cudaEventRecord(h->ev[1], h->stream));
-    CU(h, launch_trace_exchange(P, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, pl.fast != 0, pl.minb, false, h->stream));
+    CU(h, launch_trace_exchange(P, pl.kernel, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, h->stream));
     CU(h, cudaEventRecord(h->ev[2], h->stream));
     R.n_launches += 2;
     unsigned long long ctl[4];

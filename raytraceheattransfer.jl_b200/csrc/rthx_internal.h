@@ -91,15 +91,11 @@ struct TraceParams {
   int32_t compact_rows;        // 1: counts row index is the owned-emitter ordinal, 0: the element index
   int32_t row_chunks;
   int32_t coarse_in_smem;
-  int32_t hist_in_smem;
   int32_t force_generic;
-  int32_t multi_bounce;        // RTHX_MULTI_BOUNCE: follow scattering / reflection events until absorption
   int32_t specular;            // MULTI_BOUNCE: mirror reflection instead of diffuse
   int32_t flush_system;        // 1: system-scope atomics for the flush (count matrix in peer memory)
   int32_t rec_bin;
   int32_t queue_refill;        // queue kernel: with the queue dry, emit the next batch once <= this many lanes still hold a ray
-  int32_t queue_depth;         // queue kernel: rays parked per lane and batch (queue slots per warp = 32 * queue_depth)
-  int32_t queue_bilinear;      // queue kernel variant bits: 8 general faces (bilinear lattices, T-junctions), 16 generic locator, 32 its 80-register build
   int32_t queue_sq;            // MULTI queue kernel: the domain is one parallelogram (1 axis-aligned, 2 general): SQ form of the step
   // The 64-bit block below starts on a 16-byte boundary of the parameter bank whatever the number of pointers above: the kernels take
   // the constants and the Philox round keys as c[0][..] operands / 128-bit uniform loads, and ptxas' register allocation depends on
@@ -137,13 +133,37 @@ struct TraceParams {
 static_assert(offsetof(TraceParams, rays_per_emitter) % 16 == 0 && offsetof(TraceParams, k_u52) % 16 == 0 && offsetof(TraceParams, rk) % 16 == 0,
               "TraceParams: constants and round keys keep their 16-byte alignment in the parameter bank");
 
-// launchers implemented in rthx_kernels.cu
-cudaError_t launch_trace_exchange(const TraceParams& p, int n_blocks, int block_threads, size_t smem_bytes, bool fast, int minb, bool sq,
-                                  cudaStream_t stream);   // minb == 6: the queue kernel with p.queue_depth in {1, 2, 4}
+// Which trace kernel runs: decided once per trace by make_plan (rthx_api.cu), mapped to its compiled instance by rthx_kernels.cu.
+struct TraceKernelSel {
+  enum Family : int {
+    LOCKSTEP,   // trace_exchange_kernel: one ray per thread, any mesh
+    SQ,         // trace_exchange_sq_kernel: the whole domain is one parallelogram face
+    QUEUE,      // trace_exchange_queue_kernel: per-warp ray queue (multi-face meshes; MULTI_BOUNCE on analytic meshes)
+    HASH,       // trace_exchange_hash_kernel: hashed row tally (rthx_trace_exchange_sparse)
+  };
+  Family family = LOCKSTEP;
+  bool hist = false;      // row histogram in shared memory (SQ and QUEUE always, HASH never)
+  bool fast = false;      // no generic locator in the kernel: every face an affine lattice with a complete neighbour table.  The
+                          // generic locator tables (ensure_generic) are needed exactly when this is false.
+  bool multi = false;     // MULTI_BOUNCE event loop
+  int depth = 0;          // QUEUE: rays parked per lane and batch (queue slots per warp = 32 * depth)
+  bool general = false;   // QUEUE: bilinear lattices or interfaces without a unique neighbour (the !fast build has them always)
+  bool operator==(const TraceKernelSel& o) const {
+    return family == o.family && hist == o.hist && fast == o.fast && multi == o.multi && depth == o.depth && general == o.general;
+  }
+  // the selections of each family, with the fields the family does not use at their defaults
+  static constexpr TraceKernelSel lockstep(bool hist, bool fast, bool multi) { return {LOCKSTEP, hist, fast, multi, 0, false}; }
+  static constexpr TraceKernelSel sq(bool multi) { return {SQ, true, true, multi, 0, false}; }
+  static constexpr TraceKernelSel queue(bool fast, bool multi, int depth, bool general) { return {QUEUE, true, fast, multi, depth, general}; }
+  static constexpr TraceKernelSel hash(bool fast) { return {HASH, false, fast, false, 0, false}; }
+};
+
+// launchers implemented in rthx_kernels.cu; a selection without a compiled instance fails with cudaErrorInvalidDeviceFunction
+cudaError_t launch_trace_exchange(const TraceParams& p, const TraceKernelSel& k, int n_blocks, int block_threads, size_t smem_bytes,
+                                  cudaStream_t stream);
 cudaError_t configure_trace_kernel(size_t smem_bytes);
 cudaError_t launch_fp64_peak(double* out, int n_blocks, int block_threads, int iters, cudaStream_t stream);
-int trace_kernel_max_blocks_per_sm(int block_threads, size_t smem_bytes, bool hist, bool fast, int minb, bool multi, bool sq, int queue_depth = 0,
-                                   bool hash = false);
+int trace_kernel_max_blocks_per_sm(const TraceKernelSel& k, int block_threads, size_t smem_bytes);
 constexpr size_t hash_table_bytes(int slots) { return 8 * (size_t)slots + 16; }   // keys + counts (u32 each) + occupied / fill / base words
 
 // hashed row tally, host side of the reduction (rthx_sparse_tally.cu)

@@ -326,15 +326,6 @@ __device__ __forceinline__ int locate_affine(const TraceParams& p, const CoarseD
   return __ldg(p.lattice + cf.lat_off + cell);
 }
 
-// the same for a face known to be a parallelogram lattice (fine index = n + m Nx, meshQuad.jl:139,151)
-__device__ __forceinline__ int locate_quad(const CoarseDev& cf, double px, double py) {
-  const double rx = px - cf.ax, ry = py - cf.ay;
-  const double s = rx * cf.g1x + ry * cf.g1y, t = rx * cf.g2x + ry * cf.g2y;
-  const int n = __double2int_rd(s), m = __double2int_rd(t);
-  if (!((s >= 0.0) & (t >= 0.0) & (n < cf.Nx) & (m < cf.Ny))) return -1;
-  return n + m * cf.Nx;
-}
-
 template <bool FAST>
 __device__ __forceinline__ int locate_fine(const TraceParams& p, const CoarseDev& cf, int c, int kind, double px, double py) {
   if (!FAST && kind == KIND_GENERIC) return find_face_generic(p, 1 + c, px, py);
@@ -447,7 +438,8 @@ __device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, uns
 //   HASH     : hashed row tally into (row, column, count) pairs (see above; HIST_SMEM == false): trace_exchange_hash_kernel
 //   FAST     : every coarse face is a verified affine lattice with a complete neighbour table and the coarse
 //              descriptors fit in shared memory -> no generic locator code in the kernel at all
-//   MINB     : minimum resident blocks per SM the register allocation is bounded for
+//   MULTI    : RTHX_MULTI_BOUNCE event loop
+// Registers are bounded for 4 resident blocks per SM (64) with the histogram and FIRST_INTERACTION, for 2 otherwise.
 // ------------------------------------------------------------------------------------------------------------
 // Block-uniform emitter description, kept in shared memory (broadcast LDS) instead of ~24 registers per thread.
 //   surface emitter: [0,1] p1, [2,3] edge p2-p1, [4,5] xVecLocal (unit edge), [6,7] yVecLocal (left normal)
@@ -455,12 +447,8 @@ __device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, uns
 //   both           : [12,13] cell midPoint
 constexpr int EM_DOUBLES = 16;
 
-//   MULTI    : RTHX_MULTI_BOUNCE event loop
-//   SQ       : the whole domain is ONE parallelogram coarse face (every square / rectangular enclosure): its descriptor
-//              is read from the kernel-parameter bank (FP64 instructions take c[0][..] operands: no LDS, no address
-//              arithmetic), there is no coarse-face loop and no per-face kind dispatch
-template <bool HIST_SMEM, bool FAST, int MINB, bool MULTI, bool SQ>
-__global__ void __launch_bounds__(256, MINB) trace_exchange_kernel(const __grid_constant__ TraceParams p) {
+template <bool HIST_SMEM, bool FAST, bool MULTI>
+__global__ void __launch_bounds__(256, HIST_SMEM && !MULTI ? 4 : 2) trace_exchange_kernel(const __grid_constant__ TraceParams p) {
   constexpr bool HASH = false;
 #include "rthx_trace_body.cuh"
 }
@@ -468,13 +456,14 @@ __global__ void __launch_bounds__(256, MINB) trace_exchange_kernel(const __grid_
 // the same kernel with the hashed row tally (FIRST_INTERACTION, no histogram; the host rejects MULTI_BOUNCE before a launch)
 template <bool FAST>
 __global__ void __launch_bounds__(256, 2) trace_exchange_hash_kernel(const __grid_constant__ TraceParams p) {
-  constexpr bool HIST_SMEM = false, MULTI = false, SQ = false, HASH = true;
+  constexpr bool HIST_SMEM = false, MULTI = false, HASH = true;
 #include "rthx_trace_body.cuh"
 }
 
 // ------------------------------------------------------------------------------------------------------------
 // K1-SQ: the fused kernel for domains that are ONE parallelogram coarse face (every square / rectangular enclosure:
-// cfg1-4).  Same arithmetic as the SQ branch of trace_exchange_kernel; what differs is the code shape:
+// cfg1-4).  Its descriptor is read from the kernel-parameter bank (FP64 instructions take c[0][..] operands: no LDS, no address
+// arithmetic); there is no coarse-face loop and no per-face kind dispatch.  The code shape:
 //   * the three block-uniform decisions — surface or volume emitter, uniform or cell-wise beta, recorder on or off —
 //     are taken ONCE, outside the ray loop, into eight specialised loop bodies.  Each loop keeps only its own
 //     constants live, so the uniform-register file no longer overflows (the single shared loop spent ~40 of 327 warp
@@ -689,17 +678,6 @@ __device__ __forceinline__ unsigned int sq_ray_loop(const TraceParams& p, const 
         absorber = sid;
       }
     }
-#ifdef RTHX_TALLY_MATCH
-    // A/B variant (tools/gpu_evidence_r2.sh builds it as a second library): warp-aggregated tally — lanes that hit the same bin
-    // elect one of them to add the group's count.  Measured on cfg3: slower than one red.shared.add.u32 per ray (DESIGN.md section 4).
-    {
-      const unsigned act = __activemask();
-      const unsigned grp = __match_any_sync(act, absorber);
-      if (absorber >= 0 && (int)(__ffs((int)grp) - 1) == (int)(threadIdx.x & 31))
-        asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(hist_s + 4u * (uint32_t)absorber), "r"((unsigned)__popc(grp)) : "memory");
-      if (absorber < 0) ++n_lost;
-    }
-#else
     if (absorber >= 0) {
       asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(hist_s + 4u * (uint32_t)absorber), "r"(1u) : "memory");
       if (REC) {
@@ -711,7 +689,6 @@ __device__ __forceinline__ unsigned int sq_ray_loop(const TraceParams& p, const 
     } else {
       ++n_lost;
     }
-#endif
     {
       const uint64_t ray_id = (uint64_t)(b.ray0 + (int64_t)(i + blockDim.x));
       w0n = philox4x32_10_rk(make_uint4((uint32_t)ray_id, (uint32_t)(ray_id >> 32), b.e, b.cw | 0u), p.rk);
@@ -1503,9 +1480,10 @@ __device__ __forceinline__ unsigned int queue_multi_dispatch(const TraceParams& 
 }
 
 // BILIN: the mesh has general convex quadrilateral faces (bilinear lattices); compiled separately so that meshes of parallelograms
-// and triangles keep the shorter traversal loop
-template <int MINB, int DEPTH, bool BILIN, bool MULTI, bool GEN = false>
-__global__ void __launch_bounds__(256, MINB) trace_exchange_queue_kernel(const __grid_constant__ TraceParams p) {
+// and triangles keep the shorter traversal loop.  GEN: faces on the generic locator (FIRST_INTERACTION).
+// Registers are bounded for 4 resident blocks per SM (64), 3 (80) for the MULTI event loop.
+template <int DEPTH, bool BILIN, bool MULTI, bool GEN>
+__global__ void __launch_bounds__(256, MULTI ? 3 : 4) trace_exchange_queue_kernel(const __grid_constant__ TraceParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const size_t coarse_bytes = sizeof(CoarseDev) * (size_t)p.n_coarse;
   double* s_em = reinterpret_cast<double*>(smem_raw + coarse_bytes);
@@ -1592,78 +1570,69 @@ __global__ void __launch_bounds__(256, MINB) trace_exchange_queue_kernel(const _
   }
 }
 
-// kernel variants: hist_in_smem x fast x multi; the register bound MINB only varies for the hot FIRST_INTERACTION FAST kernel
+// Every compiled trace-kernel instance and the selection that names it: launches and occupancy queries look the selection up here.
+// The list is also the order in which the instances are instantiated, and ptxas output depends on it (the front end numbers
+// virtual registers in that order): the same instances listed family by family in another order changed the register assignment of
+// the MULTI queue kernels.
 typedef void (*TraceKernel)(const TraceParams);
-static TraceKernel kernel_variant(bool hist, bool fast, int minb, bool multi, bool sq, int queue_depth = 0) {
-  if (sq && hist && fast && multi) return (TraceKernel)trace_exchange_sq_kernel<4, true>;   // multi-bounce on the single-quad domain
-  if (sq && hist && fast && !multi) {
-    if (minb == 3) return (TraceKernel)trace_exchange_kernel<true, true, 4, false, true>;   // RTHX_MINB=3: the shared-loop form (A/B knob)
-    return (TraceKernel)trace_exchange_sq_kernel<4, false>;
-  }
-  if (minb == 6 && hist && fast && !sq) {                                                               // per-warp ray queue (multi-face meshes; MULTI_BOUNCE on any analytic mesh)
-    const bool bilin = (queue_depth & 8) != 0;                                                          // depth + 8: bilinear faces present
-    const int d = queue_depth & 7;
-    if (queue_depth & 16) {                                                                             // depth + 16: faces on the generic locator (FIRST_INTERACTION; compiled depths 2, 4)
-      if (queue_depth & 32) return d >= 4 ? (TraceKernel)trace_exchange_queue_kernel<3, 4, true, false, true> : (TraceKernel)trace_exchange_queue_kernel<3, 2, true, false, true>;   // RTHX_GENERIC_MINB=3
-      return d >= 4 ? (TraceKernel)trace_exchange_queue_kernel<4, 4, true, false, true> : (TraceKernel)trace_exchange_queue_kernel<4, 2, true, false, true>;
-    }
-    if (multi) {                                                                                        // compiled depths: 1, 2
-      if (d >= 2) return bilin ? (TraceKernel)trace_exchange_queue_kernel<3, 2, true, true> : (TraceKernel)trace_exchange_queue_kernel<3, 2, false, true>;
-      return bilin ? (TraceKernel)trace_exchange_queue_kernel<3, 1, true, true> : (TraceKernel)trace_exchange_queue_kernel<3, 1, false, true>;
-    }
-    if (d >= 4) return bilin ? (TraceKernel)trace_exchange_queue_kernel<4, 4, true, false> : (TraceKernel)trace_exchange_queue_kernel<4, 4, false, false>;
-    if (d >= 2) return bilin ? (TraceKernel)trace_exchange_queue_kernel<4, 2, true, false> : (TraceKernel)trace_exchange_queue_kernel<4, 2, false, false>;
-    return bilin ? (TraceKernel)trace_exchange_queue_kernel<4, 1, true, false> : (TraceKernel)trace_exchange_queue_kernel<4, 1, false, false>;
-  }
-  if (multi) {
-    if (hist) return fast ? (TraceKernel)trace_exchange_kernel<true, true, 2, true, false> : (TraceKernel)trace_exchange_kernel<true, false, 2, true, false>;
-    return fast ? (TraceKernel)trace_exchange_kernel<false, true, 2, true, false> : (TraceKernel)trace_exchange_kernel<false, false, 2, true, false>;
-  }
-  if (!hist) return fast ? (TraceKernel)trace_exchange_kernel<false, true, 2, false, false> : (TraceKernel)trace_exchange_kernel<false, false, 2, false, false>;
-  if (!fast) return minb == 4 ? (TraceKernel)trace_exchange_kernel<true, false, 4, false, false>     // generic locator: 64 registers, 4 blocks per SM (default)
-                              : (TraceKernel)trace_exchange_kernel<true, false, 3, false, false>;    // 80 registers, 3 blocks per SM
-  switch (minb) {
-    case 3: return (TraceKernel)trace_exchange_kernel<true, true, 3, false, false>;
-    case 4: return (TraceKernel)trace_exchange_kernel<true, true, 4, false, false>;
-    default: return (TraceKernel)trace_exchange_kernel<true, true, 2, false, false>;
-  }
-}
+struct TraceInstance { TraceKernelSel sel; TraceKernel kernel; };
+using Sel = TraceKernelSel;
 
-static TraceKernel hash_kernel_variant(bool fast) {
-  return fast ? (TraceKernel)trace_exchange_hash_kernel<true> : (TraceKernel)trace_exchange_hash_kernel<false>;
+static const TraceInstance k_trace_instances[] = {
+    {Sel::sq(true), trace_exchange_sq_kernel<4, true>},
+    {Sel::sq(false), trace_exchange_sq_kernel<4, false>},
+    {Sel::queue(false, false, 4, true), trace_exchange_queue_kernel<4, true, false, true>},
+    {Sel::queue(false, false, 2, true), trace_exchange_queue_kernel<2, true, false, true>},
+    {Sel::queue(true, true, 2, true), trace_exchange_queue_kernel<2, true, true, false>},
+    {Sel::queue(true, true, 2, false), trace_exchange_queue_kernel<2, false, true, false>},
+    {Sel::queue(true, true, 1, true), trace_exchange_queue_kernel<1, true, true, false>},
+    {Sel::queue(true, true, 1, false), trace_exchange_queue_kernel<1, false, true, false>},
+    {Sel::queue(true, false, 4, true), trace_exchange_queue_kernel<4, true, false, false>},
+    {Sel::queue(true, false, 4, false), trace_exchange_queue_kernel<4, false, false, false>},
+    {Sel::queue(true, false, 2, true), trace_exchange_queue_kernel<2, true, false, false>},
+    {Sel::queue(true, false, 2, false), trace_exchange_queue_kernel<2, false, false, false>},
+    {Sel::queue(true, false, 1, true), trace_exchange_queue_kernel<1, true, false, false>},
+    {Sel::queue(true, false, 1, false), trace_exchange_queue_kernel<1, false, false, false>},
+    {Sel::lockstep(true, true, true), trace_exchange_kernel<true, true, true>},
+    {Sel::lockstep(true, false, true), trace_exchange_kernel<true, false, true>},
+    {Sel::lockstep(false, true, true), trace_exchange_kernel<false, true, true>},
+    {Sel::lockstep(false, false, true), trace_exchange_kernel<false, false, true>},
+    {Sel::lockstep(false, true, false), trace_exchange_kernel<false, true, false>},
+    {Sel::lockstep(false, false, false), trace_exchange_kernel<false, false, false>},
+    {Sel::lockstep(true, false, false), trace_exchange_kernel<true, false, false>},
+    {Sel::lockstep(true, true, false), trace_exchange_kernel<true, true, false>},
+    {Sel::hash(true), trace_exchange_hash_kernel<true>},
+    {Sel::hash(false), trace_exchange_hash_kernel<false>},
+};
+
+static TraceKernel trace_kernel(const TraceKernelSel& k) {
+  for (const TraceInstance& t : k_trace_instances)
+    if (t.sel == k) return t.kernel;
+  return nullptr;
 }
 
 cudaError_t configure_trace_kernel(size_t smem_bytes) {
-  for (int sq = 0; sq < 2; ++sq)
-    for (int multi = 0; multi < 2; ++multi)
-      for (int hist = 0; hist < 2; ++hist)
-        for (int fast = 0; fast < 2; ++fast)
-          for (int minb = 2; minb <= 6; ++minb)
-            for (int depth : {1, 2, 4, 9, 10, 12, 18, 20, 50, 52}) {
-              cudaError_t e = cudaFuncSetAttribute((const void*)kernel_variant(hist, fast, minb, multi, sq, depth), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-              if (e != cudaSuccess) return e;
-            }
-  for (int fast = 0; fast < 2; ++fast) {
-    cudaError_t e = cudaFuncSetAttribute((const void*)hash_kernel_variant(fast), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
+  for (const TraceInstance& t : k_trace_instances) {
+    cudaError_t e = cudaFuncSetAttribute((const void*)t.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
     if (e != cudaSuccess) return e;
   }
   return cudaSuccess;
 }
 
-int trace_kernel_max_blocks_per_sm(int block_threads, size_t smem_bytes, bool hist, bool fast, int minb, bool multi, bool sq, int queue_depth, bool hash) {
+int trace_kernel_max_blocks_per_sm(const TraceKernelSel& k, int block_threads, size_t smem_bytes) {
+  const TraceKernel f = trace_kernel(k);
   int n = 0;
-  const void* k = hash ? (const void*)hash_kernel_variant(fast) : (const void*)kernel_variant(hist, fast, minb, multi, sq, queue_depth);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, block_threads, smem_bytes) != cudaSuccess) return 0;
+  if (!f || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, (const void*)f, block_threads, smem_bytes) != cudaSuccess) return 0;
   return n;
 }
 
-cudaError_t launch_trace_exchange(const TraceParams& p, int n_blocks, int block_threads, size_t smem_bytes, bool fast, int minb, bool sq,
+cudaError_t launch_trace_exchange(const TraceParams& p, const TraceKernelSel& k, int n_blocks, int block_threads, size_t smem_bytes,
                                   cudaStream_t stream) {
+  const TraceKernel f = trace_kernel(k);
+  if (!f) return cudaErrorInvalidDeviceFunction;
   if (n_blocks <= 0) return cudaSuccess;
-  TraceKernel k = p.sk_keys ? hash_kernel_variant(fast)
-                            : kernel_variant(p.hist_in_smem != 0, fast, minb, p.multi_bounce != 0, sq, p.queue_depth + p.queue_bilinear);   // queue_bilinear: variant bits 8 | 16 | 32
   void* args[] = {(void*)&p};
-  return cudaLaunchKernel((const void*)k, dim3(n_blocks), dim3(block_threads), args, smem_bytes, stream);
+  return cudaLaunchKernel((const void*)f, dim3(n_blocks), dim3(block_threads), args, smem_bytes, stream);
 }
 
 // ------------------------------------------------------------------------------------------------------------

@@ -1,10 +1,10 @@
-// rthx_trace_body.cuh — body of K1 (rthx_kernels.cu), shared by trace_exchange_kernel<HIST_SMEM, FAST, MINB, MULTI, SQ> and
-// trace_exchange_hash_kernel<FAST>.  It is included INSIDE their function bodies, where HIST_SMEM, FAST, MULTI, SQ and HASH
+// rthx_trace_body.cuh — body of K1 (rthx_kernels.cu), shared by trace_exchange_kernel<HIST_SMEM, FAST, MULTI> and
+// trace_exchange_hash_kernel<FAST>.  It is included INSIDE their function bodies, where HIST_SMEM, FAST, MULTI and HASH
 // are compile-time constants and `p` is the __grid_constant__ parameter: inlining it through a device function taking the
 // parameter by reference changed the code ptxas generates for the existing instances, textual inclusion does not.
   extern __shared__ __align__(16) unsigned char smem_raw[];
   CoarseDev* s_coarse = reinterpret_cast<CoarseDev*>(smem_raw);
-  const bool coarse_smem = !SQ && (FAST || p.coarse_in_smem);
+  const bool coarse_smem = FAST || p.coarse_in_smem;
   const size_t coarse_bytes = coarse_smem ? sizeof(CoarseDev) * (size_t)p.n_coarse : 0;
   double* s_em = reinterpret_cast<double*>(smem_raw + coarse_bytes);
   double2* s_log = reinterpret_cast<double2*>(smem_raw + coarse_bytes + sizeof(double) * EM_DOUBLES);
@@ -139,31 +139,6 @@
     double neg_log = neg_log_table(R_S, s_log);
     int c = c0;
     int absorber = -1;
-    if constexpr (SQ) {
-      // single parallelogram face: one distToSurface2D, one decision, one fine-cell location (traceRay.jl:27-52)
-      const CoarseDev& cf = p.face0;
-      int k;
-      const double u = dist_quad(cf, px, py, dx, dy, p.k_eps, k);
-      double S = neg_log * inv_beta_u;
-      bool gas = S < u, ok = true;
-      if (!uniform) {
-        const int f0 = locate_quad(cf, px, py);              // traceRay.jl:87-100
-        ok = f0 >= 0;
-        const double local_beta = ok ? beta_band[f0] : 0.0;
-        gas = local_beta * u >= neg_log;
-        S = neg_log / local_beta;
-      }
-      // Gas and wall endings share one advance + one fine-cell location (same arithmetic as the two branches of
-      // traceRay.jl:31-52, selected per lane): a warp with both kinds of ray no longer issues the tail twice.
-      const bool hit = !gas & (u < CUDART_INF) & (cf.solid[k] != 0);   // an open edge has no neighbour face: the ray is lost
-      if (ok & (gas | hit)) {
-        const double adv = (gas ? S : u) - p.nudge;
-        px = fma(adv, dx, px);
-        py = fma(adv, dy, py);
-        const int f = locate_quad(cf, px, py);
-        if (f >= 0) absorber = gas ? p.n_surfaces + f : __ldg(p.cell_surf_id + 4 * f + k);
-      }
-    } else {
     double hit_nx = 0.0, hit_ny = 0.0;   // MULTI: outward unit normal of the wall that was hit
 #pragma unroll 1
     for (int event = 0;; ++event) {
@@ -266,7 +241,6 @@
       }
     }
     neg_log = -log(u52(v1.z, v1.w, p.k_u52));
-    }
     }
 
     // ---- stage 3/4: tally (+ record) -------------------------------------------------------------------------

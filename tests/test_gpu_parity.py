@@ -125,19 +125,18 @@ def test_variable_beta_across_faces(rthx_mod, oracle_mod, cuda_lib):
     check_exact(tr.trace(20000, seed=8), ref, 20000, budget_frac=2e-4)
 
 
-def test_non_parallelogram_quad_is_a_bilinear_lattice(rthx_mod, oracle_mod, cuda_lib, monkeypatch):
+def test_non_parallelogram_quad_is_a_bilinear_lattice(rthx_mod, oracle_mod, cuda_lib):
     """A quadrilateral that is no parallelogram is meshed by meshQuad.jl:116-136 into the bilinear image of a uniform lattice:
     located by the analytic inverse of the bilinear map in the queue kernel (next to an affine neighbour), by grid +
-    point-in-polygon under RTHX_LOCATOR_GENERIC and when the queue kernel is switched off (lock-step general kernel)."""
+    point-in-polygon under RTHX_LOCATOR_GENERIC and at block_threads=128, which the queue kernel does not take (lock-step
+    general kernel)."""
     rtm = rthx_mod.meshes.two_quads_domain(kappa=(1.0, 1.0), skew=0.3)
     flat, tr = tracer(rthx_mod, cuda_lib, rtm)
     assert tr.info["n_affine_faces"] == 1 and tr.info["n_bilinear_faces"] == 1     # the skewed quad is not a parallelogram
     ref = oracle_mod.trace(flat, 20000, seed=9)
     check_exact(tr.trace(20000, seed=9, locator=GENERIC), ref, 20000)
     check_exact(tr.trace(20000, seed=9), ref, 20000, budget_frac=2e-4)
-    monkeypatch.setenv("RTHX_QUEUE_DEPTH", "0")
-    check_exact(tr.trace(20000, seed=9), ref, 20000, budget_frac=2e-4)
-    monkeypatch.delenv("RTHX_QUEUE_DEPTH")
+    check_exact(tr.trace(20000, seed=9, block_threads=128), ref, 20000, budget_frac=2e-4)
 
 
 def test_bilinear_single_faces_trapezoid_and_general_quad(rthx_mod, oracle_mod, cuda_lib):

@@ -300,7 +300,7 @@ def test_multi_link_result_copies_equal_single_link(rthx_mod, cuda_lib):
 def test_generic_locator_on_the_ray_queue_equals_lock_step(rthx_mod, oracle_mod, cuda_lib, monkeypatch, mesh):
     """Multi-face meshes under RTHX_LOCATOR_GENERIC run in the queue kernel's generic variant (bucket grid + crossing number at
     every crossing, per-step cell lookup for cell-wise beta, wall lookup from the polygon record).  Same integers as the lock-step
-    generic kernel (RTHX_NO_QUEUE_GENERIC=1), as its 80-register build, as a coarser bucket grid, and — within the exact-parity
+    generic kernel (block_threads=128: the queue needs 256 threads), as a coarser bucket grid, and — within the exact-parity
     budget of the reference-faithful locator — as the CPU oracle."""
     m = rthx_mod.meshes
     rtm = {"cfg5": m.cfg5, "two_quads": lambda: m.two_quads_domain(skew=0.25),           # cell-wise beta, a bilinear face
@@ -308,18 +308,16 @@ def test_generic_locator_on_the_ray_queue_equals_lock_step(rthx_mod, oracle_mod,
     flat = rthx_mod.flatten_domain(rtm)
     rpe = 3000
     out = {}
-    for tag, env in (("queue", {}), ("lockstep", {"RTHX_NO_QUEUE_GENERIC": "1"}), ("queue80", {"RTHX_GENERIC_MINB": "3"}),
-                     ("coarse_grid", {"RTHX_GRID_FINE": "2"})):
-        for k in ("RTHX_NO_QUEUE_GENERIC", "RTHX_GENERIC_MINB", "RTHX_GRID_FINE"):
-            monkeypatch.delenv(k, raising=False)
+    for tag, env, kw in (("queue", {}, {}), ("lockstep", {}, {"block_threads": 128}), ("coarse_grid", {"RTHX_GRID_FINE": "2"}, {})):
+        monkeypatch.delenv("RTHX_GRID_FINE", raising=False)
         for k, v in env.items():
             monkeypatch.setenv(k, v)
         tr = rthx_mod.DeviceTracer(flat, device=0)       # (the grid knob is read when the tables are built)
-        out[tag] = tr.trace(rpe, seed=17, locator=1, rec_ids=[1, 3])
+        out[tag] = tr.trace(rpe, seed=17, locator=1, rec_ids=[1, 3], **kw)
         tr.close()
     ref = oracle_mod.trace(flat, rpe, seed=17, rec_ids=[1, 3])
     total = rpe * flat.n_elements
-    for tag in ("lockstep", "queue80", "coarse_grid"):
+    for tag in ("lockstep", "coarse_grid"):
         # the same locator arithmetic on every path: identical integers except for points within rounding of a bucket-grid decision
         nd = int(np.abs(out["queue"]["counts"].astype(np.int64) - out[tag]["counts"].astype(np.int64)).sum() // 2)
         assert nd <= max(2, total // 500_000), (tag, nd)

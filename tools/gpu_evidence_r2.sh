@@ -8,15 +8,7 @@ set -x
 nvidia-smi --query-compute-apps=pid,used_memory --format=csv,noheader
 # (1) pipe issue-rate micro-benchmark (the "three half-rate pipes" model of DESIGN.md section 4)
 (cd tools/microbench && nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o pipe_mix pipe_mix.cu && ./pipe_mix) > $O/pipe_mix.txt 2>&1
-# (2) warp-aggregated tally (__match_any_sync) against one shared-memory reduction per ray: second library from the same sources
-CS=raytraceheattransfer.jl_b200/csrc
-nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC,-O2 -shared --fmad=true -DRTHX_TALLY_MATCH -I include -I $CS \
-     -o $O/librthx_match.so $CS/rthx_api.cu $CS/rthx_kernels.cu $CS/rthx_smooth.cu $CS/rthx_solve.cu > $O/build_match.log 2>&1
-B3="python bench.py --steps 3 --warmup 2 --rays 1e9 --no-e2e --no-cpu-baseline --no-smoothing --no-extras"
-timeout 200 $B3 > $O/tally_red.json 2> $O/tally_red.err
-RTHX_LIBRARY=$PWD/$O/librthx_match.so timeout 200 $B3 > $O/tally_match.json 2> $O/tally_match.err
-rm -f $O/librthx_match.so
-# (3) launch list + full capture of the SQ kernel, full capture of the queue kernel (cfg5)
+# (2) launch list + full capture of the SQ kernel, full capture of the queue kernel (cfg5)
 BP="python bench.py --steps 2 --warmup 1 --rays 1e9 --no-e2e --no-cpu-baseline --no-extras"
 B5="python bench.py --workload cfg5 --steps 2 --warmup 1 --no-e2e --no-cpu-baseline --no-smoothing --no-extras"
 timeout 300 $BP > $O/plain3.json 2> $O/plain3.err && {
@@ -25,7 +17,7 @@ timeout 300 $BP > $O/plain3.json 2> $O/plain3.err && {
 }
 timeout 300 $B5 > $O/plain5.json 2> $O/plain5.err && \
   timeout 600 ncu --set full --clock-control none --import-source on -k regex:trace_exchange -s 2 -c 1 -f -o $O/prof_queue $B5 > $O/ncu_q.log 2>&1
-# (4) NVLink traffic of the fused row hand-over: one process, two GPUs, rows gathered on device 0 (rthx_trace_exchange_multi, counts_out = NULL)
+# (3) NVLink traffic of the fused row hand-over: one process, two GPUs, rows gathered on device 0 (rthx_trace_exchange_multi, counts_out = NULL)
 timeout 200 python tools/gpu_gather_probe.py > $O/gather_plain.log 2>&1 && \
   timeout 600 ncu --metrics nvltx__bytes.sum,nvlrx__bytes.sum,gpu__time_duration.sum,lts__t_sectors_srcunit_tex_aperture_peer_op_write.sum,lts__t_sectors_srcunit_tex_aperture_peer_op_red.sum --clock-control none -k regex:trace_exchange --csv --log-file $O/nvlink.csv python tools/gpu_gather_probe.py > $O/ncu_nv.log 2>&1
 ls -la $O

@@ -1,6 +1,6 @@
 #!/bin/bash
-# A/B sweep of the generic locator's knobs on one B200: bucket fineness (RTHX_GRID_FINE), bucket budget per face
-# (RTHX_GRID_PER_FACE) and resident blocks per SM (RTHX_GENERIC_MINB).  Prints rays/s per setting.
+# A/B sweep of the generic locator's knobs on one B200: bucket fineness (RTHX_GRID_FINE) and bucket budget per face
+# (RTHX_GRID_PER_FACE).  Prints rays/s per setting.
 O=${1:-gpurun_out/sweep}; mkdir -p $O
 run() {  # name workload env...
   local name=$1 w=$2; shift 2
@@ -14,10 +14,9 @@ except Exception as e:
 PY
 }
 for w in cfg3 cfg5; do
-  run ${w}_f8_m3 $w RTHX_GRID_FINE=8
-  run ${w}_f8_m4 $w RTHX_GRID_FINE=8 RTHX_GENERIC_MINB=4
-  run ${w}_f4_m3 $w RTHX_GRID_FINE=4
-  run ${w}_f6_m3 $w RTHX_GRID_FINE=6
-  run ${w}_f12_m3 $w RTHX_GRID_FINE=12 RTHX_GRID_PER_FACE=200
-  run ${w}_f16_m3 $w RTHX_GRID_FINE=16 RTHX_GRID_PER_FACE=320
+  run ${w}_f8 $w RTHX_GRID_FINE=8
+  run ${w}_f4 $w RTHX_GRID_FINE=4
+  run ${w}_f6 $w RTHX_GRID_FINE=6
+  run ${w}_f12 $w RTHX_GRID_FINE=12 RTHX_GRID_PER_FACE=200
+  run ${w}_f16 $w RTHX_GRID_FINE=16 RTHX_GRID_PER_FACE=320
 done
