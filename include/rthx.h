@@ -423,6 +423,26 @@ int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args* args, uint
 int rthx_trace_exchange_continue(rthx_handle* h, const rthx_trace_args* args, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* stats,
                                  rthx_sparse_stats* sparse_stats);
 
+/* Blocking trace of the emitter rows a caller names, and no others: what the surfaces-only crop of exchangeRayTracing.jl:9-11 keeps
+ * (emitters = 0..Ns-1 of a transparent enclosure, where the other Nv rows would be traced and thrown away), or the exchange factors
+ * of a few elements (one heater, one sensor).  Row y is element emitters[y]; its counts are those of the same row of a full
+ * rthx_trace_exchange with the same args, bit for bit (the RNG contract keys every ray by seed, ray id, emitter and band), and
+ * rays_per_emitter is that of the full trace (div(rays_total, N), not div(rays_total, R)).
+ *   emitters [n_emitters]: R = n_emitters >= 1 element indices, strictly ascending, in [0, N).  args as for rthx_trace_exchange (seed,
+ *       bins, mode incl. both MULTI_BOUNCE modes, locator, ray_id_offset, launch shape), except that emitter_rank / emitter_world must be
+ *       (0, 1) and rec_ids must be a subset of the list.  A violation is RTHX_ERR_ARG naming it, with nothing resident changed; a list
+ *       whose 8 R N n_bins bytes of counts do not fit in device memory is RTHX_ERR_NOMEM (split the list).
+ *   counts_out: [n_bins][R][N] uint64, row y = element emitters[y] (NULL: leave the R rows resident on the device);
+ *   lost_out:   [n_bins][N] uint64 (may be NULL), 0 for unlisted elements;  stats->rays_traced = rays_per_emitter * R * n_bins.
+ * Read-outs of the resident rows afterwards (each equal, bit for bit, to the same call after the full trace restricted to the listed rows):
+ *   rthx_counts_nnz / _csr : the R listed rows, as after a sharded trace;
+ *   rthx_counts_stats / _csc: the N x N matrix whose unlisted rows are empty (nnz and chi over the listed rows);
+ *   rthx_smooth_F / _DkAP / rthx_smooth_sparse (RTHX_SMOOTH_FROM_LAST_TRACE) with crop n: accepted when every row < n is listed, else
+ *       RTHX_ERR_ARG naming the first missing row.
+ * rthx_trace_exchange_continue after a resident rows trace continues the same list (the handle keeps it).                [0.3+] */
+int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* args, const int32_t* emitters, int32_t n_emitters,
+                             uint64_t* counts_out, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* stats);
+
 /* Peer-memory plumbing for the fused flush in one-process-per-GPU runs: rank 0 allocates the UInt64 count matrix
  * with rthx_shared_alloc and publishes the 64-byte CUDA IPC handle; every other rank maps it with rthx_shared_open
  * (peer access over NVLink is enabled lazily) and passes the mapped pointer as `counts_dev` to

@@ -90,6 +90,9 @@ def load_library():
     L.rthx_trace_exchange_continue.restype = C.c_int
     L.rthx_trace_exchange_continue.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_u64p, C.POINTER(rthx_rec_out), C.POINTER(rthx_stats),
                                                C.POINTER(rthx_sparse_stats)]
+    L.rthx_trace_exchange_rows.restype = C.c_int
+    L.rthx_trace_exchange_rows.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, C.c_int32, c_u64p, c_u64p,
+                                           C.POINTER(rthx_rec_out), C.POINTER(rthx_stats)]
     L.rthx_trace_exchange_device.restype = C.c_int
     L.rthx_trace_exchange_device.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int, C.POINTER(rthx_stats)]
@@ -306,8 +309,37 @@ class DeviceTracer:
                                                 lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                 C.byref(st)))
         self._last_shard = (int(args.emitter_rank), int(args.emitter_world))     # rows resident on the device: e = rank + y * world
+        self._last_rows = None
         self._record_resident(rays_per_emitter, kw, sparse=False)
         out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
+        if rec is not None:
+            out["origins"] = origins[: rec.n_recorded].copy()
+            out["endpoints"] = endpoints[: rec.n_recorded].copy()
+        return out
+
+    def trace_rows(self, emitters, rays_per_emitter: int, dense: bool = True, **kw):
+        """Blocking trace of the emitter rows `emitters` only (rthx_trace_exchange_rows): element indices, strictly ascending, in [0, N).
+        Row y of the result is element emitters[y], equal bit for bit to that row of `trace()` with the same keywords.  Returns the dict
+        of `trace()` with counts [nb, R, N] (None with dense=False: the R rows stay on the device for `counts_csr()` (R rows),
+        `counts_csc()` / `counts_stats()` (the N x N matrix whose other rows are empty), `smooth()` / `smooth_sparse()` with a crop n
+        whose rows are all listed, and `trace_continue()`); lost [nb, N] is 0 for unlisted elements."""
+        rows = np.ascontiguousarray(emitters, dtype=np.int32).ravel()
+        args, keep = make_trace_args(rays_per_emitter, **kw)
+        N, nb, R = self.n_elements, args.n_bins, len(rows)
+        if not dense:
+            counts = None
+        else:
+            counts = pinned_empty((nb, R, N), np.uint64) if nb * R * N > (1 << 16) else np.empty((nb, R, N), np.uint64)
+        lost = np.empty((nb, N), np.uint64)
+        st = rthx_stats()
+        rec, origins, endpoints = _recorder(kw.get("rec_ids"), rays_per_emitter)
+        self._check(self._L.rthx_trace_exchange_rows(self._h, C.byref(args), rows.ctypes.data_as(c_i32p), R,
+                                                     counts.ctypes.data_as(c_u64p) if counts is not None else None,
+                                                     lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None, C.byref(st)))
+        self._last_shard = (0, 1)
+        self._last_rows = rows.copy()
+        self._record_resident(rays_per_emitter, kw, sparse=False)
+        out = dict(counts=counts.reshape(nb, R, N) if counts is not None else None, lost=lost, stats=st.as_dict())
         if rec is not None:
             out["origins"] = origins[: rec.n_recorded].copy()
             out["endpoints"] = endpoints[: rec.n_recorded].copy()
@@ -326,6 +358,7 @@ class DeviceTracer:
         self._check(self._L.rthx_trace_exchange_sparse(self._h, C.byref(args), lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                        C.byref(st), C.byref(sst)))
         self._last_shard = (int(args.emitter_rank), int(args.emitter_world))
+        self._last_rows = None
         self._record_resident(rays_per_emitter, kw, sparse=True)
         out = dict(counts=None, lost=lost, stats=st.as_dict(), sparse_stats=sst.as_dict())
         if rec is not None:
@@ -378,12 +411,14 @@ class DeviceTracer:
     def counts_csr(self, bin: int = 0, values: bool = True, normalised: bool = True):
         """CSR read-out of the counts resident on the device (rthx_counts_nnz / rthx_counts_csr): returns
         (row_ptr [R+1] i64, cols [nnz] i32, counts [nnz] u64 or None, F_vals [nnz] f64 = count/row total or None); R = N after a
-        plain trace, the number of owned rows (elements rank + y * world) after a sharded one."""
+        plain trace, the number of owned rows (elements rank + y * world) after a sharded one, the listed rows after `trace_rows()`."""
         nnz = C.c_int64(0)
         self._check(self._L.rthx_counts_nnz(self._h, int(bin), C.byref(nnz)))
         N, k = self.n_elements, max(1, nnz.value)
         rank, world = getattr(self, "_last_shard", (0, 1))
         R = (N - rank + world - 1) // world          # after a sharded trace (a row tile) the view covers the rows e = rank + y * world
+        if getattr(self, "_last_rows", None) is not None:
+            R = len(self._last_rows)
         row_ptr = np.empty(R + 1, np.int64)
         cols = np.empty(k, np.int32)
         vals = np.empty(k, np.uint64) if values else None
@@ -583,6 +618,7 @@ def trace_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, counts_o
         msg = L.rthx_last_error(tracers[0]._h)
         raise RthxError(f"rthx_trace_exchange_multi failed ({rc}): {msg.decode() if msg else ''}")
     tracers[0]._last_shard = (0, 1)
+    tracers[0]._last_rows = None
     tracers[0]._record_resident(rays_per_emitter, kw, sparse=False)
     out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
     if rec is not None:
@@ -591,22 +627,25 @@ def trace_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, counts_o
     return out
 
 
-def merge_row_tiles(tiles, N: int, n_bins: int):
-    """Merge the CSR read-outs of interleaved row tiles (tile t holds the rows e = t (mod n_tiles), in order) into one CSR matrix per
-    traced bin.  tiles[t][k] = (row_ptr, cols, F_vals) of bin k.  Returns a list of (row_ptr [N+1], cols, F_vals)."""
+def merge_row_tiles(tiles, N: int, n_bins: int, tile_rows=None):
+    """Merge the CSR read-outs of interleaved row tiles (tile t holds the rows e = t (mod n_tiles), in order, or with `tile_rows` the
+    ascending elements tile_rows[t]; rows no tile holds stay empty) into one CSR matrix per traced bin.  tiles[t][k] = (row_ptr, cols,
+    F_vals) of bin k.  Returns a list of (row_ptr [N+1], cols, F_vals)."""
     n_tiles = len(tiles)
+    if tile_rows is None:
+        tile_rows = [np.arange(t, N, n_tiles) for t in range(n_tiles)]
     mats = []
     for k in range(n_bins):
         nnz_row = np.zeros(N, np.int64)
         for t in range(n_tiles):
-            nnz_row[t::n_tiles] = np.diff(tiles[t][k][0])
+            nnz_row[tile_rows[t]] = np.diff(tiles[t][k][0])
         row_ptr = np.zeros(N + 1, np.int64)
         np.cumsum(nnz_row, out=row_ptr[1:])
         cols = np.empty(int(row_ptr[-1]), np.int32)
         vals = np.empty(int(row_ptr[-1]), np.float64)
         for t in range(n_tiles):
             rp, c_t, f_t = tiles[t][k]
-            rows = np.arange(t, N, n_tiles)
+            rows = tile_rows[t]
             lens = np.diff(rp)
             # destination of every entry of the tile: start of its global row + offset inside the row
             dst = np.repeat(row_ptr[rows] - rp[:-1], lens) + np.arange(int(rp[-1]), dtype=np.int64)
@@ -692,6 +731,51 @@ def trace_sparse_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, r
     stats["rays_lost"] = sum(o["stats"]["rays_lost"] for o, _, _ in res)
     sparse_stats = {k: sum(o["sparse_stats"][k] for o, _, _ in res) for k in ("pairs", "nnz", "flushes", "row_groups")}
     result = dict(csr=merge_row_tiles([p for _, p, _ in res], N, nb), lost=lost, chi=chi, stats=stats, sparse_stats=sparse_stats)
+    if rec_ids:
+        result["origins"] = np.concatenate([o.get("origins", np.zeros((0, 2))) for o, _, _ in res], axis=0)
+        result["endpoints"] = np.concatenate([o.get("endpoints", np.zeros((0, 2))) for o, _, _ in res], axis=0)
+    return result
+
+
+def trace_rows_multi(tracers: Sequence[DeviceTracer], emitters, rays_per_emitter: int, refine: bool = False, **kw):
+    """The rows trace (DeviceTracer.trace_rows, counts left on the devices) of a list too large for one device, on several devices at
+    once: device r traces the r-th contiguous block of the list as its own rows trace (one host thread per handle), and only their
+    non-zeros come back; the host merges them into ONE row-normalised CSR matrix per traced bin over all N rows, unlisted rows empty
+    (merge_row_tiles).  F = count / row total is the F_raw of a single-device rows trace bit for bit.  Returns dict(csr=[(row_ptr, cols,
+    F_vals)] per bin, lost [nb, N], chi per bin, stats), plus origins / endpoints with rec_ids: the blocks ascend, so device 0's points
+    followed by device 1's ... are in ascending (emitter, ray) order, as a single-device trace records them.  refine=True continues the
+    rows left resident by the previous call (DeviceTracer.trace_continue)."""
+    from concurrent.futures import ThreadPoolExecutor
+    n = len(tracers)
+    N = tracers[0].n_elements
+    nb = len(kw.get("bins", (0,)))
+    rec_ids = kw.pop("rec_ids", None)
+    rows = np.ascontiguousarray(emitters, dtype=np.int32).ravel()
+    parts_rows = np.array_split(rows, n)
+
+    def run(r):
+        own = [e for e in (rec_ids or []) if e in set(parts_rows[r].tolist())]
+        if refine:
+            out = tracers[r].trace_continue(rays_per_emitter, rec_ids=own or None, **kw)
+        else:
+            out = tracers[r].trace_rows(parts_rows[r], rays_per_emitter, dense=False, rec_ids=own or None, **kw)
+        parts, chi = _tile_readout(tracers[r], nb, divide=True)
+        return out, parts, chi
+
+    live = [r for r in range(n) if len(parts_rows[r])]        # fewer rows than devices: the others stay idle
+    with ThreadPoolExecutor(max_workers=len(live)) as ex:
+        res = list(ex.map(run, live))
+    lost = np.zeros((nb, N), np.uint64)
+    chi = np.zeros(nb)
+    for out, _, c in res:
+        lost += out["lost"]
+        chi += c
+    stats = dict(res[0][0]["stats"])
+    stats["kernel_ms"] = max(o["stats"]["kernel_ms"] for o, _, _ in res)
+    stats["total_ms"] = max(o["stats"]["total_ms"] for o, _, _ in res)
+    stats["rays_traced"] = sum(o["stats"]["rays_traced"] for o, _, _ in res)
+    stats["rays_lost"] = sum(o["stats"]["rays_lost"] for o, _, _ in res)
+    result = dict(csr=merge_row_tiles([p for _, p, _ in res], N, nb, tile_rows=[parts_rows[r] for r in live]), lost=lost, chi=chi, stats=stats)
     if rec_ids:
         result["origins"] = np.concatenate([o.get("origins", np.zeros((0, 2))) for o, _, _ in res], axis=0)
         result["endpoints"] = np.concatenate([o.get("endpoints", np.zeros((0, 2))) for o, _, _ in res], axis=0)

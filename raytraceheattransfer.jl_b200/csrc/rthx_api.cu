@@ -38,6 +38,7 @@ struct DevRes {
   double* rec_pts_dev = nullptr;            size_t rec_pts_cap = 0;
   uint8_t* rec_valid_dev = nullptr;         size_t rec_valid_cap = 0;
   double* peak_dev = nullptr;
+  int32_t* rows_dev = nullptr;              size_t rows_cap = 0;       // emitter list of a rows trace (rthx_trace_exchange_rows)
   int* csr_nnz = nullptr;                   size_t csr_cap = 0;        // per-row nnz (int), row totals, row pointers
   unsigned long long* csr_rowsum = nullptr; long long* csr_rowptr = nullptr; unsigned long long* csr_cross = nullptr;
   unsigned int* row_done_dev = nullptr;     size_t row_done_cap = 0;   // fused peer flush: per-row hand-over tickets
@@ -94,6 +95,13 @@ struct rthx_handle : DevRes {
   int last_trace_bins = 0; size_t last_trace_rows = 0;    // resident counts: bins, rows per bin (N, or the rows of a shard)
   int last_rank = 0, last_world = 1;                      // ... row y of the resident matrix is element last_rank + y * last_world
   bool sparse_counts = false;                             // the resident counts are the hashed tally's (sk_*), not counts_dev
+  // Rows trace: `rows` (also in rows_dev) is the emitter list of the trace in progress when rows_active, and of the resident counts when
+  // res_rows (row y of the resident matrix is then element rows[y]; last_rank / last_world are 0 / 1).  row_runs cuts it into
+  // arithmetic runs {first row y0, rows, element of y0, stride}: each run is launched as a shard (emitter_rank + y * emitter_world),
+  // so the trace kernels map rows to emitters exactly as for every other trace.
+  std::vector<int32_t> rows;
+  std::vector<int4> row_runs;
+  bool rows_active = false, res_rows = false;
   long long sk_nnz = 0;                                   // ... its non-zeros over all traced bins
   // The one trace (of the contiguous ray-id range [ray_lo, ray_hi)) the resident counts are those of; rthx_trace_exchange_continue
   // extends it.  Valid while last_trace_bins > 0.
@@ -129,7 +137,7 @@ void devres_free(DevRes& r) {
   cudaFree(r.sk_pairs); cudaFree(r.sk_ctl); cudaFree(r.sk_tmp); cudaFree(r.sk_keys); cudaFree(r.sk_vals); cudaFree(r.sk_rowptr);
   cudaFree(r.sp_ptr); cudaFree(r.sp_rowval); cudaFree(r.sp_val); cudaFree(r.sp_keys); cudaFree(r.sp_xcol); cudaFree(r.sp_xval); cudaFree(r.sp_vec); cudaFree(r.sp_tmp);
   cudaFree(r.csr_nnz); cudaFree(r.csr_rowsum); cudaFree(r.csr_rowptr); cudaFree(r.csr_out); cudaFree(r.csr_cross); cudaFree(r.csc_partial); cudaFree(r.csc_colptr); cudaFree(r.row_done_dev);
-  cudaFree(r.arena); cudaFree(r.generic_arena); cudaFree(r.counts_dev); cudaFree(r.rec_pts_dev); cudaFree(r.rec_valid_dev); cudaFree(r.peak_dev);
+  cudaFree(r.arena); cudaFree(r.generic_arena); cudaFree(r.counts_dev); cudaFree(r.rec_pts_dev); cudaFree(r.rec_valid_dev); cudaFree(r.peak_dev); cudaFree(r.rows_dev);
   for (auto& e : r.ev) if (e) cudaEventDestroy(e);
   for (auto& e : r.bev) if (e) cudaEventDestroy(e);
   for (auto& e : r.cev) if (e) cudaEventDestroy(e);
@@ -984,10 +992,21 @@ int check_continue(rthx_handle* h, const rthx_trace_args* a) {
   return RTHX_OK;
 }
 
+// Thread blocks per row for a launch over `rows` (emitter, band) rows: enough blocks for ~32 waves of the resident set, but keep >= 2048
+// rays (and >= N/2, the flush scan) per block
+long long auto_row_chunks(const rthx_handle* h, const LaunchPlan& pl, const rthx_trace_args* a, long long rows) {
+  const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.kernel, pl.block_threads, pl.smem_bytes));
+  const long long target = (long long)h->prop.multiProcessorCount * per_sm * 32;
+  long long chunks = rows > 0 ? (target + rows - 1) / rows : 1;
+  const long long min_rays = std::max<long long>(2048, h->N / 2);
+  const long long max_chunks = std::max<long long>(1, a->rays_per_emitter / min_rays);
+  return std::max<long long>(1, std::min(chunks, max_chunks));
+}
+
 // hash_slots > 0: the hashed row tally (no histogram; the table takes hash_table_bytes(hash_slots))
 LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, int world, int hash_slots = 0) {
   LaunchPlan pl{};
-  pl.n_owned = (h->N - rank + world - 1) / world;
+  pl.n_owned = h->rows_active ? (int)h->rows.size() : (h->N - rank + world - 1) / world;
   if (pl.n_owned < 0) pl.n_owned = 0;
   pl.block_threads = a->block_threads ? a->block_threads : 256;
   const bool analytic = a->locator != RTHX_LOCATOR_GENERIC;
@@ -1028,15 +1047,7 @@ LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, i
   }
   const long long rows = (long long)pl.n_owned * a->n_bins;
   long long chunks = a->row_chunks;
-  if (chunks <= 0) {
-    // enough blocks for ~32 waves of the resident set, but keep >= 2048 rays (and >= N/2, the flush scan) per block
-    const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.kernel, pl.block_threads, pl.smem_bytes));
-    const long long target = (long long)h->prop.multiProcessorCount * per_sm * 32;
-    chunks = rows > 0 ? (target + rows - 1) / rows : 1;
-    const long long min_rays = std::max<long long>(2048, h->N / 2);
-    const long long max_chunks = std::max<long long>(1, a->rays_per_emitter / min_rays);
-    chunks = std::max<long long>(1, std::min(chunks, max_chunks));
-  }
+  if (chunks <= 0) chunks = auto_row_chunks(h, pl, a, rows);
   // A block's rays are counted in 32 bits (u32 row histogram, u32 loop counter advancing by blockDim.x): at most 2^31 rays per
   // block.  Auto-chosen chunk counts are raised to satisfy that; a plan that then exceeds the 1-D grid limit — or a caller-supplied
   // row_chunks that violates either bound — is rejected (n_blocks = -1 -> RTHX_ERR_ARG), never silently wrapped.
@@ -1180,10 +1191,26 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
   }
   if (with_rec && n_rec_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
   if (y1 < 0) y1 = pl.n_owned;
-  P.y_offset = y0;
-  const long long nb = (long long)(y1 - y0) * a->n_bins * pl.row_chunks;
-  CU(h, launch_trace_exchange(P, pl.kernel, (int)nb, pl.block_threads, pl.smem_bytes, stream));
-  if (nb > 0) *n_launches += 1;
+  if (!h->rows_active) {
+    P.y_offset = y0;
+    const long long nb = (long long)(y1 - y0) * a->n_bins * pl.row_chunks;
+    CU(h, launch_trace_exchange(P, pl.kernel, (int)nb, pl.block_threads, pl.smem_bytes, stream));
+    if (nb > 0) *n_launches += 1;
+  } else {
+    // one launch per run of the emitter list that meets [y0, y1): rows y of run {r0, n, e0, s} are elements e0 + (y - r0) s.  The launches
+    // of one stream run one after another, so with automatic chunking each is cut into enough blocks to fill the device on its own (the
+    // plan's row_chunks fills it with all R rows at once); counts do not depend on the launch shape.
+    for (const int4& run : h->row_runs) {
+      const int r0 = std::max(y0, run.x), r1 = std::min(y1, run.x + run.y);
+      if (r1 <= r0) continue;
+      const long long rows = (long long)(r1 - r0) * a->n_bins;
+      P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, a, rows));
+      P.emitter_world = run.w; P.emitter_rank = run.z - run.x * run.w;
+      P.y_offset = r0;
+      CU(h, launch_trace_exchange(P, pl.kernel, (int)(rows * P.row_chunks), pl.block_threads, pl.smem_bytes, stream));
+      *n_launches += 1;
+    }
+  }
   *plan_out = pl;
   return RTHX_OK;
 }
@@ -1208,13 +1235,13 @@ void batch_rows_of(int n_owned, int n_batches, int b, int& y0, int& y1) {
 int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, int rank, int world, bool with_rec, int n_slots,
                     LaunchPlan* plan_out, int* n_launches, int* n_batches_out) {
   const int N = h->N;
-  const int n_owned = (N - rank + world - 1) / world;
+  LaunchPlan pl = make_plan(h, a, rank, world);
+  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
+  const int n_owned = pl.n_owned;
   // counts_dev is about to be overwritten: whatever view an earlier trace left behind (resident bins, CSR row pointers) is void
   // until the caller re-validates it (rthx_trace_exchange does, for a complete single-device trace)
   h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false;
   CU(h, ensure(&h->counts_dev, &h->counts_cap, (size_t)a->n_bins * (size_t)n_owned * N));
-  LaunchPlan pl = make_plan(h, a, rank, world);
-  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
   // batches: >= ~2 waves of resident blocks each, at most 16 (consecutive batches alternate between two streams, so a batch's
   // draining tail overlaps the next one's head; cfg3 at 1e10 rays: 16 batches, the copy behind the last kernel is 17 MB and the
   // call ends 0.5 ms after the kernel — with 5 even batches it was 180 MB and 3.6 ms)
@@ -1267,9 +1294,9 @@ void parallel_memcpy(void* dst, const void* src, size_t bytes) {
 //   pageable destination (e.g. a Julia Array): DMA into two pinned staging buffers, the host thread moves batch b-1 to
 //       the caller's memory while batch b is in flight (a pageable cudaMemcpyAsync would block the host per batch and
 //       crawl at ~4 GB/s).
-int pipeline_copy(rthx_handle* h, const rthx_trace_args* a, int rank, int world, uint64_t* counts_out, int n_batches) {
+// With world == 1 the host matrix is [n_bins][n_owned][N]: n_owned = N for a plain trace, the R listed rows for a rows trace.
+int pipeline_copy(rthx_handle* h, const rthx_trace_args* a, int rank, int world, int n_owned, uint64_t* counts_out, int n_batches) {
   const int N = h->N;
-  const int n_owned = (N - rank + world - 1) / world;
   cudaPointerAttributes pa;
   bool pinned = cudaPointerGetAttributes(&pa, counts_out) == cudaSuccess && (pa.type == cudaMemoryTypeHost || pa.type == cudaMemoryTypeManaged);
   cudaGetLastError();
@@ -1282,7 +1309,7 @@ int pipeline_copy(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
       for (int bin = 0; bin < a->n_bins && y1 > y0; ++bin) {
         const unsigned long long* src = h->counts_dev + ((size_t)bin * n_owned + y0) * N;
         if (world == 1)
-          CU(h, cudaMemcpyAsync(counts_out + ((size_t)bin * N + y0) * N, src, row_bytes * (size_t)(y1 - y0), cudaMemcpyDeviceToHost, h->copy_stream));
+          CU(h, cudaMemcpyAsync(counts_out + ((size_t)bin * n_owned + y0) * N, src, row_bytes * (size_t)(y1 - y0), cudaMemcpyDeviceToHost, h->copy_stream));
         else
           CU(h, cudaMemcpy2DAsync(counts_out + ((size_t)bin * N + rank + (size_t)y0 * world) * N, row_bytes * world, src, row_bytes, row_bytes,
                                   (size_t)(y1 - y0), cudaMemcpyDeviceToHost, h->copy_stream));
@@ -1307,7 +1334,7 @@ int pipeline_copy(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
     const char* st = (const char*)h->stage[b & 1];
     for (int bin = 0; bin < a->n_bins && rows; ++bin) {
       const char* src = st + (size_t)bin * rows * row_bytes;
-      if (world == 1) parallel_memcpy(counts_out + ((size_t)bin * N + y0) * N, src, rows * row_bytes);
+      if (world == 1) parallel_memcpy(counts_out + ((size_t)bin * n_owned + y0) * N, src, rows * row_bytes);
       else
         for (size_t r = 0; r < rows; ++r) std::memcpy(counts_out + ((size_t)bin * N + rank + (size_t)(y0 + r) * world) * N, src + r * row_bytes, row_bytes);
     }
@@ -1366,16 +1393,12 @@ int collect_recorder(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec
   return RTHX_OK;
 }
 
-}  // namespace
-
-extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uint64_t* counts_out, uint64_t* lost_out,
-                                   rthx_rec_out* rec, rthx_stats* st) {
-  if (!h) return RTHX_ERR_ARG;
-  int rc = check_args(h, a);
-  if (rc) return rc;
+// Blocking host-output trace of the owned rows: those of the shard in `a`, or with h->rows_active the rows of the list in h->rows
+int trace_host(rthx_handle* h, const rthx_trace_args* a, uint64_t* counts_out, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
   CU(h, cudaSetDevice(h->device));
   const int N = h->N;
   int n_slots = 0, n_launches = 0;
+  int rc;
   CU(h, cudaEventRecord(h->ev[0], h->stream));
   rc = prepare_recorder(h, a, rec, &n_slots, h->stream);
   if (rc) return rc;
@@ -1384,7 +1407,7 @@ extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uin
   rc = pipeline_launch(h, a, a->emitter_rank, a->emitter_world, rec != nullptr, n_slots, &pl, &n_launches, &n_batches);
   if (rc) return rc;
   if (counts_out) {
-    rc = pipeline_copy(h, a, a->emitter_rank, a->emitter_world, counts_out, n_batches);
+    rc = pipeline_copy(h, a, a->emitter_rank, a->emitter_world, pl.n_owned, counts_out, n_batches);
     if (rc) return rc;
   } else {
     CU(h, cudaStreamWaitEvent(h->copy_stream, h->ev[2], 0));
@@ -1392,6 +1415,7 @@ extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uin
   // the (compact) rows this call owns stay resident: all of them for a plain trace, those of a shard / row tile otherwise
   h->last_trace_bins = a->n_bins;
   h->last_trace_rows = (size_t)pl.n_owned; h->last_rank = a->emitter_rank; h->last_world = a->emitter_world;
+  h->res_rows = h->rows_active;
   h->csr_bin = -1; h->csc_bin = -1;
   record_resident(h, a, counts_out ? RESIDENT_HOST : RESIDENT_DENSE);
   std::vector<uint64_t> lost_host((size_t)a->n_bins * N);
@@ -1413,6 +1437,86 @@ extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uin
     st->n_launches = n_launches;
   }
   return RTHX_OK;
+}
+
+// Marks the trace kernels' owned rows as those of the emitter list in h->rows for the duration of one call
+struct RowsScope {
+  rthx_handle* h;
+  RowsScope(rthx_handle* h_, bool on) : h(h_) { h->rows_active = on; }
+  ~RowsScope() { h->rows_active = false; }
+};
+
+// Maximal arithmetic runs {first row, rows, first element, stride} of an ascending emitter list, taken greedily from the front.  A run
+// keeps (first row + rows) * stride below 2^31, so that the kernels' int arithmetic emitter_rank + y * emitter_world cannot overflow.
+std::vector<int4> list_runs(const std::vector<int32_t>& rows) {
+  std::vector<int4> runs;
+  const int R = (int)rows.size();
+  for (int k = 0; k < R;) {
+    int n = 1, s = 1;
+    if (k + 1 < R) {
+      s = rows[k + 1] - rows[k];
+      while (k + n < R && rows[k + n] - rows[k + n - 1] == s && (long long)(k + n + 1) * s <= 0x7FFFFFFFll) ++n;
+      if (n == 1) s = 1;
+    }
+    runs.push_back(make_int4(k, n, rows[k], s));
+    k += n;
+  }
+  return runs;
+}
+
+// Checks of rthx_trace_exchange_rows that must pass before anything resident changes
+int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n) {
+  if (!emitters || n < 1) return fail(h, RTHX_ERR_ARG, "trace_rows: the emitter list is empty (n_emitters must be >= 1)");
+  for (int32_t i = 0; i < n; ++i) {
+    if (emitters[i] < 0 || emitters[i] >= h->N)
+      return fail(h, RTHX_ERR_ARG, "trace_rows: emitters[" + std::to_string(i) + "] = " + std::to_string(emitters[i]) + " is outside [0, N = " +
+                                       std::to_string(h->N) + ")");
+    if (i > 0 && emitters[i] <= emitters[i - 1])
+      return fail(h, RTHX_ERR_ARG, "trace_rows: emitters must be strictly ascending (emitters[" + std::to_string(i) + "] = " + std::to_string(emitters[i]) +
+                                       " follows " + std::to_string(emitters[i - 1]) + ")");
+  }
+  if (a->emitter_rank != 0 || a->emitter_world != 1)
+    return fail(h, RTHX_ERR_ARG, "trace_rows: emitter_rank / emitter_world must be (0, 1) with an emitter list");
+  for (int32_t k = 0; k < a->n_rec_ids; ++k)
+    if (!std::binary_search(emitters, emitters + n, a->rec_ids[k]))
+      return fail(h, RTHX_ERR_ARG, "trace_rows: rec_ids[" + std::to_string(k) + "] = " + std::to_string(a->rec_ids[k]) + " is not in the emitter list");
+  const size_t need = (size_t)n * (size_t)h->N * (size_t)a->n_bins;
+  if (need > h->counts_cap) {
+    size_t free_b = 0, total_b = 0;
+    CU(h, cudaMemGetInfo(&free_b, &total_b));
+    if ((need - h->counts_cap) * sizeof(unsigned long long) > free_b)
+      return fail(h, RTHX_ERR_NOMEM, "trace_rows: the counts of " + std::to_string(n) + " rows x " + std::to_string(h->N) + " columns x " + std::to_string(a->n_bins) +
+                                         " bins (" + std::to_string(need * 8) + " bytes) do not fit in device memory; split the emitter list");
+  }
+  return RTHX_OK;
+}
+
+}  // namespace
+
+extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uint64_t* counts_out, uint64_t* lost_out,
+                                   rthx_rec_out* rec, rthx_stats* st) {
+  if (!h) return RTHX_ERR_ARG;
+  const int rc = check_args(h, a);
+  if (rc) return rc;
+  return trace_host(h, a, counts_out, lost_out, rec, st);
+}
+
+extern "C" int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n_emitters,
+                                        uint64_t* counts_out, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
+  if (!h) return RTHX_ERR_ARG;
+  int rc = check_args(h, a);
+  if (rc) return rc;
+  CU(h, cudaSetDevice(h->device));
+  rc = check_rows(h, a, emitters, n_emitters);
+  if (rc) return rc;
+  // the resident counts are replaced from here on
+  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->res_rows = false;
+  h->rows.assign(emitters, emitters + n_emitters);
+  h->row_runs = list_runs(h->rows);
+  CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)n_emitters));
+  CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)n_emitters, cudaMemcpyHostToDevice, h->stream));
+  RowsScope scope(h, true);
+  return trace_host(h, a, counts_out, lost_out, rec, st);
 }
 
 extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args* a, void* counts_dev, void* lost_dev, void* stream,
@@ -1604,7 +1708,7 @@ int sparse_finish(rthx_handle* h, const rthx_trace_args* a, const SparseRun& R, 
   h->sparse_counts = true; h->sk_nnz = R.total;
   h->last_trace_bins = nb; h->last_trace_rows = (size_t)R.pl.n_owned; h->last_rank = a->emitter_rank; h->last_world = a->emitter_world;
   if (lost_before) h->ray_hi += a->rays_per_emitter;
-  else record_resident(h, a, RESIDENT_SPARSE);
+  else { record_resident(h, a, RESIDENT_SPARSE); h->res_rows = false; }
   if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
   int rc = collect_recorder(h, a, rec, R.n_slots, h->stream, false);
   if (rc) return rc;
@@ -1752,6 +1856,12 @@ extern "C" int rthx_trace_exchange_continue(rthx_handle* h, const rthx_trace_arg
   CU(h, cudaSetDevice(h->device));
   if (h->sparse_counts) return continue_sparse(h, a, lost_out, rec, st, sst);
   if (sst) std::memset(sst, 0, sizeof(*sst));
+  if (h->res_rows)                  // a rows trace continues its own list (on the device since that trace)
+    for (int32_t k = 0; k < a->n_rec_ids; ++k)
+      if (!std::binary_search(h->rows.begin(), h->rows.end(), a->rec_ids[k]))
+        return fail(h, RTHX_ERR_ARG, "trace_continue: rec_ids[" + std::to_string(k) + "] = " + std::to_string(a->rec_ids[k]) +
+                                         " is not in the emitter list of the resident rows trace");
+  RowsScope scope(h, h->res_rows);
   return continue_dense(h, a, lost_out, rec, st);
 }
 
@@ -1863,7 +1973,7 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
       } else {
         r = pipeline_launch(h, a, i, n, rec != nullptr, J.slots, &J.plan, &J.launches, &J.batches);
         if (r) return r;
-        r = pipeline_copy(h, a, i, n, counts_out, J.batches);
+        r = pipeline_copy(h, a, i, n, J.plan.n_owned, counts_out, J.batches);
         if (r) return r;
         J.lost.resize(lost_n);
         CU(h, cudaMemcpyAsync(J.lost.data(), h->lost_dev, sizeof(uint64_t) * lost_n, cudaMemcpyDeviceToHost, h->copy_stream));
@@ -1896,7 +2006,7 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
   if (gather) {
     CU(h0, cudaSetDevice(h0->device));
     CU(h0, cudaMemcpy(lost_sum.data(), h0->lost_dev, sizeof(uint64_t) * lost_n, cudaMemcpyDeviceToHost));
-    h0->last_trace_bins = a->n_bins; h0->last_trace_rows = (size_t)N; h0->last_rank = 0; h0->last_world = 1;
+    h0->last_trace_bins = a->n_bins; h0->last_trace_rows = (size_t)N; h0->last_rank = 0; h0->last_world = 1; h0->res_rows = false;
     record_resident(h0, a, RESIDENT_MULTI);
   } else {
     for (int i = 0; i < n; ++i)
@@ -2068,13 +2178,14 @@ extern "C" int rthx_flag_wait(const void* flags, int n, uint64_t value, double t
 // sparse read-out of the resident counts
 // ---------------------------------------------------------------------------------------------------------------
 namespace rthx {
-cudaError_t launch_row_nnz(const unsigned long long* c, int n_rows, int n_cols, size_t ld, int n_surf, int row_first, int row_stride, int* nnz,
-                           unsigned long long* rowsum, unsigned long long* cross, cudaStream_t st);
+cudaError_t launch_row_nnz(const unsigned long long* c, int n_rows, int n_cols, size_t ld, int n_surf, int row_first, int row_stride, const int* rows,
+                           int* nnz, unsigned long long* rowsum, unsigned long long* cross, cudaStream_t st);
 cudaError_t launch_row_fill(const unsigned long long* c, int n_rows, int n_cols, size_t ld, const long long* row_ptr, const unsigned long long* rowsum, int* cols,
                             unsigned long long* vals, double* fvals, cudaStream_t st);
-cudaError_t launch_csc_count(const unsigned long long* c, int n, size_t ld, int* partial, long long* colptr, cudaStream_t st);
-cudaError_t launch_csc_fill(const unsigned long long* c, int n, size_t ld, const int* partial, const long long* colptr, const unsigned long long* rowsum,
-                            int index_base, void* rowval, bool rowval_i64, unsigned long long* vals, double* fvals, cudaStream_t st);
+cudaError_t launch_csc_count(const unsigned long long* c, int n_rows, int n, size_t ld, int* partial, long long* colptr, cudaStream_t st);
+cudaError_t launch_csc_fill(const unsigned long long* c, int n_rows, int n, size_t ld, const int* rows, const int* partial, const long long* colptr,
+                            const unsigned long long* rowsum, int index_base, void* rowval, bool rowval_i64, unsigned long long* vals, double* fvals,
+                            cudaStream_t st);
 cudaError_t launch_add_base(long long* p, int n, long long base, cudaStream_t st);
 }  // namespace rthx
 
@@ -2217,7 +2328,8 @@ int prepare_rows(rthx_handle* h, int bin) {
                                 h->csr_rowsum, h->csr_cross, h->stream));
   } else {
     const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
-    CU(h, rthx::launch_row_nnz(c, R, N, (size_t)N, h->ns, h->last_rank, h->last_world, h->csr_nnz, h->csr_rowsum, h->csr_cross, h->stream));
+    CU(h, rthx::launch_row_nnz(c, R, N, (size_t)N, h->ns, h->last_rank, h->last_world, h->res_rows ? h->rows_dev : nullptr, h->csr_nnz, h->csr_rowsum,
+                               h->csr_cross, h->stream));
   }
   std::vector<int> nnz(std::max(R, 1));
   std::vector<unsigned long long> rowsum(std::max(R, 1)), cross(std::max(R, 1));
@@ -2363,7 +2475,7 @@ extern "C" int rthx_counts_csr(rthx_handle* h, int bin, int64_t* row_ptr, int32_
 
 extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, uint64_t* vals, double* F_vals) {
   if (!h || !colptr || !rowval || (index_base != 0 && index_base != 1)) return RTHX_ERR_ARG;
-  if (h->last_trace_bins > 0 && (h->last_world != 1 || (int)h->last_trace_rows != h->N))
+  if (h->last_trace_bins > 0 && !h->res_rows && (h->last_world != 1 || (int)h->last_trace_rows != h->N))
     return fail(h, RTHX_ERR_ARG, "counts_csc: the resident counts are the rows of a shard (emitter_world > 1); the column view needs the whole matrix");
   int rc = prepare_rows(h, bin);              // row totals for the normalisation, nnz for the buffer sizes
   if (rc) return rc;
@@ -2372,8 +2484,9 @@ extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowv
   const size_t nnz = (size_t)h->csr_total, nz1 = std::max<size_t>(1, nnz);
   if (!rowval_is_i64 && (size_t)N + (size_t)index_base > 0x7FFFFFFFull) return fail(h, RTHX_ERR_ARG, "counts_csc: 32-bit row indices overflow");
   if (h->sparse_counts) { rc = counts_csc_sparse(h, bin, index_base, rowval_is_i64, colptr, rowval, vals, F_vals); if (rc) return rc; h->csc_bin = bin; return RTHX_OK; }
-  const int n_tiles = (N + 63) / 64;
-  CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)n_tiles * (size_t)N));
+  const int R = (int)h->last_trace_rows;                      // N, or the listed rows of a rows trace (the other rows are empty)
+  const int n_tiles = (R + 63) / 64;
+  CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)std::max(n_tiles, 1) * (size_t)N));
   CU(h, ensure(&h->csc_colptr, &h->csc_colptr_cap, (size_t)N + 1));
   const size_t need = nz1 * (sizeof(long long) + (vals ? sizeof(unsigned long long) : 0) + (F_vals ? sizeof(double) : 0));
   if (h->csr_out_cap < need) {
@@ -2385,8 +2498,9 @@ extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowv
   unsigned long long* d_vals = vals ? (unsigned long long*)(d_rows + nz1) : nullptr;
   double* d_f = F_vals ? (double*)(d_rows + nz1 + (vals ? nz1 : 0)) : nullptr;
   const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
-  CU(h, rthx::launch_csc_count(c, N, (size_t)N, h->csc_partial, h->csc_colptr, h->stream));
-  CU(h, rthx::launch_csc_fill(c, N, (size_t)N, h->csc_partial, h->csc_colptr, h->csr_rowsum, index_base, d_rows, rowval_is_i64 != 0, d_vals, d_f, h->stream));
+  CU(h, rthx::launch_csc_count(c, R, N, (size_t)N, h->csc_partial, h->csc_colptr, h->stream));
+  CU(h, rthx::launch_csc_fill(c, R, N, (size_t)N, h->res_rows ? h->rows_dev : nullptr, h->csc_partial, h->csc_colptr, h->csr_rowsum, index_base, d_rows,
+                              rowval_is_i64 != 0, d_vals, d_f, h->stream));
   if (index_base) CU(h, rthx::launch_add_base(h->csc_colptr, N + 1, (long long)index_base, h->stream));
   if ((rc = copy_out(h, colptr, h->csc_colptr, sizeof(long long) * ((size_t)N + 1), h->stream))) return rc;
   if (nnz) {
@@ -2414,6 +2528,19 @@ cudaError_t run_dykstra(const unsigned long long* src_counts, const double* src_
 cudaError_t time_scale_pass(double* X, double* u, double* r, int n, size_t ldx, int reps, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, double* ms_per_pass);
 }  // namespace rthx
 
+namespace {
+// After a rows trace the crop n of a FROM_LAST_TRACE smoothing must be traced in full: rows 0..n-1 listed, so that resident row y < n is
+// element y and the leading n x n block lies where it lies after a full trace
+int check_crop_rows(rthx_handle* h, int n, const char* who) {
+  if (!h->res_rows) return RTHX_OK;
+  for (int y = 0; y < n; ++y)
+    if (y >= (int)h->rows.size() || h->rows[y] != y)
+      return fail(h, RTHX_ERR_ARG, std::string(who) + ": row " + std::to_string(y) + " of the crop n = " + std::to_string(n) +
+                                       " was not traced (it is not in the emitter list of the resident rows trace)");
+  return RTHX_OK;
+}
+}  // namespace
+
 extern "C" int rthx_smooth_F(rthx_handle* h, int source, const void* src_host, int bin, int n, const double* w, int max_iters, double target,
                              int measure_pass, double* F_out, rthx_smooth_stats* st) {
   return rthx_smooth_DkAP(h, source, src_host, bin, n, w, 0, max_iters, target, measure_pass, F_out, st);
@@ -2431,8 +2558,10 @@ extern "C" int rthx_smooth_DkAP(rthx_handle* h, int source, const void* src_host
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
     if (h->sparse_counts)
       return fail(h, RTHX_ERR_ARG, "smooth: the resident counts are the sparse form of rthx_trace_exchange_sparse (smooth them with rthx_smooth_sparse)");
-    if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev || n > h->N || h->last_world != 1 || (int)h->last_trace_rows != h->N)
+    if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev || n > h->N || (!h->res_rows && (h->last_world != 1 || (int)h->last_trace_rows != h->N)))
       return fail(h, RTHX_ERR_ARG, "smooth: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
+    const int rc = check_crop_rows(h, n, "smooth");
+    if (rc) return rc;
     src_counts = h->counts_dev + (size_t)bin * h->last_trace_rows * h->N;
     ld = (size_t)h->N;
   } else if (source == RTHX_SMOOTH_FROM_COUNTS || source == RTHX_SMOOTH_FROM_F) {
@@ -2513,8 +2642,11 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
   if (n < 1 || !w || !nnz_out || max_iters < 0) return fail(h, RTHX_ERR_ARG, "smooth_sparse: bad argument");
   long long nnz_f = 0;
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
-    if (bin < 0 || bin >= h->last_trace_bins || (!h->counts_dev && !h->sparse_counts) || n > h->N || h->last_world != 1 || (int)h->last_trace_rows != h->N)
+    if (bin < 0 || bin >= h->last_trace_bins || (!h->counts_dev && !h->sparse_counts) || n > h->N ||
+        (!h->res_rows && (h->last_world != 1 || (int)h->last_trace_rows != h->N)))
       return fail(h, RTHX_ERR_ARG, "smooth_sparse: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
+    const int rc = check_crop_rows(h, n, "smooth_sparse");
+    if (rc) return rc;
   } else if (source == RTHX_SMOOTH_FROM_CSC) {
     // the whole matrix is checked here, before anything is uploaded: a bad index must never reach a kernel
     if (!colptr) return fail(h, RTHX_ERR_ARG, "smooth_sparse: colptr is NULL");
@@ -2556,14 +2688,14 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
     unsigned long long* rowsum = reinterpret_cast<unsigned long long*>(vec + n);   // u and u' are free until the iteration
     int* row_nnz = reinterpret_cast<int*>(vec + 2 * (size_t)n);
     CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)((n + 63) / 64) * (size_t)n));
-    CU(h, rthx::launch_row_nnz(c, n, n, ld, h->ns, 0, 1, row_nnz, rowsum, nullptr, h->stream));
-    CU(h, rthx::launch_csc_count(c, n, ld, h->csc_partial, cp, h->stream));
+    CU(h, rthx::launch_row_nnz(c, n, n, ld, h->ns, 0, 1, nullptr, row_nnz, rowsum, nullptr, h->stream));
+    CU(h, rthx::launch_csc_count(c, n, n, ld, h->csc_partial, cp, h->stream));
     CU(h, cudaMemcpyAsync(&nnz_f, cp + n, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
     CU(h, cudaStreamSynchronize(h->stream));
     if (nnz_f > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "smooth_sparse: more than 2^31 - 1 non-zeros");
     CU(h, ensure(&h->sp_rowval, &h->sp_rowval_cap, (size_t)std::max<long long>(nnz_f, 1)));
     CU(h, ensure(&h->sp_val, &h->sp_val_cap, 2 * (size_t)std::max<long long>(nnz_f, 1)));
-    CU(h, rthx::launch_csc_fill(c, n, ld, h->csc_partial, cp, rowsum, 0, h->sp_rowval, false, nullptr, h->sp_val, h->stream));
+    CU(h, rthx::launch_csc_fill(c, n, n, ld, nullptr, h->csc_partial, cp, rowsum, 0, h->sp_rowval, false, nullptr, h->sp_val, h->stream));
   } else {
     CU(h, ensure(&h->sp_rowval, &h->sp_rowval_cap, (size_t)std::max<long long>(nnz_f, 1)));
     CU(h, ensure(&h->sp_val, &h->sp_val_cap, 2 * (size_t)std::max<long long>(nnz_f, 1)));

@@ -157,15 +157,16 @@ __global__ void __launch_bounds__(ROW_THREADS) recover_kernel(double* __restrict
 // ---------------------------------------------------------------------------------------------------------------
 // one warp per row: number of non-zero tallies, the row total and — for cross_coupling_chi (smoothExchangeFactors.jl:212-241) —
 // the tallies that couple a surface with a gas cell (exactly one of row / column index below n_surf).  The matrix may hold only
-// the rows of a shard (row y = element row_first + y * row_stride), n_rows x n_cols with leading dimension ld.
+// the rows of a shard (row y = element row_first + y * row_stride) or of a rows trace (row y = element rows[y]), n_rows x n_cols with
+// leading dimension ld.
 __global__ void __launch_bounds__(256) row_nnz_kernel(const unsigned long long* __restrict__ c, int n_rows, int n_cols, size_t ld, int n_surf, int row_first,
-                                                      int row_stride, int* __restrict__ nnz, unsigned long long* __restrict__ rowsum,
-                                                      unsigned long long* __restrict__ cross) {
+                                                      int row_stride, const int* __restrict__ rows, int* __restrict__ nnz,
+                                                      unsigned long long* __restrict__ rowsum, unsigned long long* __restrict__ cross) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= n_rows) return;
   int cnt = 0;
   unsigned long long s = 0, x = 0;
-  const bool row_surf = row_first + row * row_stride < n_surf;
+  const bool row_surf = (rows ? rows[row] : row_first + row * row_stride) < n_surf;
   for (int j = lane; j < n_cols; j += 32) {
     const unsigned long long v = c[(size_t)row * ld + j];
     cnt += v != 0; s += v;
@@ -199,9 +200,9 @@ __global__ void __launch_bounds__(256) row_fill_kernel(const unsigned long long*
   }
 }
 
-cudaError_t launch_row_nnz(const unsigned long long* c, int n_rows, int n_cols, size_t ld, int n_surf, int row_first, int row_stride, int* nnz,
-                           unsigned long long* rowsum, unsigned long long* cross, cudaStream_t st) {
-  if (n_rows > 0) row_nnz_kernel<<<(n_rows + 7) / 8, 256, 0, st>>>(c, n_rows, n_cols, ld, n_surf, row_first, row_stride, nnz, rowsum, cross);
+cudaError_t launch_row_nnz(const unsigned long long* c, int n_rows, int n_cols, size_t ld, int n_surf, int row_first, int row_stride, const int* rows,
+                           int* nnz, unsigned long long* rowsum, unsigned long long* cross, cudaStream_t st) {
+  if (n_rows > 0) row_nnz_kernel<<<(n_rows + 7) / 8, 256, 0, st>>>(c, n_rows, n_cols, ld, n_surf, row_first, row_stride, rows, nnz, rowsum, cross);
   return cudaGetLastError();
 }
 cudaError_t launch_row_fill(const unsigned long long* c, int n_rows, int n_cols, size_t ld, const long long* row_ptr, const unsigned long long* rowsum, int* cols,
@@ -215,14 +216,15 @@ cudaError_t launch_row_fill(const unsigned long long* c, int n_rows, int n_cols,
 // that the host neither transposes a CSR matrix nor runs sparse(I, J, V) over ~1e8 triplets (parallelRayTracing.jl:144-154 takes
 // seconds there for cfg3).  Rows are cut into tiles of CSC_TILE; thread (tile, column) counts, then writes, its own run of the
 // column, so both passes read the row-major matrix coalesced (consecutive threads = consecutive columns) and every column comes
-// out in ascending row order.
+// out in ascending row order.  The matrix may hold only the rows of a rows trace (n_rows x n columns, row i = element rows[i], rows
+// ascending): the column view is then that of the n x n matrix whose other rows are empty.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int CSC_TILE = 64;
 
-__global__ void __launch_bounds__(256) col_nnz_partial_kernel(const unsigned long long* __restrict__ c, int n, size_t ld, int* __restrict__ partial) {
+__global__ void __launch_bounds__(256) col_nnz_partial_kernel(const unsigned long long* __restrict__ c, int n_rows, int n, size_t ld, int* __restrict__ partial) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x, t = blockIdx.y;
   if (j >= n) return;
-  const int i0 = t * CSC_TILE, i1 = min(n, i0 + CSC_TILE);
+  const int i0 = t * CSC_TILE, i1 = min(n_rows, i0 + CSC_TILE);
   int cnt = 0;
   for (int i = i0; i < i1; ++i) cnt += c[(size_t)i * ld + j] != 0ull;
   partial[(size_t)t * n + j] = cnt;
@@ -260,17 +262,18 @@ __global__ void __launch_bounds__(1024) exclusive_scan_kernel(const long long* i
 }
 
 template <class IDX>
-__global__ void __launch_bounds__(256) col_fill_kernel(const unsigned long long* __restrict__ c, int n, size_t ld, const int* __restrict__ partial,
-                                                       const long long* __restrict__ colptr, const unsigned long long* __restrict__ rowsum, int index_base,
-                                                       IDX* __restrict__ rowval, unsigned long long* __restrict__ vals, double* __restrict__ fvals) {
+__global__ void __launch_bounds__(256) col_fill_kernel(const unsigned long long* __restrict__ c, int n_rows, int n, size_t ld, const int* __restrict__ rows,
+                                                       const int* __restrict__ partial, const long long* __restrict__ colptr,
+                                                       const unsigned long long* __restrict__ rowsum, int index_base, IDX* __restrict__ rowval,
+                                                       unsigned long long* __restrict__ vals, double* __restrict__ fvals) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x, t = blockIdx.y;
   if (j >= n) return;
-  const int i0 = t * CSC_TILE, i1 = min(n, i0 + CSC_TILE);
+  const int i0 = t * CSC_TILE, i1 = min(n_rows, i0 + CSC_TILE);
   long long k = colptr[j] + partial[(size_t)t * n + j];
   for (int i = i0; i < i1; ++i) {
     const unsigned long long v = c[(size_t)i * ld + j];
     if (v) {
-      rowval[k] = (IDX)(i + index_base);
+      rowval[k] = (IDX)((rows ? rows[i] : i) + index_base);
       if (vals) vals[k] = v;
       if (fvals) fvals[k] = (double)v / (double)rowsum[i];      // count / row total: parallelRayTracing.jl:144-146 + row_normalize! :161-169
       ++k;
@@ -278,21 +281,24 @@ __global__ void __launch_bounds__(256) col_fill_kernel(const unsigned long long*
   }
 }
 
-// column pointers of bin `c` (n x n, leading dimension ld) into colptr[0..n] (0-based, device); partial is [n_tiles][n] ints
-cudaError_t launch_csc_count(const unsigned long long* c, int n, size_t ld, int* partial, long long* colptr, cudaStream_t st) {
-  const int n_tiles = (n + CSC_TILE - 1) / CSC_TILE;
+// column pointers of bin `c` (n_rows x n, leading dimension ld) into colptr[0..n] (0-based, device); partial is [n_tiles][n] ints,
+// n_tiles = ceil(n_rows / 64)
+cudaError_t launch_csc_count(const unsigned long long* c, int n_rows, int n, size_t ld, int* partial, long long* colptr, cudaStream_t st) {
+  const int n_tiles = (n_rows + CSC_TILE - 1) / CSC_TILE;
   const dim3 grid((unsigned)((n + 255) / 256), (unsigned)n_tiles);
-  col_nnz_partial_kernel<<<grid, 256, 0, st>>>(c, n, ld, partial);
+  col_nnz_partial_kernel<<<grid, 256, 0, st>>>(c, n_rows, n, ld, partial);
   col_offsets_kernel<<<(n + 255) / 256, 256, 0, st>>>(partial, n, n_tiles, colptr);
   exclusive_scan_kernel<<<1, 1024, 0, st>>>(colptr, n, colptr);
   return cudaGetLastError();
 }
-cudaError_t launch_csc_fill(const unsigned long long* c, int n, size_t ld, const int* partial, const long long* colptr, const unsigned long long* rowsum,
-                            int index_base, void* rowval, bool rowval_i64, unsigned long long* vals, double* fvals, cudaStream_t st) {
-  const int n_tiles = (n + CSC_TILE - 1) / CSC_TILE;
+// rows (may be nullptr): element index of each of the n_rows rows
+cudaError_t launch_csc_fill(const unsigned long long* c, int n_rows, int n, size_t ld, const int* rows, const int* partial, const long long* colptr,
+                            const unsigned long long* rowsum, int index_base, void* rowval, bool rowval_i64, unsigned long long* vals, double* fvals,
+                            cudaStream_t st) {
+  const int n_tiles = (n_rows + CSC_TILE - 1) / CSC_TILE;
   const dim3 grid((unsigned)((n + 255) / 256), (unsigned)n_tiles);
-  if (rowval_i64) col_fill_kernel<long long><<<grid, 256, 0, st>>>(c, n, ld, partial, colptr, rowsum, index_base, (long long*)rowval, vals, fvals);
-  else col_fill_kernel<int><<<grid, 256, 0, st>>>(c, n, ld, partial, colptr, rowsum, index_base, (int*)rowval, vals, fvals);
+  if (rowval_i64) col_fill_kernel<long long><<<grid, 256, 0, st>>>(c, n_rows, n, ld, rows, partial, colptr, rowsum, index_base, (long long*)rowval, vals, fvals);
+  else col_fill_kernel<int><<<grid, 256, 0, st>>>(c, n_rows, n, ld, rows, partial, colptr, rowsum, index_base, (int*)rowval, vals, fvals);
   return cudaGetLastError();
 }
 // colptr += base (1-based pointers for Julia), in place

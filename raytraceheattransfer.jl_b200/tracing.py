@@ -104,12 +104,17 @@ def auto_row_tiles(n_elements: int, n_bins: int, budget_bytes: float = 48e9) -> 
     return max(1, int(np.ceil(8.0 * n_elements * n_elements * n_bins / budget_bytes)))
 
 
+def rows_fit_one_device(n_rows: int, n_elements: int, n_bins: int, budget_bytes: float = 48e9) -> bool:
+    """Whether the resident UInt64 counts of a rows trace (8 R N bytes per traced bin) stay within `budget_bytes` of one device."""
+    return 8.0 * n_rows * n_elements * n_bins <= budget_bytes
+
+
 def _same_flat(a, b) -> bool:
     keys = [k for k in a.__dict__ if k != "c"]
     return keys == [k for k in b.__dict__ if k != "c"] and all(np.array_equal(np.asarray(a.__dict__[k]), np.asarray(b.__dict__[k])) for k in keys)
 
 
-def _refine_state(rtm, seed, devices, locator, row_tiles, nudge):
+def _refine_state(rtm, seed, devices, locator, row_tiles, nudge, emitters=None):
     """The state of the previous call that `refine=True` continues; ValueError when it cannot be continued with these keywords."""
     state = getattr(rtm, "_trace_state", None)
     if state is None or not getattr(rtm, "_devices", None):
@@ -121,6 +126,9 @@ def _refine_state(rtm, seed, devices, locator, row_tiles, nudge):
     for name, given in (("seed", seed), ("devices", devices), ("locator", locator), ("row_tiles", row_tiles), ("nudge", nudge)):
         if given is not None and given != state[name]:
             raise ValueError(f"refine=True: {name}={given!r} differs from the previous call's {state[name]!r}")
+    prev = state.get("emitters")
+    if (emitters is None) != (prev is None) or (emitters is not None and not np.array_equal(emitters, prev)):
+        raise ValueError("refine=True: the traced emitter rows differ from the previous call's")
     if not _same_flat(flatten_domain(rtm), rtm._devices[0].flat):
         raise ValueError("refine=True: the domain changed since the previous call (its flattened mesh differs)")
     return state
@@ -129,9 +137,10 @@ def _refine_state(rtm, seed, devices, locator, row_tiles, nudge):
 def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectral_bins: Sequence[int],
                                verbose: bool, rec, seed: int, device: int = 0,
                                locator: int = RTHX_LOCATOR_AUTO, devices=None, row_tiles: Optional[int] = None,
-                               refine: bool = False) -> List[sp.csc_matrix]:
+                               refine: bool = False, emitters=None) -> List[sp.csc_matrix]:
     """Batched form of computeExchangeFactorsBin: traces every requested (1-based) bin in one launch per device.  refine=True adds
-    the rays to the counts the previous call left resident (parallelRayTracing checks that it can)."""
+    the rays to the counts the previous call left resident (parallelRayTracing checks that it can).  emitters (0-based, ascending):
+    trace only those rows; the other rows of every returned N x N matrix are empty."""
     import time
     if refine:
         state = rtm._trace_state
@@ -156,14 +165,29 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
         n_tiles = state["n_tiles"]
     else:
         n_tiles = auto_row_tiles(tr.n_elements, len(spectral_bins)) if row_tiles is None else int(row_tiles)
+    if emitters is not None:
+        n_tiles = 1                  # R x N counts: the rows of a surfaces-only trace fit where the N x N matrix would not
+    n_rows = len(emitters) if emitters is not None else tr.n_elements
     new_state = dict(seed=seed, devices=devs, locator=locator, row_tiles=row_tiles, nudge=nudge, n_tiles=n_tiles,
-                     dense_multi=n_tiles == 1 and len(trs) > 1, rays_per_emitter_total=rpe_total)
+                     dense_multi=n_tiles == 1 and len(trs) > 1 and emitters is None, rays_per_emitter_total=rpe_total,
+                     emitters=None if emitters is None else np.array(emitters, dtype=np.int32))
     sparse_multi = row_tiles is None and n_tiles > 1 and len(trs) > 1
-    if n_tiles > 1 and (row_tiles is not None or sparse_multi):
+    # listed rows whose counts fit one device are traced there, whatever the number of devices: they stay resident on it and are smoothed
+    # from there, as the counts a multi-device full trace gathers on the first device are; only a list beyond one device is split
+    rows_multi = emitters is not None and len(trs) > 1 and not rows_fit_one_device(n_rows, tr.n_elements, len(spectral_bins))
+    if rows_multi or (n_tiles > 1 and (row_tiles is not None or sparse_multi)):
         # N >> 57 k elements: the dense count matrix is the limit, not the tally (SURVEY.md section 5).  Several devices: each traces
         # its emitter shard with the hashed row tally and only the non-zeros come back.  An explicit row_tiles: the rows are traced in
         # tiles on one device, keeping only each tile's non-zeros; the recorder is not available there.
-        if sparse_multi:
+        if rows_multi:
+            # several devices, a list beyond one device: device r traces the r-th contiguous block of it; only their non-zeros come back
+            from ._lib import trace_rows_multi
+            res = trace_rows_multi(trs, emitters, rays_per_emitter, refine=refine, **kw)
+            stats = dict(res["stats"], devices=len(trs), rays_per_emitter_total=rpe_total)
+            if rec is not None and "origins" in res:
+                rec.origins[0] = np.concatenate([rec.origins[0], res["origins"]], axis=0)
+                rec.endpoints[0] = np.concatenate([rec.endpoints[0], res["endpoints"]], axis=0)
+        elif sparse_multi:
             from ._lib import trace_sparse_multi
             res = trace_sparse_multi(trs, rays_per_emitter, refine=refine, **kw)
             stats = dict(res["stats"], tally="sparse", devices=len(trs), sparse=res["sparse_stats"], rays_per_emitter_total=rpe_total)
@@ -179,7 +203,7 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
             stats = dict(res["stats"], row_tiles=n_tiles, rays_per_emitter_total=rpe_total)
         t1 = time.perf_counter()
         rtm._trace_state = new_state
-        rtm.last_trace_stats = stats
+        rtm.last_trace_stats = dict(stats, rows=n_rows)
         rtm.last_lost = res["lost"]
         N = tr.n_elements
         mats = []
@@ -195,6 +219,8 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
         # one device, dense matrix beyond the budget: the hashed row tally keeps the counts on the device in sparse form
         out = tr.trace_continue(rays_per_emitter, **kw) if refine else tr.trace_sparse(rays_per_emitter, **kw)
         out["stats"] = dict(out["stats"], tally="sparse", sparse=out["sparse_stats"])
+    elif emitters is not None:
+        out = tr.trace_continue(rays_per_emitter, **kw) if refine else tr.trace_rows(emitters, rays_per_emitter, dense=False, **kw)
     elif len(trs) == 1:
         out = tr.trace_continue(rays_per_emitter, **kw) if refine else tr.trace(rays_per_emitter, dense=False, **kw)
     else:
@@ -203,7 +229,7 @@ def computeExchangeFactorsBins(rtm, rays_per_emitter: int, nudge: float, spectra
         tr.set_copy_helpers(trs[1:])           # the read-outs below leave through every device's PCIe link
     t1 = time.perf_counter()
     rtm._trace_state = new_state
-    rtm.last_trace_stats = dict(out["stats"], rays_per_emitter_total=rpe_total)
+    rtm.last_trace_stats = dict(out["stats"], rays_per_emitter_total=rpe_total, rows=n_rows)
     rtm.last_lost = out["lost"]
     if rec is not None and "origins" in out:
         # parallelRayTracing.jl:120-123 push into rec.origins[tid]; any slot works for collect_rays
@@ -239,18 +265,25 @@ def computeExchangeFactorsBin(rtm, rays_per_emitter: int, nudge: float, spectral
 
 def parallelRayTracing(rtm, rays_total: int, nudge: Optional[float], verbose: bool, rec=None, seed: Optional[int] = None,
                        device: Optional[int] = None, locator: Optional[int] = None, devices=None, row_tiles: Optional[int] = None,
-                       refine: bool = False):
+                       refine: bool = False, emitters=None):
     """parallelRayTracing(rtm, rays_total, nudge, verbose; rec) -> (F_raw, rays_per_emitter).  refine=True (new): add
     rays_total // N rays per emitter to the counts the previous call left on the device(s) — same handles, seed, bins, nudge and
     locator — and return the F_raw of ONE trace of all rays so far, with their number per emitter.  ValueError when there is no
     previous call, it traced explicit row_tiles or gathered dense counts from several devices, the flattened mesh changed, or
-    seed / devices / device / locator / row_tiles / nudge are given and differ (`device=d` stands for `devices=[d]`)."""
+    seed / devices / device / locator / row_tiles / nudge / emitters are given and differ (`device=d` stands for `devices=[d]`).
+    emitters (new): 0-based element indices, strictly ascending; only those rows are traced (rthx_trace_exchange_rows) and F_raw is the
+    N x N matrix whose other rows are empty, each listed row equal bit for bit to that row of the full trace.  rays_per_emitter stays
+    rays_total // N.  The printed loss line is then the maximum over the traced rows."""
     num_emitters = rtm.num_elements
     rays_per_emitter = rays_total // num_emitters                        # parallelRayTracing.jl:6
     n_bins = rtm.n_spectral_bins
+    if emitters is not None:
+        emitters = np.ascontiguousarray(emitters, dtype=np.int32).ravel()
+        if row_tiles is not None:
+            raise ValueError("emitters and row_tiles cannot be combined (a rows trace keeps R x N counts on the device)")
     if refine:
         given = resolve_devices(devices, 0, rays_total) if devices is not None else ([int(device)] if device is not None else None)
-        state = _refine_state(rtm, seed, given, locator, row_tiles, nudge)
+        state = _refine_state(rtm, seed, given, locator, row_tiles, nudge, emitters)
         seed, devices, locator, nudge = state["seed"], state["devices"], state["locator"], state["nudge"]
         device = devices[0]
     else:
@@ -268,7 +301,7 @@ def parallelRayTracing(rtm, rays_total: int, nudge: Optional[float], verbose: bo
         groups, reps, nonuniform = group_uniform_bins(rtm.uniform_across_bin)
         to_trace = list(nonuniform) + [g[0] for g in groups]
         mats = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, to_trace, verbose, rec, seed, device, locator, devices, row_tiles,
-                                          refine)
+                                          refine, emitters)
         rtm._traced_bins = list(to_trace)
         F_raw_vector: List[Optional[sp.csc_matrix]] = [None] * n_bins
         for b, F in zip(to_trace[: len(nonuniform)], mats[: len(nonuniform)]):
@@ -281,7 +314,8 @@ def parallelRayTracing(rtm, rays_total: int, nudge: Optional[float], verbose: bo
         verbose and print(f"Computing single F matrix for uniform spectral extinction ({n_bins} bins)")
     else:
         verbose and print("Computing single F matrix for grey extinction")
-    F_raw = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, [1], verbose, rec, seed, device, locator, devices, row_tiles, refine)[0]
+    F_raw = computeExchangeFactorsBins(rtm, rays_per_emitter, nudge, [1], verbose, rec, seed, device, locator, devices, row_tiles, refine,
+                                       emitters)[0]
     rtm._traced_bins = [1]
     return F_raw, rtm._trace_state["rays_per_emitter_total"]
 
@@ -328,8 +362,10 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
     """smooth_F on the GPU for traced bin number `k` (0-based position in the last launch).  Dense branch (density > 0.25,
     smoothExchangeFactors.jl:432-434): straight from the counts the trace left on the device.  Sparse branch with AP only
     (k_dykstra nothing or 0): AP on the non-zero pattern, from the resident counts (dense, or the hashed tally's of a single-device
-    trace), or from the host CSC F_raw after a trace in row tiles or a multi-device hashed-tally trace (only one shard is resident).  Returns None where the host path applies: sparse Dykstra rounds, or a dense
-    F traced in row tiles or with the hashed row tally."""
+    trace), or from the host CSC F_raw after a trace in row tiles, a multi-device hashed-tally trace or a list of rows split over several
+    devices (only one shard is resident).  Returns None where the host path (smooth_F on the CPU) applies: sparse Dykstra rounds, or a
+    dense F traced in row tiles, with the hashed row tally, or as a list of rows split over several devices.  A rows trace whose counts
+    fit one device (every surfaces-only route of exchangeRayTracing) is resident there and takes the device paths above."""
     tr = getattr(rtm, "_device", None)
     n = F_raw.shape[0]
     if tr is None or max_iters <= 0:
@@ -337,7 +373,7 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
     trace_stats = getattr(rtm, "last_trace_stats", None) or {}
     row_tiled = trace_stats.get("row_tiles", 1) > 1
     sparse_tally = trace_stats.get("tally") == "sparse"
-    resident = not row_tiled and not (sparse_tally and trace_stats.get("devices", 1) > 1)   # all rows of F_raw on this device
+    resident = not row_tiled and trace_stats.get("devices", 1) == 1      # all rows of F_raw on this device
     wn = w[:n] / np.min(w[:n])
     if F_raw.nnz / float(n * n) <= 0.25:
         if k_dykstra not in (None, 0):
@@ -353,8 +389,8 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
         verbose and print(f"AP: {st['iterations']} iterations, delta_R {st['delta_init']:.3e} -> {st['delta']:.3e}, "
                           f"{st['total_ms']:.1f} ms on the device")
         return F_smooth
-    if row_tiled or sparse_tally:
-        return None                                          # a dense F traced in row tiles or with the hashed tally: no dense counts resident
+    if not resident or sparse_tally:
+        return None                                          # a dense F traced in row tiles, on several devices or with the hashed tally: no dense counts resident
     if k_dykstra is None:       # smooth_F :441-450: one Dykstra round when surfaces and gas are strongly coupled, else AP only
         stats = getattr(rtm, "last_counts_stats", None)
         if rtm.surfaces_only:
@@ -380,15 +416,24 @@ def _smooth_on_device(rtm, k: int, F_raw, w, ns: int, max_iters: int, verbose: b
 
 def exchangeRayTracing(rtm, rays_tot: int, nudge: Optional[float], max_iters: int, k_dykstra, verbose: bool, rec,
                        seed: Optional[int] = None, device: Optional[int] = None, locator: Optional[int] = None,
-                       smooth: bool = True, devices=None, row_tiles: Optional[int] = None, refine: bool = False):
+                       smooth: bool = True, devices=None, row_tiles: Optional[int] = None, refine: bool = False,
+                       trace_volume_rows: bool = False):
     """exchangeRayTracing!(rtm, rays_tot, nudge, max_iters, k_dykstra, verbose, rec): trace, optional
-    surfaces-only crop (:9-11), smooth (:14-70), store rtm.F_raw / rtm.F_smooth (:73-74).  refine=True: see parallelRayTracing."""
+    surfaces-only crop (:9-11), smooth (:14-70), store rtm.F_raw / rtm.F_smooth (:73-74).  refine=True: see parallelRayTracing.
+    A surfaces-only domain (one F for all bins) traces only the Ns surface rows the crop keeps (parallelRayTracing(emitters=0..Ns-1)):
+    rtm.F_raw, rtm.F_smooth and the recorder are bit-identical to those of the full trace, and the loss line is the maximum over the
+    surface rows.  The surface rows are traced on the first resolved device alone, whatever the number of devices: their counts stay
+    resident there and are smoothed there, as the full trace's gathered counts are.  The full trace is taken when a RayRecorder names a
+    volume element, row_tiles is given, trace_volume_rows=True, or the surface rows' 8 Ns N bytes of counts would not fit one device."""
     import time
     from .smoothing import smooth_F
-    F_raw, rays_per_emitter = parallelRayTracing(rtm, rays_tot, nudge, verbose, rec=rec, seed=seed, device=device,
-                                                 locator=locator, devices=devices, row_tiles=row_tiles, refine=refine)
-    t0 = time.perf_counter()
     ns = rtm.num_surfaces
+    rows_only = (rtm.surfaces_only and rtm.spectral_mode != "spectral_variable" and ns > 0 and not trace_volume_rows and row_tiles is None
+                 and (rec is None or all(int(i) - 1 < ns for i in rec.ids)) and rows_fit_one_device(ns, rtm.num_elements, 1))
+    F_raw, rays_per_emitter = parallelRayTracing(rtm, rays_tot, nudge, verbose, rec=rec, seed=seed, device=device,
+                                                 locator=locator, devices=devices, row_tiles=row_tiles, refine=refine,
+                                                 emitters=np.arange(ns, dtype=np.int32) if rows_only else None)
+    t0 = time.perf_counter()
     if rtm.surfaces_only and not isinstance(F_raw, list):
         F_raw = F_raw[:ns, :ns]
 
