@@ -269,6 +269,7 @@ class DeviceTracer:
         self._check(self._L.rthx_get_info(self._h, C.byref(info)))
         self.info = info.as_dict()
         self.n_elements = info.n_elements
+        self._resident = None          # the trace whose counts the library keeps on the device (_set_resident)
 
     def _check(self, rc: int):
         if rc != 0:
@@ -308,14 +309,8 @@ class DeviceTracer:
         self._check(self._L.rthx_trace_exchange(self._h, C.byref(args), counts.ctypes.data_as(c_u64p) if counts is not None else None,
                                                 lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                 C.byref(st)))
-        self._last_shard = (int(args.emitter_rank), int(args.emitter_world))     # rows resident on the device: e = rank + y * world
-        self._last_rows = None
-        self._record_resident(rays_per_emitter, kw, sparse=False)
-        out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
-        if rec is not None:
-            out["origins"] = origins[: rec.n_recorded].copy()
-            out["endpoints"] = endpoints[: rec.n_recorded].copy()
-        return out
+        self._set_resident(rays_per_emitter, kw, len(range(args.emitter_rank, N, args.emitter_world)))   # rows e = rank + y * world
+        return _recorded(dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict()), rec, origins, endpoints)
 
     def trace_rows(self, emitters, rays_per_emitter: int, dense: bool = True, **kw):
         """Blocking trace of the emitter rows `emitters` only (rthx_trace_exchange_rows): element indices, strictly ascending, in [0, N).
@@ -336,14 +331,8 @@ class DeviceTracer:
         self._check(self._L.rthx_trace_exchange_rows(self._h, C.byref(args), rows.ctypes.data_as(c_i32p), R,
                                                      counts.ctypes.data_as(c_u64p) if counts is not None else None,
                                                      lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None, C.byref(st)))
-        self._last_shard = (0, 1)
-        self._last_rows = rows.copy()
-        self._record_resident(rays_per_emitter, kw, sparse=False)
-        out = dict(counts=counts.reshape(nb, R, N) if counts is not None else None, lost=lost, stats=st.as_dict())
-        if rec is not None:
-            out["origins"] = origins[: rec.n_recorded].copy()
-            out["endpoints"] = endpoints[: rec.n_recorded].copy()
-        return out
+        self._set_resident(rays_per_emitter, kw, R)
+        return _recorded(dict(counts=counts.reshape(nb, R, N) if counts is not None else None, lost=lost, stats=st.as_dict()), rec, origins, endpoints)
 
     def trace_sparse(self, rays_per_emitter: int, **kw):
         """Blocking trace with the hashed row tally (rthx_trace_exchange_sparse): the counts never exist in dense form and stay on
@@ -357,21 +346,17 @@ class DeviceTracer:
         rec, origins, endpoints = _recorder(kw.get("rec_ids"), rays_per_emitter)
         self._check(self._L.rthx_trace_exchange_sparse(self._h, C.byref(args), lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None,
                                                        C.byref(st), C.byref(sst)))
-        self._last_shard = (int(args.emitter_rank), int(args.emitter_world))
-        self._last_rows = None
-        self._record_resident(rays_per_emitter, kw, sparse=True)
-        out = dict(counts=None, lost=lost, stats=st.as_dict(), sparse_stats=sst.as_dict())
-        if rec is not None:
-            out["origins"] = origins[: rec.n_recorded].copy()
-            out["endpoints"] = endpoints[: rec.n_recorded].copy()
-        return out
+        self._set_resident(rays_per_emitter, kw, len(range(args.emitter_rank, self.n_elements, args.emitter_world)), sparse=True)
+        return _recorded(dict(counts=None, lost=lost, stats=st.as_dict(), sparse_stats=sst.as_dict()), rec, origins, endpoints)
 
     # keywords that fix the resident trace's ray stream; trace_continue repeats them unless given
     _STREAM_KW = ("seed", "bins", "nudge", "mode", "locator", "emitter_rank", "emitter_world")
 
-    def _record_resident(self, rays_per_emitter: int, kw, sparse: bool):
+    def _set_resident(self, rays_per_emitter: int, kw, rows: int, sparse: bool = False):
+        """Record the trace whose counts the library now keeps on the device: its stream keywords and the end of its ray-id range (what
+        trace_continue repeats and continues), its form, and its rows per bin (the R of counts_csr)."""
         lo = int(kw.get("ray_id_offset", 0))
-        self._resident = dict(kw={k: kw[k] for k in self._STREAM_KW if k in kw}, hi=lo + int(rays_per_emitter), sparse=sparse)
+        self._resident = dict(kw={k: kw[k] for k in self._STREAM_KW if k in kw}, hi=lo + int(rays_per_emitter), sparse=sparse, rows=int(rows))
 
     def trace_continue(self, rays_per_emitter: int, **kw):
         """Add `rays_per_emitter` rays per owned emitter to the counts resident from the last `trace(dense=False)`, `trace_sparse()` or
@@ -380,7 +365,7 @@ class DeviceTracer:
         resident ray-id range.  Afterwards every read-out of the resident counts equals, bit for bit, the read-out after ONE trace of
         the whole range.  Returns the dict of the trace that left the counts resident (sparse_stats after a hashed one), with lost
         cumulative over the whole range; origins / endpoints hold this call's recorded rays."""
-        res = getattr(self, "_resident", None) or dict(kw={}, hi=0, sparse=False)
+        res = self._resident or dict(kw={}, hi=0, sparse=False)
         kw = {**res["kw"], "ray_id_offset": res["hi"], **kw}
         args, keep = make_trace_args(rays_per_emitter, **kw)
         lost = np.empty((args.n_bins, self.n_elements), np.uint64)
@@ -392,10 +377,7 @@ class DeviceTracer:
         out = dict(counts=None, lost=lost, stats=st.as_dict())
         if res["sparse"]:
             out["sparse_stats"] = sst.as_dict()
-        if rec is not None:
-            out["origins"] = origins[: rec.n_recorded].copy()
-            out["endpoints"] = endpoints[: rec.n_recorded].copy()
-        return out
+        return _recorded(out, rec, origins, endpoints)
 
     def trace_device(self, rays_per_emitter: int, counts_ptr: int, lost_ptr: int, stream: int = 0,
                      zero_first=True, **kw):
@@ -415,10 +397,7 @@ class DeviceTracer:
         nnz = C.c_int64(0)
         self._check(self._L.rthx_counts_nnz(self._h, int(bin), C.byref(nnz)))
         N, k = self.n_elements, max(1, nnz.value)
-        rank, world = getattr(self, "_last_shard", (0, 1))
-        R = (N - rank + world - 1) // world          # after a sharded trace (a row tile) the view covers the rows e = rank + y * world
-        if getattr(self, "_last_rows", None) is not None:
-            R = len(self._last_rows)
+        R = self._resident["rows"] if self._resident else N
         row_ptr = np.empty(R + 1, np.int64)
         cols = np.empty(k, np.int32)
         vals = np.empty(k, np.uint64) if values else None
@@ -579,6 +558,14 @@ def _recorder(rec_ids, rays_per_emitter: int):
     return rthx_rec_out(cap, origins.ctypes.data_as(c_f64p), endpoints.ctypes.data_as(c_f64p), 0), origins, endpoints
 
 
+def _recorded(out, rec, origins, endpoints):
+    """`out` with the rays the recorder caught (origins / endpoints of _recorder's arrays) when recording was on."""
+    if rec is not None:
+        out["origins"] = origins[: rec.n_recorded].copy()
+        out["endpoints"] = endpoints[: rec.n_recorded].copy()
+    return out
+
+
 def create_multi(flat, devices: Sequence[int]):
     """One DeviceTracer per device from ONE host-side mesh preparation (rthx_create_multi)."""
     L = load_library()
@@ -617,14 +604,8 @@ def trace_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, counts_o
     if rc != 0:
         msg = L.rthx_last_error(tracers[0]._h)
         raise RthxError(f"rthx_trace_exchange_multi failed ({rc}): {msg.decode() if msg else ''}")
-    tracers[0]._last_shard = (0, 1)
-    tracers[0]._last_rows = None
-    tracers[0]._record_resident(rays_per_emitter, kw, sparse=False)
-    out = dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict())
-    if rec is not None:
-        out["origins"] = origins[: rec.n_recorded].copy()
-        out["endpoints"] = endpoints[: rec.n_recorded].copy()
-    return out
+    tracers[0]._set_resident(rays_per_emitter, kw, N)
+    return _recorded(dict(counts=counts.reshape(nb, N, N) if counts is not None else None, lost=lost, stats=st.as_dict()), rec, origins, endpoints)
 
 
 def merge_row_tiles(tiles, N: int, n_bins: int, tile_rows=None):
@@ -719,21 +700,8 @@ def trace_sparse_multi(tracers: Sequence[DeviceTracer], rays_per_emitter: int, r
 
     with ThreadPoolExecutor(max_workers=n) as ex:
         res = list(ex.map(run, range(n)))
-    lost = np.zeros((nb, N), np.uint64)
-    chi = np.zeros(nb)
-    for out, _, c in res:
-        lost += out["lost"]
-        chi += c
-    stats = dict(res[0][0]["stats"])
-    stats["kernel_ms"] = max(o["stats"]["kernel_ms"] for o, _, _ in res)
-    stats["total_ms"] = max(o["stats"]["total_ms"] for o, _, _ in res)
-    stats["rays_traced"] = sum(o["stats"]["rays_traced"] for o, _, _ in res)
-    stats["rays_lost"] = sum(o["stats"]["rays_lost"] for o, _, _ in res)
-    sparse_stats = {k: sum(o["sparse_stats"][k] for o, _, _ in res) for k in ("pairs", "nnz", "flushes", "row_groups")}
-    result = dict(csr=merge_row_tiles([p for _, p, _ in res], N, nb), lost=lost, chi=chi, stats=stats, sparse_stats=sparse_stats)
-    if rec_ids:
-        result["origins"] = np.concatenate([o.get("origins", np.zeros((0, 2))) for o, _, _ in res], axis=0)
-        result["endpoints"] = np.concatenate([o.get("endpoints", np.zeros((0, 2))) for o, _, _ in res], axis=0)
+    result = _combine_shards(res, N, nb, bool(rec_ids))
+    result["sparse_stats"] = {k: sum(o["sparse_stats"][k] for o, _, _ in res) for k in ("pairs", "nnz", "flushes", "row_groups")}
     return result
 
 
@@ -765,20 +733,26 @@ def trace_rows_multi(tracers: Sequence[DeviceTracer], emitters, rays_per_emitter
     live = [r for r in range(n) if len(parts_rows[r])]        # fewer rows than devices: the others stay idle
     with ThreadPoolExecutor(max_workers=len(live)) as ex:
         res = list(ex.map(run, live))
+    return _combine_shards(res, N, nb, bool(rec_ids), tile_rows=[parts_rows[r] for r in live])
+
+
+def _combine_shards(res, N: int, nb: int, recorded: bool, tile_rows=None):
+    """One result from the per-device runs res = [(trace output, CSR pieces, chi)] of trace_sparse_multi / trace_rows_multi: the pieces
+    merged into one CSR matrix per bin (merge_row_tiles), lost and chi summed, device 0's stats with the ray counts summed and the times of
+    the slowest device, and with `recorded` the recorded rays of every device in device order."""
+    outs = [o for o, _, _ in res]
     lost = np.zeros((nb, N), np.uint64)
     chi = np.zeros(nb)
     for out, _, c in res:
         lost += out["lost"]
         chi += c
-    stats = dict(res[0][0]["stats"])
-    stats["kernel_ms"] = max(o["stats"]["kernel_ms"] for o, _, _ in res)
-    stats["total_ms"] = max(o["stats"]["total_ms"] for o, _, _ in res)
-    stats["rays_traced"] = sum(o["stats"]["rays_traced"] for o, _, _ in res)
-    stats["rays_lost"] = sum(o["stats"]["rays_lost"] for o, _, _ in res)
-    result = dict(csr=merge_row_tiles([p for _, p, _ in res], N, nb, tile_rows=[parts_rows[r] for r in live]), lost=lost, chi=chi, stats=stats)
-    if rec_ids:
-        result["origins"] = np.concatenate([o.get("origins", np.zeros((0, 2))) for o, _, _ in res], axis=0)
-        result["endpoints"] = np.concatenate([o.get("endpoints", np.zeros((0, 2))) for o, _, _ in res], axis=0)
+    stats = dict(outs[0]["stats"])
+    for k, agg in (("kernel_ms", max), ("total_ms", max), ("rays_traced", sum), ("rays_lost", sum)):
+        stats[k] = agg(o["stats"][k] for o in outs)
+    result = dict(csr=merge_row_tiles([p for _, p, _ in res], N, nb, tile_rows), lost=lost, chi=chi, stats=stats)
+    if recorded:
+        for k in ("origins", "endpoints"):
+            result[k] = np.concatenate([o.get(k, np.zeros((0, 2))) for o in outs], axis=0)
     return result
 
 

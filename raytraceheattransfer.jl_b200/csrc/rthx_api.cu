@@ -76,6 +76,27 @@ struct DevRes {
 
 namespace { struct HostImage; }
 
+// where the resident counts come from
+enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4 };
+
+// The emitter rows a trace owns: row y is element rank + y * world (a shard), or with `listed` element rows[y] of the handle's emitter
+// list (a rows trace; rank / world are then 0 / 1)
+struct OwnedRows { int rank = 0, world = 1; bool listed = false; };
+
+// The counts resident on the device (counts_dev, or the hashed tally's sk_* set for RESIDENT_SPARSE) and the one trace, of the
+// contiguous ray-id range [ray_lo, ray_hi), they are those of; rthx_trace_exchange_continue extends it.  Set only by set_resident and
+// voided only by drop_resident; kind == RESIDENT_NONE: nothing is resident.
+struct Resident {
+  int kind = RESIDENT_NONE;
+  OwnedRows own;                       // what row y of the resident matrix is
+  int n_rows = 0;                      // rows per bin: N, the rows of a shard, or the listed rows
+  long long nnz = 0;                   // the hashed set's non-zeros over all traced bins
+  uint64_t seed = 0; double nudge = 0.0; int mode = 0, locator = 0;
+  std::vector<int32_t> bins;           // the traced bins
+  int64_t ray_lo = 0, ray_hi = 0;
+  int n_bins() const { return (int)bins.size(); }
+};
+
 struct rthx_handle : DevRes {
   int device = 0;
   std::shared_ptr<HostImage> image;    // host image of the mesh tables (shared by the handles of one rthx_create_multi call)
@@ -92,27 +113,15 @@ struct rthx_handle : DevRes {
   bool fast_ok = false;        // every coarse face affine + complete neighbour table + descriptors fit in smem
   size_t mesh_bytes = 0;
   TraceParams base{};          // mesh pointers filled once
-  int last_trace_bins = 0; size_t last_trace_rows = 0;    // resident counts: bins, rows per bin (N, or the rows of a shard)
-  int last_rank = 0, last_world = 1;                      // ... row y of the resident matrix is element last_rank + y * last_world
-  bool sparse_counts = false;                             // the resident counts are the hashed tally's (sk_*), not counts_dev
-  // Rows trace: `rows` (also in rows_dev) is the emitter list of the trace in progress when rows_active, and of the resident counts when
-  // res_rows (row y of the resident matrix is then element rows[y]; last_rank / last_world are 0 / 1).  row_runs cuts it into
-  // arithmetic runs {first row y0, rows, element of y0, stride}: each run is launched as a shard (emitter_rank + y * emitter_world),
-  // so the trace kernels map rows to emitters exactly as for every other trace.
+  Resident res;                                           // the resident counts
+  // Emitter list of the last rows trace (also in rows_dev): the resident rows when res.own.listed.  row_runs cuts it into arithmetic
+  // runs {first row y0, rows, element of y0, stride}: each run is launched as a shard (emitter_rank + y * emitter_world), so the trace
+  // kernels map rows to emitters exactly as for every other trace.
   std::vector<int32_t> rows;
   std::vector<int4> row_runs;
-  bool rows_active = false, res_rows = false;
-  long long sk_nnz = 0;                                   // ... its non-zeros over all traced bins
-  // The one trace (of the contiguous ray-id range [ray_lo, ray_hi)) the resident counts are those of; rthx_trace_exchange_continue
-  // extends it.  Valid while last_trace_bins > 0.
-  int resident_kind = 0;                                  // RESIDENT_*
-  uint64_t res_seed = 0; double res_nudge = 0.0; int res_mode = 0, res_locator = 0;
-  std::vector<int32_t> res_bins;
-  int64_t ray_lo = 0, ray_hi = 0;
   int smooth_n = 0; size_t smooth_ldx = 0;                // F_smooth resident in smooth_X after rthx_smooth_F (0: none)
   int sparse_n = 0; long long sparse_nnz = 0;             // sparse F_smooth resident in sp_* after rthx_smooth_sparse (0: none)
-  int csr_bin = -1; long long csr_total = 0;              // bin whose row pointers are prepared on the device
-  int csc_bin = -1;                                       // bin whose column pointers are prepared on the device
+  int csr_bin = -1; long long csr_total = 0;              // bin of the resident counts whose row pointers are prepared on the device
   double csr_chi = 0.0;                                   // surface-gas cross-coupling of that bin's row-normalised F
   // views into the arena
   unsigned long long* lost_dev = nullptr;   size_t lost_cap = 0;
@@ -959,36 +968,50 @@ int check_args(rthx_handle* h, const rthx_trace_args* a) {
   return RTHX_OK;
 }
 
-// where the resident counts come from
-enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4 };
+OwnedRows shard_of(const rthx_trace_args* a) { return {a->emitter_rank, a->emitter_world, false}; }
 
-void record_resident(rthx_handle* h, const rthx_trace_args* a, int kind) {
-  h->resident_kind = kind;
-  h->res_seed = a->seed; h->res_nudge = a->nudge; h->res_mode = a->mode; h->res_locator = a->locator;
-  h->res_bins.assign(a->bins, a->bins + a->n_bins);
-  h->ray_lo = a->ray_id_offset; h->ray_hi = a->ray_id_offset + a->rays_per_emitter;
+// counts_dev or the hashed set is about to be overwritten: nothing is resident (and no bin's row pointers prepared) until set_resident
+void drop_resident(rthx_handle* h) {
+  h->res = Resident{};
+  h->csr_bin = -1;
+}
+
+// The trace `a` of the rows `own` (n_rows per bin) has finished and its counts are resident, in the form `kind`
+void set_resident(rthx_handle* h, const rthx_trace_args* a, int kind, OwnedRows own, int n_rows) {
+  Resident& r = h->res;
+  r.kind = kind; r.own = own; r.n_rows = n_rows; r.nnz = 0;
+  r.seed = a->seed; r.nudge = a->nudge; r.mode = a->mode; r.locator = a->locator;
+  r.bins.assign(a->bins, a->bins + a->n_bins);
+  r.ray_lo = a->ray_id_offset; r.ray_hi = a->ray_id_offset + a->rays_per_emitter;
+}
+
+// The continuation `a` of the trace `kept` (dropped while it ran) has finished: that trace is resident again, over the longer range
+void resume_resident(rthx_handle* h, Resident kept, const rthx_trace_args* a) {
+  kept.ray_hi += a->rays_per_emitter;
+  h->res = std::move(kept);
 }
 
 // Preconditions of rthx_trace_exchange_continue: the resident counts are one trace of [ray_lo, ray_hi) that `a` continues
 int check_continue(rthx_handle* h, const rthx_trace_args* a) {
-  if (h->last_trace_bins <= 0 || h->resident_kind == RESIDENT_NONE)
+  const Resident& r = h->res;
+  if (r.kind == RESIDENT_NONE)
     return fail(h, RTHX_ERR_ARG, "trace_continue: no resident counts (run rthx_trace_exchange with counts_out == NULL or rthx_trace_exchange_sparse first)");
-  if (h->resident_kind == RESIDENT_HOST)
+  if (r.kind == RESIDENT_HOST)
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts come from a host-output trace (counts_out != NULL); trace with counts_out == NULL to continue");
-  if (h->resident_kind == RESIDENT_MULTI)
+  if (r.kind == RESIDENT_MULTI)
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts were gathered from several devices (rthx_trace_exchange_multi), whose peer hand-over stores rows instead of adding them");
-  if (a->seed != h->res_seed) return fail(h, RTHX_ERR_ARG, "trace_continue: seed differs from the resident trace's");
-  if (a->nudge != h->res_nudge) return fail(h, RTHX_ERR_ARG, "trace_continue: nudge differs from the resident trace's");
-  if (a->mode != h->res_mode) return fail(h, RTHX_ERR_ARG, "trace_continue: mode differs from the resident trace's");
-  if (a->locator != h->res_locator) return fail(h, RTHX_ERR_ARG, "trace_continue: locator differs from the resident trace's");
-  if (a->n_bins != (int)h->res_bins.size() || !std::equal(a->bins, a->bins + a->n_bins, h->res_bins.begin()))
+  if (a->seed != r.seed) return fail(h, RTHX_ERR_ARG, "trace_continue: seed differs from the resident trace's");
+  if (a->nudge != r.nudge) return fail(h, RTHX_ERR_ARG, "trace_continue: nudge differs from the resident trace's");
+  if (a->mode != r.mode) return fail(h, RTHX_ERR_ARG, "trace_continue: mode differs from the resident trace's");
+  if (a->locator != r.locator) return fail(h, RTHX_ERR_ARG, "trace_continue: locator differs from the resident trace's");
+  if (a->n_bins != r.n_bins() || !std::equal(a->bins, a->bins + a->n_bins, r.bins.begin()))
     return fail(h, RTHX_ERR_ARG, "trace_continue: bins differ from the resident trace's");
-  if (a->emitter_rank != h->last_rank || a->emitter_world != h->last_world)
+  if (a->emitter_rank != r.own.rank || a->emitter_world != r.own.world)
     return fail(h, RTHX_ERR_ARG, "trace_continue: emitter shard (emitter_rank / emitter_world) differs from the resident trace's");
-  if (a->ray_id_offset != h->ray_hi)
+  if (a->ray_id_offset != r.ray_hi)
     return fail(h, RTHX_ERR_ARG, "trace_continue: ray_id_offset " + std::to_string(a->ray_id_offset) + " does not continue the resident ray-id range [" +
-                                     std::to_string(h->ray_lo) + ", " + std::to_string(h->ray_hi) + ")");
-  if (a->rays_per_emitter > INT64_MAX - h->ray_hi) return fail(h, RTHX_ERR_ARG, "trace_continue: ray ids past 2^63");
+                                     std::to_string(r.ray_lo) + ", " + std::to_string(r.ray_hi) + ")");
+  if (a->rays_per_emitter > INT64_MAX - r.ray_hi) return fail(h, RTHX_ERR_ARG, "trace_continue: ray ids past 2^63");
   return RTHX_OK;
 }
 
@@ -1004,9 +1027,9 @@ long long auto_row_chunks(const rthx_handle* h, const LaunchPlan& pl, const rthx
 }
 
 // hash_slots > 0: the hashed row tally (no histogram; the table takes hash_table_bytes(hash_slots))
-LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, int rank, int world, int hash_slots = 0) {
+LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, OwnedRows own, int hash_slots = 0) {
   LaunchPlan pl{};
-  pl.n_owned = h->rows_active ? (int)h->rows.size() : (h->N - rank + world - 1) / world;
+  pl.n_owned = own.listed ? (int)h->rows.size() : (h->N - own.rank + own.world - 1) / own.world;
   if (pl.n_owned < 0) pl.n_owned = 0;
   pl.block_threads = a->block_threads ? a->block_threads : 256;
   const bool analytic = a->locator != RTHX_LOCATOR_GENERIC;
@@ -1119,20 +1142,26 @@ cudaError_t ensure(T** ptr, size_t* cap, size_t need) {
   return e;
 }
 
-void fill_stats(rthx_stats* st, const LaunchPlan& pl, const rthx_trace_args* a) {
+// rthx_stats of a trace: its plan, the lost counters read back (none: rays_lost 0), its launches and its kernel and call times
+void fill_stats(rthx_stats* st, const rthx_trace_args* a, const LaunchPlan& pl, const std::vector<uint64_t>& lost, int n_launches, double kernel_ms,
+                double total_ms) {
   if (!st) return;
   std::memset(st, 0, sizeof(*st));
   st->rays_traced = (int64_t)pl.n_owned * a->n_bins * a->rays_per_emitter;
   st->n_blocks = pl.n_blocks; st->block_threads = pl.block_threads; st->row_chunks = pl.row_chunks;
   st->smem_bytes = (int32_t)pl.smem_bytes; st->hist_in_smem = pl.kernel.hist;
+  for (uint64_t v : lost) st->rays_lost += (int64_t)v;
+  st->n_launches = n_launches;
+  st->kernel_ms = kernel_ms; st->total_ms = total_ms;
 }
 
 // Enqueue (zero +) kernel for one handle on `stream`; counts layout compact (owned rows) or full.
 // [y0, y1) restricts the launch to a range of owned-emitter ordinals (y1 < 0: all rows).
-int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world, bool compact, unsigned long long* counts,
+int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, bool compact, unsigned long long* counts,
                   unsigned long long* lost, int zero_first, bool with_rec, int n_rec_slots, cudaStream_t stream,
                   LaunchPlan* plan_out, int* n_launches, int y0 = 0, int y1 = -1, bool upload_bins = true) {
-  LaunchPlan pl = make_plan(h, a, rank, world);
+  const int rank = own.rank, world = own.world;
+  LaunchPlan pl = make_plan(h, a, own);
   if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
   if (!pl.kernel.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }     // the generic locator reads the reference-faithful tables
   if (upload_bins) CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)a->n_bins, cudaMemcpyHostToDevice, stream));
@@ -1152,7 +1181,7 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
   unsigned long long* stage_counts = nullptr;
   unsigned int* row_done = nullptr;
   if (staged) {
-    h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false;   // counts_dev becomes the staging matrix
+    drop_resident(h);                                                    // counts_dev becomes the staging matrix
     const size_t n_rows = (size_t)a->n_bins * (size_t)pl.n_owned;
     if (pl.row_chunks > 1) {
       CU(h, ensure(&h->counts_dev, &h->counts_cap, n_rows * (size_t)h->N));
@@ -1191,7 +1220,7 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, int rank, int world,
   }
   if (with_rec && n_rec_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
   if (y1 < 0) y1 = pl.n_owned;
-  if (!h->rows_active) {
+  if (!own.listed) {
     P.y_offset = y0;
     const long long nb = (long long)(y1 - y0) * a->n_bins * pl.row_chunks;
     CU(h, launch_trace_exchange(P, pl.kernel, (int)nb, pl.block_threads, pl.smem_bytes, stream));
@@ -1232,15 +1261,13 @@ void batch_rows_of(int n_owned, int n_batches, int b, int& y0, int& y1) {
   y0 = (int)((long long)n_owned * edge(b) / units); y1 = (int)((long long)n_owned * edge(b + 1) / units);
 }
 
-int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, int rank, int world, bool with_rec, int n_slots,
+int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, bool with_rec, int n_slots,
                     LaunchPlan* plan_out, int* n_launches, int* n_batches_out) {
   const int N = h->N;
-  LaunchPlan pl = make_plan(h, a, rank, world);
+  LaunchPlan pl = make_plan(h, a, own);
   if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
   const int n_owned = pl.n_owned;
-  // counts_dev is about to be overwritten: whatever view an earlier trace left behind (resident bins, CSR row pointers) is void
-  // until the caller re-validates it (rthx_trace_exchange does, for a complete single-device trace)
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false;
+  drop_resident(h);
   CU(h, ensure(&h->counts_dev, &h->counts_cap, (size_t)a->n_bins * (size_t)n_owned * N));
   // batches: >= ~2 waves of resident blocks each, at most 16 (consecutive batches alternate between two streams, so a batch's
   // draining tail overlaps the next one's head; cfg3 at 1e10 rays: 16 batches, the copy behind the last kernel is 17 MB and the
@@ -1261,7 +1288,7 @@ int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, int rank, int worl
     batch_rows_of(n_owned, n_batches, b, y0, y1);
     cudaStream_t cs = (b & 1) ? h->stream2 : h->stream;
     LaunchPlan tmp{};
-    int rc = enqueue_trace(h, a, rank, world, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, with_rec, n_slots, cs, &tmp, n_launches, y0, y1,
+    int rc = enqueue_trace(h, a, own, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, with_rec, n_slots, cs, &tmp, n_launches, y0, y1,
                            /*upload_bins=*/false);
     if (rc) return rc;
     CU(h, cudaEventRecord(h->bev[b], cs));
@@ -1393,58 +1420,61 @@ int collect_recorder(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec
   return RTHX_OK;
 }
 
-// Blocking host-output trace of the owned rows: those of the shard in `a`, or with h->rows_active the rows of the list in h->rows
-int trace_host(rthx_handle* h, const rthx_trace_args* a, uint64_t* counts_out, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
-  CU(h, cudaSetDevice(h->device));
-  const int N = h->N;
-  int n_slots = 0, n_launches = 0;
-  int rc;
-  CU(h, cudaEventRecord(h->ev[0], h->stream));
-  rc = prepare_recorder(h, a, rec, &n_slots, h->stream);
-  if (rc) return rc;
+// What the launches of one trace did, for its tail (finish_trace)
+struct TraceRun {
   LaunchPlan pl{};
-  int n_batches = 1;
-  rc = pipeline_launch(h, a, a->emitter_rank, a->emitter_world, rec != nullptr, n_slots, &pl, &n_launches, &n_batches);
-  if (rc) return rc;
-  if (counts_out) {
-    rc = pipeline_copy(h, a, a->emitter_rank, a->emitter_world, pl.n_owned, counts_out, n_batches);
-    if (rc) return rc;
-  } else {
-    CU(h, cudaStreamWaitEvent(h->copy_stream, h->ev[2], 0));
-  }
-  // the (compact) rows this call owns stay resident: all of them for a plain trace, those of a shard / row tile otherwise
-  h->last_trace_bins = a->n_bins;
-  h->last_trace_rows = (size_t)pl.n_owned; h->last_rank = a->emitter_rank; h->last_world = a->emitter_world;
-  h->res_rows = h->rows_active;
-  h->csr_bin = -1; h->csc_bin = -1;
-  record_resident(h, a, counts_out ? RESIDENT_HOST : RESIDENT_DENSE);
-  std::vector<uint64_t> lost_host((size_t)a->n_bins * N);
-  CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->copy_stream));
-  CU(h, cudaEventRecord(h->ev[3], h->copy_stream));
-  CU(h, cudaStreamSynchronize(h->copy_stream));
-  CU(h, cudaStreamSynchronize(h->stream));
-  if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
-  rc = collect_recorder(h, a, rec, n_slots, h->stream, false);
+  int n_slots = 0, n_launches = 0;     // recorder slots; launches and memsets
+  double kernel_ms = 0;
+  std::vector<uint64_t> lost;          // the lost counters, read back
+};
+
+// End of a trace whose kernels ran from ev[1] to ev[2]: the lost counters to the host behind everything enqueued on `stream` so far,
+// ev[3] as the end of the call's device work, and the kernel time
+int read_lost(rthx_handle* h, const rthx_trace_args* a, cudaStream_t stream, TraceRun& R) {
+  R.lost.resize((size_t)a->n_bins * h->N);
+  CU(h, cudaMemcpyAsync(R.lost.data(), h->lost_dev, sizeof(uint64_t) * R.lost.size(), cudaMemcpyDeviceToHost, stream));
+  CU(h, cudaEventRecord(h->ev[3], stream));
+  CU(h, cudaStreamSynchronize(stream));
+  float ms = 0;
+  CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2]));
+  R.kernel_ms = ms;
+  return RTHX_OK;
+}
+
+// Tail of a finished trace: lost_out, the recorded rays, and rthx_stats with the call's time from ev[0] to ev[3]
+int finish_trace(rthx_handle* h, const rthx_trace_args* a, const TraceRun& R, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
+  if (lost_out) std::memcpy(lost_out, R.lost.data(), sizeof(uint64_t) * R.lost.size());
+  const int rc = collect_recorder(h, a, rec, R.n_slots, h->stream, false);
   if (rc) return rc;
   if (st) {
-    fill_stats(st, pl, a);
     float ms = 0;
-    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); st->kernel_ms = ms;
-    CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3])); st->total_ms = ms;
-    int64_t nl = 0;
-    for (uint64_t v : lost_host) nl += (int64_t)v;
-    st->rays_lost = nl;
-    st->n_launches = n_launches;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3]));
+    fill_stats(st, a, R.pl, R.lost, R.n_launches, R.kernel_ms, ms);
   }
   return RTHX_OK;
 }
 
-// Marks the trace kernels' owned rows as those of the emitter list in h->rows for the duration of one call
-struct RowsScope {
-  rthx_handle* h;
-  RowsScope(rthx_handle* h_, bool on) : h(h_) { h->rows_active = on; }
-  ~RowsScope() { h->rows_active = false; }
-};
+// Blocking host-output trace of the owned rows `own`; with counts_out == NULL they stay resident
+int trace_host(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, uint64_t* counts_out, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
+  CU(h, cudaSetDevice(h->device));
+  TraceRun R;
+  CU(h, cudaEventRecord(h->ev[0], h->stream));
+  int rc = prepare_recorder(h, a, rec, &R.n_slots, h->stream);
+  if (rc) return rc;
+  int n_batches = 1;
+  rc = pipeline_launch(h, a, own, rec != nullptr, R.n_slots, &R.pl, &R.n_launches, &n_batches);
+  if (rc) return rc;
+  if (counts_out) {
+    rc = pipeline_copy(h, a, own.rank, own.world, R.pl.n_owned, counts_out, n_batches);
+    if (rc) return rc;
+  } else {
+    CU(h, cudaStreamWaitEvent(h->copy_stream, h->ev[2], 0));
+  }
+  if ((rc = read_lost(h, a, h->copy_stream, R))) return rc;
+  CU(h, cudaStreamSynchronize(h->stream));
+  set_resident(h, a, counts_out ? RESIDENT_HOST : RESIDENT_DENSE, own, R.pl.n_owned);
+  return finish_trace(h, a, R, lost_out, rec, st);
+}
 
 // Maximal arithmetic runs {first row, rows, first element, stride} of an ascending emitter list, taken greedily from the front.  A run
 // keeps (first row + rows) * stride below 2^31, so that the kernels' int arithmetic emitter_rank + y * emitter_world cannot overflow.
@@ -1498,7 +1528,7 @@ extern "C" int rthx_trace_exchange(rthx_handle* h, const rthx_trace_args* a, uin
   if (!h) return RTHX_ERR_ARG;
   const int rc = check_args(h, a);
   if (rc) return rc;
-  return trace_host(h, a, counts_out, lost_out, rec, st);
+  return trace_host(h, a, shard_of(a), counts_out, lost_out, rec, st);
 }
 
 extern "C" int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n_emitters,
@@ -1509,14 +1539,12 @@ extern "C" int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* a
   CU(h, cudaSetDevice(h->device));
   rc = check_rows(h, a, emitters, n_emitters);
   if (rc) return rc;
-  // the resident counts are replaced from here on
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->res_rows = false;
+  drop_resident(h);                  // the resident counts are replaced from here on
   h->rows.assign(emitters, emitters + n_emitters);
   h->row_runs = list_runs(h->rows);
   CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)n_emitters));
   CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)n_emitters, cudaMemcpyHostToDevice, h->stream));
-  RowsScope scope(h, true);
-  return trace_host(h, a, counts_out, lost_out, rec, st);
+  return trace_host(h, a, OwnedRows{0, 1, true}, counts_out, lost_out, rec, st);
 }
 
 extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args* a, void* counts_dev, void* lost_dev, void* stream,
@@ -1528,10 +1556,10 @@ extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args*
   CU(h, cudaSetDevice(h->device));
   LaunchPlan pl{};
   int n_launches = 0;
-  rc = enqueue_trace(h, a, a->emitter_rank, a->emitter_world, /*compact=*/false, (unsigned long long*)counts_dev,
-                     (unsigned long long*)lost_dev, zero_first, false, 0, (cudaStream_t)stream, &pl, &n_launches);
+  rc = enqueue_trace(h, a, shard_of(a), /*compact=*/false, (unsigned long long*)counts_dev, (unsigned long long*)lost_dev, zero_first, false, 0,
+                     (cudaStream_t)stream, &pl, &n_launches);
   if (rc) return rc;
-  if (st) { fill_stats(st, pl, a); st->n_launches = n_launches; }
+  fill_stats(st, a, pl, {}, n_launches, 0, 0);
   return RTHX_OK;
 }
 
@@ -1560,12 +1588,14 @@ cudaError_t grow_keep(T** ptr, size_t* cap, size_t need, size_t keep, cudaStream
 
 namespace {
 // What one hashed-tally pass over the rows of a call did (sparse_trace_rows)
-struct SparseRun {
-  LaunchPlan pl{};
-  int log2s = 0, groups = 0, n_slots = 0, n_launches = 0;
+struct SparseRun : TraceRun {
+  int log2s = 0, groups = 0;
   long long cap = 0, n_rows = 0, total = 0, pairs = 0, flushes = 0;
-  double kernel_ms = 0, reduce_ms = 0;
+  double reduce_ms = 0;
 };
+
+// The resident trace a hashed continuation extends, held while it runs: its record and its lost counters
+struct HeldSparse { Resident res; std::vector<uint64_t> lost; };
 
 // A device array freed when it goes out of scope (scratch of rthx_trace_exchange_continue)
 template <class T>
@@ -1594,7 +1624,7 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     if (v > 0) { log2s = 0; while ((1ll << log2s) < v) ++log2s; forced = true; }
   }
   log2s = std::max(log2s, min_log2s);
-  LaunchPlan pl = make_plan(h, a, rank, world, 1 << log2s);
+  LaunchPlan pl = make_plan(h, a, shard_of(a), 1 << log2s);
   if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
   if (!forced) {                                             // a block with few rays needs no large table: clearing and scanning it is the cost
     const long long per_block = (a->rays_per_emitter + pl.row_chunks - 1) / pl.row_chunks;
@@ -1689,39 +1719,27 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
 }
 
 // Second half of a hashed-tally trace or continuation whose sorted unique pairs (R.total of them) are in sk_keys / sk_vals: row
-// pointers, lost read-out, handle state, recorder and statistics.  lost_before (continuation): the lost counts of the resident
-// trace, added to this call's.
-int sparse_finish(rthx_handle* h, const rthx_trace_args* a, const SparseRun& R, const std::vector<uint64_t>* lost_before, uint64_t* lost_out,
-                  rthx_rec_out* rec, rthx_stats* st, rthx_sparse_stats* sst) {
-  const int N = h->N, nb = a->n_bins;
+// pointers, lost read-out, handle state, recorder and statistics.  held (continuation): the resident trace it continues, whose lost
+// counts are added to this call's.
+int sparse_finish(rthx_handle* h, const rthx_trace_args* a, SparseRun& R, const HeldSparse* held, uint64_t* lost_out, rthx_rec_out* rec,
+                  rthx_stats* st, rthx_sparse_stats* sst) {
   CU(h, ensure(&h->sk_rowptr, &h->sk_rowptr_cap, (size_t)R.n_rows + 1));
   CU(h, tally_row_ptr(h->sk_keys, R.total, R.n_rows, h->sk_rowptr, h->stream));
-  std::vector<uint64_t> lost_host((size_t)nb * N);
-  CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->stream));
-  if (lost_before) {
+  std::vector<uint64_t>& lost = R.lost;
+  lost.resize((size_t)a->n_bins * h->N);
+  CU(h, cudaMemcpyAsync(lost.data(), h->lost_dev, sizeof(uint64_t) * lost.size(), cudaMemcpyDeviceToHost, h->stream));
+  if (held) {
     CU(h, cudaStreamSynchronize(h->stream));
-    for (size_t k = 0; k < lost_host.size(); ++k) lost_host[k] += (*lost_before)[k];
-    CU(h, cudaMemcpyAsync(h->lost_dev, lost_host.data(), sizeof(uint64_t) * lost_host.size(), cudaMemcpyHostToDevice, h->stream));
+    for (size_t k = 0; k < lost.size(); ++k) lost[k] += held->lost[k];
+    CU(h, cudaMemcpyAsync(h->lost_dev, lost.data(), sizeof(uint64_t) * lost.size(), cudaMemcpyHostToDevice, h->stream));
   }
   CU(h, cudaEventRecord(h->ev[3], h->stream));
   CU(h, cudaStreamSynchronize(h->stream));
-  h->sparse_counts = true; h->sk_nnz = R.total;
-  h->last_trace_bins = nb; h->last_trace_rows = (size_t)R.pl.n_owned; h->last_rank = a->emitter_rank; h->last_world = a->emitter_world;
-  if (lost_before) h->ray_hi += a->rays_per_emitter;
-  else { record_resident(h, a, RESIDENT_SPARSE); h->res_rows = false; }
-  if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
-  int rc = collect_recorder(h, a, rec, R.n_slots, h->stream, false);
+  if (held) resume_resident(h, held->res, a);
+  else set_resident(h, a, RESIDENT_SPARSE, shard_of(a), R.pl.n_owned);
+  h->res.nnz = R.total;
+  const int rc = finish_trace(h, a, R, lost_out, rec, st);
   if (rc) return rc;
-  if (st) {
-    fill_stats(st, R.pl, a);
-    st->kernel_ms = R.kernel_ms;
-    float ms = 0;
-    CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3])); st->total_ms = ms;
-    int64_t nl = 0;
-    for (uint64_t v : lost_host) nl += (int64_t)v;
-    st->rays_lost = nl;
-    st->n_launches = R.n_launches;
-  }
   if (sst) {
     std::memset(sst, 0, sizeof(*sst));
     sst->pairs = R.pairs; sst->nnz = R.total; sst->flushes = R.flushes; sst->pair_capacity = R.cap;
@@ -1774,59 +1792,40 @@ int continue_sparse_merge(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out
 // Continuation of a hashed-tally trace.  Until the merged set replaces it the resident set is untouched, so a failure before that
 // point leaves it resident, with its lost counters restored.
 int continue_sparse(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st, rthx_sparse_stats* sst) {
-  std::vector<uint64_t> lost_before((size_t)a->n_bins * h->N);
-  CU(h, cudaMemcpyAsync(lost_before.data(), h->lost_dev, sizeof(uint64_t) * lost_before.size(), cudaMemcpyDeviceToHost, h->stream));
+  HeldSparse held{h->res, std::vector<uint64_t>((size_t)a->n_bins * h->N)};
+  CU(h, cudaMemcpyAsync(held.lost.data(), h->lost_dev, sizeof(uint64_t) * held.lost.size(), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaStreamSynchronize(h->stream));
-  const long long old_nnz = h->sk_nnz;
-  const int old_bins = h->last_trace_bins;
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1;  // incomplete until the merge has landed
+  drop_resident(h);                  // incomplete until the merge has landed
   SparseRun R;
-  const int rc = continue_sparse_merge(h, a, rec, old_nnz, R);
+  const int rc = continue_sparse_merge(h, a, rec, held.res.nnz, R);
   if (rc) {
-    if (cudaMemcpy(h->lost_dev, lost_before.data(), sizeof(uint64_t) * lost_before.size(), cudaMemcpyHostToDevice) == cudaSuccess)
-      h->last_trace_bins = old_bins;
+    if (cudaMemcpy(h->lost_dev, held.lost.data(), sizeof(uint64_t) * held.lost.size(), cudaMemcpyHostToDevice) == cudaSuccess)
+      h->res = held.res;
     else
       cudaGetLastError();
     return rc;
   }
-  return sparse_finish(h, a, R, &lost_before, lost_out, rec, st, sst);
+  return sparse_finish(h, a, R, &held, lost_out, rec, st, sst);
 }
 
 // Continuation of a dense resident trace: the same launches as rthx_trace_exchange(counts_out == NULL) without clearing the counts or
 // the lost counters.  Every flush into a matrix on the handle's own device adds (shared-memory histogram rows, global atomics,
 // row_chunks == 1 alike), so the counts add up to those of one trace of the whole range.
 int continue_dense(rthx_handle* h, const rthx_trace_args* a, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* st) {
-  int n_slots = 0, n_launches = 0;
+  TraceRun R;
   CU(h, cudaEventRecord(h->ev[0], h->stream));
-  int rc = prepare_recorder(h, a, rec, &n_slots, h->stream);
+  int rc = prepare_recorder(h, a, rec, &R.n_slots, h->stream);
   if (rc) return rc;
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1;  // incomplete until the kernels have finished
+  Resident kept = h->res;
+  drop_resident(h);                  // incomplete until the kernels have finished
   CU(h, cudaEventRecord(h->ev[1], h->stream));
-  LaunchPlan pl{};
-  rc = enqueue_trace(h, a, a->emitter_rank, a->emitter_world, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, rec != nullptr, n_slots,
-                     h->stream, &pl, &n_launches);
+  rc = enqueue_trace(h, a, kept.own, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, rec != nullptr, R.n_slots, h->stream, &R.pl,
+                     &R.n_launches);
   if (rc) return rc;
   CU(h, cudaEventRecord(h->ev[2], h->stream));
-  std::vector<uint64_t> lost_host((size_t)a->n_bins * h->N);
-  CU(h, cudaMemcpyAsync(lost_host.data(), h->lost_dev, sizeof(uint64_t) * lost_host.size(), cudaMemcpyDeviceToHost, h->stream));
-  CU(h, cudaEventRecord(h->ev[3], h->stream));
-  CU(h, cudaStreamSynchronize(h->stream));
-  h->last_trace_bins = a->n_bins;
-  h->ray_hi += a->rays_per_emitter;
-  if (lost_out) std::memcpy(lost_out, lost_host.data(), sizeof(uint64_t) * lost_host.size());
-  rc = collect_recorder(h, a, rec, n_slots, h->stream, false);
-  if (rc) return rc;
-  if (st) {
-    fill_stats(st, pl, a);
-    float ms = 0;
-    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); st->kernel_ms = ms;
-    CU(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[3])); st->total_ms = ms;
-    int64_t nl = 0;
-    for (uint64_t v : lost_host) nl += (int64_t)v;
-    st->rays_lost = nl;
-    st->n_launches = n_launches;
-  }
-  return RTHX_OK;
+  if ((rc = read_lost(h, a, h->stream, R))) return rc;
+  resume_resident(h, std::move(kept), a);
+  return finish_trace(h, a, R, lost_out, rec, st);
 }
 }  // namespace
 
@@ -1838,8 +1837,7 @@ extern "C" int rthx_trace_exchange_sparse(rthx_handle* h, const rthx_trace_args*
   if (a->mode != RTHX_FIRST_INTERACTION)
     return fail(h, RTHX_ERR_ARG, "trace_sparse: the hashed tally supports RTHX_FIRST_INTERACTION only (trace MULTI_BOUNCE with rthx_trace_exchange)");
   CU(h, cudaSetDevice(h->device));
-  // whatever counts were resident (dense or sparse) are void from here on
-  h->last_trace_bins = 0; h->csr_bin = -1; h->csc_bin = -1; h->sparse_counts = false; h->sk_nnz = 0;
+  drop_resident(h);                  // whatever counts were resident (dense or sparse) are void from here on
   SparseRun R;
   rc = sparse_trace_rows(h, a, rec, &h->sk_keys, &h->sk_keys_cap, &h->sk_vals, &h->sk_vals_cap, R);
   if (rc) return rc;
@@ -1854,27 +1852,24 @@ extern "C" int rthx_trace_exchange_continue(rthx_handle* h, const rthx_trace_arg
   rc = check_continue(h, a);
   if (rc) return rc;
   CU(h, cudaSetDevice(h->device));
-  if (h->sparse_counts) return continue_sparse(h, a, lost_out, rec, st, sst);
+  if (h->res.kind == RESIDENT_SPARSE) return continue_sparse(h, a, lost_out, rec, st, sst);
   if (sst) std::memset(sst, 0, sizeof(*sst));
-  if (h->res_rows)                  // a rows trace continues its own list (on the device since that trace)
+  if (h->res.own.listed)             // a rows trace continues its own list (on the device since that trace)
     for (int32_t k = 0; k < a->n_rec_ids; ++k)
       if (!std::binary_search(h->rows.begin(), h->rows.end(), a->rec_ids[k]))
         return fail(h, RTHX_ERR_ARG, "trace_continue: rec_ids[" + std::to_string(k) + "] = " + std::to_string(a->rec_ids[k]) +
                                          " is not in the emitter list of the resident rows trace");
-  RowsScope scope(h, h->res_rows);
   return continue_dense(h, a, lost_out, rec, st);
 }
 
 namespace {
 
 // Per-device outcome of rthx_trace_exchange_multi (one host thread drives each device).
-struct MultiJob {
+struct MultiJob : TraceRun {
   int rc = RTHX_OK;
   std::string err;
-  LaunchPlan plan{};
-  int slots = 0, batches = 1, launches = 0;
-  double kernel_ms = 0, total_ms = 0;
-  std::vector<uint64_t> lost;
+  int batches = 1;
+  double total_ms = 0;
 };
 
 // Recorder read-back of one device in a multi-device trace: every device holds slots for all recorded elements, only the rows it
@@ -1938,11 +1933,10 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
   if (gather) {
     // the full matrix lives on hs[0]; the other devices need peer access to it
     CU(h0, cudaSetDevice(h0->device));
-    h0->last_trace_bins = 0; h0->csr_bin = -1; h0->csc_bin = -1; h0->sparse_counts = false;
+    for (int i = 0; i < n; ++i) drop_resident(hs[i]);
     CU(h0, ensure(&h0->counts_dev, &h0->counts_cap, (size_t)a->n_bins * (size_t)N * N));
     shared_counts = h0->counts_dev;
     for (int i = 1; i < n; ++i) {
-      hs[i]->last_trace_bins = 0; hs[i]->csr_bin = -1; hs[i]->csc_bin = -1; hs[i]->sparse_counts = false;
       if (hs[i]->device == h0->device) continue;
       int can = 0;
       CU(h0, cudaDeviceCanAccessPeer(&can, hs[i]->device, h0->device));
@@ -1961,24 +1955,23 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
     auto run = [&]() -> int {
       CU(h, cudaSetDevice(h->device));
       CU(h, cudaEventRecord(h->ev[0], h->stream));
-      int r = prepare_recorder(h, a, rec, &J.slots, h->stream);
+      int r = prepare_recorder(h, a, rec, &J.n_slots, h->stream);
       if (r) return r;
+      const OwnedRows own{i, n, false};
       if (gather) {
         CU(h, cudaEventRecord(h->ev[1], h->stream));
-        r = enqueue_trace(h, a, i, n, /*compact=*/false, shared_counts, h0->lost_dev, RTHX_ZERO_OWN_ROWS, rec != nullptr, J.slots, h->stream, &J.plan, &J.launches);
+        r = enqueue_trace(h, a, own, /*compact=*/false, shared_counts, h0->lost_dev, RTHX_ZERO_OWN_ROWS, rec != nullptr, J.n_slots, h->stream, &J.pl,
+                          &J.n_launches);
         if (r) return r;
         CU(h, cudaEventRecord(h->ev[2], h->stream));
         CU(h, cudaEventRecord(h->ev[3], h->stream));
         CU(h, cudaStreamSynchronize(h->stream));
       } else {
-        r = pipeline_launch(h, a, i, n, rec != nullptr, J.slots, &J.plan, &J.launches, &J.batches);
+        r = pipeline_launch(h, a, own, rec != nullptr, J.n_slots, &J.pl, &J.n_launches, &J.batches);
         if (r) return r;
-        r = pipeline_copy(h, a, i, n, J.plan.n_owned, counts_out, J.batches);
+        r = pipeline_copy(h, a, i, n, J.pl.n_owned, counts_out, J.batches);
         if (r) return r;
-        J.lost.resize(lost_n);
-        CU(h, cudaMemcpyAsync(J.lost.data(), h->lost_dev, sizeof(uint64_t) * lost_n, cudaMemcpyDeviceToHost, h->copy_stream));
-        CU(h, cudaEventRecord(h->ev[3], h->copy_stream));
-        CU(h, cudaStreamSynchronize(h->copy_stream));
+        if ((r = read_lost(h, a, h->copy_stream, J))) return r;
         CU(h, cudaStreamSynchronize(h->stream));
       }
       float ms = 0;
@@ -2006,8 +1999,7 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
   if (gather) {
     CU(h0, cudaSetDevice(h0->device));
     CU(h0, cudaMemcpy(lost_sum.data(), h0->lost_dev, sizeof(uint64_t) * lost_n, cudaMemcpyDeviceToHost));
-    h0->last_trace_bins = a->n_bins; h0->last_trace_rows = (size_t)N; h0->last_rank = 0; h0->last_world = 1; h0->res_rows = false;
-    record_resident(h0, a, RESIDENT_MULTI);
+    set_resident(h0, a, RESIDENT_MULTI, OwnedRows{}, N);
   } else {
     for (int i = 0; i < n; ++i)
       for (size_t k = 0; k < lost_n; ++k) lost_sum[k] += jobs[i].lost[k];
@@ -2018,7 +2010,7 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
     std::vector<RecChunk> chunks;
     for (int i = 0; i < n; ++i) {
       CU(h0, cudaSetDevice(hs[i]->device));
-      rc = gather_recorder(hs[i], a, i, n, jobs[i].slots, chunks);
+      rc = gather_recorder(hs[i], a, i, n, jobs[i].n_slots, chunks);
       if (rc) return fail(h0, rc, hs[i]->err);
     }
     std::sort(chunks.begin(), chunks.end(), [](const RecChunk& x, const RecChunk& y) { return x.elem < y.elem; });
@@ -2032,16 +2024,12 @@ extern "C" int rthx_trace_exchange_multi(rthx_handle** hs, int n, const rthx_tra
   }
   if (lost_out) std::memcpy(lost_out, lost_sum.data(), sizeof(uint64_t) * lost_n);
   if (st) {
-    fill_stats(st, jobs[0].plan, a);
-    st->rays_traced = (int64_t)N * a->n_bins * a->rays_per_emitter;
-    int64_t nl = 0;
-    for (uint64_t v : lost_sum) nl += (int64_t)v;
-    st->rays_lost = nl;
     int nbk = 0, nlaunch = 0;
     double kmax = 0, tmax = 0;
-    for (auto& J : jobs) { nbk += J.plan.n_blocks; nlaunch += J.launches; kmax = std::max(kmax, J.kernel_ms); tmax = std::max(tmax, J.total_ms); }
-    st->n_blocks = nbk; st->n_launches = nlaunch;
-    st->kernel_ms = kmax; st->total_ms = tmax;     // the slowest device
+    for (auto& J : jobs) { nbk += J.pl.n_blocks; nlaunch += J.n_launches; kmax = std::max(kmax, J.kernel_ms); tmax = std::max(tmax, J.total_ms); }
+    fill_stats(st, a, jobs[0].pl, lost_sum, nlaunch, kmax, tmax);     // times: the slowest device
+    st->rays_traced = (int64_t)N * a->n_bins * a->rays_per_emitter;
+    st->n_blocks = nbk;
   }
   return RTHX_OK;
 }
@@ -2305,15 +2293,46 @@ int copy_out(rthx_handle* h, void* dst, const void* src_dev, size_t bytes, cudaS
   return copy_out_2d(h, dst, bytes, src_dev, bytes, bytes, 1, stream);
 }
 
+// The read-outs of the resident counts
+enum ReadOut { READ_ROWS, READ_COLUMNS, READ_SMOOTH, READ_SMOOTH_SPARSE };
+
+// Precondition of a read-out of the resident counts of `bin`.  The row read-outs take any resident rows.  The others need the whole
+// matrix: not the rows of a shard, but the listed rows of a rows trace (its other rows are empty).  rthx_smooth_F / _DkAP take the
+// dense form only.  The smoothings read the leading n x n block, so after a rows trace every row < n must be listed: resident row
+// y < n is then element y, and the block lies where it lies after a full trace.
+int need_resident(rthx_handle* h, ReadOut what, int bin, int n = 0) {
+  const Resident& r = h->res;
+  const bool have = r.kind != RESIDENT_NONE && bin >= 0 && bin < r.n_bins();
+  const bool shard = !r.own.listed && r.own.world != 1;
+  if (what == READ_COLUMNS && shard)
+    return fail(h, RTHX_ERR_ARG, "counts_csc: the resident counts are the rows of a shard (emitter_world > 1); the column view needs the whole matrix");
+  if (what == READ_ROWS || what == READ_COLUMNS)
+    return have ? RTHX_OK : fail(h, RTHX_ERR_ARG, "counts: no resident counts for that bin (run rthx_trace_exchange with counts_out == NULL, rthx_trace_exchange_multi with counts_out == NULL, or rthx_trace_exchange_sparse first)");
+  const std::string who = what == READ_SMOOTH ? "smooth" : "smooth_sparse";
+  if (what == READ_SMOOTH && r.kind == RESIDENT_SPARSE)
+    return fail(h, RTHX_ERR_ARG, "smooth: the resident counts are the sparse form of rthx_trace_exchange_sparse (smooth them with rthx_smooth_sparse)");
+  if (!have || n > h->N || shard) return fail(h, RTHX_ERR_ARG, who + ": no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
+  if (r.own.listed)
+    for (int y = 0; y < n; ++y)
+      if (y >= (int)h->rows.size() || h->rows[y] != y)
+        return fail(h, RTHX_ERR_ARG, who + ": row " + std::to_string(y) + " of the crop n = " + std::to_string(n) +
+                                         " was not traced (it is not in the emitter list of the resident rows trace)");
+  return RTHX_OK;
+}
+
+// The dense resident counts of `bin`: n_rows rows of N
+const unsigned long long* resident_counts(const rthx_handle* h, int bin) { return h->counts_dev + (size_t)bin * h->res.n_rows * h->N; }
+
 // Row pass over the resident counts of `bin`: non-zeros and total per row, row pointers on the device, and the surface-gas
 // cross-coupling chi of the row-normalised F (cross_coupling_chi, smoothExchangeFactors.jl:212-241).  After a sharded trace
 // (emitter_world > 1: one row tile of a matrix too large to hold at once) the rows are those of the shard and chi is their share.
 int prepare_rows(rthx_handle* h, int bin) {
-  if (bin < 0 || bin >= h->last_trace_bins || (!h->counts_dev && !h->sparse_counts))
-    return fail(h, RTHX_ERR_ARG, "counts: no resident counts for that bin (run rthx_trace_exchange with counts_out == NULL, rthx_trace_exchange_multi with counts_out == NULL, or rthx_trace_exchange_sparse first)");
+  const int rc = need_resident(h, READ_ROWS, bin);
+  if (rc) return rc;
   if (h->csr_bin == bin) return RTHX_OK;
   CU(h, cudaSetDevice(h->device));
-  const int N = h->N, R = (int)h->last_trace_rows;
+  const Resident& res = h->res;
+  const int N = h->N, R = res.n_rows;
   if (h->csr_cap < (size_t)N + 1) {
     cudaFree(h->csr_nnz); cudaFree(h->csr_rowsum); cudaFree(h->csr_rowptr); cudaFree(h->csr_cross);
     h->csr_nnz = nullptr; h->csr_rowsum = nullptr; h->csr_rowptr = nullptr; h->csr_cross = nullptr; h->csr_cap = 0;
@@ -2323,13 +2342,12 @@ int prepare_rows(rthx_handle* h, int bin) {
     CU(h, cudaMalloc(&h->csr_rowptr, sizeof(long long) * ((size_t)N + 1)));
     h->csr_cap = (size_t)N + 1;
   }
-  if (h->sparse_counts) {
-    CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, R, N, h->ns, h->last_rank, h->last_world, h->csr_nnz,
+  if (res.kind == RESIDENT_SPARSE) {
+    CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, res.n_bins(), bin, R, N, h->ns, res.own.rank, res.own.world, h->csr_nnz,
                                 h->csr_rowsum, h->csr_cross, h->stream));
   } else {
-    const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
-    CU(h, rthx::launch_row_nnz(c, R, N, (size_t)N, h->ns, h->last_rank, h->last_world, h->res_rows ? h->rows_dev : nullptr, h->csr_nnz, h->csr_rowsum,
-                               h->csr_cross, h->stream));
+    CU(h, rthx::launch_row_nnz(resident_counts(h, bin), R, N, (size_t)N, h->ns, res.own.rank, res.own.world, res.own.listed ? h->rows_dev : nullptr,
+                               h->csr_nnz, h->csr_rowsum, h->csr_cross, h->stream));
   }
   std::vector<int> nnz(std::max(R, 1));
   std::vector<unsigned long long> rowsum(std::max(R, 1)), cross(std::max(R, 1));
@@ -2364,10 +2382,10 @@ namespace {
 // rowval -> sp_rowval, F = count / row total over the block -> sp_val (the values rthx_counts_csc computes); *nnz_out its non-zeros.
 // The CSR of the block is transposed by the radix sort of rthx_smooth_sparse (sparse_transpose), so rows ascend within each column.
 // With counts != nullptr the count of every entry (as bits) is sorted along instead of F.  vec: 3 n scratch words.
-int sparse_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long long* rptr, void* vec, bool counts, long long* nnz_out) {
+int hashed_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long long* rptr, void* vec, bool counts, long long* nnz_out) {
   unsigned long long* rowsum = reinterpret_cast<unsigned long long*>(vec);
   int* row_nnz = reinterpret_cast<int*>(rowsum + n);
-  CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, n, n, h->ns, 0, 1, row_nnz, rowsum, nullptr, h->stream));
+  CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, n, n, h->ns, 0, 1, row_nnz, rowsum, nullptr, h->stream));
   std::vector<int> rn((size_t)n);
   CU(h, cudaMemcpyAsync(rn.data(), row_nnz, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaStreamSynchronize(h->stream));
@@ -2382,7 +2400,7 @@ int sparse_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long lon
   CU(h, ensure(&h->sp_keys, &h->sp_keys_cap, 2 * nz1));
   const size_t tmp_bytes = rthx::sparse_sort_temp_bytes((int)nnz, n);
   CU(h, ensure(reinterpret_cast<char**>(&h->sp_tmp), &h->sp_tmp_cap, tmp_bytes));
-  CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, n, n, rptr, rowsum, true, h->sp_rowval,
+  CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, n, n, rptr, rowsum, true, h->sp_rowval,
                              counts ? reinterpret_cast<unsigned long long*>(h->sp_val) : nullptr, counts ? nullptr : h->sp_val, h->stream));
   CU(h, rthx::sparse_transpose(n, (int)nnz, rptr, h->sp_rowval, h->sp_val, h->sp_keys, h->sp_keys + nz1, h->sp_val + nz1, cp, h->sp_tmp, tmp_bytes,
                                h->stream));
@@ -2403,11 +2421,11 @@ int counts_csc_sparse(rthx_handle* h, int bin, int index_base, int rowval_is_i64
   long long* rptr = reinterpret_cast<long long*>(h->csr_out);
   void* vec = rptr + (size_t)N + 1;
   long long nnz = 0;
-  int rc = sparse_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, false, &nnz);
+  int rc = hashed_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, false, &nnz);
   if (rc) return rc;
   if (F_vals && nnz && (rc = copy_out(h, F_vals, h->sp_val + std::max<long long>(nnz, 1), sizeof(double) * (size_t)nnz, h->stream))) return rc;
   if (vals) {                                                // the counts ride along a second sort of the same keys
-    if ((rc = sparse_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, true, &nnz))) return rc;
+    if ((rc = hashed_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, true, &nnz))) return rc;
     if (nnz && (rc = copy_out(h, vals, h->sp_val + std::max<long long>(nnz, 1), sizeof(uint64_t) * (size_t)nnz, h->stream))) return rc;
   }
   const size_t nz1 = (size_t)std::max<long long>(nnz, 1);
@@ -2454,13 +2472,12 @@ extern "C" int rthx_counts_csr(rthx_handle* h, int bin, int64_t* row_ptr, int32_
   unsigned long long* d_vals = (unsigned long long*)h->csr_out;
   double* d_f = (double*)(d_vals + std::max<size_t>(1, nnz));
   int* d_cols = (int*)(d_f + std::max<size_t>(1, nnz));
-  const int R = (int)h->last_trace_rows;
-  if (h->sparse_counts) {
-    CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->last_trace_bins, bin, R, N, h->csr_rowptr, h->csr_rowsum, false, d_cols, d_vals,
+  const int R = h->res.n_rows;
+  if (h->res.kind == RESIDENT_SPARSE) {
+    CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, R, N, h->csr_rowptr, h->csr_rowsum, false, d_cols, d_vals,
                                F_vals ? d_f : nullptr, h->stream));
   } else {
-    const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
-    CU(h, rthx::launch_row_fill(c, R, N, (size_t)N, h->csr_rowptr, h->csr_rowsum, d_cols, d_vals, F_vals ? d_f : nullptr, h->stream));
+    CU(h, rthx::launch_row_fill(resident_counts(h, bin), R, N, (size_t)N, h->csr_rowptr, h->csr_rowsum, d_cols, d_vals, F_vals ? d_f : nullptr, h->stream));
   }
   rc = copy_out(h, row_ptr, h->csr_rowptr, sizeof(long long) * ((size_t)R + 1), h->stream);
   if (rc) return rc;
@@ -2475,16 +2492,15 @@ extern "C" int rthx_counts_csr(rthx_handle* h, int bin, int64_t* row_ptr, int32_
 
 extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, uint64_t* vals, double* F_vals) {
   if (!h || !colptr || !rowval || (index_base != 0 && index_base != 1)) return RTHX_ERR_ARG;
-  if (h->last_trace_bins > 0 && !h->res_rows && (h->last_world != 1 || (int)h->last_trace_rows != h->N))
-    return fail(h, RTHX_ERR_ARG, "counts_csc: the resident counts are the rows of a shard (emitter_world > 1); the column view needs the whole matrix");
-  int rc = prepare_rows(h, bin);              // row totals for the normalisation, nnz for the buffer sizes
+  int rc = need_resident(h, READ_COLUMNS, bin);
   if (rc) return rc;
+  if ((rc = prepare_rows(h, bin))) return rc;   // row totals for the normalisation, nnz for the buffer sizes
   CU(h, cudaSetDevice(h->device));
   const int N = h->N;
   const size_t nnz = (size_t)h->csr_total, nz1 = std::max<size_t>(1, nnz);
   if (!rowval_is_i64 && (size_t)N + (size_t)index_base > 0x7FFFFFFFull) return fail(h, RTHX_ERR_ARG, "counts_csc: 32-bit row indices overflow");
-  if (h->sparse_counts) { rc = counts_csc_sparse(h, bin, index_base, rowval_is_i64, colptr, rowval, vals, F_vals); if (rc) return rc; h->csc_bin = bin; return RTHX_OK; }
-  const int R = (int)h->last_trace_rows;                      // N, or the listed rows of a rows trace (the other rows are empty)
+  if (h->res.kind == RESIDENT_SPARSE) return counts_csc_sparse(h, bin, index_base, rowval_is_i64, colptr, rowval, vals, F_vals);
+  const int R = h->res.n_rows;                                // N, or the listed rows of a rows trace (the other rows are empty)
   const int n_tiles = (R + 63) / 64;
   CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)std::max(n_tiles, 1) * (size_t)N));
   CU(h, ensure(&h->csc_colptr, &h->csc_colptr_cap, (size_t)N + 1));
@@ -2497,9 +2513,9 @@ extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowv
   long long* d_rows = (long long*)h->csr_out;                 // 8 bytes per entry reserved, holds int or long long indices
   unsigned long long* d_vals = vals ? (unsigned long long*)(d_rows + nz1) : nullptr;
   double* d_f = F_vals ? (double*)(d_rows + nz1 + (vals ? nz1 : 0)) : nullptr;
-  const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * N;
+  const unsigned long long* c = resident_counts(h, bin);
   CU(h, rthx::launch_csc_count(c, R, N, (size_t)N, h->csc_partial, h->csc_colptr, h->stream));
-  CU(h, rthx::launch_csc_fill(c, R, N, (size_t)N, h->res_rows ? h->rows_dev : nullptr, h->csc_partial, h->csc_colptr, h->csr_rowsum, index_base, d_rows,
+  CU(h, rthx::launch_csc_fill(c, R, N, (size_t)N, h->res.own.listed ? h->rows_dev : nullptr, h->csc_partial, h->csc_colptr, h->csr_rowsum, index_base, d_rows,
                               rowval_is_i64 != 0, d_vals, d_f, h->stream));
   if (index_base) CU(h, rthx::launch_add_base(h->csc_colptr, N + 1, (long long)index_base, h->stream));
   if ((rc = copy_out(h, colptr, h->csc_colptr, sizeof(long long) * ((size_t)N + 1), h->stream))) return rc;
@@ -2509,7 +2525,6 @@ extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowv
     if (F_vals && (rc = copy_out(h, F_vals, d_f, sizeof(double) * nnz, h->stream))) return rc;
   }
   CU(h, cudaStreamSynchronize(h->stream));
-  h->csc_bin = bin;
   return RTHX_OK;
 }
 
@@ -2528,19 +2543,6 @@ cudaError_t run_dykstra(const unsigned long long* src_counts, const double* src_
 cudaError_t time_scale_pass(double* X, double* u, double* r, int n, size_t ldx, int reps, cudaStream_t st, cudaEvent_t e0, cudaEvent_t e1, double* ms_per_pass);
 }  // namespace rthx
 
-namespace {
-// After a rows trace the crop n of a FROM_LAST_TRACE smoothing must be traced in full: rows 0..n-1 listed, so that resident row y < n is
-// element y and the leading n x n block lies where it lies after a full trace
-int check_crop_rows(rthx_handle* h, int n, const char* who) {
-  if (!h->res_rows) return RTHX_OK;
-  for (int y = 0; y < n; ++y)
-    if (y >= (int)h->rows.size() || h->rows[y] != y)
-      return fail(h, RTHX_ERR_ARG, std::string(who) + ": row " + std::to_string(y) + " of the crop n = " + std::to_string(n) +
-                                       " was not traced (it is not in the emitter list of the resident rows trace)");
-  return RTHX_OK;
-}
-}  // namespace
-
 extern "C" int rthx_smooth_F(rthx_handle* h, int source, const void* src_host, int bin, int n, const double* w, int max_iters, double target,
                              int measure_pass, double* F_out, rthx_smooth_stats* st) {
   return rthx_smooth_DkAP(h, source, src_host, bin, n, w, 0, max_iters, target, measure_pass, F_out, st);
@@ -2556,13 +2558,9 @@ extern "C" int rthx_smooth_DkAP(rthx_handle* h, int source, const void* src_host
   const double* src_F = nullptr;
   size_t ld = (size_t)n;
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
-    if (h->sparse_counts)
-      return fail(h, RTHX_ERR_ARG, "smooth: the resident counts are the sparse form of rthx_trace_exchange_sparse (smooth them with rthx_smooth_sparse)");
-    if (bin < 0 || bin >= h->last_trace_bins || !h->counts_dev || n > h->N || (!h->res_rows && (h->last_world != 1 || (int)h->last_trace_rows != h->N)))
-      return fail(h, RTHX_ERR_ARG, "smooth: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
-    const int rc = check_crop_rows(h, n, "smooth");
+    const int rc = need_resident(h, READ_SMOOTH, bin, n);
     if (rc) return rc;
-    src_counts = h->counts_dev + (size_t)bin * h->last_trace_rows * h->N;
+    src_counts = resident_counts(h, bin);
     ld = (size_t)h->N;
   } else if (source == RTHX_SMOOTH_FROM_COUNTS || source == RTHX_SMOOTH_FROM_F) {
     if (!src_host) return fail(h, RTHX_ERR_ARG, "smooth: src_host is NULL");
@@ -2642,10 +2640,7 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
   if (n < 1 || !w || !nnz_out || max_iters < 0) return fail(h, RTHX_ERR_ARG, "smooth_sparse: bad argument");
   long long nnz_f = 0;
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
-    if (bin < 0 || bin >= h->last_trace_bins || (!h->counts_dev && !h->sparse_counts) || n > h->N ||
-        (!h->res_rows && (h->last_world != 1 || (int)h->last_trace_rows != h->N)))
-      return fail(h, RTHX_ERR_ARG, "smooth_sparse: no resident counts for that bin (run rthx_trace_exchange on all emitters first)");
-    const int rc = check_crop_rows(h, n, "smooth_sparse");
+    const int rc = need_resident(h, READ_SMOOTH_SPARSE, bin, n);
     if (rc) return rc;
   } else if (source == RTHX_SMOOTH_FROM_CSC) {
     // the whole matrix is checked here, before anything is uploaded: a bad index must never reach a kernel
@@ -2674,16 +2669,16 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
   double* vec = w_dev + n;                                     // r | u | u' | part | scalars
   CU(h, cudaMemcpyAsync(w_dev, w, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
   CU(h, cudaEventRecord(h->ev[0], h->stream));
-  if (source == RTHX_SMOOTH_FROM_LAST_TRACE && h->sparse_counts) {
+  if (source == RTHX_SMOOTH_FROM_LAST_TRACE && h->res.kind == RESIDENT_SPARSE) {
     // the hashed tally's rows cropped to n, F = count / row total over the crop, transposed to CSC (same values and order as below)
-    int rc = sparse_counts_to_csc(h, bin, n, cp, rptr, vec + n, false, &nnz_f);
+    int rc = hashed_counts_to_csc(h, bin, n, cp, rptr, vec + n, false, &nnz_f);
     if (rc) return rc;
     const size_t nz1 = (size_t)std::max<long long>(nnz_f, 1);
     CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz_f, 0, h->sp_rowval, false, h->stream));
     if (nnz_f) CU(h, cudaMemcpyAsync(h->sp_val, h->sp_val + nz1, sizeof(double) * (size_t)nnz_f, cudaMemcpyDeviceToDevice, h->stream));
   } else if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
     // F = counts / row total over the crop, compacted to CSC by the read-out kernels of rthx_counts_csc
-    const unsigned long long* c = h->counts_dev + (size_t)bin * h->last_trace_rows * h->N;
+    const unsigned long long* c = resident_counts(h, bin);
     const size_t ld = (size_t)h->N;
     unsigned long long* rowsum = reinterpret_cast<unsigned long long*>(vec + n);   // u and u' are free until the iteration
     int* row_nnz = reinterpret_cast<int*>(vec + 2 * (size_t)n);
