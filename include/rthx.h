@@ -48,7 +48,7 @@ enum {
  * algebraically later by the unchanged host solver. */
 enum {
   RTHX_FIRST_INTERACTION = 0,
-  /* Optional total-exchange mode (the analogue of method=:direct's traceSingleRay.jl:7-81 without re-emission): after
+  /* Optional total-exchange mode (the analogue of method=:direct's traceSingleRay.jl:7-81 without re-emission; rthx_trace_direct adds it): after
    * every first interaction the ray is absorbed with probability 1 - omega (gas, omega = sigma_s/(kappa+sigma_s)) or
    * epsilon (wall); otherwise it scatters isotropically (isotropicScatter2D.jl:1-4) or is reflected — diffusely about
    * the inward wall normal, or specularly — and is traced on to its next interaction.  counts[i][j] then is the number
@@ -442,6 +442,26 @@ int rthx_trace_exchange_continue(rthx_handle* h, const rthx_trace_args* args, ui
  * rthx_trace_exchange_continue after a resident rows trace continues the same list (the handle keeps it).                [0.3+] */
 int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* args, const int32_t* emitters, int32_t n_emitters,
                              uint64_t* counts_out, uint64_t* lost_out, rthx_rec_out* rec, rthx_stats* stats);
+
+/* method=:direct of the reference's functor, grey: energy bundles traced to absorption, re-emitted by every element whose temperature is
+ * unknown.  Source y is element sources[y] and traces rays[y] bundles (ray ids [ray_id_offset, ray_id_offset + rays[y])) with the events
+ * of RTHX_MULTI_BOUNCE[_SPECULAR] (args->mode).  A bundle absorbed by element k is tallied in row y, column k; if reemit[k] != 0 it then
+ * leaves k again as a fresh emission of k (uniform point, Lambert about the inward normal / isotropic, emission nudge, new free path) and
+ * goes on, else it ends.  Re-emission m of a bundle draws Philox calls 0x8000 + 2m and 0x8001 + 2m (counter word 2 stays the source), so
+ * with no absorption at a re-emitting element the counts are, bit for bit, those of rthx_trace_exchange_rows(sources) with the same mode.
+ * The event counter runs over the whole chain: roulette after 1000 events also ends chains in an enclosure without a sink.
+ *   sources [n_sources]: strictly ascending element indices; rays [n_sources] >= 1; reemit [N] flags; bundle_energy [n_sources] >= 0;
+ *   absorbed_out [N]: Abs_k = sum_y bundle_energy[y] count[y][k], summed on the device in ascending y with every product and sum
+ *       rounded on its own — bit-identical for any launch shape, and to the same sum over rows read out with rthx_counts_csr;
+ *   lost_out [N] (may be NULL): bundles of source element e lost (escaped, roulette, 16000 events); events_out (may be NULL): traversal
+ *       segments of all bundles (one per interaction or loss); stats (may be NULL): rays_traced = sum of rays.
+ * args: n_bins = 1, n_rec_ids = 0, emitter_rank / emitter_world (0, 1); seed, nudge, locator, ray_id_offset, block_threads and
+ * row_chunks as for a trace.  A violation is RTHX_ERR_ARG naming it, with nothing resident changed.  Afterwards the counts of the
+ * sources stay resident as the listed rows of a rows trace: rthx_counts_nnz / _csr / _stats / _csc read them;
+ * rthx_trace_exchange_continue and the smoothings refuse them.                                                          [0.3+] */
+int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* args, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                      const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, uint64_t* lost_out, int64_t* events_out,
+                      rthx_stats* stats);
 
 /* Peer-memory plumbing for the fused flush in one-process-per-GPU runs: rank 0 allocates the UInt64 count matrix
  * with rthx_shared_alloc and publishes the 64-byte CUDA IPC handle; every other rank maps it with rthx_shared_open

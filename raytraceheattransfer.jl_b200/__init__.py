@@ -11,6 +11,7 @@ from ._lib import (make_trace_args, load_library, library_path, build_library, D
 from .tracing import (parallelRayTracing, exchangeRayTracing, computeExchangeFactorsBin, group_uniform_bins,
                       counts_to_F, get_w, get_b)
 from .equilibrium import solveEquilibrium, equilibriumGrey2D, buildSystemMatrix
+from .direct import directRayTracing
 from . import meshes, smoothing
 
 __all__ = [
@@ -18,5 +19,5 @@ __all__ = [
     "flatten_domain", "FlatMesh", "make_trace_args", "load_library", "library_path", "build_library",
     "DeviceTracer", "RthxError", "parallelRayTracing", "exchangeRayTracing", "computeExchangeFactorsBin",
     "group_uniform_bins", "counts_to_F", "get_w", "get_b", "meshes",
-    "solveEquilibrium", "equilibriumGrey2D", "buildSystemMatrix",
+    "solveEquilibrium", "equilibriumGrey2D", "buildSystemMatrix", "directRayTracing",
 ]

@@ -93,6 +93,9 @@ def load_library():
     L.rthx_trace_exchange_rows.restype = C.c_int
     L.rthx_trace_exchange_rows.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, C.c_int32, c_u64p, c_u64p,
                                            C.POINTER(rthx_rec_out), C.POINTER(rthx_stats)]
+    L.rthx_trace_direct.restype = C.c_int
+    L.rthx_trace_direct.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, c_i64p, C.c_int32, C.POINTER(C.c_uint8), c_f64p, c_f64p,
+                                    c_u64p, c_i64p, C.POINTER(rthx_stats)]
     L.rthx_trace_exchange_device.restype = C.c_int
     L.rthx_trace_exchange_device.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int, C.POINTER(rthx_stats)]
@@ -333,6 +336,31 @@ class DeviceTracer:
                                                      lost.ctypes.data_as(c_u64p), C.byref(rec) if rec else None, C.byref(st)))
         self._set_resident(rays_per_emitter, kw, R)
         return _recorded(dict(counts=counts.reshape(nb, R, N) if counts is not None else None, lost=lost, stats=st.as_dict()), rec, origins, endpoints)
+
+    def trace_direct(self, sources, rays, reemit, bundle_energy, specular: bool = False, **kw):
+        """method=:direct on the device (rthx_trace_direct): source y = element sources[y] (strictly ascending) traces rays[y] bundles of
+        energy bundle_energy[y] through the MULTI_BOUNCE events (specular=True: mirror reflection); a bundle absorbed by element k with
+        reemit[k] is emitted again from k.  Keywords of `trace()` (seed, nudge, locator, block_threads, row_chunks, ray_id_offset).
+        Returns dict(absorbed [N] f64 = sum_y bundle_energy[y] counts[y][k] in ascending y, lost [N] u64 per source element,
+        events, stats).  The counts stay resident as the listed rows of a rows trace (`counts_csr()`: R = len(sources) rows)."""
+        from ._abi import RTHX_MULTI_BOUNCE, RTHX_MULTI_BOUNCE_SPECULAR
+        rows = np.ascontiguousarray(sources, dtype=np.int32).ravel()
+        R, N = len(rows), self.n_elements
+        nr = np.ascontiguousarray(rays, dtype=np.int64).ravel()
+        re_ = np.ascontiguousarray(reemit, dtype=np.uint8).ravel()
+        w = np.ascontiguousarray(bundle_energy, dtype=np.float64).ravel()
+        if len(nr) != R or len(w) != R or len(re_) != N:
+            raise ValueError(f"trace_direct: rays and bundle_energy need {R} entries (one per source), reemit {N} (one per element)")
+        args, keep = make_trace_args(0, mode=RTHX_MULTI_BOUNCE_SPECULAR if specular else RTHX_MULTI_BOUNCE, **kw)
+        absorbed = np.empty(N, np.float64)
+        lost = np.empty(N, np.uint64)
+        events = C.c_int64(0)
+        st = rthx_stats()
+        self._check(self._L.rthx_trace_direct(self._h, C.byref(args), rows.ctypes.data_as(c_i32p), nr.ctypes.data_as(c_i64p), R,
+                                              re_.ctypes.data_as(C.POINTER(C.c_uint8)), w.ctypes.data_as(c_f64p), absorbed.ctypes.data_as(c_f64p),
+                                              lost.ctypes.data_as(c_u64p), C.byref(events), C.byref(st)))
+        self._resident = dict(kw={}, hi=0, sparse=False, rows=R)
+        return dict(absorbed=absorbed, lost=lost, events=int(events.value), stats=st.as_dict())
 
     def trace_sparse(self, rays_per_emitter: int, **kw):
         """Blocking trace with the hashed row tally (rthx_trace_exchange_sparse): the counts never exist in dense form and stay on

@@ -39,6 +39,7 @@ struct DevRes {
   uint8_t* rec_valid_dev = nullptr;         size_t rec_valid_cap = 0;
   double* peak_dev = nullptr;
   int32_t* rows_dev = nullptr;              size_t rows_cap = 0;       // emitter list of a rows trace (rthx_trace_exchange_rows)
+  char* dr_buf = nullptr;                   size_t dr_cap = 0;          // rthx_trace_direct: bundles and energy per row, Abs, events, re-emit flags (bytes)
   int* csr_nnz = nullptr;                   size_t csr_cap = 0;        // per-row nnz (int), row totals, row pointers
   unsigned long long* csr_rowsum = nullptr; long long* csr_rowptr = nullptr; unsigned long long* csr_cross = nullptr;
   unsigned int* row_done_dev = nullptr;     size_t row_done_cap = 0;   // fused peer flush: per-row hand-over tickets
@@ -77,7 +78,7 @@ struct DevRes {
 namespace { struct HostImage; }
 
 // where the resident counts come from
-enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4 };
+enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4, RESIDENT_DIRECT = 5 };
 
 // The emitter rows a trace owns: row y is element rank + y * world (a shard), or with `listed` element rows[y] of the handle's emitter
 // list (a rows trace; rank / world are then 0 / 1)
@@ -147,6 +148,7 @@ void devres_free(DevRes& r) {
   cudaFree(r.sp_ptr); cudaFree(r.sp_rowval); cudaFree(r.sp_val); cudaFree(r.sp_keys); cudaFree(r.sp_xcol); cudaFree(r.sp_xval); cudaFree(r.sp_vec); cudaFree(r.sp_tmp);
   cudaFree(r.csr_nnz); cudaFree(r.csr_rowsum); cudaFree(r.csr_rowptr); cudaFree(r.csr_out); cudaFree(r.csr_cross); cudaFree(r.csc_partial); cudaFree(r.csc_colptr); cudaFree(r.row_done_dev);
   cudaFree(r.arena); cudaFree(r.generic_arena); cudaFree(r.counts_dev); cudaFree(r.rec_pts_dev); cudaFree(r.rec_valid_dev); cudaFree(r.peak_dev); cudaFree(r.rows_dev);
+  cudaFree(r.dr_buf);
   for (auto& e : r.ev) if (e) cudaEventDestroy(e);
   for (auto& e : r.bev) if (e) cudaEventDestroy(e);
   for (auto& e : r.cev) if (e) cudaEventDestroy(e);
@@ -1000,6 +1002,8 @@ int check_continue(rthx_handle* h, const rthx_trace_args* a) {
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts come from a host-output trace (counts_out != NULL); trace with counts_out == NULL to continue");
   if (r.kind == RESIDENT_MULTI)
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts were gathered from several devices (rthx_trace_exchange_multi), whose peer hand-over stores rows instead of adding them");
+  if (r.kind == RESIDENT_DIRECT)
+    return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts are those of a direct trace (rthx_trace_direct), which cannot be continued");
   if (a->seed != r.seed) return fail(h, RTHX_ERR_ARG, "trace_continue: seed differs from the resident trace's");
   if (a->nudge != r.nudge) return fail(h, RTHX_ERR_ARG, "trace_continue: nudge differs from the resident trace's");
   if (a->mode != r.mode) return fail(h, RTHX_ERR_ARG, "trace_continue: mode differs from the resident trace's");
@@ -1495,28 +1499,28 @@ std::vector<int4> list_runs(const std::vector<int32_t>& rows) {
 }
 
 // Checks of rthx_trace_exchange_rows that must pass before anything resident changes
-int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n) {
-  if (!emitters || n < 1) return fail(h, RTHX_ERR_ARG, "trace_rows: the emitter list is empty (n_emitters must be >= 1)");
+int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n, const std::string& who = "trace_rows", const char* list = "emitter") {
+  if (!emitters || n < 1) return fail(h, RTHX_ERR_ARG, who + ": the " + list + " list is empty (n_" + list + "s must be >= 1)");
   for (int32_t i = 0; i < n; ++i) {
     if (emitters[i] < 0 || emitters[i] >= h->N)
-      return fail(h, RTHX_ERR_ARG, "trace_rows: emitters[" + std::to_string(i) + "] = " + std::to_string(emitters[i]) + " is outside [0, N = " +
+      return fail(h, RTHX_ERR_ARG, who + ": " + list + "s[" + std::to_string(i) + "] = " + std::to_string(emitters[i]) + " is outside [0, N = " +
                                        std::to_string(h->N) + ")");
     if (i > 0 && emitters[i] <= emitters[i - 1])
-      return fail(h, RTHX_ERR_ARG, "trace_rows: emitters must be strictly ascending (emitters[" + std::to_string(i) + "] = " + std::to_string(emitters[i]) +
+      return fail(h, RTHX_ERR_ARG, who + ": " + list + "s must be strictly ascending (" + list + "s[" + std::to_string(i) + "] = " + std::to_string(emitters[i]) +
                                        " follows " + std::to_string(emitters[i - 1]) + ")");
   }
   if (a->emitter_rank != 0 || a->emitter_world != 1)
-    return fail(h, RTHX_ERR_ARG, "trace_rows: emitter_rank / emitter_world must be (0, 1) with an emitter list");
+    return fail(h, RTHX_ERR_ARG, who + ": emitter_rank / emitter_world must be (0, 1) with " + (list[0] == 'e' ? "an " : "a ") + list + " list");
   for (int32_t k = 0; k < a->n_rec_ids; ++k)
     if (!std::binary_search(emitters, emitters + n, a->rec_ids[k]))
-      return fail(h, RTHX_ERR_ARG, "trace_rows: rec_ids[" + std::to_string(k) + "] = " + std::to_string(a->rec_ids[k]) + " is not in the emitter list");
+      return fail(h, RTHX_ERR_ARG, who + ": rec_ids[" + std::to_string(k) + "] = " + std::to_string(a->rec_ids[k]) + " is not in the " + list + " list");
   const size_t need = (size_t)n * (size_t)h->N * (size_t)a->n_bins;
   if (need > h->counts_cap) {
     size_t free_b = 0, total_b = 0;
     CU(h, cudaMemGetInfo(&free_b, &total_b));
     if ((need - h->counts_cap) * sizeof(unsigned long long) > free_b)
-      return fail(h, RTHX_ERR_NOMEM, "trace_rows: the counts of " + std::to_string(n) + " rows x " + std::to_string(h->N) + " columns x " + std::to_string(a->n_bins) +
-                                         " bins (" + std::to_string(need * 8) + " bytes) do not fit in device memory; split the emitter list");
+      return fail(h, RTHX_ERR_NOMEM, who + ": the counts of " + std::to_string(n) + " rows x " + std::to_string(h->N) + " columns x " + std::to_string(a->n_bins) +
+                                         " bins (" + std::to_string(need * 8) + " bytes) do not fit in device memory; split the " + list + " list");
   }
   return RTHX_OK;
 }
@@ -1545,6 +1549,131 @@ extern "C" int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* a
   CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)n_emitters));
   CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)n_emitters, cudaMemcpyHostToDevice, h->stream));
   return trace_host(h, a, OwnedRows{0, 1, true}, counts_out, lost_out, rec, st);
+}
+
+namespace {
+
+// Bundles a block traces at most with the direct kernel: every bundle tallies at most one absorption per event (< 16001 events), so the
+// block's u32 row histogram cannot wrap
+constexpr long long kDirectRaysPerBlock = 1ll << 17;
+
+// Checks of rthx_trace_direct that must pass before anything resident changes
+int check_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n, const uint8_t* reemit,
+                 const double* energy, const double* absorbed_out) {
+  if (a->mode != RTHX_MULTI_BOUNCE && a->mode != RTHX_MULTI_BOUNCE_SPECULAR)
+    return fail(h, RTHX_ERR_ARG, "trace_direct: mode must be RTHX_MULTI_BOUNCE or RTHX_MULTI_BOUNCE_SPECULAR");
+  if (a->n_bins != 1) return fail(h, RTHX_ERR_ARG, "trace_direct: exactly one bin (n_bins = 1): the direct method is grey");
+  if (a->n_rec_ids != 0) return fail(h, RTHX_ERR_ARG, "trace_direct: recording rays is not available (n_rec_ids must be 0)");
+  if (!rays || !reemit || !energy || !absorbed_out) return fail(h, RTHX_ERR_ARG, "trace_direct: rays, reemit, bundle_energy and absorbed_out must not be NULL");
+  if (a->ray_id_offset < 0) return fail(h, RTHX_ERR_ARG, "trace_direct: ray_id_offset < 0");
+  int rc = check_rows(h, a, sources, n, "trace_direct", "source");
+  if (rc) return rc;
+  for (int32_t i = 0; i < n; ++i) {
+    if (rays[i] < 1 || rays[i] > INT64_MAX - a->ray_id_offset)
+      return fail(h, RTHX_ERR_ARG, "trace_direct: rays[" + std::to_string(i) + "] = " + std::to_string(rays[i]) + " (every source traces >= 1 bundle)");
+    if (!(energy[i] >= 0.0) || !std::isfinite(energy[i]))
+      return fail(h, RTHX_ERR_ARG, "trace_direct: bundle_energy[" + std::to_string(i) + "] is negative or not finite");
+  }
+  return RTHX_OK;
+}
+
+// Launch plan of a direct trace of the listed source rows: the lock-step body with re-emission, histogram in shared memory when the
+// row fits, chunks for the longest row
+LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long long max_rays) {
+  LaunchPlan pl{};
+  pl.n_owned = (int)h->rows.size();
+  pl.block_threads = a->block_threads ? a->block_threads : 256;
+  const size_t coarse_bytes = h->coarse_fits_smem ? sizeof(CoarseDev) * (size_t)h->n_coarse : 0;
+  const size_t hist_bytes = sizeof(uint32_t) * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;
+  bool hist = coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
+  if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) hist = false; }
+  pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0);
+  pl.kernel = TraceKernelSel::direct(hist, h->fast_ok && a->locator != RTHX_LOCATOR_GENERIC);
+  rthx_trace_args longest = *a;
+  longest.rays_per_emitter = max_rays;
+  long long chunks = a->row_chunks > 0 ? a->row_chunks : auto_row_chunks(h, pl, &longest, pl.n_owned);
+  chunks = std::max(chunks, (max_rays + kDirectRaysPerBlock - 1) / kDirectRaysPerBlock);
+  pl.row_chunks = (int)std::min<long long>(chunks, 0x7FFFFFFFll);
+  pl.n_blocks = (long long)pl.n_owned * chunks > 0x7FFFFFFFll ? -1 : (int)(pl.n_owned * chunks);
+  return pl;
+}
+
+}  // namespace
+
+extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                                 const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, uint64_t* lost_out,
+                                 int64_t* events_out, rthx_stats* st) {
+  if (!h) return RTHX_ERR_ARG;
+  int rc = check_args(h, a);
+  if (rc) return rc;
+  CU(h, cudaSetDevice(h->device));
+  rc = check_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out);
+  if (rc) return rc;
+  const int N = h->N, R = n_sources;
+  const long long max_rays = *std::max_element(rays, rays + R);
+  drop_resident(h);                  // the resident counts are replaced from here on
+  h->rows.assign(sources, sources + R);
+  h->row_runs = list_runs(h->rows);
+  const LaunchPlan pl = make_direct_plan(h, a, max_rays);
+  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace_direct: too many bundles for one launch (a launch has at most 2^31 blocks)");
+  if (!pl.kernel.fast) { rc = ensure_generic(h); if (rc) return rc; }
+  // dr_buf: rays [R] i64 | bundle energy [R] f64 | Abs [N] f64 | events u64 | re-emit flags [N] u8
+  const size_t off_w = 8 * (size_t)R, off_abs = off_w + 8 * (size_t)R, off_ev = off_abs + 8 * (size_t)N, off_re = off_ev + 8;
+  CU(h, ensure(&h->dr_buf, &h->dr_cap, off_re + (size_t)N));
+  char* buf = h->dr_buf;
+  CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)R));
+  CU(h, ensure(&h->counts_dev, &h->counts_cap, (size_t)R * N));
+  cudaStream_t s = h->stream;
+  int n_launches = 0;
+  CU(h, cudaEventRecord(h->ev[0], s));
+  CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)R, cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemcpyAsync(buf, rays, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemcpyAsync(buf + off_w, bundle_energy, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemcpyAsync(buf + off_re, reemit, (size_t)N, cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemsetAsync(h->counts_dev, 0, sizeof(unsigned long long) * (size_t)R * N, s));
+  CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)N, s));
+  CU(h, cudaMemsetAsync(buf + off_ev, 0, 8, s));
+  n_launches += 3;
+  TraceParams P;
+  fill_params(h, a, pl, 0, 1, /*compact=*/true, h->counts_dev, h->lost_dev, P);
+  P.dr_rays = reinterpret_cast<const int64_t*>(buf);
+  P.dr_reemit = reinterpret_cast<const uint8_t*>(buf + off_re);
+  P.dr_events = reinterpret_cast<unsigned long long*>(buf + off_ev);
+  CU(h, cudaEventRecord(h->ev[1], s));
+  for (const int4& run : h->row_runs) {      // one launch per arithmetic run of the source list, as rthx_trace_exchange_rows
+    const int4 r = run;
+    rthx_trace_args longest = *a;
+    longest.rays_per_emitter = max_rays;
+    P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r.y));
+    P.emitter_world = r.w; P.emitter_rank = r.z - r.x * r.w;
+    P.y_offset = r.x;
+    if ((long long)r.y * P.row_chunks > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "trace_direct: too many bundles for one launch (a launch has at most 2^31 blocks)");
+    CU(h, launch_trace_exchange(P, pl.kernel, r.y * P.row_chunks, pl.block_threads, pl.smem_bytes, s));
+    ++n_launches;
+  }
+  CU(h, cudaEventRecord(h->ev[2], s));
+  CU(h, launch_direct_absorbed(h->counts_dev, R, N, reinterpret_cast<const double*>(buf + off_w), reinterpret_cast<double*>(buf + off_abs), s));
+  ++n_launches;
+  std::vector<uint64_t> lost(N);
+  unsigned long long events = 0;
+  CU(h, cudaMemcpyAsync(absorbed_out, buf + off_abs, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  CU(h, cudaMemcpyAsync(lost.data(), h->lost_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  CU(h, cudaMemcpyAsync(&events, buf + off_ev, 8, cudaMemcpyDeviceToHost, s));
+  CU(h, cudaEventRecord(h->ev[3], s));
+  CU(h, cudaStreamSynchronize(s));
+  set_resident(h, a, RESIDENT_DIRECT, OwnedRows{0, 1, true}, R);
+  if (lost_out) std::memcpy(lost_out, lost.data(), 8 * (size_t)N);
+  if (events_out) *events_out = (int64_t)events;
+  if (st) {
+    float k_ms = 0, t_ms = 0;
+    CU(h, cudaEventElapsedTime(&k_ms, h->ev[1], h->ev[2]));
+    CU(h, cudaEventElapsedTime(&t_ms, h->ev[0], h->ev[3]));
+    fill_stats(st, a, pl, lost, n_launches, k_ms, t_ms);
+    st->rays_traced = 0;
+    for (int32_t i = 0; i < R; ++i) st->rays_traced += rays[i];
+  }
+  return RTHX_OK;
 }
 
 extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args* a, void* counts_dev, void* lost_dev, void* stream,
@@ -2309,6 +2438,8 @@ int need_resident(rthx_handle* h, ReadOut what, int bin, int n = 0) {
   if (what == READ_ROWS || what == READ_COLUMNS)
     return have ? RTHX_OK : fail(h, RTHX_ERR_ARG, "counts: no resident counts for that bin (run rthx_trace_exchange with counts_out == NULL, rthx_trace_exchange_multi with counts_out == NULL, or rthx_trace_exchange_sparse first)");
   const std::string who = what == READ_SMOOTH ? "smooth" : "smooth_sparse";
+  if (r.kind == RESIDENT_DIRECT)
+    return fail(h, RTHX_ERR_ARG, who + ": the resident counts are those of a direct trace (rthx_trace_direct): absorptions with re-emission, not exchange factors");
   if (what == READ_SMOOTH && r.kind == RESIDENT_SPARSE)
     return fail(h, RTHX_ERR_ARG, "smooth: the resident counts are the sparse form of rthx_trace_exchange_sparse (smooth them with rthx_smooth_sparse)");
   if (!have || n > h->N || shard) return fail(h, RTHX_ERR_ARG, who + ": no resident counts for that bin (run rthx_trace_exchange on all emitters first)");

@@ -128,6 +128,10 @@ struct TraceParams {
   unsigned long long sk_cap;   // pair-buffer capacity
   int32_t sk_slots_log2;       // hash slots per block = 1 << sk_slots_log2 (>= 2 blockDim.x)
   int32_t sk_pad_;
+  // method=:direct (rthx_trace_direct), behind everything else as well
+  const int64_t* dr_rays;      // [listed rows] bundles of source row y
+  const uint8_t* dr_reemit;    // [N] 1: the element's temperature is unknown, a bundle it absorbs is emitted again from it
+  unsigned long long* dr_events;  // [1] traversal segments of all bundles (one per interaction, or per loss)
 };
 
 static_assert(offsetof(TraceParams, rays_per_emitter) % 16 == 0 && offsetof(TraceParams, k_u52) % 16 == 0 && offsetof(TraceParams, rk) % 16 == 0,
@@ -140,6 +144,7 @@ struct TraceKernelSel {
     SQ,         // trace_exchange_sq_kernel: the whole domain is one parallelogram face
     QUEUE,      // trace_exchange_queue_kernel: per-warp ray queue (multi-face meshes; MULTI_BOUNCE on analytic meshes)
     HASH,       // trace_exchange_hash_kernel: hashed row tally (rthx_trace_exchange_sparse)
+    DIRECT,     // trace_direct_kernel: MULTI_BOUNCE with re-emission (rthx_trace_direct)
   };
   Family family = LOCKSTEP;
   bool hist = false;      // row histogram in shared memory (SQ and QUEUE always, HASH never)
@@ -156,6 +161,7 @@ struct TraceKernelSel {
   static constexpr TraceKernelSel sq(bool multi) { return {SQ, true, true, multi, 0, false}; }
   static constexpr TraceKernelSel queue(bool fast, bool multi, int depth, bool general) { return {QUEUE, true, fast, multi, depth, general}; }
   static constexpr TraceKernelSel hash(bool fast) { return {HASH, false, fast, false, 0, false}; }
+  static constexpr TraceKernelSel direct(bool hist, bool fast) { return {DIRECT, hist, fast, true, 0, false}; }
 };
 
 // launchers implemented in rthx_kernels.cu; a selection without a compiled instance fails with cudaErrorInvalidDeviceFunction
@@ -164,6 +170,8 @@ cudaError_t launch_trace_exchange(const TraceParams& p, const TraceKernelSel& k,
 cudaError_t configure_trace_kernel(size_t smem_bytes);
 cudaError_t launch_fp64_peak(double* out, int n_blocks, int block_threads, int iters, cudaStream_t stream);
 int trace_kernel_max_blocks_per_sm(const TraceKernelSel& k, int block_threads, size_t smem_bytes);
+// Abs[k] = sum_i w[i] counts[i][k] over R rows of N, in ascending row order (rthx_trace_direct)
+cudaError_t launch_direct_absorbed(const unsigned long long* counts, int R, int N, const double* w, double* absorbed, cudaStream_t stream);
 constexpr size_t hash_table_bytes(int slots) { return 8 * (size_t)slots + 16; }   // keys + counts (u32 each) + occupied / fill / base words
 
 // hashed row tally, host side of the reduction (rthx_sparse_tally.cu)

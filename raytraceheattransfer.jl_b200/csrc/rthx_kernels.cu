@@ -447,17 +447,97 @@ __device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, uns
 //   both           : [12,13] cell midPoint
 constexpr int EM_DOUBLES = 16;
 
+// method=:direct re-emission: the bundle of source row `count_row` was absorbed by element k, whose temperature is unknown.  The
+// absorption is tallied in column k, and the bundle leaves k again as a fresh emission of k: uniform point of the wall / cell, Lambert
+// direction about the inward normal (wall) or isotropic (gas), emission nudge, new free path — the arithmetic of the block prologue and
+// stage 1 of the trace body, with k's geometry read from the mesh tables instead of shared memory.  Its Philox words are calls
+// 0x8000 + 2m and 0x8001 + 2m (m-th re-emission of the bundle), in the upper half of the call field, disjoint from the event calls
+// 2 + 2n, 3 + 2n (n < 16000).
+template <bool HIST_SMEM>
+__device__ __forceinline__ void direct_reemit(const TraceParams& p, uint32_t* hist, unsigned long long* count_row, int k, uint32_t c_lo,
+                                              uint32_t c_hi, uint32_t e, uint32_t cw, int m, const double2* s_log, double& px, double& py,
+                                              double& dx, double& dy, double& neg_log, int& c) {
+  if (HIST_SMEM) atomicAdd(&hist[k], 1u);
+  else atomicAdd(&count_row[k], 1ULL);
+  const uint4 w0 = philox4x32_10_rk(make_uint4(c_lo, c_hi, e, cw | (uint32_t)(0x8000 + 2 * m)), p.rk);
+  const uint4 w1 = philox4x32_10_rk(make_uint4(c_lo, c_hi, e, cw | (uint32_t)(0x8001 + 2 * m)), p.rk);
+  const int g = __ldg(p.em_cell + k), wall = __ldg(p.em_wall + k);
+  c = __ldg(p.em_coarse + k);
+  const double* vx = p.poly_vx + 4 * g;
+  const double* vy = p.poly_vy + 4 * g;
+  const int nv = __ldg(p.poly_nv + g);
+  double R_S;
+  if (wall >= 0) {
+    const int j = (wall + 1 == nv) ? 0 : wall + 1;
+    const double ex = vx[j] - vx[wall], ey = vy[j] - vy[wall];
+    const double len = sqrt(ex * ex + ey * ey);
+    const double R = u32d(w0.x, p.k_u32);
+    px = fma(ex, R, vx[wall]);
+    py = fma(ey, R, vy[wall]);
+    const float cosT = __fsqrt_rn(u23(w0.y));
+    const float cos2 = __fmul_rn(cosT, cosT);
+    const double sinT = sqrt_pos(1.0 - (double)cos2);
+    const double xdir = sinT * cos2pi_unit((double)u23(w0.z));
+    const double zdir = (double)cosT;
+    dx = (ex / len) * xdir + (-(ey / len)) * zdir;
+    dy = (ey / len) * xdir + (ex / len) * zdir;
+    R_S = u52(w1.x, w1.y, p.k_u52);
+  } else {
+    const double sel = nv == 3 ? 2.0 : 0.5 * (vx[0] * (vy[1] - vy[2]) + vx[1] * (vy[2] - vy[0]) + vx[2] * (vy[0] - vy[1])) / p.cell_volume[g];
+    const int t0 = (u32d(w0.z, p.k_u32) < sel) ? 0 : 2;        // triangle ABC (V0, V1, V2) or CDA (V2, V3, V0)
+    const int t1 = t0 + 1, t2 = (t0 + 2) & 3;
+    const double R1 = u32d(w0.x, p.k_u32), R2 = u32d(w0.y, p.k_u32);
+    const double sq = sqrt_pos(R1);
+    const double a2 = sq * R2, a1 = sq - a2;
+    px = fma(a2, vx[t2] - vx[t0], fma(a1, vx[t1] - vx[t0], vx[t0]));
+    py = fma(a2, vy[t2] - vy[t0], fma(a1, vy[t1] - vy[t0], vy[t0]));
+    const double Rt = u52(w1.x, w1.y, p.k_u52);
+    const double sinT = 2.0 * sqrt_pos(Rt * (1.0 - Rt));
+    dx = sinT * cos2pi_unit(u32d(w0.w, p.k_u32));
+    dy = fma(Rt, -2.0, 1.0);
+    R_S = u52(w1.z, w1.w, p.k_u52);
+  }
+  px = fma(p.cell_mid[2 * g] - px, p.nudge, px);
+  py = fma(p.cell_mid[2 * g + 1] - py, p.nudge, py);
+  neg_log = neg_log_table(R_S, s_log);
+}
+
 template <bool HIST_SMEM, bool FAST, bool MULTI>
 __global__ void __launch_bounds__(256, HIST_SMEM && !MULTI ? 4 : 2) trace_exchange_kernel(const __grid_constant__ TraceParams p) {
-  constexpr bool HASH = false;
+  constexpr bool HASH = false, REEMIT = false;
 #include "rthx_trace_body.cuh"
 }
 
 // the same kernel with the hashed row tally (FIRST_INTERACTION, no histogram; the host rejects MULTI_BOUNCE before a launch)
 template <bool FAST>
 __global__ void __launch_bounds__(256, 2) trace_exchange_hash_kernel(const __grid_constant__ TraceParams p) {
-  constexpr bool HIST_SMEM = false, MULTI = false, HASH = true;
+  constexpr bool HIST_SMEM = false, MULTI = false, HASH = true, REEMIT = false;
 #include "rthx_trace_body.cuh"
+}
+
+// method=:direct (rthx_trace_direct): the MULTI_BOUNCE event loop with re-emission from elements of unknown temperature.  One block
+// per (source row, chunk) of the listed source rows; row y traces p.dr_rays[y] bundles.
+template <bool HIST_SMEM, bool FAST>
+__global__ void __launch_bounds__(256, 2) trace_direct_kernel(const __grid_constant__ TraceParams p) {
+  constexpr bool MULTI = true, HASH = false, REEMIT = true;
+#include "rthx_trace_body.cuh"
+}
+
+// Absorbed power of every element, Abs[k] = sum_i w[i] count[i][k] over the R resident source rows, summed in ascending row order
+// with every product and sum rounded on its own (no FMA contraction): the same sum, bit for bit, as a host loop over the rows.
+__global__ void __launch_bounds__(256) direct_absorbed_kernel(const unsigned long long* __restrict__ counts, int R, int N,
+                                                             const double* __restrict__ w, double* __restrict__ absorbed) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= N) return;
+  double acc = 0.0;
+  for (int i = 0; i < R; ++i) acc = __dadd_rn(acc, __dmul_rn(w[i], (double)counts[(size_t)i * N + k]));
+  absorbed[k] = acc;
+}
+
+cudaError_t launch_direct_absorbed(const unsigned long long* counts, int R, int N, const double* w, double* absorbed, cudaStream_t stream) {
+  if (N <= 0) return cudaSuccess;
+  direct_absorbed_kernel<<<(N + 255) / 256, 256, 0, stream>>>(counts, R, N, w, absorbed);
+  return cudaGetLastError();
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1603,6 +1683,10 @@ static const TraceInstance k_trace_instances[] = {
     {Sel::lockstep(true, true, false), trace_exchange_kernel<true, true, false>},
     {Sel::hash(true), trace_exchange_hash_kernel<true>},
     {Sel::hash(false), trace_exchange_hash_kernel<false>},
+    {Sel::direct(true, true), trace_direct_kernel<true, true>},
+    {Sel::direct(true, false), trace_direct_kernel<true, false>},
+    {Sel::direct(false, true), trace_direct_kernel<false, true>},
+    {Sel::direct(false, false), trace_direct_kernel<false, false>},
 };
 
 static TraceKernel trace_kernel(const TraceKernelSel& k) {

@@ -1,6 +1,6 @@
-// rthx_trace_body.cuh — body of K1 (rthx_kernels.cu), shared by trace_exchange_kernel<HIST_SMEM, FAST, MULTI> and
-// trace_exchange_hash_kernel<FAST>.  It is included INSIDE their function bodies, where HIST_SMEM, FAST, MULTI and HASH
-// are compile-time constants and `p` is the __grid_constant__ parameter: inlining it through a device function taking the
+// rthx_trace_body.cuh — body of K1 (rthx_kernels.cu), shared by trace_exchange_kernel<HIST_SMEM, FAST, MULTI>,
+// trace_exchange_hash_kernel<FAST> and trace_direct_kernel<HIST_SMEM, FAST>.  It is included INSIDE their function bodies, where
+// HIST_SMEM, FAST, MULTI, HASH and REEMIT are compile-time constants and `p` is the __grid_constant__ parameter: inlining it through a device function taking the
 // parameter by reference changed the code ptxas generates for the existing instances, textual inclusion does not.
   extern __shared__ __align__(16) unsigned char smem_raw[];
   CoarseDev* s_coarse = reinterpret_cast<CoarseDev*>(smem_raw);
@@ -59,11 +59,12 @@
     s_em[12] = p.cell_mid[2 * g]; s_em[13] = p.cell_mid[2 * g + 1];
   }
 
-  // ray range of this chunk
-  const int64_t per = (p.rays_per_emitter + p.row_chunks - 1) / p.row_chunks;
+  // ray range of this chunk (REEMIT: every source row has its own bundle count)
+  const int64_t row_rays = REEMIT ? p.dr_rays[y] : p.rays_per_emitter;
+  const int64_t per = (row_rays + p.row_chunks - 1) / p.row_chunks;
   const int64_t r_begin = (int64_t)chunk * per;
   int64_t r_end = r_begin + per;
-  if (r_end > p.rays_per_emitter) r_end = p.rays_per_emitter;
+  if (r_end > row_rays) r_end = row_rays;
 
   const double ub = p.uniform_beta[band];
   const bool uniform = ub > -0.1;                      // traceRay.jl:4
@@ -78,6 +79,7 @@
 
   const uint32_t cw = ((uint32_t)band << 16);
   unsigned int n_lost = 0;
+  [[maybe_unused]] unsigned int n_events = 0;   // REEMIT: traversal segments (one per interaction, or per loss)
   const unsigned long long row_key = HASH ? (unsigned long long)y * (unsigned long long)p.n_bins + (unsigned long long)bi : 0ull;
 
   // HASH: block-synchronous rounds (every thread runs every round; lanes past r_end only take part in the flush)
@@ -136,12 +138,16 @@
     // ---- stage 2: first-interaction traversal (traceRayUniform / traceRayVariable) --------------------------
     // MULTI (RTHX_MULTI_BOUNCE): the traversal is repeated from every scattering / reflection event until the ray is
     // absorbed (traceSingleRay.jl:7-81 without the re-emission branches); otherwise the body runs exactly once.
+    // REEMIT (method=:direct): an absorption by an element of unknown temperature is tallied and the bundle is emitted
+    // again from that element (direct_reemit); the event counter runs on over the whole chain.
     double neg_log = neg_log_table(R_S, s_log);
     int c = c0;
     int absorber = -1;
     double hit_nx = 0.0, hit_ny = 0.0;   // MULTI: outward unit normal of the wall that was hit
+    [[maybe_unused]] int n_reemit = 0;   // REEMIT: re-emissions of this bundle so far
 #pragma unroll 1
     for (int event = 0;; ++event) {
+    if constexpr (REEMIT) ++n_events;
     double S = uniform ? neg_log * inv_beta_u : 0.0;   // remaining free path (uniform); beta = 0 -> Inf
     double acc = 0.0;                                  // accumulated tau (variable)
     absorber = -1;
@@ -217,14 +223,30 @@
     if (event >= 1000 && u32d(v0.w, p.k_u32) > 0.8) { absorber = -1; break; }   // Russian roulette, traceSingleRay.jl:11
     const double dec = u32d(v0.x, p.k_u32);
     if (absorber >= p.n_surfaces) {
-      if (!(dec < p.omega[(size_t)band * p.n_cells + (absorber - p.n_surfaces)])) break;   // absorbed in the gas
+      if (!(dec < p.omega[(size_t)band * p.n_cells + (absorber - p.n_surfaces)])) {        // absorbed in the gas
+        if constexpr (REEMIT) {
+          if (p.dr_reemit[absorber]) {
+            direct_reemit<HIST_SMEM>(p, hist, count_row, absorber, c_lo, c_hi, (uint32_t)e, cw, n_reemit++, s_log, px, py, dx, dy, neg_log, c);
+            continue;
+          }
+        }
+        break;
+      }
       // isotropicScatter2D.jl:1-4: theta = acos(2R-1), phi = 2 pi R
       const double Rt = u52(v1.x, v1.y, p.k_u52);
       const double sinT = 2.0 * sqrt(Rt * (1.0 - Rt));
       dx = sinT * cospi(2.0 * u32d(v0.y, p.k_u32));
       dy = fma(Rt, 2.0, -1.0);
     } else {
-      if (dec < p.eps[(size_t)band * p.n_surfaces + absorber]) break;                       // absorbed by the wall
+      if (dec < p.eps[(size_t)band * p.n_surfaces + absorber]) {                           // absorbed by the wall
+        if constexpr (REEMIT) {
+          if (p.dr_reemit[absorber]) {
+            direct_reemit<HIST_SMEM>(p, hist, count_row, absorber, c_lo, c_hi, (uint32_t)e, cw, n_reemit++, s_log, px, py, dx, dy, neg_log, c);
+            continue;
+          }
+        }
+        break;
+      }
       if (p.specular) {
         const double dn = dx * hit_nx + dy * hit_ny;            // mirror the in-plane components; the axial one is unchanged
         dx = fma(-2.0 * dn, hit_nx, dx);
@@ -267,6 +289,7 @@
     if (p.flush_system) atomicAdd_system(&p.lost[(size_t)bi * N + e], (unsigned long long)n_lost);
     else atomicAdd(&p.lost[(size_t)bi * N + e], (unsigned long long)n_lost);
   }
+  if constexpr (REEMIT) { if (n_events) atomicAdd(p.dr_events, (unsigned long long)n_events); }
   if (HIST_SMEM) {
     __syncthreads();
     if (p.peer_counts != nullptr) { handover_row_hist(p, hist, reinterpret_cast<unsigned int*>(s_em + 15) + 1); return; }

@@ -472,10 +472,13 @@ def exchangeRayTracing(rtm, rays_tot: int, nudge: Optional[float], max_iters: in
 def dispatch_ray_trace(rtm, rays_tot: int, method: str = "exchange", nudge: Optional[float] = None,
                        k_dykstra=None, max_iters: int = 1000, verbose: bool = True, rec=None, **kw):
     """(rtm)(rays_tot; method, nudge, k_dykstra, max_iters, verbose, rec) — multiDispatchRayTrace2D.jl:1-18.  New keyword
-    refine=True (method=:exchange): add rays_tot // N rays per emitter to the previous call's trace and smooth again (parallelRayTracing)."""
+    refine=True (method=:exchange): add rays_tot // N rays per emitter to the previous call's trace and smooth again (parallelRayTracing).
+    method=:direct traces energy bundles with re-emission and writes the temperatures itself (direct.directRayTracing; grey domains;
+    keywords seed, device / devices, locator, specular)."""
     method = method.lstrip(":")
     if method == "exchange":
         return exchangeRayTracing(rtm, rays_tot, nudge, max_iters, k_dykstra, verbose, rec, **kw)
     if method == "direct":
-        raise NotImplementedError("method=:direct is outside the scope of this drop-in (exchange path only)")
+        from .direct import directRayTracing
+        return directRayTracing(rtm, rays_tot, nudge, verbose, rec, **kw)
     raise ValueError(f"Unknown ray tracing method: {method}, must be :exchange or :direct")
