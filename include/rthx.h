@@ -463,6 +463,20 @@ int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* args, const int32_t
                       const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, uint64_t* lost_out, int64_t* events_out,
                       rthx_stats* stats);
 
+/* rthx_trace_direct with the redirection tally, for the radiosity, irradiation and intensity fields.  A redirection is an event at
+ * element k that neither ends nor re-emits the bundle: a scattering in cell k (dec < omega_k) or a reflection at surface k
+ * (dec >= eps_k).  Each one is tallied in row y, column k of a second count block, from the decision already drawn (no new Philox
+ * draw), so the absorption counts, absorbed_out, lost_out and events_out are bit for bit those of rthx_trace_direct with the same
+ * arguments, and events = sum of absorption counts + sum of redirection counts + sum of lost.
+ *   redirected_out [N] (not NULL): r_k = sum_y bundle_energy[y] redir[y][k], the fixed-order sum of absorbed_out over the second block.
+ * Arguments and checks otherwise those of rthx_trace_direct.  The two blocks take 16 R N bytes of device memory; if they cannot fit the
+ * call is RTHX_ERR_NOMEM naming the bytes, with nothing resident changed.  Afterwards the resident record holds two bins: bin 0 the
+ * absorption counts, bin 1 the redirection counts, both read by rthx_counts_nnz / _csr / _stats / _csc (after rthx_trace_direct, bin 1
+ * is RTHX_ERR_ARG); rthx_trace_exchange_continue and the smoothings refuse them.                                        [0.3+] */
+int rthx_trace_direct_fields(rthx_handle* h, const rthx_trace_args* args, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                             const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, double* redirected_out,
+                             uint64_t* lost_out, int64_t* events_out, rthx_stats* stats);
+
 /* Peer-memory plumbing for the fused flush in one-process-per-GPU runs: rank 0 allocates the UInt64 count matrix
  * with rthx_shared_alloc and publishes the 64-byte CUDA IPC handle; every other rank maps it with rthx_shared_open
  * (peer access over NVLink is enabled lazily) and passes the mapped pointer as `counts_dev` to

@@ -96,6 +96,9 @@ def load_library():
     L.rthx_trace_direct.restype = C.c_int
     L.rthx_trace_direct.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, c_i64p, C.c_int32, C.POINTER(C.c_uint8), c_f64p, c_f64p,
                                     c_u64p, c_i64p, C.POINTER(rthx_stats)]
+    L.rthx_trace_direct_fields.restype = C.c_int
+    L.rthx_trace_direct_fields.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, c_i64p, C.c_int32, C.POINTER(C.c_uint8), c_f64p, c_f64p,
+                                           c_f64p, c_u64p, c_i64p, C.POINTER(rthx_stats)]
     L.rthx_trace_exchange_device.restype = C.c_int
     L.rthx_trace_exchange_device.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int, C.POINTER(rthx_stats)]
@@ -337,12 +340,15 @@ class DeviceTracer:
         self._set_resident(rays_per_emitter, kw, R)
         return _recorded(dict(counts=counts.reshape(nb, R, N) if counts is not None else None, lost=lost, stats=st.as_dict()), rec, origins, endpoints)
 
-    def trace_direct(self, sources, rays, reemit, bundle_energy, specular: bool = False, **kw):
+    def trace_direct(self, sources, rays, reemit, bundle_energy, specular: bool = False, redirected: bool = False, **kw):
         """method=:direct on the device (rthx_trace_direct): source y = element sources[y] (strictly ascending) traces rays[y] bundles of
         energy bundle_energy[y] through the MULTI_BOUNCE events (specular=True: mirror reflection); a bundle absorbed by element k with
         reemit[k] is emitted again from k.  Keywords of `trace()` (seed, nudge, locator, block_threads, row_chunks, ray_id_offset).
         Returns dict(absorbed [N] f64 = sum_y bundle_energy[y] counts[y][k] in ascending y, lost [N] u64 per source element,
-        events, stats).  The counts stay resident as the listed rows of a rows trace (`counts_csr()`: R = len(sources) rows)."""
+        events, stats).  The counts stay resident as the listed rows of a rows trace (`counts_csr()`: R = len(sources) rows).
+        redirected=True (rthx_trace_direct_fields) also tallies every scattering and reflection at element k in a second count block,
+        read out with `counts_csr(bin=1)`, and adds redirected [N] f64, the same fixed-order sum over that block; everything else is
+        bit for bit the result of redirected=False."""
         from ._abi import RTHX_MULTI_BOUNCE, RTHX_MULTI_BOUNCE_SPECULAR
         rows = np.ascontiguousarray(sources, dtype=np.int32).ravel()
         R, N = len(rows), self.n_elements
@@ -353,14 +359,22 @@ class DeviceTracer:
             raise ValueError(f"trace_direct: rays and bundle_energy need {R} entries (one per source), reemit {N} (one per element)")
         args, keep = make_trace_args(0, mode=RTHX_MULTI_BOUNCE_SPECULAR if specular else RTHX_MULTI_BOUNCE, **kw)
         absorbed = np.empty(N, np.float64)
+        red = np.empty(N, np.float64) if redirected else None
         lost = np.empty(N, np.uint64)
         events = C.c_int64(0)
         st = rthx_stats()
-        self._check(self._L.rthx_trace_direct(self._h, C.byref(args), rows.ctypes.data_as(c_i32p), nr.ctypes.data_as(c_i64p), R,
-                                              re_.ctypes.data_as(C.POINTER(C.c_uint8)), w.ctypes.data_as(c_f64p), absorbed.ctypes.data_as(c_f64p),
-                                              lost.ctypes.data_as(c_u64p), C.byref(events), C.byref(st)))
+        head = (self._h, C.byref(args), rows.ctypes.data_as(c_i32p), nr.ctypes.data_as(c_i64p), R, re_.ctypes.data_as(C.POINTER(C.c_uint8)),
+                w.ctypes.data_as(c_f64p), absorbed.ctypes.data_as(c_f64p))
+        tail = (lost.ctypes.data_as(c_u64p), C.byref(events), C.byref(st))
+        if redirected:
+            self._check(self._L.rthx_trace_direct_fields(*head, red.ctypes.data_as(c_f64p), *tail))
+        else:
+            self._check(self._L.rthx_trace_direct(*head, *tail))
         self._resident = dict(kw={}, hi=0, sparse=False, rows=R)
-        return dict(absorbed=absorbed, lost=lost, events=int(events.value), stats=st.as_dict())
+        out = dict(absorbed=absorbed, lost=lost, events=int(events.value), stats=st.as_dict())
+        if redirected:
+            out["redirected"] = red
+        return out
 
     def trace_sparse(self, rays_per_emitter: int, **kw):
         """Blocking trace with the hashed row tally (rthx_trace_exchange_sparse): the counts never exist in dense form and stay on
@@ -421,7 +435,8 @@ class DeviceTracer:
     def counts_csr(self, bin: int = 0, values: bool = True, normalised: bool = True):
         """CSR read-out of the counts resident on the device (rthx_counts_nnz / rthx_counts_csr): returns
         (row_ptr [R+1] i64, cols [nnz] i32, counts [nnz] u64 or None, F_vals [nnz] f64 = count/row total or None); R = N after a
-        plain trace, the number of owned rows (elements rank + y * world) after a sharded one, the listed rows after `trace_rows()`."""
+        plain trace, the number of owned rows (elements rank + y * world) after a sharded one, the listed rows after `trace_rows()`.
+        After `trace_direct()` bin 0 holds the absorption counts of the sources, and with redirected=True bin 1 their redirections."""
         nnz = C.c_int64(0)
         self._check(self._L.rthx_counts_nnz(self._h, int(bin), C.byref(nnz)))
         N, k = self.n_elements, max(1, nnz.value)

@@ -39,7 +39,7 @@ struct DevRes {
   uint8_t* rec_valid_dev = nullptr;         size_t rec_valid_cap = 0;
   double* peak_dev = nullptr;
   int32_t* rows_dev = nullptr;              size_t rows_cap = 0;       // emitter list of a rows trace (rthx_trace_exchange_rows)
-  char* dr_buf = nullptr;                   size_t dr_cap = 0;          // rthx_trace_direct: bundles and energy per row, Abs, events, re-emit flags (bytes)
+  char* dr_buf = nullptr;                   size_t dr_cap = 0;          // rthx_trace_direct: bundles and energy per row, Abs, redirected power, events, re-emit flags (bytes)
   int* csr_nnz = nullptr;                   size_t csr_cap = 0;        // per-row nnz (int), row totals, row pointers
   unsigned long long* csr_rowsum = nullptr; long long* csr_rowptr = nullptr; unsigned long long* csr_cross = nullptr;
   unsigned int* row_done_dev = nullptr;     size_t row_done_cap = 0;   // fused peer flush: per-row hand-over tickets
@@ -1553,38 +1553,42 @@ extern "C" int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* a
 
 namespace {
 
-// Bundles a block traces at most with the direct kernel: every bundle tallies at most one absorption per event (< 16001 events), so the
-// block's u32 row histogram cannot wrap
+// Bundles a block traces at most with the direct kernel: every traversal segment of a bundle ends in at most one tally, an absorption
+// or (rthx_trace_direct_fields) a redirection, and a bundle has at most 16001 segments, so absorption and redirection tallies together
+// are <= 16001 per bundle: with 2^17 bundles a block's u32 histogram entries stay below 16001 * 2^17 < 2^32 and cannot wrap
 constexpr long long kDirectRaysPerBlock = 1ll << 17;
 
-// Checks of rthx_trace_direct that must pass before anything resident changes
+// Checks of rthx_trace_direct / _fields (`who`) that must pass before anything resident changes; `blocks` count blocks per source row
+// (2 with the redirection tally), laid out and checked against free memory as the bins of a rows trace
 int check_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n, const uint8_t* reemit,
-                 const double* energy, const double* absorbed_out) {
+                 const double* energy, const double* absorbed_out, const std::string& who, int blocks) {
   if (a->mode != RTHX_MULTI_BOUNCE && a->mode != RTHX_MULTI_BOUNCE_SPECULAR)
-    return fail(h, RTHX_ERR_ARG, "trace_direct: mode must be RTHX_MULTI_BOUNCE or RTHX_MULTI_BOUNCE_SPECULAR");
-  if (a->n_bins != 1) return fail(h, RTHX_ERR_ARG, "trace_direct: exactly one bin (n_bins = 1): the direct method is grey");
-  if (a->n_rec_ids != 0) return fail(h, RTHX_ERR_ARG, "trace_direct: recording rays is not available (n_rec_ids must be 0)");
-  if (!rays || !reemit || !energy || !absorbed_out) return fail(h, RTHX_ERR_ARG, "trace_direct: rays, reemit, bundle_energy and absorbed_out must not be NULL");
-  if (a->ray_id_offset < 0) return fail(h, RTHX_ERR_ARG, "trace_direct: ray_id_offset < 0");
-  int rc = check_rows(h, a, sources, n, "trace_direct", "source");
+    return fail(h, RTHX_ERR_ARG, who + ": mode must be RTHX_MULTI_BOUNCE or RTHX_MULTI_BOUNCE_SPECULAR");
+  if (a->n_bins != 1) return fail(h, RTHX_ERR_ARG, who + ": exactly one bin (n_bins = 1): the direct method is grey");
+  if (a->n_rec_ids != 0) return fail(h, RTHX_ERR_ARG, who + ": recording rays is not available (n_rec_ids must be 0)");
+  if (!rays || !reemit || !energy || !absorbed_out) return fail(h, RTHX_ERR_ARG, who + ": rays, reemit, bundle_energy and absorbed_out must not be NULL");
+  if (a->ray_id_offset < 0) return fail(h, RTHX_ERR_ARG, who + ": ray_id_offset < 0");
+  rthx_trace_args laid_out = *a;
+  laid_out.n_bins = blocks;
+  int rc = check_rows(h, &laid_out, sources, n, who, "source");
   if (rc) return rc;
   for (int32_t i = 0; i < n; ++i) {
     if (rays[i] < 1 || rays[i] > INT64_MAX - a->ray_id_offset)
-      return fail(h, RTHX_ERR_ARG, "trace_direct: rays[" + std::to_string(i) + "] = " + std::to_string(rays[i]) + " (every source traces >= 1 bundle)");
+      return fail(h, RTHX_ERR_ARG, who + ": rays[" + std::to_string(i) + "] = " + std::to_string(rays[i]) + " (every source traces >= 1 bundle)");
     if (!(energy[i] >= 0.0) || !std::isfinite(energy[i]))
-      return fail(h, RTHX_ERR_ARG, "trace_direct: bundle_energy[" + std::to_string(i) + "] is negative or not finite");
+      return fail(h, RTHX_ERR_ARG, who + ": bundle_energy[" + std::to_string(i) + "] is negative or not finite");
   }
   return RTHX_OK;
 }
 
 // Launch plan of a direct trace of the listed source rows: the lock-step body with re-emission, histogram in shared memory when the
-// row fits, chunks for the longest row
-LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long long max_rays) {
+// row fits (both halves with the redirection tally), chunks for the longest row
+LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long long max_rays, int blocks) {
   LaunchPlan pl{};
   pl.n_owned = (int)h->rows.size();
   pl.block_threads = a->block_threads ? a->block_threads : 256;
   const size_t coarse_bytes = h->coarse_fits_smem ? sizeof(CoarseDev) * (size_t)h->n_coarse : 0;
-  const size_t hist_bytes = sizeof(uint32_t) * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;
+  const size_t hist_bytes = sizeof(uint32_t) * (size_t)blocks * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;
   bool hist = coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
   if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) hist = false; }
   pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0);
@@ -1598,31 +1602,35 @@ LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long
   return pl;
 }
 
-}  // namespace
-
-extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources,
-                                 const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, uint64_t* lost_out,
-                                 int64_t* events_out, rthx_stats* st) {
-  if (!h) return RTHX_ERR_ARG;
+// rthx_trace_direct, and with redirected_out != NULL (fields) rthx_trace_direct_fields: the redirections are tallied in a second
+// count block, counts_dev = [2][R][N], and reduced to redirected_out as the absorptions are to absorbed_out
+int trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources, const uint8_t* reemit,
+                 const double* bundle_energy, double* absorbed_out, double* redirected_out, uint64_t* lost_out, int64_t* events_out, rthx_stats* st,
+                 bool fields) {
+  const std::string who = fields ? "trace_direct_fields" : "trace_direct";
+  const int blocks = fields ? 2 : 1;
   int rc = check_args(h, a);
   if (rc) return rc;
   CU(h, cudaSetDevice(h->device));
-  rc = check_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out);
+  if (fields && !redirected_out) return fail(h, RTHX_ERR_ARG, who + ": redirected_out must not be NULL");
+  rc = check_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, who, blocks);
   if (rc) return rc;
   const int N = h->N, R = n_sources;
+  const size_t RN = (size_t)R * N;
   const long long max_rays = *std::max_element(rays, rays + R);
   drop_resident(h);                  // the resident counts are replaced from here on
   h->rows.assign(sources, sources + R);
   h->row_runs = list_runs(h->rows);
-  const LaunchPlan pl = make_direct_plan(h, a, max_rays);
-  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace_direct: too many bundles for one launch (a launch has at most 2^31 blocks)");
+  const LaunchPlan pl = make_direct_plan(h, a, max_rays, blocks);
+  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, who + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
   if (!pl.kernel.fast) { rc = ensure_generic(h); if (rc) return rc; }
-  // dr_buf: rays [R] i64 | bundle energy [R] f64 | Abs [N] f64 | events u64 | re-emit flags [N] u8
-  const size_t off_w = 8 * (size_t)R, off_abs = off_w + 8 * (size_t)R, off_ev = off_abs + 8 * (size_t)N, off_re = off_ev + 8;
+  // dr_buf: rays [R] i64 | bundle energy [R] f64 | Abs [N] f64 | redirected power [N] f64 | events u64 | re-emit flags [N] u8
+  const size_t off_w = 8 * (size_t)R, off_abs = off_w + 8 * (size_t)R, off_red = off_abs + 8 * (size_t)N, off_ev = off_red + 8 * (size_t)N,
+               off_re = off_ev + 8;
   CU(h, ensure(&h->dr_buf, &h->dr_cap, off_re + (size_t)N));
   char* buf = h->dr_buf;
   CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)R));
-  CU(h, ensure(&h->counts_dev, &h->counts_cap, (size_t)R * N));
+  CU(h, ensure(&h->counts_dev, &h->counts_cap, blocks * RN));
   cudaStream_t s = h->stream;
   int n_launches = 0;
   CU(h, cudaEventRecord(h->ev[0], s));
@@ -1631,7 +1639,7 @@ extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const
   CU(h, cudaMemcpyAsync(buf + off_w, bundle_energy, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
   CU(h, cudaMemcpyAsync(buf + off_re, reemit, (size_t)N, cudaMemcpyHostToDevice, s));
   CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t), cudaMemcpyHostToDevice, s));
-  CU(h, cudaMemsetAsync(h->counts_dev, 0, sizeof(unsigned long long) * (size_t)R * N, s));
+  CU(h, cudaMemsetAsync(h->counts_dev, 0, sizeof(unsigned long long) * blocks * RN, s));
   CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)N, s));
   CU(h, cudaMemsetAsync(buf + off_ev, 0, 8, s));
   n_launches += 3;
@@ -1640,6 +1648,7 @@ extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const
   P.dr_rays = reinterpret_cast<const int64_t*>(buf);
   P.dr_reemit = reinterpret_cast<const uint8_t*>(buf + off_re);
   P.dr_events = reinterpret_cast<unsigned long long*>(buf + off_ev);
+  P.dr_redirect = fields ? 1 : 0;
   CU(h, cudaEventRecord(h->ev[1], s));
   for (const int4& run : h->row_runs) {      // one launch per arithmetic run of the source list, as rthx_trace_exchange_rows
     const int4 r = run;
@@ -1648,21 +1657,27 @@ extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const
     P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r.y));
     P.emitter_world = r.w; P.emitter_rank = r.z - r.x * r.w;
     P.y_offset = r.x;
-    if ((long long)r.y * P.row_chunks > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "trace_direct: too many bundles for one launch (a launch has at most 2^31 blocks)");
+    if ((long long)r.y * P.row_chunks > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, who + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
     CU(h, launch_trace_exchange(P, pl.kernel, r.y * P.row_chunks, pl.block_threads, pl.smem_bytes, s));
     ++n_launches;
   }
   CU(h, cudaEventRecord(h->ev[2], s));
   CU(h, launch_direct_absorbed(h->counts_dev, R, N, reinterpret_cast<const double*>(buf + off_w), reinterpret_cast<double*>(buf + off_abs), s));
   ++n_launches;
+  if (fields) {                              // the same fixed-order sum over the second block
+    CU(h, launch_direct_absorbed(h->counts_dev + RN, R, N, reinterpret_cast<const double*>(buf + off_w), reinterpret_cast<double*>(buf + off_red), s));
+    ++n_launches;
+  }
   std::vector<uint64_t> lost(N);
   unsigned long long events = 0;
   CU(h, cudaMemcpyAsync(absorbed_out, buf + off_abs, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  if (fields) CU(h, cudaMemcpyAsync(redirected_out, buf + off_red, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
   CU(h, cudaMemcpyAsync(lost.data(), h->lost_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
   CU(h, cudaMemcpyAsync(&events, buf + off_ev, 8, cudaMemcpyDeviceToHost, s));
   CU(h, cudaEventRecord(h->ev[3], s));
   CU(h, cudaStreamSynchronize(s));
   set_resident(h, a, RESIDENT_DIRECT, OwnedRows{0, 1, true}, R);
+  if (fields) h->res.bins.push_back(a->bins[0]);   // the redirection block reads out as bin 1
   if (lost_out) std::memcpy(lost_out, lost.data(), 8 * (size_t)N);
   if (events_out) *events_out = (int64_t)events;
   if (st) {
@@ -1674,6 +1689,22 @@ extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const
     for (int32_t i = 0; i < R; ++i) st->rays_traced += rays[i];
   }
   return RTHX_OK;
+}
+
+}  // namespace
+
+extern "C" int rthx_trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                                 const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, uint64_t* lost_out,
+                                 int64_t* events_out, rthx_stats* st) {
+  if (!h) return RTHX_ERR_ARG;
+  return trace_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, nullptr, lost_out, events_out, st, false);
+}
+
+extern "C" int rthx_trace_direct_fields(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                                        const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, double* redirected_out,
+                                        uint64_t* lost_out, int64_t* events_out, rthx_stats* st) {
+  if (!h) return RTHX_ERR_ARG;
+  return trace_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, redirected_out, lost_out, events_out, st, true);
 }
 
 extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args* a, void* counts_dev, void* lost_dev, void* stream,

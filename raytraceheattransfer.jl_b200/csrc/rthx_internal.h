@@ -132,6 +132,10 @@ struct TraceParams {
   const int64_t* dr_rays;      // [listed rows] bundles of source row y
   const uint8_t* dr_reemit;    // [N] 1: the element's temperature is unknown, a bundle it absorbs is emitted again from it
   unsigned long long* dr_events;  // [1] traversal segments of all bundles (one per interaction, or per loss)
+  // method=:direct with the redirection tally (rthx_trace_direct_fields), behind the fields above
+  int32_t dr_redirect;         // 1: every scattering / reflection at element k is tallied in row y, column k of the second count block
+                               // (rows n_owned + y: the compact layout of a two-bin rows trace)
+  int32_t dr_pad_;
 };
 
 static_assert(offsetof(TraceParams, rays_per_emitter) % 16 == 0 && offsetof(TraceParams, k_u52) % 16 == 0 && offsetof(TraceParams, rk) % 16 == 0,

@@ -516,7 +516,8 @@ __global__ void __launch_bounds__(256, 2) trace_exchange_hash_kernel(const __gri
 }
 
 // method=:direct (rthx_trace_direct): the MULTI_BOUNCE event loop with re-emission from elements of unknown temperature.  One block
-// per (source row, chunk) of the listed source rows; row y traces p.dr_rays[y] bundles.
+// per (source row, chunk) of the listed source rows; row y traces p.dr_rays[y] bundles.  With p.dr_redirect (rthx_trace_direct_fields)
+// the scatterings and reflections are tallied as well, into the second count block (and the second half of a 2N-entry histogram).
 template <bool HIST_SMEM, bool FAST>
 __global__ void __launch_bounds__(256, 2) trace_direct_kernel(const __grid_constant__ TraceParams p) {
   constexpr bool MULTI = true, HASH = false, REEMIT = true;

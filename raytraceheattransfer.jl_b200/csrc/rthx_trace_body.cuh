@@ -29,6 +29,10 @@
   }
   if (HIST_SMEM)
     for (int i = threadIdx.x; i < N; i += blockDim.x) hist[i] = 0u;
+  if constexpr (REEMIT) {                              // the redirection half of the histogram, [N, 2N)
+    if (HIST_SMEM && p.dr_redirect)
+      for (int i = threadIdx.x; i < N; i += blockDim.x) hist[N + i] = 0u;
+  }
   if (HASH)
     for (int i = threadIdx.x; i < (2 << p.sk_slots_log2) + 2; i += blockDim.x) hist[i] = 0u;
   for (int i = threadIdx.x; i < LOGTAB_N; i += blockDim.x) s_log[i] = c_logtab[i];
@@ -139,7 +143,9 @@
     // MULTI (RTHX_MULTI_BOUNCE): the traversal is repeated from every scattering / reflection event until the ray is
     // absorbed (traceSingleRay.jl:7-81 without the re-emission branches); otherwise the body runs exactly once.
     // REEMIT (method=:direct): an absorption by an element of unknown temperature is tallied and the bundle is emitted
-    // again from that element (direct_reemit); the event counter runs on over the whole chain.
+    // again from that element (direct_reemit); the event counter runs on over the whole chain.  With p.dr_redirect every event that
+    // neither ends nor re-emits the bundle (a scattering or a reflection) is tallied in the second count block, from the decision
+    // already drawn: every segment then ends in exactly one absorption tally, redirection tally or loss.
     double neg_log = neg_log_table(R_S, s_log);
     int c = c0;
     int absorber = -1;
@@ -262,6 +268,12 @@
         dy = -nxi * xdir + nyi * zdir;
       }
     }
+    if constexpr (REEMIT) {                     // a redirection (scattering or reflection) at `absorber`: second count block
+      if (p.dr_redirect) {
+        if (HIST_SMEM) atomicAdd(&hist[N + absorber], 1u);
+        else atomicAdd(&count_row[(size_t)p.n_owned * N + absorber], 1ULL);
+      }
+    }
     neg_log = -log(u52(v1.z, v1.w, p.k_u52));
     }
 
@@ -299,5 +311,12 @@
         if (p.flush_system) atomicAdd_system(&count_row[i], (unsigned long long)v);   // red.sys: matrix lives on a peer GPU
         else atomicAdd(&count_row[i], (unsigned long long)v);                          // red.gpu.global.add.u64, result unused
       }
+    }
+    if constexpr (REEMIT) {
+      if (p.dr_redirect)
+        for (int i = threadIdx.x; i < N; i += blockDim.x) {
+          const uint32_t v = hist[N + i];
+          if (v) atomicAdd(&count_row[(size_t)p.n_owned * N + i], (unsigned long long)v);
+        }
     }
   }

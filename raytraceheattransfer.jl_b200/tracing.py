@@ -474,7 +474,8 @@ def dispatch_ray_trace(rtm, rays_tot: int, method: str = "exchange", nudge: Opti
     """(rtm)(rays_tot; method, nudge, k_dykstra, max_iters, verbose, rec) — multiDispatchRayTrace2D.jl:1-18.  New keyword
     refine=True (method=:exchange): add rays_tot // N rays per emitter to the previous call's trace and smooth again (parallelRayTracing).
     method=:direct traces energy bundles with re-emission and writes the temperatures itself (direct.directRayTracing; grey domains;
-    keywords seed, device / devices, locator, specular)."""
+    keywords seed, device / devices, locator, specular, and all_fields=True to tally scatterings and reflections too and write j, r, g
+    and i as the grey solve does)."""
     method = method.lstrip(":")
     if method == "exchange":
         return exchangeRayTracing(rtm, rays_tot, nudge, max_iters, k_dykstra, verbose, rec, **kw)

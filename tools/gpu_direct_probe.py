@@ -2,7 +2,8 @@
 
   python tools/gpu_direct_probe.py [--out DIR] [--bundles 1e9] [--reps 3]
 
-Rates (DeviceTracer.trace_direct, kernel time from CUDA events, after one warm-up call):
+Rates (DeviceTracer.trace_direct, kernel time from CUDA events, after one warm-up call of each kind), without and with the
+redirection tally (redirected=True), alternated rep by rep on one handle:
   cs101   101 x 101, kappa = 1, black walls, bottom at 1000 K, gas of zero net emission (the Crosbie & Schrenker set-up);
   refl41  41 x 41, kappa = 1, eps = (1, .5, .5, .5), bottom at 1000 K (a reflecting enclosure), gas of zero net emission.
 Whole call on cs101: rtm(B; method=:direct) against rtm(B; method=:exchange) + solveEquilibrium, host wall time of each, and each
@@ -40,21 +41,27 @@ def domain(name):
 
 
 def rates(name, bundles, reps):
+    """Each rep traces the same bundles without and with the redirection tally (redirected=True), alternately, on one handle."""
     rtm = domain(name)
     flat = rthx.flatten_domain(rtm)
     ws, known_T, E, src, rays, w = direct_sources(rtm, bundles)
     reemit = np.zeros(flat.n_elements, np.uint8)
     reemit[:len(known_T)] = ~known_T
     tr = rthx.DeviceTracer(flat, device=0)
-    tr.trace_direct(src, np.minimum(rays, 1000), reemit, w, seed=1)
+    for tally in (False, True):
+        tr.trace_direct(src, np.minimum(rays, 1000), reemit, w, seed=1, redirected=tally)
     runs = []
     for r in range(reps):
-        out = tr.trace_direct(src, rays, reemit, w, seed=100 + r)
-        ms = out["stats"]["kernel_ms"]
-        runs.append(dict(kernel_ms=ms, total_ms=out["stats"]["total_ms"], bundles=int(rays.sum()), events=out["events"],
-                         lost=int(out["lost"].sum()), bundles_per_s=rays.sum() / (ms * 1e-3), events_per_s=out["events"] / (ms * 1e-3)))
+        for tally in (False, True):
+            out = tr.trace_direct(src, rays, reemit, w, seed=100 + r, redirected=tally)
+            ms = out["stats"]["kernel_ms"]
+            runs.append(dict(tally=tally, kernel_ms=ms, total_ms=out["stats"]["total_ms"], bundles=int(rays.sum()), events=out["events"],
+                             lost=int(out["lost"].sum()), bundles_per_s=rays.sum() / (ms * 1e-3), events_per_s=out["events"] / (ms * 1e-3)))
     tr.close()
-    return dict(domain=name, N=flat.n_elements, sources=len(src), runs=runs)
+    median = {str(t): {k: float(np.median([x[k] for x in runs if x["tally"] == t])) for k in ("kernel_ms", "bundles_per_s", "events_per_s")}
+              for t in (False, True)}
+    return dict(domain=name, N=flat.n_elements, sources=len(src), runs=runs, median_without_tally=median["False"], median_with_tally=median["True"],
+                tally_cost=median["True"]["kernel_ms"] / median["False"]["kernel_ms"] - 1.0)
 
 
 def centre_line_error(rtm):
