@@ -477,6 +477,28 @@ int rthx_trace_direct_fields(rthx_handle* h, const rthx_trace_args* args, const 
                              const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, double* redirected_out,
                              uint64_t* lost_out, int64_t* events_out, rthx_stats* stats);
 
+/* rthx_trace_direct (redirected_out == NULL) or rthx_trace_direct_fields (redirected_out != NULL) on the hashed row tally of
+ * rthx_trace_exchange_sparse, for source lists whose 8 R N bytes of dense counts (16 R N with the redirection tally) do not fit: an
+ * isothermal or prescribed-temperature medium makes every element a source, R = N.  Each block tallies its source row in a
+ * shared-memory hash table; the table is flushed between rounds of bundles once it is half full, and inside a round a tally that finds
+ * neither its key nor an empty slot within a fixed probe length is appended to the pair buffer as its own (key, 1) pair (a bundle
+ * tallies at every absorption by a re-emitting element and every redirection, with no block-wide point to flush at).  The pairs are
+ * sorted and reduced by key, so the totals do not depend on where a tally landed.  Row y's absorptions are row key y * blocks, its
+ * redirections y * blocks + 1 (blocks = 1, or 2 with the redirection tally).  The pair buffer takes at most half the free device
+ * memory; a group of source rows whose pairs overrun it is traced again split in two, and one source row that overruns it alone is
+ * RTHX_ERR_NOMEM naming the source, with nothing resident (as rthx_trace_exchange_sparse).
+ *   absorbed_out / redirected_out: the sums of rthx_trace_direct(_fields), bit for bit: the sorted set is transposed to columns and
+ *       each column summed in ascending source row, with every product and sum rounded on its own (a zero count adds +0.0);
+ *   lost_out, events_out, stats: as rthx_trace_direct, counted once however often a group was traced; sparse_stats (may be NULL):
+ *       the tally, as rthx_trace_exchange_sparse reports it.
+ * Arguments and checks are those of rthx_trace_direct(_fields) without the check of the dense counts against free memory.  Afterwards
+ * rthx_counts_nnz / _csr / _stats / _csc for bins 0 (and 1) return what they return after rthx_trace_direct(_fields) with the same
+ * arguments, bit for bit; rthx_trace_exchange_continue and the smoothings refuse the counts.  A set of more than 2^31 - 1
+ * non-zeros in one count block cannot be summed (RTHX_ERR_ARG naming the limit).                                       [0.3+] */
+int rthx_trace_direct_sparse(rthx_handle* h, const rthx_trace_args* args, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                             const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, double* redirected_out,
+                             uint64_t* lost_out, int64_t* events_out, rthx_stats* stats, rthx_sparse_stats* sparse_stats);
+
 /* Peer-memory plumbing for the fused flush in one-process-per-GPU runs: rank 0 allocates the UInt64 count matrix
  * with rthx_shared_alloc and publishes the 64-byte CUDA IPC handle; every other rank maps it with rthx_shared_open
  * (peer access over NVLink is enabled lazily) and passes the mapped pointer as `counts_dev` to

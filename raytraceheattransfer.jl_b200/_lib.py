@@ -99,6 +99,9 @@ def load_library():
     L.rthx_trace_direct_fields.restype = C.c_int
     L.rthx_trace_direct_fields.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, c_i64p, C.c_int32, C.POINTER(C.c_uint8), c_f64p, c_f64p,
                                            c_f64p, c_u64p, c_i64p, C.POINTER(rthx_stats)]
+    L.rthx_trace_direct_sparse.restype = C.c_int
+    L.rthx_trace_direct_sparse.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), c_i32p, c_i64p, C.c_int32, C.POINTER(C.c_uint8), c_f64p, c_f64p,
+                                           c_f64p, c_u64p, c_i64p, C.POINTER(rthx_stats), C.POINTER(rthx_sparse_stats)]
     L.rthx_trace_exchange_device.restype = C.c_int
     L.rthx_trace_exchange_device.argtypes = [C.c_void_p, C.POINTER(rthx_trace_args), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int, C.POINTER(rthx_stats)]
@@ -340,7 +343,7 @@ class DeviceTracer:
         self._set_resident(rays_per_emitter, kw, R)
         return _recorded(dict(counts=counts.reshape(nb, R, N) if counts is not None else None, lost=lost, stats=st.as_dict()), rec, origins, endpoints)
 
-    def trace_direct(self, sources, rays, reemit, bundle_energy, specular: bool = False, redirected: bool = False, **kw):
+    def trace_direct(self, sources, rays, reemit, bundle_energy, specular: bool = False, redirected: bool = False, sparse: bool = False, **kw):
         """method=:direct on the device (rthx_trace_direct): source y = element sources[y] (strictly ascending) traces rays[y] bundles of
         energy bundle_energy[y] through the MULTI_BOUNCE events (specular=True: mirror reflection); a bundle absorbed by element k with
         reemit[k] is emitted again from k.  Keywords of `trace()` (seed, nudge, locator, block_threads, row_chunks, ray_id_offset).
@@ -348,7 +351,10 @@ class DeviceTracer:
         events, stats).  The counts stay resident as the listed rows of a rows trace (`counts_csr()`: R = len(sources) rows).
         redirected=True (rthx_trace_direct_fields) also tallies every scattering and reflection at element k in a second count block,
         read out with `counts_csr(bin=1)`, and adds redirected [N] f64, the same fixed-order sum over that block; everything else is
-        bit for bit the result of redirected=False."""
+        bit for bit the result of redirected=False.
+        sparse=True (rthx_trace_direct_sparse) tallies the counts into the hashed row tally instead of dense [R][N] rows, for source
+        lists whose 8 R N bytes (16 R N with redirected=True) do not fit; every result and read-out is bit for bit that of sparse=False,
+        and the dict adds `sparse_stats` (pairs, flushes, row groups)."""
         from ._abi import RTHX_MULTI_BOUNCE, RTHX_MULTI_BOUNCE_SPECULAR
         rows = np.ascontiguousarray(sources, dtype=np.int32).ravel()
         R, N = len(rows), self.n_elements
@@ -366,14 +372,19 @@ class DeviceTracer:
         head = (self._h, C.byref(args), rows.ctypes.data_as(c_i32p), nr.ctypes.data_as(c_i64p), R, re_.ctypes.data_as(C.POINTER(C.c_uint8)),
                 w.ctypes.data_as(c_f64p), absorbed.ctypes.data_as(c_f64p))
         tail = (lost.ctypes.data_as(c_u64p), C.byref(events), C.byref(st))
-        if redirected:
+        sst = rthx_sparse_stats()
+        if sparse:
+            self._check(self._L.rthx_trace_direct_sparse(*head, red.ctypes.data_as(c_f64p) if redirected else None, *tail, C.byref(sst)))
+        elif redirected:
             self._check(self._L.rthx_trace_direct_fields(*head, red.ctypes.data_as(c_f64p), *tail))
         else:
             self._check(self._L.rthx_trace_direct(*head, *tail))
-        self._resident = dict(kw={}, hi=0, sparse=False, rows=R)
+        self._resident = dict(kw={}, hi=0, sparse=bool(sparse), rows=R)
         out = dict(absorbed=absorbed, lost=lost, events=int(events.value), stats=st.as_dict())
         if redirected:
             out["redirected"] = red
+        if sparse:
+            out["sparse_stats"] = sst.as_dict()
         return out
 
     def trace_sparse(self, rays_per_emitter: int, **kw):

@@ -77,14 +77,14 @@ struct DevRes {
 
 namespace { struct HostImage; }
 
-// where the resident counts come from
-enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4, RESIDENT_DIRECT = 5 };
+// where the resident counts come from (RESIDENT_DIRECT_SPARSE: a direct trace with the hashed row tally, rthx_trace_direct_sparse)
+enum { RESIDENT_NONE = 0, RESIDENT_DENSE = 1, RESIDENT_SPARSE = 2, RESIDENT_HOST = 3, RESIDENT_MULTI = 4, RESIDENT_DIRECT = 5, RESIDENT_DIRECT_SPARSE = 6 };
 
 // The emitter rows a trace owns: row y is element rank + y * world (a shard), or with `listed` element rows[y] of the handle's emitter
 // list (a rows trace; rank / world are then 0 / 1)
 struct OwnedRows { int rank = 0, world = 1; bool listed = false; };
 
-// The counts resident on the device (counts_dev, or the hashed tally's sk_* set for RESIDENT_SPARSE) and the one trace, of the
+// The counts resident on the device (counts_dev, or the hashed tally's sk_* set when hashed()) and the one trace, of the
 // contiguous ray-id range [ray_lo, ray_hi), they are those of; rthx_trace_exchange_continue extends it.  Set only by set_resident and
 // voided only by drop_resident; kind == RESIDENT_NONE: nothing is resident.
 struct Resident {
@@ -96,6 +96,8 @@ struct Resident {
   std::vector<int32_t> bins;           // the traced bins
   int64_t ray_lo = 0, ray_hi = 0;
   int n_bins() const { return (int)bins.size(); }
+  bool hashed() const { return kind == RESIDENT_SPARSE || kind == RESIDENT_DIRECT_SPARSE; }   // the sorted (key, total) set in sk_*
+  bool direct() const { return kind == RESIDENT_DIRECT || kind == RESIDENT_DIRECT_SPARSE; }   // absorptions with re-emission
 };
 
 struct rthx_handle : DevRes {
@@ -1002,7 +1004,7 @@ int check_continue(rthx_handle* h, const rthx_trace_args* a) {
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts come from a host-output trace (counts_out != NULL); trace with counts_out == NULL to continue");
   if (r.kind == RESIDENT_MULTI)
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts were gathered from several devices (rthx_trace_exchange_multi), whose peer hand-over stores rows instead of adding them");
-  if (r.kind == RESIDENT_DIRECT)
+  if (r.direct())
     return fail(h, RTHX_ERR_ARG, "trace_continue: the resident counts are those of a direct trace (rthx_trace_direct), which cannot be continued");
   if (a->seed != r.seed) return fail(h, RTHX_ERR_ARG, "trace_continue: seed differs from the resident trace's");
   if (a->nudge != r.nudge) return fail(h, RTHX_ERR_ARG, "trace_continue: nudge differs from the resident trace's");
@@ -1432,6 +1434,25 @@ struct TraceRun {
   std::vector<uint64_t> lost;          // the lost counters, read back
 };
 
+// What one hashed-tally pass over the rows of a call did (sparse_trace_rows)
+struct SparseRun : TraceRun {
+  int log2s = 0, groups = 0;
+  long long cap = 0, n_rows = 0, total = 0, pairs = 0, flushes = 0;
+  double reduce_ms = 0;
+  unsigned long long events = 0;       // direct: traversal segments of the launches that were kept
+};
+
+// A direct trace on the hashed tally (rthx_trace_direct_sparse), as sparse_trace_rows traces it: the listed source rows of the handle,
+// `blocks` count blocks per row (row keys y * blocks + block), the per-row bundles and re-emit flags on the device, the event counter
+// (cleared before every launch of a group, and read after it)
+struct DirectRows {
+  int blocks;
+  long long max_rays;
+  const int64_t* rays;
+  const uint8_t* reemit;
+  unsigned long long* events;
+};
+
 // End of a trace whose kernels ran from ev[1] to ev[2]: the lost counters to the host behind everything enqueued on `stream` so far,
 // ev[3] as the end of the call's device work, and the kernel time
 int read_lost(rthx_handle* h, const rthx_trace_args* a, cudaStream_t stream, TraceRun& R) {
@@ -1499,7 +1520,9 @@ std::vector<int4> list_runs(const std::vector<int32_t>& rows) {
 }
 
 // Checks of rthx_trace_exchange_rows that must pass before anything resident changes
-int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n, const std::string& who = "trace_rows", const char* list = "emitter") {
+// (dense == false: the counts are not held densely, so their size is not checked against free memory)
+int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n, const std::string& who = "trace_rows", const char* list = "emitter",
+               bool dense = true) {
   if (!emitters || n < 1) return fail(h, RTHX_ERR_ARG, who + ": the " + list + " list is empty (n_" + list + "s must be >= 1)");
   for (int32_t i = 0; i < n; ++i) {
     if (emitters[i] < 0 || emitters[i] >= h->N)
@@ -1515,7 +1538,7 @@ int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters
     if (!std::binary_search(emitters, emitters + n, a->rec_ids[k]))
       return fail(h, RTHX_ERR_ARG, who + ": rec_ids[" + std::to_string(k) + "] = " + std::to_string(a->rec_ids[k]) + " is not in the " + list + " list");
   const size_t need = (size_t)n * (size_t)h->N * (size_t)a->n_bins;
-  if (need > h->counts_cap) {
+  if (dense && need > h->counts_cap) {
     size_t free_b = 0, total_b = 0;
     CU(h, cudaMemGetInfo(&free_b, &total_b));
     if ((need - h->counts_cap) * sizeof(unsigned long long) > free_b)
@@ -1558,10 +1581,10 @@ namespace {
 // are <= 16001 per bundle: with 2^17 bundles a block's u32 histogram entries stay below 16001 * 2^17 < 2^32 and cannot wrap
 constexpr long long kDirectRaysPerBlock = 1ll << 17;
 
-// Checks of rthx_trace_direct / _fields (`who`) that must pass before anything resident changes; `blocks` count blocks per source row
-// (2 with the redirection tally), laid out and checked against free memory as the bins of a rows trace
+// Checks of rthx_trace_direct / _fields / _sparse (`who`) that must pass before anything resident changes; `blocks` count blocks per
+// source row (2 with the redirection tally), laid out and (dense) checked against free memory as the bins of a rows trace
 int check_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n, const uint8_t* reemit,
-                 const double* energy, const double* absorbed_out, const std::string& who, int blocks) {
+                 const double* energy, const double* absorbed_out, const std::string& who, int blocks, bool dense) {
   if (a->mode != RTHX_MULTI_BOUNCE && a->mode != RTHX_MULTI_BOUNCE_SPECULAR)
     return fail(h, RTHX_ERR_ARG, who + ": mode must be RTHX_MULTI_BOUNCE or RTHX_MULTI_BOUNCE_SPECULAR");
   if (a->n_bins != 1) return fail(h, RTHX_ERR_ARG, who + ": exactly one bin (n_bins = 1): the direct method is grey");
@@ -1570,7 +1593,7 @@ int check_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* source
   if (a->ray_id_offset < 0) return fail(h, RTHX_ERR_ARG, who + ": ray_id_offset < 0");
   rthx_trace_args laid_out = *a;
   laid_out.n_bins = blocks;
-  int rc = check_rows(h, &laid_out, sources, n, who, "source");
+  int rc = check_rows(h, &laid_out, sources, n, who, "source", dense);
   if (rc) return rc;
   for (int32_t i = 0; i < n; ++i) {
     if (rays[i] < 1 || rays[i] > INT64_MAX - a->ray_id_offset)
@@ -1582,17 +1605,19 @@ int check_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* source
 }
 
 // Launch plan of a direct trace of the listed source rows: the lock-step body with re-emission, histogram in shared memory when the
-// row fits (both halves with the redirection tally), chunks for the longest row
-LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long long max_rays, int blocks) {
+// row fits (both halves with the redirection tally), chunks for the longest row.  hash_slots > 0: the hashed row tally instead
+// (trace_direct_hash_kernel, no histogram; the table takes hash_table_bytes(hash_slots))
+LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long long max_rays, int blocks, int hash_slots = 0) {
   LaunchPlan pl{};
   pl.n_owned = (int)h->rows.size();
   pl.block_threads = a->block_threads ? a->block_threads : 256;
   const size_t coarse_bytes = h->coarse_fits_smem ? sizeof(CoarseDev) * (size_t)h->n_coarse : 0;
   const size_t hist_bytes = sizeof(uint32_t) * (size_t)blocks * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;
-  bool hist = coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
+  bool hist = hash_slots == 0 && coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
   if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) hist = false; }
-  pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0);
-  pl.kernel = TraceKernelSel::direct(hist, h->fast_ok && a->locator != RTHX_LOCATOR_GENERIC);
+  pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0) + (hash_slots > 0 ? hash_table_bytes(hash_slots) : 0);
+  const bool fast = h->fast_ok && a->locator != RTHX_LOCATOR_GENERIC;
+  pl.kernel = hash_slots > 0 ? TraceKernelSel::direct_hash(fast) : TraceKernelSel::direct(hist, fast);
   rthx_trace_args longest = *a;
   longest.rays_per_emitter = max_rays;
   long long chunks = a->row_chunks > 0 ? a->row_chunks : auto_row_chunks(h, pl, &longest, pl.n_owned);
@@ -1602,18 +1627,24 @@ LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long
   return pl;
 }
 
+int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec, unsigned long long** out_keys, size_t* keys_cap,
+                      unsigned long long** out_vals, size_t* vals_cap, SparseRun& R, const DirectRows* direct = nullptr);
+int direct_column_sums(rthx_handle* h, int block, int R, const double* w, double* out);
+
 // rthx_trace_direct, and with redirected_out != NULL (fields) rthx_trace_direct_fields: the redirections are tallied in a second
-// count block, counts_dev = [2][R][N], and reduced to redirected_out as the absorptions are to absorbed_out
+// count block, counts_dev = [2][R][N], and reduced to redirected_out as the absorptions are to absorbed_out.  hashed
+// (rthx_trace_direct_sparse, fields when redirected_out != NULL): the count blocks are tallied into the hashed row tally instead
+// (sparse_trace_rows), and summed from its sorted set (direct_column_sums); sst receives the tally's statistics.
 int trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources, const uint8_t* reemit,
                  const double* bundle_energy, double* absorbed_out, double* redirected_out, uint64_t* lost_out, int64_t* events_out, rthx_stats* st,
-                 bool fields) {
-  const std::string who = fields ? "trace_direct_fields" : "trace_direct";
+                 bool fields, bool hashed = false, rthx_sparse_stats* sst = nullptr) {
+  const std::string who = hashed ? "trace_direct_sparse" : fields ? "trace_direct_fields" : "trace_direct";
   const int blocks = fields ? 2 : 1;
   int rc = check_args(h, a);
   if (rc) return rc;
   CU(h, cudaSetDevice(h->device));
   if (fields && !redirected_out) return fail(h, RTHX_ERR_ARG, who + ": redirected_out must not be NULL");
-  rc = check_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, who, blocks);
+  rc = check_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, who, blocks, !hashed);
   if (rc) return rc;
   const int N = h->N, R = n_sources;
   const size_t RN = (size_t)R * N;
@@ -1630,7 +1661,7 @@ int trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* source
   CU(h, ensure(&h->dr_buf, &h->dr_cap, off_re + (size_t)N));
   char* buf = h->dr_buf;
   CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)R));
-  CU(h, ensure(&h->counts_dev, &h->counts_cap, blocks * RN));
+  if (!hashed) CU(h, ensure(&h->counts_dev, &h->counts_cap, blocks * RN));
   cudaStream_t s = h->stream;
   int n_launches = 0;
   CU(h, cudaEventRecord(h->ev[0], s));
@@ -1638,55 +1669,88 @@ int trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* source
   CU(h, cudaMemcpyAsync(buf, rays, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
   CU(h, cudaMemcpyAsync(buf + off_w, bundle_energy, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
   CU(h, cudaMemcpyAsync(buf + off_re, reemit, (size_t)N, cudaMemcpyHostToDevice, s));
-  CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t), cudaMemcpyHostToDevice, s));
-  CU(h, cudaMemsetAsync(h->counts_dev, 0, sizeof(unsigned long long) * blocks * RN, s));
-  CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)N, s));
-  CU(h, cudaMemsetAsync(buf + off_ev, 0, 8, s));
-  n_launches += 3;
-  TraceParams P;
-  fill_params(h, a, pl, 0, 1, /*compact=*/true, h->counts_dev, h->lost_dev, P);
-  P.dr_rays = reinterpret_cast<const int64_t*>(buf);
-  P.dr_reemit = reinterpret_cast<const uint8_t*>(buf + off_re);
-  P.dr_events = reinterpret_cast<unsigned long long*>(buf + off_ev);
-  P.dr_redirect = fields ? 1 : 0;
-  CU(h, cudaEventRecord(h->ev[1], s));
-  for (const int4& run : h->row_runs) {      // one launch per arithmetic run of the source list, as rthx_trace_exchange_rows
-    const int4 r = run;
-    rthx_trace_args longest = *a;
-    longest.rays_per_emitter = max_rays;
-    P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r.y));
-    P.emitter_world = r.w; P.emitter_rank = r.z - r.x * r.w;
-    P.y_offset = r.x;
-    if ((long long)r.y * P.row_chunks > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, who + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
-    CU(h, launch_trace_exchange(P, pl.kernel, r.y * P.row_chunks, pl.block_threads, pl.smem_bytes, s));
+  const double* w_dev = reinterpret_cast<const double*>(buf + off_w);
+  double* abs_dev = reinterpret_cast<double*>(buf + off_abs);
+  double* red_dev = reinterpret_cast<double*>(buf + off_red);
+  unsigned long long* events_dev = reinterpret_cast<unsigned long long*>(buf + off_ev);
+  SparseRun S;
+  float k_ms = 0;
+  unsigned long long events = 0;
+  if (hashed) {
+    // row groups, overflow splits, sort and reduce as rthx_trace_exchange_sparse, one launch per arithmetic run of the source list
+    const DirectRows dr{blocks, max_rays, reinterpret_cast<const int64_t*>(buf), reinterpret_cast<const uint8_t*>(buf + off_re), events_dev};
+    rc = sparse_trace_rows(h, a, nullptr, &h->sk_keys, &h->sk_keys_cap, &h->sk_vals, &h->sk_vals_cap, S, &dr);
+    if (rc) return rc;
+    CU(h, ensure(&h->sk_rowptr, &h->sk_rowptr_cap, (size_t)S.n_rows + 1));
+    CU(h, tally_row_ptr(h->sk_keys, S.total, S.n_rows, h->sk_rowptr, s));
+    // the set is resident in the record's key layout from here on: the sums read it through the read-out paths
+    set_resident(h, a, RESIDENT_DIRECT_SPARSE, OwnedRows{0, 1, true}, R);
+    if (fields) h->res.bins.push_back(a->bins[0]);
+    h->res.nnz = S.total;
+    if ((rc = direct_column_sums(h, 0, R, w_dev, abs_dev)) || (fields && (rc = direct_column_sums(h, 1, R, w_dev, red_dev)))) {
+      drop_resident(h);
+      return rc;
+    }
+    n_launches = S.n_launches + (fields ? 2 : 1);
+    k_ms = (float)S.kernel_ms;
+    events = S.events;
+  } else {
+    CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    CU(h, cudaMemsetAsync(h->counts_dev, 0, sizeof(unsigned long long) * blocks * RN, s));
+    CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)N, s));
+    CU(h, cudaMemsetAsync(events_dev, 0, 8, s));
+    n_launches += 3;
+    TraceParams P;
+    fill_params(h, a, pl, 0, 1, /*compact=*/true, h->counts_dev, h->lost_dev, P);
+    P.dr_rays = reinterpret_cast<const int64_t*>(buf);
+    P.dr_reemit = reinterpret_cast<const uint8_t*>(buf + off_re);
+    P.dr_events = events_dev;
+    P.dr_redirect = fields ? 1 : 0;
+    CU(h, cudaEventRecord(h->ev[1], s));
+    for (const int4& run : h->row_runs) {      // one launch per arithmetic run of the source list, as rthx_trace_exchange_rows
+      const int4 r = run;
+      rthx_trace_args longest = *a;
+      longest.rays_per_emitter = max_rays;
+      P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r.y));
+      P.emitter_world = r.w; P.emitter_rank = r.z - r.x * r.w;
+      P.y_offset = r.x;
+      if ((long long)r.y * P.row_chunks > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, who + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
+      CU(h, launch_trace_exchange(P, pl.kernel, r.y * P.row_chunks, pl.block_threads, pl.smem_bytes, s));
+      ++n_launches;
+    }
+    CU(h, cudaEventRecord(h->ev[2], s));
+    CU(h, launch_direct_absorbed(h->counts_dev, R, N, w_dev, abs_dev, s));
     ++n_launches;
-  }
-  CU(h, cudaEventRecord(h->ev[2], s));
-  CU(h, launch_direct_absorbed(h->counts_dev, R, N, reinterpret_cast<const double*>(buf + off_w), reinterpret_cast<double*>(buf + off_abs), s));
-  ++n_launches;
-  if (fields) {                              // the same fixed-order sum over the second block
-    CU(h, launch_direct_absorbed(h->counts_dev + RN, R, N, reinterpret_cast<const double*>(buf + off_w), reinterpret_cast<double*>(buf + off_red), s));
-    ++n_launches;
+    if (fields) {                              // the same fixed-order sum over the second block
+      CU(h, launch_direct_absorbed(h->counts_dev + RN, R, N, w_dev, red_dev, s));
+      ++n_launches;
+    }
+    CU(h, cudaMemcpyAsync(&events, events_dev, 8, cudaMemcpyDeviceToHost, s));
   }
   std::vector<uint64_t> lost(N);
-  unsigned long long events = 0;
-  CU(h, cudaMemcpyAsync(absorbed_out, buf + off_abs, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
-  if (fields) CU(h, cudaMemcpyAsync(redirected_out, buf + off_red, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  CU(h, cudaMemcpyAsync(absorbed_out, abs_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  if (fields) CU(h, cudaMemcpyAsync(redirected_out, red_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
   CU(h, cudaMemcpyAsync(lost.data(), h->lost_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
-  CU(h, cudaMemcpyAsync(&events, buf + off_ev, 8, cudaMemcpyDeviceToHost, s));
   CU(h, cudaEventRecord(h->ev[3], s));
   CU(h, cudaStreamSynchronize(s));
-  set_resident(h, a, RESIDENT_DIRECT, OwnedRows{0, 1, true}, R);
-  if (fields) h->res.bins.push_back(a->bins[0]);   // the redirection block reads out as bin 1
+  if (!hashed) {
+    set_resident(h, a, RESIDENT_DIRECT, OwnedRows{0, 1, true}, R);
+    if (fields) h->res.bins.push_back(a->bins[0]);   // the redirection block reads out as bin 1
+  }
   if (lost_out) std::memcpy(lost_out, lost.data(), 8 * (size_t)N);
   if (events_out) *events_out = (int64_t)events;
   if (st) {
-    float k_ms = 0, t_ms = 0;
-    CU(h, cudaEventElapsedTime(&k_ms, h->ev[1], h->ev[2]));
+    float t_ms = 0;
+    if (!hashed) CU(h, cudaEventElapsedTime(&k_ms, h->ev[1], h->ev[2]));
     CU(h, cudaEventElapsedTime(&t_ms, h->ev[0], h->ev[3]));
-    fill_stats(st, a, pl, lost, n_launches, k_ms, t_ms);
+    fill_stats(st, a, hashed ? S.pl : pl, lost, n_launches, k_ms, t_ms);
     st->rays_traced = 0;
     for (int32_t i = 0; i < R; ++i) st->rays_traced += rays[i];
+  }
+  if (sst) {
+    std::memset(sst, 0, sizeof(*sst));
+    sst->pairs = S.pairs; sst->nnz = S.total; sst->flushes = S.flushes; sst->pair_capacity = S.cap;
+    sst->row_groups = S.groups; sst->hash_slots = 1 << S.log2s; sst->reduce_ms = S.reduce_ms;
   }
   return RTHX_OK;
 }
@@ -1705,6 +1769,14 @@ extern "C" int rthx_trace_direct_fields(rthx_handle* h, const rthx_trace_args* a
                                         uint64_t* lost_out, int64_t* events_out, rthx_stats* st) {
   if (!h) return RTHX_ERR_ARG;
   return trace_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, redirected_out, lost_out, events_out, st, true);
+}
+
+extern "C" int rthx_trace_direct_sparse(rthx_handle* h, const rthx_trace_args* a, const int32_t* sources, const int64_t* rays, int32_t n_sources,
+                                        const uint8_t* reemit, const double* bundle_energy, double* absorbed_out, double* redirected_out,
+                                        uint64_t* lost_out, int64_t* events_out, rthx_stats* st, rthx_sparse_stats* sst) {
+  if (!h) return RTHX_ERR_ARG;
+  return trace_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, redirected_out, lost_out, events_out, st,
+                      redirected_out != nullptr, true, sst);
 }
 
 extern "C" int rthx_trace_exchange_device(rthx_handle* h, const rthx_trace_args* a, void* counts_dev, void* lost_dev, void* stream,
@@ -1747,13 +1819,6 @@ cudaError_t grow_keep(T** ptr, size_t* cap, size_t need, size_t keep, cudaStream
 }  // namespace
 
 namespace {
-// What one hashed-tally pass over the rows of a call did (sparse_trace_rows)
-struct SparseRun : TraceRun {
-  int log2s = 0, groups = 0;
-  long long cap = 0, n_rows = 0, total = 0, pairs = 0, flushes = 0;
-  double reduce_ms = 0;
-};
-
 // The resident trace a hashed continuation extends, held while it runs: its record and its lost counters
 struct HeldSparse { Resident res; std::vector<uint64_t> lost; };
 
@@ -1771,37 +1836,42 @@ struct DevBuf {
 // Trace the rows of `a` with the hashed row tally and append the sorted unique (key, u64 total) pairs of every row group to
 // (*out_keys, *out_vals), growing them as needed; lost_dev is cleared first and counts the rays of this call.  A group whose pairs
 // overran the pair buffer is traced again split in two.  ev[0] marks the start of the call's device work.
+// direct != nullptr (rthx_trace_direct_sparse): the listed source rows of a direct trace instead of the rows of a shard, with
+// `direct->blocks` row keys per source row; ev[0] is then the caller's.
 int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec, unsigned long long** out_keys, size_t* keys_cap,
-                      unsigned long long** out_vals, size_t* vals_cap, SparseRun& R) {
+                      unsigned long long** out_vals, size_t* vals_cap, SparseRun& R, const DirectRows* direct) {
   const int N = h->N, nb = a->n_bins, rank = a->emitter_rank, world = a->emitter_world;
+  const int nk = direct ? direct->blocks : nb;               // row keys per traced row
   const int bt = a->block_threads ? a->block_threads : 256;
   int log2s = 12;                                            // 4096 slots: 32 KB of table
   int min_log2s = 1;
-  while ((1 << min_log2s) < 2 * bt) ++min_log2s;             // a round of blockDim.x inserts must fit below half full
+  // a round of blockDim.x inserts must fit below half full (direct: an insert that finds no slot spills, any size works)
+  if (direct) min_log2s = 5;
+  else while ((1 << min_log2s) < 2 * bt) ++min_log2s;
   bool forced = false;
   if (const char* ev = std::getenv("RTHX_SPARSE_HASH_SLOTS")) {   // test knob: small tables flush many times
     const long long v = std::atoll(ev);
     if (v > 0) { log2s = 0; while ((1ll << log2s) < v) ++log2s; forced = true; }
   }
   log2s = std::max(log2s, min_log2s);
-  LaunchPlan pl = make_plan(h, a, shard_of(a), 1 << log2s);
+  LaunchPlan pl = direct ? make_direct_plan(h, a, direct->max_rays, direct->blocks, 1 << log2s) : make_plan(h, a, shard_of(a), 1 << log2s);
   if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
   if (!forced) {                                             // a block with few rays needs no large table: clearing and scanning it is the cost
-    const long long per_block = (a->rays_per_emitter + pl.row_chunks - 1) / pl.row_chunks;
-    const long long distinct = std::min<long long>(per_block, N);
+    // direct: a re-emitted bundle tallies many columns, so only the row's count blocks bound the distinct keys
+    const long long distinct = direct ? (long long)direct->blocks * N : std::min<long long>((a->rays_per_emitter + pl.row_chunks - 1) / pl.row_chunks, N);
     const int old = log2s;
     while (log2s > min_log2s && (1ll << (log2s - 1)) >= 2 * distinct) --log2s;
     pl.smem_bytes = pl.smem_bytes - hash_table_bytes(1 << old) + hash_table_bytes(1 << log2s);
   }
   if (pl.smem_bytes > h->prop.sharedMemPerBlockOptin) return fail(h, RTHX_ERR_ARG, "trace_sparse: hash table does not fit in shared memory");
   if (!pl.kernel.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }
-  // pair buffer: at most one pair per tallied ray, and at most half the free device memory (24 bytes a pair with the sort's
-  // alternate buffers); the other half is left for the resident totals
+  // pair buffer: at most half the free device memory (24 bytes a pair with the sort's alternate buffers), the other half is left for the
+  // resident totals; an exchange trace flushes at most one pair per tallied ray, a direct bundle has no such bound
   long long cap = 0x7FFFFFFFll;
   {
     size_t free_b = 0, total_b = 0;
     CU(h, cudaMemGetInfo(&free_b, &total_b));
-    const double rays = (double)pl.n_owned * nb * (double)a->rays_per_emitter;
+    const double rays = direct ? (double)cap : (double)pl.n_owned * nb * (double)a->rays_per_emitter;
     cap = (long long)std::min<double>((double)cap, std::min(rays, (double)(free_b / 2 + h->sk_pairs_cap * 24) / 24.0));
     if (const char* ev = std::getenv("RTHX_SPARSE_PAIR_CAP")) { const long long v = std::atoll(ev); if (v > 0) cap = std::min(cap, v); }   // test knob: forces row-group splits
     cap = std::max<long long>(cap, 1);
@@ -1818,11 +1888,11 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
   unsigned long long* keys_alt = keys + cap;
   uint32_t* cnt = (uint32_t*)(keys_alt + cap);
   uint32_t* cnt_alt = cnt + cap;
-  const long long n_rows = (long long)pl.n_owned * nb;       // row key y * n_bins + bi
+  const long long n_rows = (long long)pl.n_owned * nk;       // row key y * nk + bin (or count block)
   int end_bit = 32;
   while ((1ll << (end_bit - 32)) < n_rows) ++end_bit;
 
-  CU(h, cudaEventRecord(h->ev[0], h->stream));
+  if (!direct) CU(h, cudaEventRecord(h->ev[0], h->stream));
   int rc = prepare_recorder(h, a, rec, &R.n_slots, h->stream);
   if (rc) return rc;
   CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)nb, cudaMemcpyHostToDevice, h->stream));
@@ -1832,6 +1902,20 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
   fill_params(h, a, pl, rank, world, true, nullptr, h->lost_dev, P);
   if (R.n_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
   P.sk_keys = keys; P.sk_cnt = cnt; P.sk_ctl = h->sk_ctl; P.sk_cap = (unsigned long long)cap; P.sk_slots_log2 = log2s;
+  if (direct) {
+    P.dr_rays = direct->rays; P.dr_reemit = direct->reemit; P.dr_events = direct->events; P.dr_redirect = direct->blocks - 1;
+  }
+  // The row runs that meet rows [y0, y1): a shard is one run {0, n_owned, rank, world}, a source list cut into arithmetic runs
+  // (rthx_trace_exchange_rows) has one per run.  Row y of run {r0, n, e0, s} is element e0 + (y - r0) s.
+  const std::vector<int4> shard_run{make_int4(0, pl.n_owned, rank, world)};
+  const std::vector<int4>& runs = direct ? h->row_runs : shard_run;
+  auto for_runs = [&](int y0, int y1, auto&& f) -> int {
+    for (const int4& run : runs) {
+      const int r0 = std::max(y0, run.x), r1 = std::min(y1, run.x + run.y);
+      if (r1 > r0) { const int rcf = f(run, r0, r1); if (rcf) return rcf; }
+    }
+    return RTHX_OK;
+  };
 
   // row groups in ascending order: a group whose pairs overran the buffer is traced again as two halves
   std::vector<std::pair<int, int>> todo{{0, pl.n_owned}};
@@ -1841,27 +1925,55 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     todo.erase(todo.begin());
     if (y1 <= y0) continue;
     CU(h, cudaMemsetAsync(h->sk_ctl, 0, 4 * sizeof(unsigned long long), h->stream));
-    P.y_offset = y0;
+    if (direct) CU(h, cudaMemsetAsync(direct->events, 0, sizeof(unsigned long long), h->stream));
     CU(h, cudaEventRecord(h->ev[1], h->stream));
-    CU(h, launch_trace_exchange(P, pl.kernel, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, h->stream));
+    if (!direct) {
+      P.y_offset = y0;
+      CU(h, launch_trace_exchange(P, pl.kernel, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, h->stream));
+      R.n_launches += 2;
+    } else {                                                 // one launch per arithmetic run of the source list, as rthx_trace_direct
+      rthx_trace_args longest = *a;
+      longest.rays_per_emitter = direct->max_rays;
+      rc = for_runs(y0, y1, [&](const int4& run, int r0, int r1) -> int {
+        P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r1 - r0));
+        P.emitter_world = run.w; P.emitter_rank = run.z - run.x * run.w;
+        P.y_offset = r0;
+        if ((long long)(r1 - r0) * P.row_chunks > 0x7FFFFFFFll)
+          return fail(h, RTHX_ERR_ARG, "trace_direct_sparse: too many bundles for one launch (a launch has at most 2^31 blocks)");
+        CU(h, launch_trace_exchange(P, pl.kernel, (r1 - r0) * P.row_chunks, pl.block_threads, pl.smem_bytes, h->stream));
+        R.n_launches += 1;
+        return RTHX_OK;
+      });
+      if (rc) return rc;
+      R.n_launches += 2;
+    }
     CU(h, cudaEventRecord(h->ev[2], h->stream));
-    R.n_launches += 2;
-    unsigned long long ctl[4];
+    unsigned long long ctl[4], events = 0;
     CU(h, cudaMemcpyAsync(ctl, h->sk_ctl, sizeof(ctl), cudaMemcpyDeviceToHost, h->stream));
+    if (direct) CU(h, cudaMemcpyAsync(&events, direct->events, sizeof(events), cudaMemcpyDeviceToHost, h->stream));
     CU(h, cudaStreamSynchronize(h->stream));
     float ms = 0;
     CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2])); R.kernel_ms += ms;
     if (ctl[1]) {
-      if (y1 - y0 == 1) return fail(h, RTHX_ERR_NOMEM, "trace_sparse: the pairs of one emitter row exceed the pair buffer (" + std::to_string(cap) + " pairs)");
+      if (y1 - y0 == 1) {
+        if (direct)
+          return fail(h, RTHX_ERR_NOMEM, "trace_direct_sparse: the pairs of source row " + std::to_string(y0) + " (element " + std::to_string(h->rows[y0]) +
+                                             ") exceed the pair buffer (" + std::to_string(cap) + " pairs)");
+        return fail(h, RTHX_ERR_NOMEM, "trace_sparse: the pairs of one emitter row exceed the pair buffer (" + std::to_string(cap) + " pairs)");
+      }
       for (int b = 0; b < nb; ++b)                          // the lost rays of the group are counted again
-        CU(h, cudaMemset2DAsync(h->lost_dev + (size_t)b * N + rank + (size_t)y0 * world, sizeof(unsigned long long) * world, 0,
-                                sizeof(unsigned long long), (size_t)(y1 - y0), h->stream));
+        rc = for_runs(y0, y1, [&](const int4& run, int r0, int r1) -> int {
+          CU(h, cudaMemset2DAsync(h->lost_dev + (size_t)b * N + run.z + (size_t)(r0 - run.x) * run.w, sizeof(unsigned long long) * run.w, 0,
+                                  sizeof(unsigned long long), (size_t)(r1 - r0), h->stream));
+          return RTHX_OK;
+        });
+      if (rc) return rc;
       const int mid = y0 + (y1 - y0) / 2;
       todo.insert(todo.begin(), {{y0, mid}, {mid, y1}});
       continue;
     }
     const long long n = (long long)ctl[0];
-    ++R.groups; R.pairs += n; R.flushes += (long long)ctl[2];
+    ++R.groups; R.pairs += n; R.flushes += (long long)ctl[2]; R.events += events;
     CU(h, grow_keep(out_keys, keys_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
     CU(h, grow_keep(out_vals, vals_cap, (size_t)(total + std::max(n, 1ll)), (size_t)total, h->stream));
     CU(h, cudaEventRecord(h->ev[1], h->stream));
@@ -2469,7 +2581,7 @@ int need_resident(rthx_handle* h, ReadOut what, int bin, int n = 0) {
   if (what == READ_ROWS || what == READ_COLUMNS)
     return have ? RTHX_OK : fail(h, RTHX_ERR_ARG, "counts: no resident counts for that bin (run rthx_trace_exchange with counts_out == NULL, rthx_trace_exchange_multi with counts_out == NULL, or rthx_trace_exchange_sparse first)");
   const std::string who = what == READ_SMOOTH ? "smooth" : "smooth_sparse";
-  if (r.kind == RESIDENT_DIRECT)
+  if (r.direct())
     return fail(h, RTHX_ERR_ARG, who + ": the resident counts are those of a direct trace (rthx_trace_direct): absorptions with re-emission, not exchange factors");
   if (what == READ_SMOOTH && r.kind == RESIDENT_SPARSE)
     return fail(h, RTHX_ERR_ARG, "smooth: the resident counts are the sparse form of rthx_trace_exchange_sparse (smooth them with rthx_smooth_sparse)");
@@ -2504,9 +2616,9 @@ int prepare_rows(rthx_handle* h, int bin) {
     CU(h, cudaMalloc(&h->csr_rowptr, sizeof(long long) * ((size_t)N + 1)));
     h->csr_cap = (size_t)N + 1;
   }
-  if (res.kind == RESIDENT_SPARSE) {
-    CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, res.n_bins(), bin, R, N, h->ns, res.own.rank, res.own.world, h->csr_nnz,
-                                h->csr_rowsum, h->csr_cross, h->stream));
+  if (res.hashed()) {
+    CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, res.n_bins(), bin, R, N, h->ns, res.own.rank, res.own.world,
+                                res.own.listed ? h->rows_dev : nullptr, h->csr_nnz, h->csr_rowsum, h->csr_cross, h->stream));
   } else {
     CU(h, rthx::launch_row_nnz(resident_counts(h, bin), R, N, (size_t)N, h->ns, res.own.rank, res.own.world, res.own.listed ? h->rows_dev : nullptr,
                                h->csr_nnz, h->csr_rowsum, h->csr_cross, h->stream));
@@ -2540,19 +2652,22 @@ cudaError_t sparse_transpose(int n, int nnz, const long long* colptr, const int*
 }  // namespace rthx
 
 namespace {
-// Leading n x n block of the hashed tally's rows (bin `bin`, all emitters) as CSC in the sparse smoothing's scratch: colptr -> cp [n+1],
-// rowval -> sp_rowval, F = count / row total over the block -> sp_val (the values rthx_counts_csc computes); *nnz_out its non-zeros.
-// The CSR of the block is transposed by the radix sort of rthx_smooth_sparse (sparse_transpose), so rows ascend within each column.
+// The first n_rows resident rows of the hashed tally (bin `bin`), over the columns < n, as CSC in the sparse smoothing's scratch:
+// colptr -> cp [n+1], rowval -> sp_rowval, F = count / row total over the block -> sp_val (the values rthx_counts_csc computes);
+// *nnz_out its non-zeros.  n_rows = n: the leading n x n block (all emitters); n_rows < n: the listed rows of a direct trace, row y in
+// the low word of the sorted keys (tally_key_index maps it to its element).  The CSR of the block is transposed by the radix sort of
+// rthx_smooth_sparse (sparse_transpose), so rows ascend within each column; it takes an int nnz, a larger set is RTHX_ERR_ARG.
 // With counts != nullptr the count of every entry (as bits) is sorted along instead of F.  vec: 3 n scratch words.
-int hashed_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long long* rptr, void* vec, bool counts, long long* nnz_out) {
+int hashed_counts_to_csc(rthx_handle* h, int bin, int n_rows, int n, long long* cp, long long* rptr, void* vec, bool counts, long long* nnz_out) {
   unsigned long long* rowsum = reinterpret_cast<unsigned long long*>(vec);
   int* row_nnz = reinterpret_cast<int*>(rowsum + n);
-  CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, n, n, h->ns, 0, 1, row_nnz, rowsum, nullptr, h->stream));
-  std::vector<int> rn((size_t)n);
-  CU(h, cudaMemcpyAsync(rn.data(), row_nnz, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+  CU(h, rthx::tally_row_stats(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, n_rows, n, h->ns, 0, 1, nullptr, row_nnz, rowsum, nullptr,
+                              h->stream));
+  std::vector<int> rn((size_t)n_rows);
+  if (n_rows > 0) CU(h, cudaMemcpyAsync(rn.data(), row_nnz, sizeof(int) * (size_t)n_rows, cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaStreamSynchronize(h->stream));
-  std::vector<long long> rp((size_t)n + 1, 0);
-  for (int i = 0; i < n; ++i) rp[i + 1] = rp[i] + rn[i];
+  std::vector<long long> rp((size_t)n + 1, 0);        // rows past n_rows are empty: the transpose runs over n "columns" of the CSR
+  for (int i = 0; i < n; ++i) rp[i + 1] = rp[i] + (i < n_rows ? rn[i] : 0);
   const long long nnz = rp[n];
   if (nnz > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, "sparse counts: more than 2^31 - 1 non-zeros in one column view");
   CU(h, cudaMemcpyAsync(rptr, rp.data(), sizeof(long long) * ((size_t)n + 1), cudaMemcpyHostToDevice, h->stream));
@@ -2562,7 +2677,7 @@ int hashed_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long lon
   CU(h, ensure(&h->sp_keys, &h->sp_keys_cap, 2 * nz1));
   const size_t tmp_bytes = rthx::sparse_sort_temp_bytes((int)nnz, n);
   CU(h, ensure(reinterpret_cast<char**>(&h->sp_tmp), &h->sp_tmp_cap, tmp_bytes));
-  CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, n, n, rptr, rowsum, true, h->sp_rowval,
+  CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, n_rows, n, rptr, rowsum, true, h->sp_rowval,
                              counts ? reinterpret_cast<unsigned long long*>(h->sp_val) : nullptr, counts ? nullptr : h->sp_val, h->stream));
   CU(h, rthx::sparse_transpose(n, (int)nnz, rptr, h->sp_rowval, h->sp_val, h->sp_keys, h->sp_keys + nz1, h->sp_val + nz1, cp, h->sp_tmp, tmp_bytes,
                                h->stream));
@@ -2570,33 +2685,59 @@ int hashed_counts_to_csc(rthx_handle* h, int bin, int n, long long* cp, long lon
   return RTHX_OK;
 }
 
-// rthx_counts_csc after a sparse trace: sorted transpose keys -> rowval (+ base), sorted values -> F_vals / vals
-int counts_csc_sparse(rthx_handle* h, int bin, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, uint64_t* vals, double* F_vals) {
+// Scratch of a column view of the hashed set (hashed_counts_to_csc over N columns): csc_colptr [N+1], and in csr_out the row pointers
+// [N+1] (*rptr) followed by 3 N words of row totals / non-zeros
+int hashed_csc_scratch(rthx_handle* h, long long** rptr) {
   const int N = h->N;
   CU(h, ensure(&h->csc_colptr, &h->csc_colptr_cap, (size_t)N + 1));
-  const size_t need = (3 * (size_t)N + 1) * sizeof(unsigned long long);   // row pointers + row totals / non-zeros scratch
+  const size_t need = (3 * (size_t)N + 1) * sizeof(unsigned long long);
   if (h->csr_out_cap < need) {
     cudaFree(h->csr_out); h->csr_out = nullptr; h->csr_out_cap = 0;
     CU(h, cudaMalloc(&h->csr_out, need));
     h->csr_out_cap = need;
   }
-  long long* rptr = reinterpret_cast<long long*>(h->csr_out);
+  *rptr = reinterpret_cast<long long*>(h->csr_out);
+  return RTHX_OK;
+}
+
+// rthx_counts_csc after a sparse trace: sorted transpose keys -> rowval (+ base), sorted values -> F_vals / vals
+int counts_csc_sparse(rthx_handle* h, int bin, int index_base, int rowval_is_i64, int64_t* colptr, void* rowval, uint64_t* vals, double* F_vals) {
+  const int N = h->N;
+  long long* rptr = nullptr;
+  int rc = hashed_csc_scratch(h, &rptr);
+  if (rc) return rc;
   void* vec = rptr + (size_t)N + 1;
   long long nnz = 0;
-  int rc = hashed_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, false, &nnz);
-  if (rc) return rc;
+  const int R = h->res.n_rows;                               // N, or the listed rows of a direct trace
+  const int* rows = h->res.own.listed ? h->rows_dev : nullptr;
+  if ((rc = hashed_counts_to_csc(h, bin, R, N, h->csc_colptr, rptr, vec, false, &nnz))) return rc;
   if (F_vals && nnz && (rc = copy_out(h, F_vals, h->sp_val + std::max<long long>(nnz, 1), sizeof(double) * (size_t)nnz, h->stream))) return rc;
   if (vals) {                                                // the counts ride along a second sort of the same keys
-    if ((rc = hashed_counts_to_csc(h, bin, N, h->csc_colptr, rptr, vec, true, &nnz))) return rc;
+    if ((rc = hashed_counts_to_csc(h, bin, R, N, h->csc_colptr, rptr, vec, true, &nnz))) return rc;
     if (nnz && (rc = copy_out(h, vals, h->sp_val + std::max<long long>(nnz, 1), sizeof(uint64_t) * (size_t)nnz, h->stream))) return rc;
   }
   const size_t nz1 = (size_t)std::max<long long>(nnz, 1);
   // the indices: low words of the sorted keys, written over the unsorted keys
-  CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz, index_base, h->sp_keys, rowval_is_i64 != 0, h->stream));
+  CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz, index_base, rows, h->sp_keys, rowval_is_i64 != 0, h->stream));
   if (index_base) CU(h, rthx::launch_add_base(h->csc_colptr, N + 1, (long long)index_base, h->stream));
   if ((rc = copy_out(h, colptr, h->csc_colptr, sizeof(long long) * ((size_t)N + 1), h->stream))) return rc;
   if (nnz && (rc = copy_out(h, rowval, h->sp_keys, (rowval_is_i64 ? sizeof(long long) : sizeof(int)) * (size_t)nnz, h->stream))) return rc;
   CU(h, cudaStreamSynchronize(h->stream));
+  return RTHX_OK;
+}
+
+// rthx_trace_direct_sparse: out[k] = sum_y w[y] count[y][k] over count block `block` of the R resident source rows, in
+// ascending y with every product and sum rounded on its own — direct_absorbed_kernel's sum.  The block is transposed to columns with
+// the key sort of the CSC read-out (hashed_counts_to_csc), then one thread per column walks its entries.
+int direct_column_sums(rthx_handle* h, int block, int R, const double* w, double* out) {
+  const int N = h->N;
+  long long* rptr = nullptr;
+  long long nnz = 0;
+  int rc = hashed_csc_scratch(h, &rptr);
+  if (rc || (rc = hashed_counts_to_csc(h, block, R, N, h->csc_colptr, rptr, rptr + (size_t)N + 1, true, &nnz))) return rc;
+  const size_t nz1 = (size_t)std::max<long long>(nnz, 1);
+  CU(h, launch_direct_absorbed_sparse(h->csc_colptr, h->sp_keys + nz1, reinterpret_cast<const unsigned long long*>(h->sp_val + nz1), N, w, out,
+                                      h->stream));
   return RTHX_OK;
 }
 }  // namespace
@@ -2635,7 +2776,7 @@ extern "C" int rthx_counts_csr(rthx_handle* h, int bin, int64_t* row_ptr, int32_
   double* d_f = (double*)(d_vals + std::max<size_t>(1, nnz));
   int* d_cols = (int*)(d_f + std::max<size_t>(1, nnz));
   const int R = h->res.n_rows;
-  if (h->res.kind == RESIDENT_SPARSE) {
+  if (h->res.hashed()) {
     CU(h, rthx::tally_row_fill(h->sk_keys, h->sk_vals, h->sk_rowptr, h->res.n_bins(), bin, R, N, h->csr_rowptr, h->csr_rowsum, false, d_cols, d_vals,
                                F_vals ? d_f : nullptr, h->stream));
   } else {
@@ -2661,7 +2802,7 @@ extern "C" int rthx_counts_csc(rthx_handle* h, int bin, int index_base, int rowv
   const int N = h->N;
   const size_t nnz = (size_t)h->csr_total, nz1 = std::max<size_t>(1, nnz);
   if (!rowval_is_i64 && (size_t)N + (size_t)index_base > 0x7FFFFFFFull) return fail(h, RTHX_ERR_ARG, "counts_csc: 32-bit row indices overflow");
-  if (h->res.kind == RESIDENT_SPARSE) return counts_csc_sparse(h, bin, index_base, rowval_is_i64, colptr, rowval, vals, F_vals);
+  if (h->res.hashed()) return counts_csc_sparse(h, bin, index_base, rowval_is_i64, colptr, rowval, vals, F_vals);
   const int R = h->res.n_rows;                                // N, or the listed rows of a rows trace (the other rows are empty)
   const int n_tiles = (R + 63) / 64;
   CU(h, ensure(&h->csc_partial, &h->csc_partial_cap, (size_t)std::max(n_tiles, 1) * (size_t)N));
@@ -2833,10 +2974,10 @@ extern "C" int rthx_smooth_sparse(rthx_handle* h, int source, int bin, int n, co
   CU(h, cudaEventRecord(h->ev[0], h->stream));
   if (source == RTHX_SMOOTH_FROM_LAST_TRACE && h->res.kind == RESIDENT_SPARSE) {
     // the hashed tally's rows cropped to n, F = count / row total over the crop, transposed to CSC (same values and order as below)
-    int rc = hashed_counts_to_csc(h, bin, n, cp, rptr, vec + n, false, &nnz_f);
+    int rc = hashed_counts_to_csc(h, bin, n, n, cp, rptr, vec + n, false, &nnz_f);
     if (rc) return rc;
     const size_t nz1 = (size_t)std::max<long long>(nnz_f, 1);
-    CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz_f, 0, h->sp_rowval, false, h->stream));
+    CU(h, rthx::tally_key_index(h->sp_keys + nz1, nnz_f, 0, nullptr, h->sp_rowval, false, h->stream));
     if (nnz_f) CU(h, cudaMemcpyAsync(h->sp_val, h->sp_val + nz1, sizeof(double) * (size_t)nnz_f, cudaMemcpyDeviceToDevice, h->stream));
   } else if (source == RTHX_SMOOTH_FROM_LAST_TRACE) {
     // F = counts / row total over the crop, compacted to CSC by the read-out kernels of rthx_counts_csc

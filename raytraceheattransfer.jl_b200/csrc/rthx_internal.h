@@ -149,6 +149,7 @@ struct TraceKernelSel {
     QUEUE,      // trace_exchange_queue_kernel: per-warp ray queue (multi-face meshes; MULTI_BOUNCE on analytic meshes)
     HASH,       // trace_exchange_hash_kernel: hashed row tally (rthx_trace_exchange_sparse)
     DIRECT,     // trace_direct_kernel: MULTI_BOUNCE with re-emission (rthx_trace_direct)
+    DIRECT_HASH,  // trace_direct_hash_kernel: the same with the hashed row tally (rthx_trace_direct_sparse)
   };
   Family family = LOCKSTEP;
   bool hist = false;      // row histogram in shared memory (SQ and QUEUE always, HASH never)
@@ -166,6 +167,7 @@ struct TraceKernelSel {
   static constexpr TraceKernelSel queue(bool fast, bool multi, int depth, bool general) { return {QUEUE, true, fast, multi, depth, general}; }
   static constexpr TraceKernelSel hash(bool fast) { return {HASH, false, fast, false, 0, false}; }
   static constexpr TraceKernelSel direct(bool hist, bool fast) { return {DIRECT, hist, fast, true, 0, false}; }
+  static constexpr TraceKernelSel direct_hash(bool fast) { return {DIRECT_HASH, false, fast, true, 0, false}; }
 };
 
 // launchers implemented in rthx_kernels.cu; a selection without a compiled instance fails with cudaErrorInvalidDeviceFunction
@@ -176,6 +178,10 @@ cudaError_t launch_fp64_peak(double* out, int n_blocks, int block_threads, int i
 int trace_kernel_max_blocks_per_sm(const TraceKernelSel& k, int block_threads, size_t smem_bytes);
 // Abs[k] = sum_i w[i] counts[i][k] over R rows of N, in ascending row order (rthx_trace_direct)
 cudaError_t launch_direct_absorbed(const unsigned long long* counts, int R, int N, const double* w, double* absorbed, cudaStream_t stream);
+// the same sum over a hashed direct tally transposed to columns: colptr [N+1], keys (source row in the low word, ascending within a
+// column) and u64 counts (rthx_trace_direct_sparse)
+cudaError_t launch_direct_absorbed_sparse(const long long* colptr, const unsigned long long* keys, const unsigned long long* cnt, int N, const double* w,
+                                          double* absorbed, cudaStream_t stream);
 constexpr size_t hash_table_bytes(int slots) { return 8 * (size_t)slots + 16; }   // keys + counts (u32 each) + occupied / fill / base words
 
 // hashed row tally, host side of the reduction (rthx_sparse_tally.cu)
@@ -186,10 +192,11 @@ cudaError_t tally_reduce(unsigned long long* keys, uint32_t* cnt, unsigned long 
                          cudaStream_t st);
 // row pointers [n_rows + 1] of the sorted unique keys (row key in the high word)
 cudaError_t tally_row_ptr(const unsigned long long* keys, long long nnz, long long n_rows, long long* row_ptr, cudaStream_t st);
-// rows of bin `bin` (row key y * n_bins + bin, y < n_rows): non-zeros, total and surface-gas cross tallies over the columns < n_cols
+// rows of bin `bin` (row key y * n_bins + bin, y < n_rows): non-zeros, total and surface-gas cross tallies over the columns < n_cols.
+// Row y is element row_first + y * row_stride, or rows[y] when rows != nullptr (a rows or direct trace).
 cudaError_t tally_row_stats(const unsigned long long* keys, const unsigned long long* vals, const long long* row_ptr, int n_bins, int bin, int n_rows,
-                            int n_cols, int n_surf, int row_first, int row_stride, int* nnz, unsigned long long* rowsum, unsigned long long* cross,
-                            cudaStream_t st);
+                            int n_cols, int n_surf, int row_first, int row_stride, const int* rows, int* nnz, unsigned long long* rowsum,
+                            unsigned long long* cross, cudaStream_t st);
 // the same rows as CSR at out_ptr[row]: columns < n_cols, counts, and F = count * (1 / total) (divide == false, the CSR read-out) or
 // count / total (divide == true, the CSC read-out)
 cudaError_t tally_row_fill(const unsigned long long* keys, const unsigned long long* vals, const long long* row_ptr, int n_bins, int bin, int n_rows,
@@ -202,8 +209,9 @@ size_t tally_merge_temp_bytes(long long n_tiles);
 cudaError_t tally_merge(const unsigned long long* a_keys, const unsigned long long* a_vals, long long na, const unsigned long long* b_keys,
                         const unsigned long long* b_vals, long long nb, unsigned long long* out_keys, unsigned long long* out_vals, long long* tiles,
                         void* temp, size_t temp_bytes, cudaStream_t st);
-// low words of sorted transpose keys (the rows of a CSC) + base as int32 / int64
-cudaError_t tally_key_index(const unsigned long long* keys_sorted, long long nnz, int base, void* out, bool i64, cudaStream_t st);
+// low words of sorted transpose keys (the rows of a CSC) + base as int32 / int64; with rows != nullptr the low word y stands for
+// element rows[y] (a rows or direct trace)
+cudaError_t tally_key_index(const unsigned long long* keys_sorted, long long nnz, int base, const int* rows, void* out, bool i64, cudaStream_t st);
 
 // ---- grey equilibrium solve (rthx_solve.cu) ---------------------------------------------------------------------
 struct SolveMatrix {

@@ -395,7 +395,10 @@ __device__ __forceinline__ void hash_insert(uint32_t* tab, int log2s, int absorb
 }
 
 // Block-uniform: every thread calls it at the same point.  Returns false when the pair buffer is full (the block must stop).
-__device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, unsigned long long row_key) {
+// DIRECT (trace_direct_hash_kernel): a key carries the count block in bit 31 (direct_hash_tally); block b of row y is flushed as row key
+// row_key + b, row_key = y * count blocks (the key layout of a rows trace with n_bins = count blocks).
+template <bool DIRECT>
+__device__ __forceinline__ bool hash_flush_body(const TraceParams& p, uint32_t* tab, unsigned long long row_key) {
   const uint32_t S = 1u << p.sk_slots_log2;
   uint32_t* occ = tab + 2 * S;
   unsigned long long* base = reinterpret_cast<unsigned long long*>(tab + 2 * S + 2);
@@ -421,7 +424,8 @@ __device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, uns
     w = __shfl_sync(0xffffffffu, w, 0);
     if (k) {
       const unsigned long long d = b + w + __popc(m & ((1u << lane) - 1u));
-      p.sk_keys[d] = (row_key << 32) | (unsigned long long)(k - 1u);
+      if (DIRECT) p.sk_keys[d] = ((row_key + (k >> 31)) << 32) | (unsigned long long)((k & 0x7FFFFFFFu) - 1u);
+      else p.sk_keys[d] = (row_key << 32) | (unsigned long long)(k - 1u);
       p.sk_cnt[d] = tab[S + i];
       tab[i] = 0u; tab[S + i] = 0u;
     }
@@ -430,6 +434,40 @@ __device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, uns
   if (threadIdx.x == 0) *occ = 0u;
   __syncthreads();
   return true;
+}
+
+__device__ __noinline__ bool hash_flush(const TraceParams& p, uint32_t* tab, unsigned long long row_key) { return hash_flush_body<false>(p, tab, row_key); }
+__device__ __noinline__ bool direct_hash_flush(const TraceParams& p, uint32_t* tab, unsigned long long row_key) {
+  return hash_flush_body<true>(p, tab, row_key);
+}
+
+// method=:direct on the hashed tally (trace_direct_hash_kernel): tally one event of count block `block` (0 absorption, 1 redirection) in
+// column `col` of the block's row.  A direct bundle tallies at every absorption by a re-emitting element and, with the redirection tally,
+// at every scattering or reflection, inside an event loop where the threads of a block diverge: there is no block-wide point at which
+// the table could be flushed when it fills.  So the insert is bounded instead: a tally that finds neither its key nor an empty slot
+// within kDirectProbe slots is appended to the pair buffer as a pair (key, 1) of its own.  The sort and reduce-by-key sum equal keys,
+// so where a tally lands does not change the totals.  Key: column + 1, count block in bit 31 (N < 2^31).
+constexpr int kDirectProbe = 32;
+__device__ __forceinline__ void direct_hash_tally(const TraceParams& p, uint32_t* tab, unsigned long long row_key, int block, int col) {
+  const int log2s = p.sk_slots_log2;
+  const uint32_t mask = (1u << log2s) - 1u, key = ((uint32_t)col + 1u) | ((uint32_t)block << 31);
+  uint32_t s = (key * 0x9E3779B1u) >> (32 - log2s);
+  for (int i = 0; i < kDirectProbe; ++i) {
+    const uint32_t prev = atomicCAS(&tab[s], 0u, key);
+    if (prev == 0u || prev == key) {
+      atomicAdd(&tab[(mask + 1u) + s], 1u);
+      if (prev == 0u) atomicAdd(&tab[2 * (mask + 1u)], 1u);
+      return;
+    }
+    s = (s + 1u) & mask;
+  }
+  const unsigned long long d = atomicAdd(&p.sk_ctl[0], 1ull);
+  if (d < p.sk_cap) {
+    p.sk_keys[d] = ((row_key + (unsigned long long)block) << 32) | (unsigned long long)col;
+    p.sk_cnt[d] = 1u;
+  } else {
+    atomicExch(&p.sk_ctl[1], 1ull);              // the pair buffer is full: the host traces this group of rows again, split
+  }
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -453,11 +491,13 @@ constexpr int EM_DOUBLES = 16;
 // stage 1 of the trace body, with k's geometry read from the mesh tables instead of shared memory.  Its Philox words are calls
 // 0x8000 + 2m and 0x8001 + 2m (m-th re-emission of the bundle), in the upper half of the call field, disjoint from the event calls
 // 2 + 2n, 3 + 2n (n < 16000).
-template <bool HIST_SMEM>
+// HASH (trace_direct_hash_kernel): the absorption goes to the hashed table of row key `row_key` (direct_hash_tally).
+template <bool HIST_SMEM, bool HASH = false>
 __device__ __forceinline__ void direct_reemit(const TraceParams& p, uint32_t* hist, unsigned long long* count_row, int k, uint32_t c_lo,
                                               uint32_t c_hi, uint32_t e, uint32_t cw, int m, const double2* s_log, double& px, double& py,
-                                              double& dx, double& dy, double& neg_log, int& c) {
-  if (HIST_SMEM) atomicAdd(&hist[k], 1u);
+                                              double& dx, double& dy, double& neg_log, int& c, unsigned long long row_key = 0) {
+  if constexpr (HASH) direct_hash_tally(p, hist, row_key, 0, k);
+  else if (HIST_SMEM) atomicAdd(&hist[k], 1u);
   else atomicAdd(&count_row[k], 1ULL);
   const uint4 w0 = philox4x32_10_rk(make_uint4(c_lo, c_hi, e, cw | (uint32_t)(0x8000 + 2 * m)), p.rk);
   const uint4 w1 = philox4x32_10_rk(make_uint4(c_lo, c_hi, e, cw | (uint32_t)(0x8001 + 2 * m)), p.rk);
@@ -524,6 +564,16 @@ __global__ void __launch_bounds__(256, 2) trace_direct_kernel(const __grid_const
 #include "rthx_trace_body.cuh"
 }
 
+// method=:direct with the hashed row tally (rthx_trace_direct_sparse): the body of trace_direct_kernel with the table of
+// trace_exchange_hash_kernel in place of the histogram.  Rounds of blockDim.x bundles; the table is flushed between rounds once it is
+// half full, and inside a round a tally that finds no slot goes straight to the pair buffer (direct_hash_tally).  Row y's absorptions
+// flush as row key y * (1 + dr_redirect), its redirections as the key after it.
+template <bool FAST>
+__global__ void __launch_bounds__(256, 2) trace_direct_hash_kernel(const __grid_constant__ TraceParams p) {
+  constexpr bool HIST_SMEM = false, MULTI = true, HASH = true, REEMIT = true;
+#include "rthx_trace_body.cuh"
+}
+
 // Absorbed power of every element, Abs[k] = sum_i w[i] count[i][k] over the R resident source rows, summed in ascending row order
 // with every product and sum rounded on its own (no FMA contraction): the same sum, bit for bit, as a host loop over the rows.
 __global__ void __launch_bounds__(256) direct_absorbed_kernel(const unsigned long long* __restrict__ counts, int R, int N,
@@ -538,6 +588,26 @@ __global__ void __launch_bounds__(256) direct_absorbed_kernel(const unsigned lon
 cudaError_t launch_direct_absorbed(const unsigned long long* counts, int R, int N, const double* w, double* absorbed, cudaStream_t stream) {
   if (N <= 0) return cudaSuccess;
   direct_absorbed_kernel<<<(N + 255) / 256, 256, 0, stream>>>(counts, R, N, w, absorbed);
+  return cudaGetLastError();
+}
+
+// The same sum from a hashed direct tally (rthx_trace_direct_sparse), transposed to columns: column k's non-zero counts are at
+// [colptr[k], colptr[k+1]) with the source row in the low word of keys[p], ascending, and the count in cnt[p].  The dense sum adds
+// w[i] * 0 = +0.0 for every zero count, which leaves its partial sums (>= +0.0) unchanged, so both sums are the same bits.
+__global__ void __launch_bounds__(256) direct_absorbed_sparse_kernel(const long long* __restrict__ colptr, const unsigned long long* __restrict__ keys,
+                                                                    const unsigned long long* __restrict__ cnt, int N, const double* __restrict__ w,
+                                                                    double* __restrict__ absorbed) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= N) return;
+  double acc = 0.0;
+  for (long long q = colptr[k]; q < colptr[k + 1]; ++q) acc = __dadd_rn(acc, __dmul_rn(w[keys[q] & 0xffffffffull], (double)cnt[q]));
+  absorbed[k] = acc;
+}
+
+cudaError_t launch_direct_absorbed_sparse(const long long* colptr, const unsigned long long* keys, const unsigned long long* cnt, int N, const double* w,
+                                          double* absorbed, cudaStream_t stream) {
+  if (N <= 0) return cudaSuccess;
+  direct_absorbed_sparse_kernel<<<(N + 255) / 256, 256, 0, stream>>>(colptr, keys, cnt, N, w, absorbed);
   return cudaGetLastError();
 }
 
@@ -1688,6 +1758,8 @@ static const TraceInstance k_trace_instances[] = {
     {Sel::direct(true, false), trace_direct_kernel<true, false>},
     {Sel::direct(false, true), trace_direct_kernel<false, true>},
     {Sel::direct(false, false), trace_direct_kernel<false, false>},
+    {Sel::direct_hash(true), trace_direct_hash_kernel<true>},
+    {Sel::direct_hash(false), trace_direct_hash_kernel<false>},
 };
 
 static TraceKernel trace_kernel(const TraceKernelSel& k) {

@@ -35,13 +35,14 @@ __global__ void __launch_bounds__(256) row_ptr_kernel(const unsigned long long* 
 // one warp per row (same reductions as row_nnz_kernel: integer sums, so the order does not matter)
 __global__ void __launch_bounds__(256) tally_stats_kernel(const unsigned long long* __restrict__ keys, const unsigned long long* __restrict__ vals,
                                                           const long long* __restrict__ row_ptr, int n_bins, int bin, int n_rows, int n_cols,
-                                                          int n_surf, int row_first, int row_stride, int* __restrict__ nnz,
+                                                          int n_surf, int row_first, int row_stride, const int* __restrict__ rows,
+                                                          int* __restrict__ nnz,
                                                           unsigned long long* __restrict__ rowsum, unsigned long long* __restrict__ cross) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= n_rows) return;
   const size_t rk = (size_t)row * n_bins + bin;
   const long long b = row_ptr[rk], e = row_ptr[rk + 1];
-  const bool row_surf = row_first + row * row_stride < n_surf;
+  const bool row_surf = (rows ? rows[row] : row_first + row * row_stride) < n_surf;
   int cnt = 0;
   unsigned long long s = 0, x = 0;
   for (long long p = b + lane; p < e; p += 32) {
@@ -81,9 +82,12 @@ __global__ void __launch_bounds__(256) tally_fill_kernel(const unsigned long lon
 }
 
 template <class IDX>
-__global__ void __launch_bounds__(256) key_index_kernel(const unsigned long long* __restrict__ keys, long long nnz, int base, IDX* __restrict__ out) {
-  for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < nnz; p += (long long)gridDim.x * blockDim.x)
-    out[p] = (IDX)(keys[p] & 0xffffffffull) + base;
+__global__ void __launch_bounds__(256) key_index_kernel(const unsigned long long* __restrict__ keys, long long nnz, int base, const int* __restrict__ rows,
+                                                        IDX* __restrict__ out) {
+  for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < nnz; p += (long long)gridDim.x * blockDim.x) {
+    const int y = (int)(keys[p] & 0xffffffffull);
+    out[p] = (IDX)(rows ? rows[y] : y) + base;
+  }
 }
 
 unsigned flat_grid(long long n) { return (unsigned)std::max<long long>(1, std::min<long long>((n + 255) / 256, 148 * 32)); }
@@ -224,10 +228,11 @@ cudaError_t tally_row_ptr(const unsigned long long* keys, long long nnz, long lo
 }
 
 cudaError_t tally_row_stats(const unsigned long long* keys, const unsigned long long* vals, const long long* row_ptr, int n_bins, int bin, int n_rows,
-                            int n_cols, int n_surf, int row_first, int row_stride, int* nnz, unsigned long long* rowsum, unsigned long long* cross,
-                            cudaStream_t st) {
+                            int n_cols, int n_surf, int row_first, int row_stride, const int* rows, int* nnz, unsigned long long* rowsum,
+                            unsigned long long* cross, cudaStream_t st) {
   if (n_rows > 0)
-    tally_stats_kernel<<<(n_rows + 7) / 8, 256, 0, st>>>(keys, vals, row_ptr, n_bins, bin, n_rows, n_cols, n_surf, row_first, row_stride, nnz, rowsum, cross);
+    tally_stats_kernel<<<(n_rows + 7) / 8, 256, 0, st>>>(keys, vals, row_ptr, n_bins, bin, n_rows, n_cols, n_surf, row_first, row_stride, rows, nnz, rowsum,
+                                                         cross);
   return cudaGetLastError();
 }
 
@@ -239,10 +244,10 @@ cudaError_t tally_row_fill(const unsigned long long* keys, const unsigned long l
   return cudaGetLastError();
 }
 
-cudaError_t tally_key_index(const unsigned long long* keys_sorted, long long nnz, int base, void* out, bool i64, cudaStream_t st) {
+cudaError_t tally_key_index(const unsigned long long* keys_sorted, long long nnz, int base, const int* rows, void* out, bool i64, cudaStream_t st) {
   if (nnz <= 0) return cudaSuccess;
-  if (i64) key_index_kernel<long long><<<flat_grid(nnz), 256, 0, st>>>(keys_sorted, nnz, base, (long long*)out);
-  else key_index_kernel<int><<<flat_grid(nnz), 256, 0, st>>>(keys_sorted, nnz, base, (int*)out);
+  if (i64) key_index_kernel<long long><<<flat_grid(nnz), 256, 0, st>>>(keys_sorted, nnz, base, rows, (long long*)out);
+  else key_index_kernel<int><<<flat_grid(nnz), 256, 0, st>>>(keys_sorted, nnz, base, rows, (int*)out);
   return cudaGetLastError();
 }
 

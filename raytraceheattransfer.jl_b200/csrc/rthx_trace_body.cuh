@@ -1,5 +1,5 @@
 // rthx_trace_body.cuh — body of K1 (rthx_kernels.cu), shared by trace_exchange_kernel<HIST_SMEM, FAST, MULTI>,
-// trace_exchange_hash_kernel<FAST> and trace_direct_kernel<HIST_SMEM, FAST>.  It is included INSIDE their function bodies, where
+// trace_exchange_hash_kernel<FAST>, trace_direct_kernel<HIST_SMEM, FAST> and trace_direct_hash_kernel<FAST>.  It is included INSIDE their function bodies, where
 // HIST_SMEM, FAST, MULTI, HASH and REEMIT are compile-time constants and `p` is the __grid_constant__ parameter: inlining it through a device function taking the
 // parameter by reference changed the code ptxas generates for the existing instances, textual inclusion does not.
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -84,16 +84,20 @@
   const uint32_t cw = ((uint32_t)band << 16);
   unsigned int n_lost = 0;
   [[maybe_unused]] unsigned int n_events = 0;   // REEMIT: traversal segments (one per interaction, or per loss)
-  const unsigned long long row_key = HASH ? (unsigned long long)y * (unsigned long long)p.n_bins + (unsigned long long)bi : 0ull;
+  // HASH && REEMIT: row y's count blocks are row keys y * (1 + dr_redirect) + block (one bin: bi = 0)
+  const unsigned long long row_key = !HASH ? 0ull
+                                     : REEMIT ? (unsigned long long)y * (unsigned long long)(1 + p.dr_redirect)
+                                              : (unsigned long long)y * (unsigned long long)p.n_bins + (unsigned long long)bi;
 
   // HASH: block-synchronous rounds (every thread runs every round; lanes past r_end only take part in the flush)
   for (int64_t r = r_begin + threadIdx.x; HASH ? r - (int64_t)threadIdx.x < r_end : r < r_end; r += blockDim.x) {
     if constexpr (HASH) {
       const uint32_t S = 1u << p.sk_slots_log2;
       __syncthreads();
-      const bool flush = hist[2 * S] + blockDim.x > S / 2;   // the coming round could pass half full
+      // the coming round could pass half full (REEMIT: the table is half full; a tally that finds no slot spills, direct_hash_tally)
+      const bool flush = REEMIT ? hist[2 * S] > S / 2 : hist[2 * S] + blockDim.x > S / 2;
       __syncthreads();
-      if (flush && !hash_flush(p, hist, row_key)) return;
+      if (flush && !(REEMIT ? direct_hash_flush(p, hist, row_key) : hash_flush(p, hist, row_key))) return;
       if (r >= r_end) continue;
     }
     const uint64_t ray_id = (uint64_t)(p.ray_id_offset + r);
@@ -232,7 +236,8 @@
       if (!(dec < p.omega[(size_t)band * p.n_cells + (absorber - p.n_surfaces)])) {        // absorbed in the gas
         if constexpr (REEMIT) {
           if (p.dr_reemit[absorber]) {
-            direct_reemit<HIST_SMEM>(p, hist, count_row, absorber, c_lo, c_hi, (uint32_t)e, cw, n_reemit++, s_log, px, py, dx, dy, neg_log, c);
+            direct_reemit<HIST_SMEM, HASH>(p, hist, count_row, absorber, c_lo, c_hi, (uint32_t)e, cw, n_reemit++, s_log, px, py, dx, dy, neg_log, c,
+                                           row_key);
             continue;
           }
         }
@@ -247,7 +252,8 @@
       if (dec < p.eps[(size_t)band * p.n_surfaces + absorber]) {                           // absorbed by the wall
         if constexpr (REEMIT) {
           if (p.dr_reemit[absorber]) {
-            direct_reemit<HIST_SMEM>(p, hist, count_row, absorber, c_lo, c_hi, (uint32_t)e, cw, n_reemit++, s_log, px, py, dx, dy, neg_log, c);
+            direct_reemit<HIST_SMEM, HASH>(p, hist, count_row, absorber, c_lo, c_hi, (uint32_t)e, cw, n_reemit++, s_log, px, py, dx, dy, neg_log, c,
+                                           row_key);
             continue;
           }
         }
@@ -270,7 +276,8 @@
     }
     if constexpr (REEMIT) {                     // a redirection (scattering or reflection) at `absorber`: second count block
       if (p.dr_redirect) {
-        if (HIST_SMEM) atomicAdd(&hist[N + absorber], 1u);
+        if (HASH) direct_hash_tally(p, hist, row_key, 1, absorber);
+        else if (HIST_SMEM) atomicAdd(&hist[N + absorber], 1u);
         else atomicAdd(&count_row[(size_t)p.n_owned * N + absorber], 1ULL);
       }
     }
@@ -280,6 +287,7 @@
     // ---- stage 3/4: tally (+ record) -------------------------------------------------------------------------
     if (absorber >= 0) {
       if (HIST_SMEM) atomicAdd(&hist[absorber], 1u);
+      else if (HASH && REEMIT) direct_hash_tally(p, hist, row_key, 0, absorber);
       else if (HASH) hash_insert(hist, p.sk_slots_log2, absorber);
       else if (p.flush_system) atomicAdd_system(&count_row[absorber], 1ULL);
       else atomicAdd(&count_row[absorber], 1ULL);
@@ -295,7 +303,7 @@
   }
 
   // ---- flush --------------------------------------------------------------------------------------------------
-  if (HASH && !hash_flush(p, hist, row_key)) return;
+  if (HASH && !(REEMIT ? direct_hash_flush(p, hist, row_key) : hash_flush(p, hist, row_key))) return;
   for (int off = 16; off > 0; off >>= 1) n_lost += __shfl_down_sync(0xffffffffu, n_lost, off);
   if ((threadIdx.x & 31) == 0 && n_lost) {
     if (p.flush_system) atomicAdd_system(&p.lost[(size_t)bi * N + e], (unsigned long long)n_lost);

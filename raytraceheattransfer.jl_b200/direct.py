@@ -52,17 +52,33 @@ def _row_sum(row_ptr, cols, vals, rows, w, out):
         out[cols[s]] = out[cols[s]] + w[i] * vals[s].astype(np.float64)
 
 
+def _hashed(n_rows: int, N: int, all_fields: bool) -> bool:
+    """Whether a device block of n_rows sources takes the hashed row tally (rthx_trace_direct_sparse): its dense counts, 8 R N bytes per
+    count block (two with all_fields), would pass the budget of one device that the :exchange route keeps to."""
+    from .tracing import rows_fit_one_device
+    return not rows_fit_one_device(n_rows, N, 2 if all_fields else 1)
+
+
+def _route(n_rows: int, N: int, all_fields: bool):
+    """trace_direct keywords of a device block of n_rows sources: the redirection tally with all_fields, the hashed tally when the dense
+    counts do not fit (_hashed)."""
+    out = dict(redirected=True) if all_fields else {}
+    if _hashed(n_rows, N, all_fields):
+        out["sparse"] = True
+    return out
+
+
 def _absorbed_multi(trs, sources, rays, reemit, w, N: int, specular: bool, kw, all_fields: bool = False):
     """Contiguous blocks of the source rows, one per device; the integer counts of every block are read back and reduced on the host in
     ascending row order with the device reduction's rounding, so the result does not depend on the number of devices.  all_fields: the
-    redirection counts (bin 1) are traced, read back and reduced the same way."""
+    redirection counts (bin 1) are traced, read back and reduced the same way.  Each block takes the dense or the hashed tally on its own
+    (_route); both read out the same counts."""
     from concurrent.futures import ThreadPoolExecutor
     blocks = [b for b in np.array_split(np.arange(len(sources)), len(trs)) if len(b)]
 
     def run(k):
         b = blocks[k]
-        fields = dict(redirected=True) if all_fields else {}
-        out = trs[k].trace_direct(sources[b], rays[b], reemit, w[b], specular=specular, **fields, **kw)
+        out = trs[k].trace_direct(sources[b], rays[b], reemit, w[b], specular=specular, **_route(len(b), N, all_fields), **kw)
         out["csr"] = trs[k].counts_csr(values=True, normalised=False)
         if all_fields:
             out["csr_redirected"] = trs[k].counts_csr(bin=1, values=True, normalised=False)
@@ -70,7 +86,8 @@ def _absorbed_multi(trs, sources, rays, reemit, w, N: int, specular: bool, kw, a
 
     with ThreadPoolExecutor(len(blocks)) as ex:
         outs = list(ex.map(run, range(len(blocks))))
-    res = dict(absorbed=np.zeros(N), lost=np.zeros(N, np.uint64), events=0, kernel_ms=0.0)
+    res = dict(absorbed=np.zeros(N), lost=np.zeros(N, np.uint64), events=0, kernel_ms=0.0,
+               tally="sparse" if any(_hashed(len(b), N, all_fields) for b in blocks) else "dense")
     if all_fields:
         res.update(redirected=np.zeros(N), redirections=0)
     for b, out in zip(blocks, outs):
@@ -99,7 +116,10 @@ def directRayTracing(rtm, rays_tot: int, nudge: Optional[float] = None, verbose:
       they absorb and get e = Abs + q_in and the temperature of computeTemperaturesVariable (0 where eps A or kappa V is 0).
       specular=True reflects at walls like a mirror (RTHX_MULTI_BOUNCE_SPECULAR); seed, device / devices and locator as for
       method=:exchange.  Several devices trace contiguous blocks of the sources; the result is bit-identical to one device's.
-    rtm.last_direct_stats: bundles, events, lost bundles, lost energy, kernel ms, devices; with all_fields the redirections too."""
+      A device block of R sources whose dense counts (8 R N bytes, 16 R N with all_fields) would pass the 48 GB budget of the :exchange
+      route is tallied in the hashed row tally instead (rthx_trace_direct_sparse): every field is bit for bit the same.
+    rtm.last_direct_stats: bundles, events, lost bundles, lost energy, kernel ms, devices, tally ("dense" or "sparse"); with all_fields
+    the redirections too."""
     import secrets
     from .tracing import _tracers_for, resolve_devices
     if rtm.spectral_mode != "grey":
@@ -119,9 +139,10 @@ def directRayTracing(rtm, rays_tot: int, nudge: Optional[float] = None, verbose:
     kw = dict(seed=secrets.randbits(63) if seed is None else int(seed), nudge=DEFAULT_NUDGE if nudge is None else float(nudge),
               locator=RTHX_LOCATOR_AUTO if locator is None else int(locator), block_threads=int(block_threads))
     if len(trs) == 1:
-        fields = dict(redirected=True) if all_fields else {}
-        out = trs[0].trace_direct(sources, rays, reemit, w, specular=specular, **fields, **kw)
-        res = dict(absorbed=out["absorbed"], lost=out["lost"], events=out["events"], kernel_ms=out["stats"]["kernel_ms"])
+        route = _route(len(sources), N, all_fields)
+        out = trs[0].trace_direct(sources, rays, reemit, w, specular=specular, **route, **kw)
+        res = dict(absorbed=out["absorbed"], lost=out["lost"], events=out["events"], kernel_ms=out["stats"]["kernel_ms"],
+                   tally="sparse" if route.get("sparse") else "dense")
         if all_fields:
             res.update(redirected=out["redirected"], redirections=int(trs[0].counts_csr(bin=1, values=True, normalised=False)[2].sum()))
     else:
@@ -157,9 +178,9 @@ def directRayTracing(rtm, rays_tot: int, nudge: Optional[float] = None, verbose:
     rtm.energy_error = float(np.sum(e - Abs))
     lost_energy = float(np.sum(w * lost[sources].astype(np.float64)))
     rtm.last_direct_stats = dict(bundles=int(rays.sum()), events=int(events), lost=int(lost.sum()), lost_energy=lost_energy,
-                                 kernel_ms=float(kernel_ms), devices=len(trs), sources=len(sources))
+                                 kernel_ms=float(kernel_ms), devices=len(trs), sources=len(sources), tally=res["tally"])
     if all_fields:
         rtm.last_direct_stats["redirections"] = res["redirections"]
     say(f"method=:direct: {int(rays.sum())} bundles from {len(sources)} sources, {int(lost.sum())} lost, {events} events, "
-        f"{kernel_ms:.2f} ms on {len(trs)} device(s)")
+        f"{kernel_ms:.2f} ms on {len(trs)} device(s), {res['tally']} tally")
     return None
