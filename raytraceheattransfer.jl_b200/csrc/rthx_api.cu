@@ -1021,31 +1021,57 @@ int check_continue(rthx_handle* h, const rthx_trace_args* a) {
   return RTHX_OK;
 }
 
-// Thread blocks per row for a launch over `rows` (emitter, band) rows: enough blocks for ~32 waves of the resident set, but keep >= 2048
-// rays (and >= N/2, the flush scan) per block
-long long auto_row_chunks(const rthx_handle* h, const LaunchPlan& pl, const rthx_trace_args* a, long long rows) {
+// Bundles a block traces at most with the direct kernel: every traversal segment of a bundle ends in at most one tally, an absorption
+// or (rthx_trace_direct_fields) a redirection, and a bundle has at most 16001 segments, so absorption and redirection tallies together
+// are <= 16001 per bundle: with 2^17 bundles a block's u32 histogram entries stay below 16001 * 2^17 < 2^32 and cannot wrap
+constexpr long long kDirectRaysPerBlock = 1ll << 17;
+
+// The source rows of a direct trace (rthx_trace_direct / _fields / _sparse, `who` in messages): the handle's listed rows, `blocks` count
+// blocks per row (2 with the redirection tally; hashed: row keys y * blocks + block), the bundles of the longest row, and on the device
+// the per-row bundles, the re-emit flags and the event counter
+struct DirectRows {
+  const char* who;
+  int blocks;
+  long long max_rays;
+  const int64_t* rays;
+  const uint8_t* reemit;
+  unsigned long long* events;
+};
+
+// The error of a launch shape the device cannot take: more than 2^31 blocks in a launch, or more than 2^31 rays in a block
+int shape_error(rthx_handle* h, const DirectRows* dr) {
+  if (dr) return fail(h, RTHX_ERR_ARG, std::string(dr->who) + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
+  return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
+}
+
+// Thread blocks per row for a launch over `rows` (emitter, band) rows of at most `rays` rays: enough blocks for ~32 waves of the resident
+// set, but keep >= 2048 rays (and >= N/2, the flush scan) per block
+long long auto_row_chunks(const rthx_handle* h, const LaunchPlan& pl, long long rays, long long rows) {
   const int per_sm = std::max(1, trace_kernel_max_blocks_per_sm(pl.kernel, pl.block_threads, pl.smem_bytes));
   const long long target = (long long)h->prop.multiProcessorCount * per_sm * 32;
   long long chunks = rows > 0 ? (target + rows - 1) / rows : 1;
   const long long min_rays = std::max<long long>(2048, h->N / 2);
-  const long long max_chunks = std::max<long long>(1, a->rays_per_emitter / min_rays);
+  const long long max_chunks = std::max<long long>(1, rays / min_rays);
   return std::max<long long>(1, std::min(chunks, max_chunks));
 }
 
-// hash_slots > 0: the hashed row tally (no histogram; the table takes hash_table_bytes(hash_slots))
-LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, OwnedRows own, int hash_slots = 0) {
-  LaunchPlan pl{};
+// Launch plan of a trace of the rows `own`.  dr != nullptr: a direct trace of the listed source rows (the lock-step body with
+// re-emission, a histogram row per count block, chunks for the longest row).  hash_slots > 0: the hashed row tally (no histogram; the
+// table takes hash_table_bytes(hash_slots)).  A shape the device cannot take is RTHX_ERR_ARG.
+int make_plan(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, LaunchPlan& pl, const DirectRows* dr = nullptr, int hash_slots = 0) {
+  pl = LaunchPlan{};
   pl.n_owned = own.listed ? (int)h->rows.size() : (h->N - own.rank + own.world - 1) / own.world;
   if (pl.n_owned < 0) pl.n_owned = 0;
   pl.block_threads = a->block_threads ? a->block_threads : 256;
-  const bool analytic = a->locator != RTHX_LOCATOR_GENERIC;
+  const bool analytic = a->locator != RTHX_LOCATOR_GENERIC, fast = h->fast_ok && analytic;
   const bool multi = a->mode != RTHX_FIRST_INTERACTION;
   const size_t coarse_bytes = h->coarse_fits_smem ? sizeof(CoarseDev) * (size_t)h->n_coarse : 0;
-  const size_t hist_bytes = sizeof(uint32_t) * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;   // emitter block + log table
+  const size_t hist_bytes = sizeof(uint32_t) * (size_t)(dr ? dr->blocks : 1) * (size_t)h->N;
+  const size_t em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;   // emitter block + log table
   bool hist = hash_slots == 0 && coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
   if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) hist = false; }   // test knob: the N > ~57k path
   pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0) + (hash_slots > 0 ? hash_table_bytes(hash_slots) : 0);
-  pl.kernel = TraceKernelSel::lockstep(hist, h->fast_ok && analytic, multi);
+  pl.kernel = TraceKernelSel::lockstep(hist, fast, multi);
   // The queue kernel needs the histogram and 256 threads.  It takes multi-face meshes with analytic locators, and MULTI_BOUNCE on
   // any of them (lanes refill when their ray is absorbed).  Its generic variant takes multi-face meshes through the GENERIC locator
   // (faces without a verified lattice, RTHX_LOCATOR_GENERIC) as long as the coarse descriptors fit in shared memory: a ray crosses
@@ -1053,8 +1079,10 @@ LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, OwnedRows o
   // kernel, except for MULTI_BOUNCE at 256 threads.
   const bool queue_fast = h->queue_ok && analytic && (h->n_coarse > 1 || h->queue_general || multi);
   const bool queue_gen = !multi && (!analytic || !h->queue_ok) && h->coarse_fits_smem && h->n_coarse > 1;
-  if (hash_slots > 0) {
-    pl.kernel = TraceKernelSel::hash(h->fast_ok && analytic);
+  if (dr) {
+    pl.kernel = hash_slots > 0 ? TraceKernelSel::direct_hash(fast) : TraceKernelSel::direct(hist, fast);
+  } else if (hash_slots > 0) {
+    pl.kernel = TraceKernelSel::hash(fast);
   } else if (h->single_quad && analytic && hist && !(multi && pl.block_threads == 256)) {
     pl.kernel = TraceKernelSel::sq(multi);
   } else if (hist && pl.block_threads == 256 && (queue_fast || queue_gen)) {
@@ -1074,39 +1102,38 @@ LaunchPlan make_plan(const rthx_handle* h, const rthx_trace_args* a, OwnedRows o
       pl.smem_bytes = base + depth * per_depth;
     }
   }
-  const long long rows = (long long)pl.n_owned * a->n_bins;
-  long long chunks = a->row_chunks;
-  if (chunks <= 0) chunks = auto_row_chunks(h, pl, a, rows);
+  const long long rows = (long long)pl.n_owned * a->n_bins, rays = dr ? dr->max_rays : a->rays_per_emitter;
+  long long chunks = a->row_chunks > 0 ? a->row_chunks : auto_row_chunks(h, pl, rays, rows);
   // A block's rays are counted in 32 bits (u32 row histogram, u32 loop counter advancing by blockDim.x): at most 2^31 rays per
   // block.  Auto-chosen chunk counts are raised to satisfy that; a plan that then exceeds the 1-D grid limit — or a caller-supplied
-  // row_chunks that violates either bound — is rejected (n_blocks = -1 -> RTHX_ERR_ARG), never silently wrapped.
-  if (a->row_chunks <= 0)
-    while ((a->rays_per_emitter + chunks - 1) / chunks > 0x7FFFFFFFll) chunks *= 2;
+  // row_chunks that violates either bound — is rejected, never silently wrapped.  A direct block traces at most kDirectRaysPerBlock
+  // bundles, whatever the caller asked for.
+  if (dr)
+    chunks = std::max(chunks, (rays + kDirectRaysPerBlock - 1) / kDirectRaysPerBlock);
+  else if (a->row_chunks <= 0)
+    while ((rays + chunks - 1) / chunks > 0x7FFFFFFFll) chunks *= 2;
   pl.row_chunks = (int)std::min<long long>(chunks, 0x7FFFFFFFll);
-  if ((a->rays_per_emitter + chunks - 1) / chunks > 0x7FFFFFFFll || rows * chunks > 0x7FFFFFFFll) { pl.n_blocks = -1; return pl; }
+  if ((rays + chunks - 1) / chunks > 0x7FFFFFFFll || rows * chunks > 0x7FFFFFFFll) return shape_error(h, dr);
   pl.n_blocks = (int)(rows * chunks);
-  return pl;
+  return RTHX_OK;
 }
 
-void fill_params(const rthx_handle* h, const rthx_trace_args* a, const LaunchPlan& pl, int rank, int world, bool compact,
-                 unsigned long long* counts, unsigned long long* lost, TraceParams& P) {
+// Parameters of a trace with plan `pl`; launch_rows sets the row mapping and the chunks of each launch.  flush_system: the count matrix
+// or the lost counters live on another GPU and take system-scope reductions.  dr: a direct trace's rows.
+void fill_params(const rthx_handle* h, const rthx_trace_args* a, const LaunchPlan& pl, bool compact, unsigned long long* counts,
+                 unsigned long long* lost, bool flush_system, const DirectRows* dr, TraceParams& P) {
   P = h->base;
   P.bins = h->bins_dev;
   P.counts = counts; P.lost = lost;
   P.n_bins = a->n_bins;
-  P.emitter_rank = rank; P.emitter_world = world; P.n_owned = pl.n_owned; P.y_offset = 0;
+  P.n_owned = pl.n_owned;
   P.compact_rows = compact ? 1 : 0;
-  P.row_chunks = pl.row_chunks;
   P.queue_refill = 24;
   P.coarse_in_smem = h->coarse_fits_smem ? 1 : 0;
   P.force_generic = a->locator == RTHX_LOCATOR_GENERIC ? 1 : 0;
   P.specular = a->mode == RTHX_MULTI_BOUNCE_SPECULAR ? 1 : 0;
-  // a count matrix that lives on another GPU (fused peer flush) is updated with system-scope reductions
-  P.flush_system = 0;
-  cudaPointerAttributes pa;
-  if (counts && cudaPointerGetAttributes(&pa, counts) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device != h->device) P.flush_system = 1;
-  else cudaGetLastError();
-  if (const char* ev = std::getenv("RTHX_FLUSH_SYSTEM")) P.flush_system = std::atoi(ev) ? 1 : 0;
+  P.flush_system = flush_system ? 1 : 0;
+  if (dr) { P.dr_rays = dr->rays; P.dr_reemit = dr->reemit; P.dr_events = dr->events; P.dr_redirect = dr->blocks - 1; }
   P.rec_bin = a->rec_bin;
   P.rays_per_emitter = a->rays_per_emitter;
   P.ray_id_offset = a->ray_id_offset;
@@ -1161,28 +1188,61 @@ void fill_stats(rthx_stats* st, const rthx_trace_args* a, const LaunchPlan& pl, 
   st->kernel_ms = kernel_ms; st->total_ms = total_ms;
 }
 
+// Calls f(run, r0, r1) for every row run of the rows `own` that meets the traced rows [y0, y1), with [r0, r1) the rows they share.  Row y
+// of run {first row f, rows, element e of row f, stride s} is element e + (y - f) s.  A shard of n_owned rows is the one run
+// {0, n_owned, rank, world}; a listed trace has the arithmetic runs of the handle's list (list_runs).
+template <class F>
+int for_runs(const rthx_handle* h, OwnedRows own, int n_owned, int y0, int y1, F&& f) {
+  const int4 shard = make_int4(0, n_owned, own.rank, own.world);
+  const int4* first = own.listed ? h->row_runs.data() : &shard;
+  const int4* last = own.listed ? first + h->row_runs.size() : &shard + 1;
+  for (const int4* run = first; run != last; ++run) {
+    const int r0 = std::max(y0, run->x), r1 = std::min(y1, run->x + run->y);
+    if (r1 > r0) { const int rc = f(*run, r0, r1); if (rc) return rc; }
+  }
+  return RTHX_OK;
+}
+
+// Launch the trace kernel of plan `pl` with the parameters P over the traced rows [y0, y1) of the rows `own`: one launch per row run
+// that meets them, each as a shard of its own (emitter_rank + y * emitter_world is the run's element of row y).  The launches of one
+// stream run one after another, so with automatic chunking a listed run is cut into enough blocks to fill the device on its own (the
+// plan's row_chunks fills it with all rows at once); a shard keeps the plan's chunks, which the pipelined batches share.  Counts do
+// not depend on the launch shape.
+int launch_rows(rthx_handle* h, const rthx_trace_args* a, const LaunchPlan& pl, OwnedRows own, const DirectRows* dr, TraceParams& P, int y0, int y1,
+                cudaStream_t stream, int* n_launches) {
+  const long long rays = dr ? dr->max_rays : a->rays_per_emitter;
+  return for_runs(h, own, pl.n_owned, y0, y1, [&](const int4& run, int r0, int r1) -> int {
+    const long long rows = (long long)(r1 - r0) * a->n_bins;
+    P.row_chunks = own.listed && a->row_chunks <= 0 ? (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, rays, rows)) : pl.row_chunks;
+    if (rows * P.row_chunks > 0x7FFFFFFFll) return shape_error(h, dr);
+    P.emitter_rank = run.z - run.x * run.w; P.emitter_world = run.w;
+    P.y_offset = r0;
+    CU(h, launch_trace_exchange(P, pl.kernel, (int)(rows * P.row_chunks), pl.block_threads, pl.smem_bytes, stream));
+    *n_launches += 1;
+    return RTHX_OK;
+  });
+}
+
 // Enqueue (zero +) kernel for one handle on `stream`; counts layout compact (owned rows) or full.
 // [y0, y1) restricts the launch to a range of owned-emitter ordinals (y1 < 0: all rows).
 int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, bool compact, unsigned long long* counts,
                   unsigned long long* lost, int zero_first, bool with_rec, int n_rec_slots, cudaStream_t stream,
                   LaunchPlan* plan_out, int* n_launches, int y0 = 0, int y1 = -1, bool upload_bins = true) {
   const int rank = own.rank, world = own.world;
-  LaunchPlan pl = make_plan(h, a, own);
-  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
-  if (!pl.kernel.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }     // the generic locator reads the reference-faithful tables
+  LaunchPlan pl;
+  int rc = make_plan(h, a, own, pl);
+  if (rc) return rc;
+  if (!pl.kernel.fast && (rc = ensure_generic(h))) return rc;     // the generic locator reads the reference-faithful tables
   if (upload_bins) CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)a->n_bins, cudaMemcpyHostToDevice, stream));
   // A matrix in peer memory (fused multi-GPU flush) is never the target of reductions: the chunks of a row add up in a local
   // compact staging matrix and the finished row is handed over with plain stores (flush_row_hist) — so the peer rows need no
   // clearing either.  Without the shared-memory histogram (N > ~57 k) the old path stays: system-scope atomics into zeroed rows.
   // (a CUDA-IPC mapping reports the mapping device, not the owner: such callers say so with RTHX_DEST_PEER)
-  bool peer = (zero_first & RTHX_DEST_PEER) != 0;
+  cudaPointerAttributes pa;
+  const bool remote = counts && cudaPointerGetAttributes(&pa, counts) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device != h->device;
+  if (!remote) cudaGetLastError();
+  const bool peer = remote || (zero_first & RTHX_DEST_PEER) != 0;
   zero_first &= ~RTHX_DEST_PEER;
-  {
-    cudaPointerAttributes pa;
-    if (counts && cudaPointerGetAttributes(&pa, counts) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device != h->device) peer = true;
-    else cudaGetLastError();
-    if (const char* ev = std::getenv("RTHX_FLUSH_SYSTEM")) peer = std::atoi(ev) != 0;     // test knob: exercise the hand-over on one GPU
-  }
   const bool staged = peer && pl.kernel.hist && !compact;
   unsigned long long* stage_counts = nullptr;
   unsigned int* row_done = nullptr;
@@ -1218,34 +1278,13 @@ int enqueue_trace(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, bool 
     }
   }
   TraceParams P;
-  fill_params(h, a, pl, rank, world, compact, counts, lost, P);
+  fill_params(h, a, pl, compact, counts, lost, /*flush_system=*/remote || staged, nullptr, P);   // staged: the lost counters live next to the peer matrix
   if (staged) {
     P.peer_counts = counts; P.row_done = row_done;
     P.counts = stage_counts; P.compact_rows = 1;                         // nullptr with row_chunks == 1: rows are written out directly
-    P.flush_system = 1;                                                  // the lost counters live next to the peer matrix
   }
   if (with_rec && n_rec_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
-  if (y1 < 0) y1 = pl.n_owned;
-  if (!own.listed) {
-    P.y_offset = y0;
-    const long long nb = (long long)(y1 - y0) * a->n_bins * pl.row_chunks;
-    CU(h, launch_trace_exchange(P, pl.kernel, (int)nb, pl.block_threads, pl.smem_bytes, stream));
-    if (nb > 0) *n_launches += 1;
-  } else {
-    // one launch per run of the emitter list that meets [y0, y1): rows y of run {r0, n, e0, s} are elements e0 + (y - r0) s.  The launches
-    // of one stream run one after another, so with automatic chunking each is cut into enough blocks to fill the device on its own (the
-    // plan's row_chunks fills it with all R rows at once); counts do not depend on the launch shape.
-    for (const int4& run : h->row_runs) {
-      const int r0 = std::max(y0, run.x), r1 = std::min(y1, run.x + run.y);
-      if (r1 <= r0) continue;
-      const long long rows = (long long)(r1 - r0) * a->n_bins;
-      P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, a, rows));
-      P.emitter_world = run.w; P.emitter_rank = run.z - run.x * run.w;
-      P.y_offset = r0;
-      CU(h, launch_trace_exchange(P, pl.kernel, (int)(rows * P.row_chunks), pl.block_threads, pl.smem_bytes, stream));
-      *n_launches += 1;
-    }
-  }
+  if ((rc = launch_rows(h, a, pl, own, nullptr, P, y0, y1 < 0 ? pl.n_owned : y1, stream, n_launches))) return rc;
   *plan_out = pl;
   return RTHX_OK;
 }
@@ -1270,8 +1309,9 @@ void batch_rows_of(int n_owned, int n_batches, int b, int& y0, int& y1) {
 int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, bool with_rec, int n_slots,
                     LaunchPlan* plan_out, int* n_launches, int* n_batches_out) {
   const int N = h->N;
-  LaunchPlan pl = make_plan(h, a, own);
-  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
+  LaunchPlan pl;
+  int rc = make_plan(h, a, own, pl);
+  if (rc) return rc;
   const int n_owned = pl.n_owned;
   drop_resident(h);
   CU(h, ensure(&h->counts_dev, &h->counts_cap, (size_t)a->n_bins * (size_t)n_owned * N));
@@ -1294,8 +1334,8 @@ int pipeline_launch(rthx_handle* h, const rthx_trace_args* a, OwnedRows own, boo
     batch_rows_of(n_owned, n_batches, b, y0, y1);
     cudaStream_t cs = (b & 1) ? h->stream2 : h->stream;
     LaunchPlan tmp{};
-    int rc = enqueue_trace(h, a, own, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, with_rec, n_slots, cs, &tmp, n_launches, y0, y1,
-                           /*upload_bins=*/false);
+    rc = enqueue_trace(h, a, own, /*compact=*/true, h->counts_dev, h->lost_dev, RTHX_ZERO_NONE, with_rec, n_slots, cs, &tmp, n_launches, y0, y1,
+                       /*upload_bins=*/false);
     if (rc) return rc;
     CU(h, cudaEventRecord(h->bev[b], cs));
   }
@@ -1442,16 +1482,13 @@ struct SparseRun : TraceRun {
   unsigned long long events = 0;       // direct: traversal segments of the launches that were kept
 };
 
-// A direct trace on the hashed tally (rthx_trace_direct_sparse), as sparse_trace_rows traces it: the listed source rows of the handle,
-// `blocks` count blocks per row (row keys y * blocks + block), the per-row bundles and re-emit flags on the device, the event counter
-// (cleared before every launch of a group, and read after it)
-struct DirectRows {
-  int blocks;
-  long long max_rays;
-  const int64_t* rays;
-  const uint8_t* reemit;
-  unsigned long long* events;
-};
+// rthx_sparse_stats of a hashed-tally pass
+void fill_sparse_stats(rthx_sparse_stats* sst, const SparseRun& R) {
+  if (!sst) return;
+  std::memset(sst, 0, sizeof(*sst));
+  sst->pairs = R.pairs; sst->nnz = R.total; sst->flushes = R.flushes; sst->pair_capacity = R.cap;
+  sst->row_groups = R.groups; sst->hash_slots = 1 << R.log2s; sst->reduce_ms = R.reduce_ms;
+}
 
 // End of a trace whose kernels ran from ev[1] to ev[2]: the lost counters to the host behind everything enqueued on `stream` so far,
 // ev[3] as the end of the call's device work, and the kernel time
@@ -1519,6 +1556,17 @@ std::vector<int4> list_runs(const std::vector<int32_t>& rows) {
   return runs;
 }
 
+// The handle's emitter list becomes the n ascending elements `list`: on the host, cut into row runs, and in rows_dev.  The rows of a
+// resident listed trace are that list, so the resident counts are replaced from here on.
+int set_rows(rthx_handle* h, const int32_t* list, int32_t n) {
+  drop_resident(h);
+  h->rows.assign(list, list + n);
+  h->row_runs = list_runs(h->rows);
+  CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)n));
+  CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, h->stream));
+  return RTHX_OK;
+}
+
 // Checks of rthx_trace_exchange_rows that must pass before anything resident changes
 // (dense == false: the counts are not held densely, so their size is not checked against free memory)
 int check_rows(rthx_handle* h, const rthx_trace_args* a, const int32_t* emitters, int32_t n, const std::string& who = "trace_rows", const char* list = "emitter",
@@ -1565,21 +1613,11 @@ extern "C" int rthx_trace_exchange_rows(rthx_handle* h, const rthx_trace_args* a
   if (rc) return rc;
   CU(h, cudaSetDevice(h->device));
   rc = check_rows(h, a, emitters, n_emitters);
-  if (rc) return rc;
-  drop_resident(h);                  // the resident counts are replaced from here on
-  h->rows.assign(emitters, emitters + n_emitters);
-  h->row_runs = list_runs(h->rows);
-  CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)n_emitters));
-  CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)n_emitters, cudaMemcpyHostToDevice, h->stream));
+  if (rc || (rc = set_rows(h, emitters, n_emitters))) return rc;
   return trace_host(h, a, OwnedRows{0, 1, true}, counts_out, lost_out, rec, st);
 }
 
 namespace {
-
-// Bundles a block traces at most with the direct kernel: every traversal segment of a bundle ends in at most one tally, an absorption
-// or (rthx_trace_direct_fields) a redirection, and a bundle has at most 16001 segments, so absorption and redirection tallies together
-// are <= 16001 per bundle: with 2^17 bundles a block's u32 histogram entries stay below 16001 * 2^17 < 2^32 and cannot wrap
-constexpr long long kDirectRaysPerBlock = 1ll << 17;
 
 // Checks of rthx_trace_direct / _fields / _sparse (`who`) that must pass before anything resident changes; `blocks` count blocks per
 // source row (2 with the redirection tally), laid out and (dense) checked against free memory as the bins of a rows trace
@@ -1604,29 +1642,6 @@ int check_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* source
   return RTHX_OK;
 }
 
-// Launch plan of a direct trace of the listed source rows: the lock-step body with re-emission, histogram in shared memory when the
-// row fits (both halves with the redirection tally), chunks for the longest row.  hash_slots > 0: the hashed row tally instead
-// (trace_direct_hash_kernel, no histogram; the table takes hash_table_bytes(hash_slots))
-LaunchPlan make_direct_plan(const rthx_handle* h, const rthx_trace_args* a, long long max_rays, int blocks, int hash_slots = 0) {
-  LaunchPlan pl{};
-  pl.n_owned = (int)h->rows.size();
-  pl.block_threads = a->block_threads ? a->block_threads : 256;
-  const size_t coarse_bytes = h->coarse_fits_smem ? sizeof(CoarseDev) * (size_t)h->n_coarse : 0;
-  const size_t hist_bytes = sizeof(uint32_t) * (size_t)blocks * (size_t)h->N, em_bytes = sizeof(double) * 16 + 16 * (size_t)LOGTAB_N;
-  bool hist = hash_slots == 0 && coarse_bytes + em_bytes + hist_bytes <= h->prop.sharedMemPerBlockOptin;
-  if (const char* ev = std::getenv("RTHX_FORCE_GLOBAL_TALLY")) { if (std::atoi(ev)) hist = false; }
-  pl.smem_bytes = coarse_bytes + em_bytes + (hist ? hist_bytes : 0) + (hash_slots > 0 ? hash_table_bytes(hash_slots) : 0);
-  const bool fast = h->fast_ok && a->locator != RTHX_LOCATOR_GENERIC;
-  pl.kernel = hash_slots > 0 ? TraceKernelSel::direct_hash(fast) : TraceKernelSel::direct(hist, fast);
-  rthx_trace_args longest = *a;
-  longest.rays_per_emitter = max_rays;
-  long long chunks = a->row_chunks > 0 ? a->row_chunks : auto_row_chunks(h, pl, &longest, pl.n_owned);
-  chunks = std::max(chunks, (max_rays + kDirectRaysPerBlock - 1) / kDirectRaysPerBlock);
-  pl.row_chunks = (int)std::min<long long>(chunks, 0x7FFFFFFFll);
-  pl.n_blocks = (long long)pl.n_owned * chunks > 0x7FFFFFFFll ? -1 : (int)(pl.n_owned * chunks);
-  return pl;
-}
-
 int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec, unsigned long long** out_keys, size_t* keys_cap,
                       unsigned long long** out_vals, size_t* vals_cap, SparseRun& R, const DirectRows* direct = nullptr);
 int direct_column_sums(rthx_handle* h, int block, int R, const double* w, double* out);
@@ -1645,113 +1660,72 @@ int trace_direct(rthx_handle* h, const rthx_trace_args* a, const int32_t* source
   CU(h, cudaSetDevice(h->device));
   if (fields && !redirected_out) return fail(h, RTHX_ERR_ARG, who + ": redirected_out must not be NULL");
   rc = check_direct(h, a, sources, rays, n_sources, reemit, bundle_energy, absorbed_out, who, blocks, !hashed);
-  if (rc) return rc;
+  if (rc || (rc = set_rows(h, sources, n_sources))) return rc;     // the resident counts are replaced from here on
   const int N = h->N, R = n_sources;
   const size_t RN = (size_t)R * N;
-  const long long max_rays = *std::max_element(rays, rays + R);
-  drop_resident(h);                  // the resident counts are replaced from here on
-  h->rows.assign(sources, sources + R);
-  h->row_runs = list_runs(h->rows);
-  const LaunchPlan pl = make_direct_plan(h, a, max_rays, blocks);
-  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, who + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
-  if (!pl.kernel.fast) { rc = ensure_generic(h); if (rc) return rc; }
+  const OwnedRows listed{0, 1, true};
   // dr_buf: rays [R] i64 | bundle energy [R] f64 | Abs [N] f64 | redirected power [N] f64 | events u64 | re-emit flags [N] u8
   const size_t off_w = 8 * (size_t)R, off_abs = off_w + 8 * (size_t)R, off_red = off_abs + 8 * (size_t)N, off_ev = off_red + 8 * (size_t)N,
                off_re = off_ev + 8;
   CU(h, ensure(&h->dr_buf, &h->dr_cap, off_re + (size_t)N));
   char* buf = h->dr_buf;
-  CU(h, ensure(&h->rows_dev, &h->rows_cap, (size_t)R));
-  if (!hashed) CU(h, ensure(&h->counts_dev, &h->counts_cap, blocks * RN));
-  cudaStream_t s = h->stream;
-  int n_launches = 0;
-  CU(h, cudaEventRecord(h->ev[0], s));
-  CU(h, cudaMemcpyAsync(h->rows_dev, h->rows.data(), sizeof(int32_t) * (size_t)R, cudaMemcpyHostToDevice, s));
-  CU(h, cudaMemcpyAsync(buf, rays, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
-  CU(h, cudaMemcpyAsync(buf + off_w, bundle_energy, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
-  CU(h, cudaMemcpyAsync(buf + off_re, reemit, (size_t)N, cudaMemcpyHostToDevice, s));
+  const DirectRows dr{who.c_str(), blocks, *std::max_element(rays, rays + R), reinterpret_cast<const int64_t*>(buf),
+                      reinterpret_cast<const uint8_t*>(buf + off_re), reinterpret_cast<unsigned long long*>(buf + off_ev)};
   const double* w_dev = reinterpret_cast<const double*>(buf + off_w);
   double* abs_dev = reinterpret_cast<double*>(buf + off_abs);
   double* red_dev = reinterpret_cast<double*>(buf + off_red);
-  unsigned long long* events_dev = reinterpret_cast<unsigned long long*>(buf + off_ev);
-  SparseRun S;
-  float k_ms = 0;
-  unsigned long long events = 0;
+  cudaStream_t s = h->stream;
+  CU(h, cudaEventRecord(h->ev[0], s));
+  CU(h, cudaMemcpyAsync(buf, rays, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemcpyAsync(buf + off_w, bundle_energy, 8 * (size_t)R, cudaMemcpyHostToDevice, s));
+  CU(h, cudaMemcpyAsync(buf + off_re, reemit, (size_t)N, cudaMemcpyHostToDevice, s));
+  SparseRun S;                         // dense: the plan, launches, kernel time and events of the one pass
   if (hashed) {
-    // row groups, overflow splits, sort and reduce as rthx_trace_exchange_sparse, one launch per arithmetic run of the source list
-    const DirectRows dr{blocks, max_rays, reinterpret_cast<const int64_t*>(buf), reinterpret_cast<const uint8_t*>(buf + off_re), events_dev};
+    // row groups, overflow splits, sort and reduce as rthx_trace_exchange_sparse
     rc = sparse_trace_rows(h, a, nullptr, &h->sk_keys, &h->sk_keys_cap, &h->sk_vals, &h->sk_vals_cap, S, &dr);
     if (rc) return rc;
     CU(h, ensure(&h->sk_rowptr, &h->sk_rowptr_cap, (size_t)S.n_rows + 1));
     CU(h, tally_row_ptr(h->sk_keys, S.total, S.n_rows, h->sk_rowptr, s));
-    // the set is resident in the record's key layout from here on: the sums read it through the read-out paths
-    set_resident(h, a, RESIDENT_DIRECT_SPARSE, OwnedRows{0, 1, true}, R);
-    if (fields) h->res.bins.push_back(a->bins[0]);
-    h->res.nnz = S.total;
-    if ((rc = direct_column_sums(h, 0, R, w_dev, abs_dev)) || (fields && (rc = direct_column_sums(h, 1, R, w_dev, red_dev)))) {
-      drop_resident(h);
-      return rc;
-    }
-    n_launches = S.n_launches + (fields ? 2 : 1);
-    k_ms = (float)S.kernel_ms;
-    events = S.events;
   } else {
+    if ((rc = make_plan(h, a, listed, S.pl, &dr))) return rc;
+    if (!S.pl.kernel.fast && (rc = ensure_generic(h))) return rc;
+    CU(h, ensure(&h->counts_dev, &h->counts_cap, blocks * RN));
     CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CU(h, cudaMemsetAsync(h->counts_dev, 0, sizeof(unsigned long long) * blocks * RN, s));
     CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)N, s));
-    CU(h, cudaMemsetAsync(events_dev, 0, 8, s));
-    n_launches += 3;
+    CU(h, cudaMemsetAsync(dr.events, 0, 8, s));
+    S.n_launches += 3;
     TraceParams P;
-    fill_params(h, a, pl, 0, 1, /*compact=*/true, h->counts_dev, h->lost_dev, P);
-    P.dr_rays = reinterpret_cast<const int64_t*>(buf);
-    P.dr_reemit = reinterpret_cast<const uint8_t*>(buf + off_re);
-    P.dr_events = events_dev;
-    P.dr_redirect = fields ? 1 : 0;
+    fill_params(h, a, S.pl, /*compact=*/true, h->counts_dev, h->lost_dev, false, &dr, P);
     CU(h, cudaEventRecord(h->ev[1], s));
-    for (const int4& run : h->row_runs) {      // one launch per arithmetic run of the source list, as rthx_trace_exchange_rows
-      const int4 r = run;
-      rthx_trace_args longest = *a;
-      longest.rays_per_emitter = max_rays;
-      P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r.y));
-      P.emitter_world = r.w; P.emitter_rank = r.z - r.x * r.w;
-      P.y_offset = r.x;
-      if ((long long)r.y * P.row_chunks > 0x7FFFFFFFll) return fail(h, RTHX_ERR_ARG, who + ": too many bundles for one launch (a launch has at most 2^31 blocks)");
-      CU(h, launch_trace_exchange(P, pl.kernel, r.y * P.row_chunks, pl.block_threads, pl.smem_bytes, s));
-      ++n_launches;
-    }
+    if ((rc = launch_rows(h, a, S.pl, listed, &dr, P, 0, S.pl.n_owned, s, &S.n_launches))) return rc;
     CU(h, cudaEventRecord(h->ev[2], s));
-    CU(h, launch_direct_absorbed(h->counts_dev, R, N, w_dev, abs_dev, s));
-    ++n_launches;
-    if (fields) {                              // the same fixed-order sum over the second block
-      CU(h, launch_direct_absorbed(h->counts_dev + RN, R, N, w_dev, red_dev, s));
-      ++n_launches;
-    }
-    CU(h, cudaMemcpyAsync(&events, events_dev, 8, cudaMemcpyDeviceToHost, s));
   }
-  std::vector<uint64_t> lost(N);
+  // the counts are resident from here on, in the record's layout: the sums read them through it
+  set_resident(h, a, hashed ? RESIDENT_DIRECT_SPARSE : RESIDENT_DIRECT, listed, R);
+  if (fields) h->res.bins.push_back(a->bins[0]);   // the redirection block reads out as bin 1
+  h->res.nnz = S.total;
+  for (int b = 0; b < blocks; ++b, ++S.n_launches)
+    if ((rc = direct_column_sums(h, b, R, w_dev, b ? red_dev : abs_dev))) { drop_resident(h); return rc; }
+  S.lost.resize(N);
   CU(h, cudaMemcpyAsync(absorbed_out, abs_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
   if (fields) CU(h, cudaMemcpyAsync(redirected_out, red_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
-  CU(h, cudaMemcpyAsync(lost.data(), h->lost_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  CU(h, cudaMemcpyAsync(S.lost.data(), h->lost_dev, 8 * (size_t)N, cudaMemcpyDeviceToHost, s));
+  if (!hashed) CU(h, cudaMemcpyAsync(&S.events, dr.events, 8, cudaMemcpyDeviceToHost, s));   // hashed: summed over the groups that were kept
   CU(h, cudaEventRecord(h->ev[3], s));
   CU(h, cudaStreamSynchronize(s));
-  if (!hashed) {
-    set_resident(h, a, RESIDENT_DIRECT, OwnedRows{0, 1, true}, R);
-    if (fields) h->res.bins.push_back(a->bins[0]);   // the redirection block reads out as bin 1
+  if (!hashed) {                       // hashed: the kernel times of the groups, summed
+    float ms = 0;
+    CU(h, cudaEventElapsedTime(&ms, h->ev[1], h->ev[2]));
+    S.kernel_ms = ms;
   }
-  if (lost_out) std::memcpy(lost_out, lost.data(), 8 * (size_t)N);
-  if (events_out) *events_out = (int64_t)events;
-  if (st) {
-    float t_ms = 0;
-    if (!hashed) CU(h, cudaEventElapsedTime(&k_ms, h->ev[1], h->ev[2]));
-    CU(h, cudaEventElapsedTime(&t_ms, h->ev[0], h->ev[3]));
-    fill_stats(st, a, hashed ? S.pl : pl, lost, n_launches, k_ms, t_ms);
+  if (events_out) *events_out = (int64_t)S.events;
+  if ((rc = finish_trace(h, a, S, lost_out, nullptr, st))) return rc;
+  if (st) {                            // the sources trace different numbers of bundles
     st->rays_traced = 0;
     for (int32_t i = 0; i < R; ++i) st->rays_traced += rays[i];
   }
-  if (sst) {
-    std::memset(sst, 0, sizeof(*sst));
-    sst->pairs = S.pairs; sst->nnz = S.total; sst->flushes = S.flushes; sst->pair_capacity = S.cap;
-    sst->row_groups = S.groups; sst->hash_slots = 1 << S.log2s; sst->reduce_ms = S.reduce_ms;
-  }
+  fill_sparse_stats(sst, S);
   return RTHX_OK;
 }
 
@@ -1840,8 +1814,9 @@ struct DevBuf {
 // `direct->blocks` row keys per source row; ev[0] is then the caller's.
 int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* rec, unsigned long long** out_keys, size_t* keys_cap,
                       unsigned long long** out_vals, size_t* vals_cap, SparseRun& R, const DirectRows* direct) {
-  const int N = h->N, nb = a->n_bins, rank = a->emitter_rank, world = a->emitter_world;
+  const int N = h->N, nb = a->n_bins;
   const int nk = direct ? direct->blocks : nb;               // row keys per traced row
+  const OwnedRows own = direct ? OwnedRows{0, 1, true} : shard_of(a);
   const int bt = a->block_threads ? a->block_threads : 256;
   int log2s = 12;                                            // 4096 slots: 32 KB of table
   int min_log2s = 1;
@@ -1854,8 +1829,9 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     if (v > 0) { log2s = 0; while ((1ll << log2s) < v) ++log2s; forced = true; }
   }
   log2s = std::max(log2s, min_log2s);
-  LaunchPlan pl = direct ? make_direct_plan(h, a, direct->max_rays, direct->blocks, 1 << log2s) : make_plan(h, a, shard_of(a), 1 << log2s);
-  if (pl.n_blocks < 0) return fail(h, RTHX_ERR_ARG, "trace: rays_per_emitter / row_chunks out of range (a block traces at most 2^31 rays, a launch at most 2^31 blocks)");
+  LaunchPlan pl;
+  int rc = make_plan(h, a, own, pl, direct, 1 << log2s);
+  if (rc) return rc;
   if (!forced) {                                             // a block with few rays needs no large table: clearing and scanning it is the cost
     // direct: a re-emitted bundle tallies many columns, so only the row's count blocks bound the distinct keys
     const long long distinct = direct ? (long long)direct->blocks * N : std::min<long long>((a->rays_per_emitter + pl.row_chunks - 1) / pl.row_chunks, N);
@@ -1864,7 +1840,7 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     pl.smem_bytes = pl.smem_bytes - hash_table_bytes(1 << old) + hash_table_bytes(1 << log2s);
   }
   if (pl.smem_bytes > h->prop.sharedMemPerBlockOptin) return fail(h, RTHX_ERR_ARG, "trace_sparse: hash table does not fit in shared memory");
-  if (!pl.kernel.fast) { const int rcg = ensure_generic(h); if (rcg) return rcg; }
+  if (!pl.kernel.fast && (rc = ensure_generic(h))) return rc;
   // pair buffer: at most half the free device memory (24 bytes a pair with the sort's alternate buffers), the other half is left for the
   // resident totals; an exchange trace flushes at most one pair per tallied ray, a direct bundle has no such bound
   long long cap = 0x7FFFFFFFll;
@@ -1893,29 +1869,15 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
   while ((1ll << (end_bit - 32)) < n_rows) ++end_bit;
 
   if (!direct) CU(h, cudaEventRecord(h->ev[0], h->stream));
-  int rc = prepare_recorder(h, a, rec, &R.n_slots, h->stream);
+  rc = prepare_recorder(h, a, rec, &R.n_slots, h->stream);
   if (rc) return rc;
   CU(h, cudaMemcpyAsync(h->bins_dev, a->bins, sizeof(int32_t) * (size_t)nb, cudaMemcpyHostToDevice, h->stream));
   CU(h, cudaMemsetAsync(h->lost_dev, 0, sizeof(unsigned long long) * (size_t)nb * N, h->stream));
   R.n_launches += 1;
   TraceParams P;
-  fill_params(h, a, pl, rank, world, true, nullptr, h->lost_dev, P);
+  fill_params(h, a, pl, true, nullptr, h->lost_dev, false, direct, P);
   if (R.n_slots > 0) { P.rec_slot = h->rec_slot_dev; P.rec_pts = h->rec_pts_dev; P.rec_valid = h->rec_valid_dev; }
   P.sk_keys = keys; P.sk_cnt = cnt; P.sk_ctl = h->sk_ctl; P.sk_cap = (unsigned long long)cap; P.sk_slots_log2 = log2s;
-  if (direct) {
-    P.dr_rays = direct->rays; P.dr_reemit = direct->reemit; P.dr_events = direct->events; P.dr_redirect = direct->blocks - 1;
-  }
-  // The row runs that meet rows [y0, y1): a shard is one run {0, n_owned, rank, world}, a source list cut into arithmetic runs
-  // (rthx_trace_exchange_rows) has one per run.  Row y of run {r0, n, e0, s} is element e0 + (y - r0) s.
-  const std::vector<int4> shard_run{make_int4(0, pl.n_owned, rank, world)};
-  const std::vector<int4>& runs = direct ? h->row_runs : shard_run;
-  auto for_runs = [&](int y0, int y1, auto&& f) -> int {
-    for (const int4& run : runs) {
-      const int r0 = std::max(y0, run.x), r1 = std::min(y1, run.x + run.y);
-      if (r1 > r0) { const int rcf = f(run, r0, r1); if (rcf) return rcf; }
-    }
-    return RTHX_OK;
-  };
 
   // row groups in ascending order: a group whose pairs overran the buffer is traced again as two halves
   std::vector<std::pair<int, int>> todo{{0, pl.n_owned}};
@@ -1927,26 +1889,8 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
     CU(h, cudaMemsetAsync(h->sk_ctl, 0, 4 * sizeof(unsigned long long), h->stream));
     if (direct) CU(h, cudaMemsetAsync(direct->events, 0, sizeof(unsigned long long), h->stream));
     CU(h, cudaEventRecord(h->ev[1], h->stream));
-    if (!direct) {
-      P.y_offset = y0;
-      CU(h, launch_trace_exchange(P, pl.kernel, (int)((long long)(y1 - y0) * nb * pl.row_chunks), pl.block_threads, pl.smem_bytes, h->stream));
-      R.n_launches += 2;
-    } else {                                                 // one launch per arithmetic run of the source list, as rthx_trace_direct
-      rthx_trace_args longest = *a;
-      longest.rays_per_emitter = direct->max_rays;
-      rc = for_runs(y0, y1, [&](const int4& run, int r0, int r1) -> int {
-        P.row_chunks = a->row_chunks > 0 ? pl.row_chunks : (int)std::max<long long>(pl.row_chunks, auto_row_chunks(h, pl, &longest, r1 - r0));
-        P.emitter_world = run.w; P.emitter_rank = run.z - run.x * run.w;
-        P.y_offset = r0;
-        if ((long long)(r1 - r0) * P.row_chunks > 0x7FFFFFFFll)
-          return fail(h, RTHX_ERR_ARG, "trace_direct_sparse: too many bundles for one launch (a launch has at most 2^31 blocks)");
-        CU(h, launch_trace_exchange(P, pl.kernel, (r1 - r0) * P.row_chunks, pl.block_threads, pl.smem_bytes, h->stream));
-        R.n_launches += 1;
-        return RTHX_OK;
-      });
-      if (rc) return rc;
-      R.n_launches += 2;
-    }
+    if ((rc = launch_rows(h, a, pl, own, direct, P, y0, y1, h->stream, &R.n_launches))) return rc;
+    R.n_launches += direct ? 2 : 1;                          // the clearing of the control words (and of the event counter)
     CU(h, cudaEventRecord(h->ev[2], h->stream));
     unsigned long long ctl[4], events = 0;
     CU(h, cudaMemcpyAsync(ctl, h->sk_ctl, sizeof(ctl), cudaMemcpyDeviceToHost, h->stream));
@@ -1961,8 +1905,8 @@ int sparse_trace_rows(rthx_handle* h, const rthx_trace_args* a, rthx_rec_out* re
                                              ") exceed the pair buffer (" + std::to_string(cap) + " pairs)");
         return fail(h, RTHX_ERR_NOMEM, "trace_sparse: the pairs of one emitter row exceed the pair buffer (" + std::to_string(cap) + " pairs)");
       }
-      for (int b = 0; b < nb; ++b)                          // the lost rays of the group are counted again
-        rc = for_runs(y0, y1, [&](const int4& run, int r0, int r1) -> int {
+      for (int b = 0; b < nb && !rc; ++b)                   // the lost rays of the group are counted again
+        rc = for_runs(h, own, pl.n_owned, y0, y1, [&](const int4& run, int r0, int r1) -> int {
           CU(h, cudaMemset2DAsync(h->lost_dev + (size_t)b * N + run.z + (size_t)(r0 - run.x) * run.w, sizeof(unsigned long long) * run.w, 0,
                                   sizeof(unsigned long long), (size_t)(r1 - r0), h->stream));
           return RTHX_OK;
@@ -2012,11 +1956,7 @@ int sparse_finish(rthx_handle* h, const rthx_trace_args* a, SparseRun& R, const 
   h->res.nnz = R.total;
   const int rc = finish_trace(h, a, R, lost_out, rec, st);
   if (rc) return rc;
-  if (sst) {
-    std::memset(sst, 0, sizeof(*sst));
-    sst->pairs = R.pairs; sst->nnz = R.total; sst->flushes = R.flushes; sst->pair_capacity = R.cap;
-    sst->row_groups = R.groups; sst->hash_slots = 1 << R.log2s; sst->reduce_ms = R.reduce_ms;
-  }
+  fill_sparse_stats(sst, R);
   return RTHX_OK;
 }
 
@@ -2726,11 +2666,15 @@ int counts_csc_sparse(rthx_handle* h, int bin, int index_base, int rowval_is_i64
   return RTHX_OK;
 }
 
-// rthx_trace_direct_sparse: out[k] = sum_y w[y] count[y][k] over count block `block` of the R resident source rows, in
-// ascending y with every product and sum rounded on its own — direct_absorbed_kernel's sum.  The block is transposed to columns with
-// the key sort of the CSC read-out (hashed_counts_to_csc), then one thread per column walks its entries.
+// rthx_trace_direct: out[k] = sum_y w[y] count[y][k] over count block `block` of the R resident source rows, in ascending y with every
+// product and sum rounded on its own (direct_absorbed_kernel over the dense rows).  Hashed (rthx_trace_direct_sparse): the block is
+// transposed to columns with the key sort of the CSC read-out (hashed_counts_to_csc), then one thread per column walks its entries.
 int direct_column_sums(rthx_handle* h, int block, int R, const double* w, double* out) {
   const int N = h->N;
+  if (!h->res.hashed()) {
+    CU(h, launch_direct_absorbed(h->counts_dev + (size_t)block * R * N, R, N, w, out, h->stream));
+    return RTHX_OK;
+  }
   long long* rptr = nullptr;
   long long nnz = 0;
   int rc = hashed_csc_scratch(h, &rptr);
